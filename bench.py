@@ -9,11 +9,11 @@ streams1080p` = configs[4] (64 x 1080p streams in total, sharded 64/N per GPU, s
 
 A "step" is one frame of every resident stream through the whole model: the first layer's change
 detection is launched on the frame where it lies in HBM, the other launches replay as one CUDA graph.
-  value : frames/s with the frames already resident in HBM: blocks of exactly K steps, each
-          bracketed by barrier + synchronize and device-timed (max over ranks), repeated until
-          --min-seconds of device time were measured; the median block is reported
+  value : frames/s with the frames already resident in HBM: exactly K = --steps steps after
+          max(W, 3) warm-up steps (W = --warmup), bracketed by barrier + synchronize and device-timed
+          (max over ranks)
   e2e   : frames/s through the public module call with HOST (pinned) frames: per step one H2D copy
-          of the step's frames and one D2H read of the step's logits inside the timed region
+          of the step's frames and one D2H read of the step's logits inside the timed region (K steps)
   e2e_u8_ingest : the same with uint8 host frames, normalised inside the detection kernel
   parity_max_rel: the benchmarked configuration against the reference flow (unmodified reference
           CUDA kernels of oracle/_ref + fp32 torch.matmul, tests/ref_flow.py), outside the timed region
@@ -22,6 +22,13 @@ detection is launched on the frame where it lies in HBM, the other launches repl
 `--impl reference` times that CPU path alone on the same config; it never imports the product.
 
 Launch: python bench.py --gpus N --steps K --warmup W      (N>1: via torch.distributed.run)
+
+`--dump-outputs DIR` writes what the timed path returned in its last timed step -- the logits
+[streams, 8, H/4, W/4] -- as DIR/output.npy (float32; DIR/output_rank<r>.npy per rank when N > 1;
+split4k: the stitched [1, 8, H/4, W/4] of its last timed frame, written by rank 0).
+The model, the video and the thresholds are seeded, so the same arguments give the same inputs and
+two builds can be compared output for output.  Above 64 MB in all the file holds a fixed sample: every
+s-th element of the flattened logits, s the smallest stride that fits.
 """
 import argparse
 import json
@@ -71,10 +78,12 @@ def parse():
                          "(ncu --profile-from-start off); prints no bench line")
     ap.add_argument("--no-extras", action="store_true", help="skip dense/latency/kernel/cpu/check legs")
     ap.add_argument("--no-check", action="store_true", help="skip the parity leg against the reference flow")
-    ap.add_argument("--min-seconds", type=float, default=0.25,
-                    help="repeat the K-step timed block until this much device time was measured (median block reported)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the logits of the last timed step to DIR/output.npy (float32)")
     ap.add_argument("--cpu-seconds", type=float, default=15.0)
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "ours" or args.profile):
+        ap.error("--dump-outputs needs --impl ours and a timed run (no --profile)")
     if args.workload in WORKLOADS:
         wl = WORKLOADS[args.workload]
         args.height = args.height or wl["h"]
@@ -423,7 +432,8 @@ def main():
     if args.impl == "reference":
         return run_reference(args)
     if args.workload == "split4k":
-        sys.argv = [sys.argv[0], "--rate", str(args.rate), "--check"]
+        sys.argv = [sys.argv[0], "--rate", str(args.rate), "--check"] + (
+            ["--dump-outputs", args.dump_outputs] if args.dump_outputs else [])
         from benchmarks import split_4k
         return split_4k.main()
 
@@ -510,32 +520,24 @@ def main():
         torch.cuda.profiler.stop()
         print(json.dumps({"profiled_steps": args.profile, "launches_per_step": my_launches_per_step}))
         return
-    # ---- timed region: blocks of EXACTLY K steps, each bracketed by barrier + synchronize and timed
-    #      on the device (max over ranks); blocks repeat until >= min_seconds were measured, the median
-    #      block is reported ------------------------------------------------------------------------
+    # ---- timed region: EXACTLY K steps, bracketed by barrier + synchronize and timed on the device
+    #      (max over ranks) ----------------------------------------------------------------------------
     sampler = ClockSampler(local)
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    blocks, fps_blocks = [], []
     barrier()
     sampler.start()
-    while True:
-        barrier()
-        e0.record()
-        for _ in range(K):
-            step(t)
-            t += 1
-        e1.record()
-        barrier()
-        # whole-job rate: frames of all ranks / slowest rank's device time
-        fps_b, ms_b = streams.whole_job_rate(S * K, e0.elapsed_time(e1), dev)
-        blocks.append(ms_b)
-        fps_blocks.append(fps_b)
-        if sum(blocks) >= args.min_seconds * 1e3 or len(blocks) >= 500:
-            break
+    e0.record()
+    for _ in range(K):
+        step(t)
+        t += 1
+    e1.record()
+    barrier()
+    # whole-job rate: frames of all ranks / slowest rank's device time
+    fps, elapsed_ms = streams.whole_job_rate(S * K, e0.elapsed_time(e1), dev)
     clocks = sampler.stop()
-    order = sorted(range(len(blocks)), key=lambda i: blocks[i])
-    mid = order[len(order) // 2]
-    fps, elapsed_ms = fps_blocks[mid], blocks[mid]
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, step_obj.out, "output" if world == 1 else "output_rank%d" % rank,
+                     DUMP_BYTES // world)
     counts = [int(m._scratch["count"].item()) for m in model.modules() if type(m) is cb.CBConv2d]
     state_mb = sum(x.numel() * x.element_size() for x in cb.getStateTensors(model)) / 1e6
 
@@ -567,32 +569,26 @@ def main():
         for i in range(1, Wm + 1):
             pipe.submit(pin[fidx(i)])
         pipe.drain()
-        i0, walls, last = Wm + 1, [], None
-        while True:
-            barrier()
-            t0 = time.perf_counter()
-            for i in range(i0, i0 + K):
-                last = pipe.submit(pin[fidx(i)])
-            pipe.wait(last)
-            pipe.drain()
-            wall_ms = (time.perf_counter() - t0) * 1e3
-            barrier()
-            # host wall clock from first submit to last result on the host (a device event pair on
-            # the default stream does not see the side streams)
-            walls.append(streams.whole_job_rate(S * K, wall_ms, dev))
-            i0 += K
-            if sum(w[1] for w in walls) >= args.min_seconds * 1e3 or len(walls) >= 200:
-                break
-        walls.sort(key=lambda w: w[1])
-        f_, ms_ = walls[len(walls) // 2]
+        last = None
+        barrier()
+        t0 = time.perf_counter()
+        for i in range(Wm + 1, Wm + 1 + K):
+            last = pipe.submit(pin[fidx(i)])
+        pipe.wait(last)
+        pipe.drain()
+        wall_ms = (time.perf_counter() - t0) * 1e3
+        barrier()
+        # host wall clock from first submit to last result on the host (a device event pair on
+        # the default stream does not see the side streams)
+        f_, ms_ = streams.whole_job_rate(S * K, wall_ms, dev)
         d2h_ = pipe.out_host[0].numel() * pipe.out_host[0].element_size()
         chk = float(pipe.out_host[last].float().abs().sum())
         del pipe
-        return f_, ms_, d2h_, chk, len(walls)
+        return f_, ms_, d2h_, chk
 
     h2d = pinned[0].numel() * pinned[0].element_size()
     ceiling_gbs = copy_only_gbs(pinned, frames[0])
-    e2e_fps, e2e_ms, d2h, e2e_checksum, e2e_blocks = e2e_leg(pinned, frames[0])
+    e2e_fps, e2e_ms, d2h, e2e_checksum = e2e_leg(pinned, frames[0])
 
     # ---- e2e with uint8 host frames (what a camera / decoder delivers): the first layer's detection
     #      kernel normalises u8/255 on the fly (cb_change_detect_u8), so a quarter of the bytes cross
@@ -603,7 +599,7 @@ def main():
         first = [m for m in model.modules() if type(m) is cb.CBConv2d][0]
         first.inputNorm = (255.0, 0.0)
         pinned8 = [f.mul(255.0).round().to(torch.uint8).pin_memory() for f in frames_cpu]
-        u8_fps, u8_ms, _, u8_chk, _ = e2e_leg(pinned8, pinned8[0].to(dev))
+        u8_fps, u8_ms, _, u8_chk = e2e_leg(pinned8, pinned8[0].to(dev))
         e2e_u8 = {"value": u8_fps, "unit": "frames/s", "ms_per_step": u8_ms / K,
                   "h2d_gbs": pinned8[0].numel() / (u8_ms / K * 1e-3) / 1e9,
                   "h2d_bytes_per_step": pinned8[0].numel(), "d2h_bytes_per_step": d2h,
@@ -623,7 +619,7 @@ def main():
             def forward(self, x):
                 return self.m(x).argmax(1).to(torch.uint8)
 
-        lb_fps, lb_ms, lb_d2h, lb_chk, _ = e2e_leg(pinned8, pinned8[0].to(dev), LabelHead(model))
+        lb_fps, lb_ms, lb_d2h, lb_chk = e2e_leg(pinned8, pinned8[0].to(dev), LabelHead(model))
         e2e_u8["labels_out"] = {"value": lb_fps, "unit": "frames/s", "ms_per_step": lb_ms / K,
                                 "h2d_bytes_per_step": pinned8[0].numel(), "d2h_bytes_per_step": lb_d2h,
                                 "checksum": lb_chk,
@@ -645,22 +641,20 @@ def main():
                                "HBM, the other launches replayed as one CUDA graph") if args.eager_detect else
                               ("per step ONE CUDA-graph launch: a graph per input slot of the %d-frame ring holds the "
                                "first-layer detection on that slot (read in place) and the rest of the model" % nframes),
-                       timing="median of %d timed blocks of %d steps each (blocks repeat until %.2f s of device "
-                              "time); min %.4f / max %.4f ms per step" % (
-                                  len(blocks), K, args.min_seconds, min(blocks) / K, max(blocks) / K),
+                       timing="one device-timed block of %d steps after %d warm-up steps" % (K, Wm),
                        thresholds=[round(x, 5) for x in thresholds],
                        changed_pixels_last_frame=counts),
-        "timed_blocks": len(blocks), "timed_region_s": sum(blocks) * 1e-3,
+        "timed_region_s": elapsed_ms * 1e-3,
         "clocks": clocks,
         "e2e": {"value": e2e_fps, "unit": "frames/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h,
-                "ms_per_step": e2e_ms / K, "checksum": e2e_checksum, "timed_blocks": e2e_blocks,
+                "ms_per_step": e2e_ms / K, "checksum": e2e_checksum,
                 "h2d_gbs": h2d / (e2e_ms / K * 1e-3) / 1e9,     # PCIe roofline of this leg (Gen5 x16 ~ 55 GB/s)
                 # the box's host-side ceiling at this N: the same pinned frames copied H2D by all ranks
                 # at once without any compute (one GPU alone ~55 GB/s; 8 GPUs share ~190 GB/s)
                 "host_h2d_copy_only_gbs_per_gpu": ceiling_gbs,
                 "path": "runtime.FramePipeline: per step pinned H2D of the frames, one graph replay, D2H of the "
                         "logits; copies of neighbouring steps overlap compute (3 streams); host wall clock"},
-        "gpu_launches": my_launches_per_step * K * len(blocks),
+        "gpu_launches": my_launches_per_step * K,
     }
     if e2e_u8 is not None:
         result["e2e_u8_ingest"] = e2e_u8
@@ -718,6 +712,21 @@ def main():
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
+
+
+DUMP_BYTES = 64_000_000       # all files of one --dump-outputs run together
+
+
+def dump_outputs(directory, out, name, budget):
+    """DIR/<name>.npy: `out` as float32; if it exceeds `budget` bytes, every s-th element of the
+    flattened array with the smallest stride s that fits"""
+    import numpy as np
+    a = out.detach().float().cpu().numpy()
+    stride = -(-a.size // ((budget - 4096) // a.itemsize))          # 4 KB for the .npy header
+    if stride > 1:
+        a = np.ascontiguousarray(a.reshape(-1)[::stride])
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, name + ".npy"), a)
 
 
 def kernels_in_step(args, model, frames, reps=40):

@@ -20,6 +20,8 @@ def main():
     ap.add_argument("--frames", type=int, default=12)
     ap.add_argument("--rate", type=float, default=0.05)
     ap.add_argument("--check", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the gathered output of the last timed frame to DIR/output.npy (float32, rank 0)")
     args = ap.parse_args()
     world, rank, local = (int(os.environ.get(k, d)) for k, d in (("WORLD_SIZE", 1), ("RANK", 0), ("LOCAL_RANK", 0)))
     torch.cuda.set_device(local)
@@ -60,6 +62,9 @@ def main():
     res = {"workload": "%dx%d scene CBinfer, %d row bands, 24-row input halo" % (W, H, world),
            "n_gpus": world, "band_rows": hi - lo, "slab_rows": sp.slab[1] - sp.slab[0],
            "ms_per_frame_median": round(ms[len(ms) // 2], 3), "frames_per_s": round(1000.0 / ms[len(ms) // 2], 1)}
+    if args.dump_outputs and rank == 0:
+        from bench import DUMP_BYTES, dump_outputs
+        dump_outputs(args.dump_outputs, out, "output", DUMP_BYTES)
     if args.check and rank == 0:
         full = models.sceneLabelingCBinfer(base, experimentIdx=6, threshold=0.02, clonePoolOutput=False,
                                            candidateDetect=True)

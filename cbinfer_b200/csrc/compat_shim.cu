@@ -15,7 +15,8 @@
 //     bitmaps / device-side counts with scratch buffers the shim owns (grow-only, per process);
 //   * everything runs on the legacy default stream, as the reference's <<<grid, block>>> launches do.
 // Layouts are the reference's: planar CHW, batch 1.  tests/test_gpu_compat_shim.py runs the same call
-// sequences against these libraries and against the unmodified reference libraries (oracle/_ref).
+// sequences against these libraries and, where oracle/_ref is built, against the unmodified reference
+// libraries; it always checks them against their own recorded outputs (tests/golden/compat_ops_golden.npz).
 #include <cuda_fp16.h>
 #include <cuda_runtime.h>
 #include <stdint.h>

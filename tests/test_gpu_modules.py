@@ -1,7 +1,8 @@
 """GPU parity tests, module level: CBConv2d / CBPoolMax2d / converted models against the oracle's
 restatement of the reference flow (oracle.OracleCBConv2d / OracleCBPoolMax2d), against dense
 nn.Conv2d at threshold 0, and against the UNMODIFIED reference kernels (oracle/_ref, JIT-compiled
-from their compute_52/61 PTX) run on the same GPU."""
+from their compute_52/61 PTX) run on the same GPU where they are built.  The ops those tests run are
+also checked, always, against their own recorded outputs (tests/golden/compat_ops_golden.npz)."""
 import ctypes
 import os
 
@@ -11,7 +12,7 @@ import torch
 import torch.nn as nn
 import torch.nn.functional as F
 
-from tests.util import ORC_DT, TORCH_DT, perturb, rand_tensor, ref_lib, to_np, to_val, vp
+from tests.util import ORC_DT, TORCH_DT, compare_outputs, perturb, rand_tensor, to_np, to_val, vp
 
 pytestmark = pytest.mark.gpu
 
@@ -380,25 +381,22 @@ def test_full_size_properties(res):
 
 
 # ---------------------------------------------------------------------------------------------
-# the UNMODIFIED reference kernels on the same GPU (oracle/_ref, PTX JIT)
+# the UNMODIFIED reference kernels on the same GPU (oracle/_ref, PTX JIT) where they are built; the
+# ops' own recorded outputs always
 # ---------------------------------------------------------------------------------------------
 
-def _ref_or_skip(name):
-    lib = ref_lib(name)
-    if lib is None:
-        pytest.skip("oracle/_ref/%s not built (reference checkout absent at build time)" % name)
-    return lib
+CD_CASES = ((16, 400, 300, 3, 0.1), (3, 97, 131, 7, 0.3), (64, 30, 40, 1, 0.5))
 
 
-@pytest.mark.parametrize("half", [False, True])
-def test_reference_cuda_kernels_change_detection(half):
-    """bit-exact masks + feedback state vs cbconv2d_cg[_half]_backend.cu run on this GPU."""
-    from cbinfer_b200 import conv2d_cg as cg
-    lib = _ref_or_skip("cbconv2d_cg_half_backend" if half else "cbconv2d_cg_backend")
-    dt = "f16" if half else "f32"
-    for (C, H, W, k, thr) in ((16, 400, 300, 3, 0.1), (3, 97, 131, 7, 0.3), (64, 30, 40, 1, 0.5)):
-        prev = rand_tensor((1, C, H, W), dt, C)
-        x = perturb(prev, 0.05, C + 1, scale=0.7)
+def _cd_inputs(C, H, W, dt):
+    prev = rand_tensor((1, C, H, W), dt, C)
+    return prev, perturb(prev, 0.05, C + 1, scale=0.7)
+
+
+def reference_change_detection_outputs(lib, half):
+    outs = {}
+    for (C, H, W, k, thr) in CD_CASES:
+        prev, x = _cd_inputs(C, H, W, "f16" if half else "f32")
         for update in (False, True):
             st_ref = prev.clone()
             cmap_ref = torch.zeros(H, W, dtype=torch.int8, device="cuda")
@@ -406,56 +404,88 @@ def test_reference_cuda_kernels_change_detection(half):
             lib.changeDetection(1, 1, grid, 1, 1, 128, vp(x), vp(st_ref), vp(cmap_ref), W, H, C,
                                 (k - 1) // 2, (k - 1) // 2, ctypes.c_float(thr), ctypes.c_bool(update))
             torch.cuda.synchronize()
+            outs["map_%d_%d" % (C, update)] = cmap_ref
+            outs["state_%d_%d" % (C, update)] = st_ref
+    return outs
+
+
+def ops_change_detection_outputs(half):
+    from cbinfer_b200 import conv2d_cg as cg
+    outs = {}
+    for (C, H, W, k, thr) in CD_CASES:
+        prev, x = _cd_inputs(C, H, W, "f16" if half else "f32")
+        for update in (False, True):
             st = prev.clone()
             cmap = cg.changeDetection(x, st, (k, k), thr, updateInputState=update)
-            assert torch.equal(cmap, cmap_ref)
-            assert torch.equal(st, st_ref)
             idx = cg.changeIndexesExtr(cmap)
-            assert torch.equal(idx, torch.nonzero(cmap_ref.view(-1)).int().view(-1))
+            assert torch.equal(idx, torch.nonzero(cmap.view(-1)).int().view(-1))
+            outs["map_%d_%d" % (C, update)] = cmap
+            outs["state_%d_%d" % (C, update)] = st
+    return outs
 
 
-def test_reference_cuda_kernels_gather_scatter_pool():
-    from cbinfer_b200 import conv2d_cg as cg
-    lib = _ref_or_skip("cbconv2d_cg_backend")
+@pytest.mark.parametrize("half", [False, True])
+def test_reference_cuda_kernels_change_detection(half):
+    """bit-exact masks + feedback state vs cbconv2d_cg[_half]_backend.cu."""
+    compare_outputs("ops_change_detection.%s" % ("f16" if half else "f32"),
+             "cbconv2d_cg_half_backend" if half else "cbconv2d_cg_backend",
+             ops_change_detection_outputs(half), lambda L: reference_change_detection_outputs(L, half))
+
+
+def _gsp_inputs():
     C, H, W, k, Cout = 8, 37, 53, 7, 12
     x = rand_tensor((1, C, H, W), "f32", 1)
     g = torch.Generator().manual_seed(2)
     idx = torch.nonzero(torch.rand(H * W, generator=g) < 0.2).view(-1).int().cuda()
-    n = idx.numel()
-    # genXMatrix
-    X_ref = torch.zeros(n, C * k * k, device="cuda")
-    tz = 128 // (k * k)
-    lib.genXMatrix(1, 1, (n - 1) // tz + 1, k, tz, k, vp(X_ref), vp(x), vp(idx), k, k, C, W, H, n)
-    assert torch.equal(cg.genXMatrix(x, idx, (k, k)), X_ref)
-    # updateOutput
-    Yt = rand_tensor((Cout, n), "f32", 3)
-    po_ref = rand_tensor((1, Cout, H, W), "f32", 4)
-    po = po_ref.clone()
-    lib.updateOutput(1, 1, (n * Cout - 1) // 1024 + 1, 1, 1, 1024, vp(Yt), vp(po_ref), vp(idx),
-                     H * W, n, Cout, ctypes.c_bool(True))
-    cg.updateOutput(Yt, idx, po, withReLU=True)
-    assert torch.equal(po, po_ref)
+    Yt = rand_tensor((Cout, idx.numel()), "f32", 3)
+    po = rand_tensor((1, Cout, H, W), "f32", 4)
     # maxPool2d (even sizes: the reference kernel has no bounds guard for odd ones)
     xe = rand_tensor((1, C, 36, 52), "f32", 5)
     idx2 = torch.nonzero(torch.rand(36 * 52, generator=g) < 0.2).view(-1).int().cuda()
-    st_ref = torch.full((1, C, 18, 26), float("inf"), device="cuda")
-    st = st_ref.clone()
+    st = torch.full((1, C, 18, 26), float("inf"), device="cuda")
+    return (C, H, W, k, Cout), x, idx, Yt, po, xe, idx2, st
+
+
+def reference_gather_scatter_pool_outputs(lib):
+    (C, H, W, k, Cout), x, idx, Yt, po_ref, xe, idx2, st_ref = _gsp_inputs()
+    n = idx.numel()
+    X_ref = torch.zeros(n, C * k * k, device="cuda")
+    tz = 128 // (k * k)
+    lib.genXMatrix(1, 1, (n - 1) // tz + 1, k, tz, k, vp(X_ref), vp(x), vp(idx), k, k, C, W, H, n)
+    lib.updateOutput(1, 1, (n * Cout - 1) // 1024 + 1, 1, 1, 1024, vp(Yt), vp(po_ref), vp(idx),
+                     H * W, n, Cout, ctypes.c_bool(True))
     lib.maxPool2d((idx2.numel() - 1) // 64 + 1, 64, vp(xe), vp(st_ref), vp(idx2), idx2.numel(), C,
                   36, 52, 18, 26, 2, 2)
+    torch.cuda.synchronize()
+    return {"xmatrix": X_ref, "output": po_ref, "pooled": st_ref}
+
+
+def ops_gather_scatter_pool_outputs():
+    from cbinfer_b200 import conv2d_cg as cg
+    (C, H, W, k, Cout), x, idx, Yt, po, xe, idx2, st = _gsp_inputs()
+    X = cg.genXMatrix(x, idx, (k, k))
+    cg.updateOutput(Yt, idx, po, withReLU=True)
     cg.maxPool2d(xe, st, idx2)
     torch.cuda.synchronize()
-    assert torch.equal(st, st_ref)
+    return {"xmatrix": X, "output": po, "pooled": st}
 
 
-def test_reference_cuda_fg_kernels():
-    from cbinfer_b200 import conv2d_fg as fg
-    lib = _ref_or_skip("cbconv2d_fg_backend")
+def test_reference_cuda_kernels_gather_scatter_pool():
+    compare_outputs("ops_gather_scatter_pool", "cbconv2d_cg_backend", ops_gather_scatter_pool_outputs(),
+             reference_gather_scatter_pool_outputs)
+
+
+def _fg_inputs():
     Cin, Cout, H, W, k = 5, 7, 21, 26, 3
     prev = rand_tensor((1, Cin, H, W), "f32", 1)
     x = perturb(prev, 0.1, 2)
     w = rand_tensor((Cout, Cin, k, k), "f32", 3, scale=0.3)
-    out_ref = rand_tensor((1, Cout, H, W), "f32", 4)
-    out = out_ref.clone()
+    out = rand_tensor((1, Cout, H, W), "f32", 4)
+    return (Cin, Cout, H, W, k), prev, x, w, out
+
+
+def reference_fg_outputs(lib):
+    (Cin, Cout, H, W, k), prev, x, w, out_ref = _fg_inputs()
     diffs = torch.zeros_like(x)
     cmap = torch.zeros(x.shape, dtype=torch.int8, device="cuda")
     lib.changeDetectionFG(vp(x), vp(prev), vp(diffs), vp(cmap), x.numel(), ctypes.c_float(0.2))
@@ -463,11 +493,21 @@ def test_reference_cuda_fg_kernels():
     nchg = coords.numel()
     lib.updateOutputFG(1, 1, (nchg - 1) // 128 + 1, 1, 1, 128, vp(diffs), vp(w), vp(out_ref),
                        vp(coords), Cout, Cin, H, W, k, k, nchg)
+    torch.cuda.synchronize()
+    return {"changed": torch.tensor([nchg], dtype=torch.int32), "output": out_ref}
+
+
+def ops_fg_outputs():
+    from cbinfer_b200 import conv2d_fg as fg
+    _, prev, x, w, out = _fg_inputs()
     cnt = torch.zeros(1, dtype=torch.int32, device="cuda")
     fg.cbconvFG(x, prev.clone(), out, w, 0.2, cnt)
     torch.cuda.synchronize()
-    assert int(cnt.item()) == nchg
-    np.testing.assert_allclose(out.cpu().numpy(), out_ref.cpu().numpy(), rtol=1e-5, atol=1e-4)
+    return {"changed": cnt, "output": out}
+
+
+def test_reference_cuda_fg_kernels():
+    compare_outputs("ops_fg", "cbconv2d_fg_backend", ops_fg_outputs(), reference_fg_outputs, tol={"output": (1e-5, 1e-4)})
 
 
 def test_eval_tools_and_threshold_tuner(tmp_path):

@@ -1,5 +1,6 @@
 """helpers shared by the GPU parity tests: torch <-> oracle (numpy) plumbing."""
 import ctypes
+import hashlib
 import os
 import platform
 
@@ -52,6 +53,59 @@ def ref_lib(name):
     if not os.path.exists(p):
         return None
     return ctypes.CDLL(p)
+
+
+def shim_lib(name):
+    """ctypes handle of the compatibility shim that exports the reference library `name`'s symbols
+    on top of libcbinfer_sm100.so (cbinfer_b200/compat, built by build_compat)."""
+    p = os.path.join(REPO, "cbinfer_b200", "compat", "%s_%s.so" % (name, platform.machine()))
+    if not os.path.exists(p):
+        from cbinfer_b200 import build
+        build.build_compat()
+    return ctypes.CDLL(p)
+
+
+OUTPUTS_GOLDEN = os.path.join(REPO, "tests", "golden", "compat_ops_golden.npz")
+
+
+def digest(t):
+    """SHA-256 of a tensor's dtype, shape and bytes: bit-exact comparison with a recorded output."""
+    a = t.detach().contiguous().cpu()
+    h = hashlib.sha256(("%s %s " % (a.dtype, tuple(a.shape))).encode())
+    h.update(a.reshape(-1).view(torch.uint8).numpy().tobytes())
+    return h.hexdigest()
+
+
+def recorded_outputs():
+    """this project's own outputs (compat shim and ops) on the inputs of the tests that compare with
+    the reference libraries, as tests/golden/make_compat_ops_golden.py recorded them"""
+    return np.load(OUTPUTS_GOLDEN)
+
+
+def record(prefix, outs, tol=()):
+    """{prefix.name: digest} of the tensors in `outs`, an array instead for the names in `tol`"""
+    return {"%s.%s" % (prefix, n): (t.detach().float().cpu().numpy() if n in tol else np.array(digest(t)))
+            for n, t in outs.items()}
+
+
+def check_outputs(expected, prefix, outs, tol={}):
+    """`outs` ({name: tensor}) against `expected` (a record() of other outputs): bit-exact by digest,
+    or within (rtol, atol) for the names in `tol`"""
+    for name, t in outs.items():
+        key = "%s.%s" % (prefix, name)
+        if name in tol:
+            np.testing.assert_allclose(t.detach().float().cpu().numpy(), expected[key], *tol[name], err_msg=key)
+        else:
+            assert digest(t) == str(expected[key]), key
+
+
+def compare_outputs(prefix, name, outs, outputs_of, tol={}):
+    """`outs` against this project's recorded outputs and, where oracle/_ref holds the reference
+    library `name`, against `outputs_of(that library)` for the same calls"""
+    check_outputs(recorded_outputs(), prefix, outs, tol)
+    ref = ref_lib(name)
+    if ref is not None:
+        check_outputs(record(prefix, outputs_of(ref), tol), prefix, outs, tol)
 
 
 def vp(t):

@@ -12,7 +12,7 @@ echo "== our arm, N=$N"; ( time run ) > gpurun_out/contract_ours_${N}.json 2> gp
 python - <<PY
 import json
 d = json.loads([l for l in open("gpurun_out/contract_ours_${N}.json") if l.startswith("{")][-1])
-print({k: d[k] for k in ("metric", "value", "n_gpus", "steps", "warmup", "ms_per_step", "scaling", "gpu_launches", "timed_blocks", "timed_region_s")})
+print({k: d[k] for k in ("metric", "value", "n_gpus", "steps", "warmup", "ms_per_step", "scaling", "gpu_launches", "timed_region_s")})
 print("e2e", d["e2e"]["value"], d["e2e"].get("host_h2d_copy_only_gbs_per_gpu"), "u8", d["e2e_u8_ingest"]["value"], "labels", d["e2e_u8_ingest"]["labels_out"]["value"])
 print("clocks", d["clocks"], "parity", d.get("parity_max_rel"), "roofline", d.get("roofline", {}).get("frac"), "cpu", d.get("cpu_baseline", {}).get("value"))
 PY
