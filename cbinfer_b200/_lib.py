@@ -29,8 +29,7 @@ SYMBOLS = [
     "cb_fg_detect", "cb_conv_accumulate", "cb_compact_small_max_words", "cb_change_detect_sparse_compact",
     "cb_tile_ws_bytes", "cb_dilate_compact_tiles", "cb_conv_tiled_supported", "cb_conv_update_tiled",
     "cb_conv_tiled_pool_supported", "cb_conv_update_tiled_pool", "cb_dilate_tiles",
-    "cb_tail_supported", "cb_tail_update", "cb_dilate_compact_hinted",
-    "cb_conv_tiled_self_supported", "cb_conv_update_tiled_self",
+    "cb_tail_supported", "cb_tail_update",
     "cb_resize_ws_bytes", "cb_resize_bicubic_u8_init", "cb_resize_bicubic_u8", "cb_resize_bilinear_u8",
 ]
 
@@ -73,17 +72,10 @@ def _load():
         "cb_tail_update": (i32, [vp, vp, vp, vp, vp, vp, i32, f32, vp, vp, vp, vp, i32, i32, f32, vp, vp, i32, i32, i32,
                                  i32, vp, vp, vp]),
         "cb_dilate_tiles": (i32, [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32]),
-        "cb_dilate_compact_hinted": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32, i32, i32,
-                                           vp, vp, vp, vp, vp]),
         "cb_conv_tiled_pool_supported": (i32, [i32, i32, i32]),
         "cb_conv_update_tiled_pool": (i32, [vp, i32, i32, vp, vp, i32, vp, vp, vp, vp, vp, i32, i32, i32, i32,
                                             i32, i32, i32, i32, i32,
                                             vp, i64, i64, i32, i32, i32, vp, i64, i64, i32, i32, vp, vp, vp, f32, i32]),
-        "cb_conv_tiled_self_supported": (i32, [i32] * 5),
-        "cb_conv_update_tiled_self": (i32, [vp, i32, i32, vp, vp, i32, vp, vp, vp, vp, vp, i32, i32, i32, i32,
-                                            i32, i32, i32, i32, i32,
-                                            vp, i64, i64, i32, i32, i32, vp, i64, i64, i32, i32, vp, vp, vp, f32, i32,
-                                            vp, vp, vp, i32]),
         "cb_resize_ws_bytes": (sz, [i32] * 5),
         "cb_resize_bicubic_u8_init": (i32, [vp, vp, i32, i32, i32, i32, i32]),
         "cb_resize_bicubic_u8": (i32, [vp, vp, i64, i64, i64, vp, i64, i64, i64, vp, i32, i32, i32, i32, i32]),

@@ -247,7 +247,6 @@ class CBConv2d(nn.Module):
         self._fresh = True        # state holds +inf: the next detection must be a full scan
         self._lastThr = None
         self._lastChanges = None
-        self._hintCache = None
         self.changeMap = None
         if getattr(self, '_wsHolder', None) is not None:
             self._wsHolder.clear()
@@ -581,8 +580,7 @@ class CBConv2d(nn.Module):
             # halo, implicit im2col through the UMMA descriptors), rows masked by the dilated bitmap
             cg.conv_update_tiled(self._inBuf, s["tile_ws"], s["dil_bits"], packed, bias32, self._outBuf,
                                  self.in_channels, self.out_channels, self.kernel_size, self.withReLU,
-                                 gemm, lo_buf=lo_buf, planes16=planes16, pool=pool_args,
-                                 self_list=changeIndexes.__dict__.pop('selfList', None))  # :242-251
+                                 gemm, lo_buf=lo_buf, planes16=planes16, pool=pool_args)  # :242-251
             if pool_args is not None:
                 changeIndexes.pooledBy = fp[0]
         else:
@@ -738,59 +736,18 @@ class CBConv2d(nn.Module):
             cache[key] = sup >= 1 if mode == 'on' else sup == 1
         return cache[key]
 
-    def _hints(self, B, H, W, dev):
-        """L2 prefetch hints for this frame's dilation (cb_dilate_compact_hinted): the previous-input
-        state of the CB layers that will threshold the pixels this layer is about to rewrite
-        (``_prefetchNext``, wired by models.enableCandidateDetection).  Those rows were last touched
-        when the pixels last changed, so the consumer would otherwise fetch them from DRAM inside a
-        latency-bound kernel; the dilation knows the pixels one contraction earlier."""
-        nxt = getattr(self, '_prefetchNext', None)
-        # (opt-in: measured on the bench model the hinted L3 dilation costs 12 us more and saves the tail
-        #  kernel 2 us -- profiles/r02_experiments.md)
-        if not nxt or os.environ.get("CBINFER_PREFETCH", "0") != "1":
-            return None
-        tg = []
-        for m, sh in nxt:
-            buf = getattr(m, '_inBuf', None)
-            if buf is None or buf.device != dev or buf.dim() != 4 or buf.shape[0] != B:
-                continue
-            th, tw = buf.shape[1], buf.shape[2]
-            if (sh == 0 and (th, tw) == (H, W)) or \
-                    (sh == 1 and th in (H // 2, (H + 1) // 2) and tw in (W // 2, (W + 1) // 2)):
-                tg.append((buf, sh))
-        key = tuple((t.data_ptr(), tuple(t.shape), sh) for t, sh in tg)
-        hc = getattr(self, '_hintCache', None)
-        if hc is None or hc[0] != key:
-            hc = (key, cg.PrefetchHints(tg))
-            self._hintCache = hc
-        return hc[1] if hc[1].n else None
-
     def _selfTiles(self, B, H, W):
-        """dilation + tile list inside the tile contraction itself (cb_conv_update_tiled_self)?"""
-        # opt-in (CBINFER_SELF_TILES=1; =N > 1: only bitmaps of at most N words): bit-identical, but no faster --
-        # the runtime admits ONE block of a TMEM-allocating kernel per SM to a cooperative launch, and even
-        # at full occupancy (plain launch, CBINFER_SELF_COOP=0) the step does not gain (profiles/r02_experiments.md)
-        lim = int(os.environ.get("CBINFER_SELF_TILES", "0") or 0)
-        if lim <= 0 or (lim > 1 and _lib.C.cb_bitmap_words(B, H, W) > lim):
-            return False
-        return bool(_lib.C.cb_conv_tiled_self_supported(B, H, W, self.kernel_size[0], self.kernel_size[1]))
+        """Always False: no kernel lists its own tiles.  bench.py reads it to count launches."""
+        return False
 
     def _compact(self, s, B, H, W, sparse_next, tiles=False, lazy=False):
         """dilate the raw bitmap by the filter footprint and compact it to the index list."""
         if tiles and "tile_ws" not in s:
             s["tile_ws"] = cg.alloc_tile_ws((B, H, W), s["idx"].device)
-        hints = self._hints(B, H, W, s["idx"].device)
-        if tiles and lazy and self._selfTiles(B, H, W):
-            # nothing to launch: the tile contraction dilates the raw bitmap and lists its tiles itself
-            # (cb_conv_update_tiled_self); bitmap, tile list and count exist once it has run
-            s["raw_clear"] = sparse_next
-            ci = ChangeIndexes(s["idx"], s["count"], (B, H, W), bits=s["dil_bits"], ws=s["ws"], listed=False)
-            ci.selfList = dict(raw_bits=s["raw_bits"], count=s["count"], ws=s["ws"], clear_raw=sparse_next)
-            return ci
         if tiles and lazy:
             # tiles + dilated bitmap + count only; the ordered list is compacted if somebody asks
             cg.dilate_tiles(s["raw_bits"], (B, H, W), self.kernel_size, s["count"], s["ws"], s["dil_bits"],
-                            s["tile_ws"], clear_raw=sparse_next, hints=hints)
+                            s["tile_ws"], clear_raw=sparse_next)
             s["raw_clear"] = sparse_next
             return ChangeIndexes(s["idx"], s["count"], (B, H, W), bits=s["dil_bits"], ws=s["ws"], listed=False)
         dil_map = s.get("dil_map") if self.saveChangeMap else None
@@ -798,7 +755,7 @@ class CBConv2d(nn.Module):
         # consumed, so the next frame's candidate detection needs no memset
         cg.dilate_compact(s["raw_bits"], (B, H, W), self.kernel_size, s["idx"], s["count"],
                           s["ws"], dil_bits=s["dil_bits"], dil_map=dil_map, clear_raw=sparse_next,
-                          tile_ws=s["tile_ws"] if tiles else None, hints=hints)
+                          tile_ws=s["tile_ws"] if tiles else None)
         s["raw_clear"] = sparse_next
         if self.saveChangeMap:
             self.changeMap = dil_map[0] if B == 1 else dil_map

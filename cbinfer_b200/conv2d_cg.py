@@ -209,63 +209,20 @@ def pool_compact(in_bits, in_shape, out_shape, idx, count, ws, out_bits=None):
                             idx.data_ptr(), count.data_ptr(), ws.data_ptr(), B, H, W, oH, oW))
 
 
-class PrefetchHints(object):
-    """L2 prefetch hints of cb_dilate_compact_hinted: pixel-major maps ``[B, tH, tW, pitch]`` (contiguous)
-    whose rows at the changed pixels a later kernel will read -- ``(buffer, shift)`` pairs, shift 1 for a
-    map at the 2x2-pooled resolution.  Holds the ctypes argument arrays (and the buffers alive)."""
-    MAX = 3
-
-    def __init__(self, targets):
-        import ctypes
-        targets = [(t, int(sh)) for t, sh in targets
-                   if t is not None and t.dim() == 4 and t.is_contiguous() and t.data_ptr() % 16 == 0
-                   and (t.shape[3] * t.element_size()) % 16 == 0 and t.numel() > 0][:self.MAX]
-        self.targets = targets
-        self.n = len(targets)
-        self.key = tuple((t.data_ptr(), tuple(t.shape), sh) for t, sh in targets)
-        self.base = (ctypes.c_void_p * max(self.n, 1))(*[t.data_ptr() for t, _ in targets])
-        ia = ctypes.c_int * max(self.n, 1)
-        self.row_bytes = ia(*[t.shape[3] * t.element_size() for t, _ in targets])
-        self.shift = ia(*[sh for _, sh in targets])
-        self.h = ia(*[t.shape[1] for t, _ in targets])
-        self.w = ia(*[t.shape[2] for t, _ in targets])
-
-
-def _dilate_hinted(raw_bits, shape, filtSize, idx, count, ws, dil_bits, dil_map, tile_ws, clear_raw, no_list,
-                   hints):
+def dilate_tiles(raw_bits, shape, filtSize, count, ws, dil_bits, tile_ws, clear_raw=False):
+    """cb_dilate_tiles: dilation + dirty-tile list + change count, no ordered index list."""
     B, H, W = shape
-    check(C.cb_dilate_compact_hinted(stream_ptr(raw_bits.device), raw_bits.data_ptr(),
-                                     dil_bits.data_ptr() if dil_bits is not None else None,
-                                     dil_map.data_ptr() if dil_map is not None else None,
-                                     idx.data_ptr() if idx is not None else None, count.data_ptr(),
-                                     ws.data_ptr(), tile_ws.data_ptr() if tile_ws is not None else None,
-                                     B, H, W, (filtSize[0] - 1) // 2, (filtSize[1] - 1) // 2,
-                                     int(bool(clear_raw)), int(bool(no_list)), hints.n, hints.base,
-                                     hints.row_bytes, hints.shift, hints.h, hints.w))
-
-
-def dilate_tiles(raw_bits, shape, filtSize, count, ws, dil_bits, tile_ws, clear_raw=False, hints=None):
-    """cb_dilate_tiles: dilation + dirty-tile list + change count, no ordered index list.  `hints`
-    (:class:`PrefetchHints`): cb_dilate_compact_hinted, same outputs."""
-    B, H, W = shape
-    if hints is not None and hints.n:
-        return _dilate_hinted(raw_bits, shape, filtSize, None, count, ws, dil_bits, None, tile_ws, clear_raw,
-                              True, hints)
     check(C.cb_dilate_tiles(stream_ptr(raw_bits.device), raw_bits.data_ptr(), dil_bits.data_ptr(),
                             count.data_ptr(), ws.data_ptr(), tile_ws.data_ptr(), B, H, W,
                             (filtSize[0] - 1) // 2, (filtSize[1] - 1) // 2, int(bool(clear_raw))))
 
 
 def dilate_compact(raw_bits, shape, filtSize, idx, count, ws, dil_bits=None, dil_map=None,
-                   clear_raw=False, tile_ws=None, hints=None):
+                   clear_raw=False, tile_ws=None):
     """cb_dilate_compact: dilation by the filter footprint + ordered compaction.  With `tile_ws`
     (cb_tile_ws_bytes of zeroed int32 device memory) the dirty 8x16 output tiles are listed as well
-    (cb_dilate_compact_tiles), for :func:`conv_update_tiled`.  `hints` (:class:`PrefetchHints`):
-    cb_dilate_compact_hinted, same outputs."""
+    (cb_dilate_compact_tiles), for :func:`conv_update_tiled`."""
     B, H, W = shape
-    if hints is not None and hints.n:
-        return _dilate_hinted(raw_bits, shape, filtSize, idx, count, ws, dil_bits, dil_map, tile_ws, clear_raw,
-                              False, hints)
     if tile_ws is not None:
         check(C.cb_dilate_compact_tiles(stream_ptr(raw_bits.device), raw_bits.data_ptr(),
                                         dil_bits.data_ptr() if dil_bits is not None else None,
@@ -443,12 +400,10 @@ def conv_accumulate(planes16, changes, packed_w, out_buf, Cin, Cout, filtSize, g
 
 
 def conv_update_tiled(state_buf, tile_ws, dil_bits, packed_w, bias_f32, out_buf, Cin, Cout, filtSize,
-                      relu, gemm, lo_buf=None, planes16=None, pool=None, self_list=None):
+                      relu, gemm, lo_buf=None, planes16=None, pool=None):
     """cb_conv_update_tiled on pixel-major buffers: the contraction over the dirty 8x16 tiles listed
     in `tile_ws` (TMA-staged halo tiles, implicit im2col), writing the pixels set in `dil_bits`.
-    Operand conventions as :func:`conv_update`.  `self_list` = dict(raw_bits, count, ws, clear_raw):
-    cb_conv_update_tiled_self -- the kernel dilates the raw bitmap and lists the tiles itself (no
-    cb_dilate_tiles launch before it); dil_bits, tile_ws and count are outputs then."""
+    Operand conventions as :func:`conv_update`."""
     B, H, W, Cp = state_buf.shape
     assert out_buf.shape[:3] == state_buf.shape[:3]
     src, src_lo, pitch = state_buf, lo_buf, Cp
@@ -460,23 +415,6 @@ def conv_update_tiled(state_buf, tile_ws, dil_bits, packed_w, bias_f32, out_buf,
         pitch = src.shape[3]
     elif gemm == _lib.GEMM_TC_3X and state_buf.dtype == torch.float32 and lo_buf is None:
         src_lo = tf32_lo(state_buf)
-    if self_list is not None:
-        pa = [None, 0, 0, 0, 0, 0, None, 0, 0, 0, 0, None, None, None, 0.0, 0]
-        if pool is not None:
-            po, ns = pool["out"], pool["next_state"]
-            assert po.stride(1) == 1 and ns.stride(1) == 1 and po.shape == ns.shape, "pixel-major maps only"
-            mode, hi, lo = _aux_args(pool.get("aux"), ns)
-            pa = [po.data_ptr(), po.stride(0), po.stride(2), po.stride(3), po.size(2), po.size(3),
-                  ns.data_ptr(), ns.stride(0), ns.stride(2), ns.stride(3), mode, hi, lo,
-                  pool["next_raw_bits"].data_ptr(), float(pool["threshold"]), int(pool["mode"])]
-        check(C.cb_conv_update_tiled_self(stream_ptr(state_buf.device), dtype_code(state_buf), gemm,
-                                          src.data_ptr(), src_lo.data_ptr() if src_lo is not None else None,
-                                          pitch, tile_ws.data_ptr(), dil_bits.data_ptr(), packed_w.data_ptr(),
-                                          bias_f32.data_ptr(), out_buf.data_ptr(), out_buf.shape[3], B, H, W,
-                                          Cin, Cout, filtSize[0], filtSize[1], int(bool(relu)), *pa,
-                                          self_list["raw_bits"].data_ptr(), self_list["count"].data_ptr(),
-                                          self_list["ws"].data_ptr(), int(bool(self_list.get("clear_raw")))))
-        return
     if pool is not None:
         # pool = dict(out=pooled map view, next_state=view, next_raw_bits, threshold, mode, aux): the
         # epilogue also re-pools the touched 2x2 windows and runs the next layer's detection on them

@@ -9,7 +9,6 @@
 #include "compact.cuh"
 #include "conv_simt.cuh"
 #include "conv_umma.cuh"
-#include "conv_pair.cuh"
 #include "conv_tile.cuh"
 #include "detect.cuh"
 #include "ingest.cuh"
@@ -41,18 +40,6 @@ int sm_count() {
   return cached > 0 ? cached : 148;
 }
 
-bool pdl_enabled() {
-  static int cached = -1;
-  if (cached < 0) {
-    // Off by default: a dependent grid that becomes resident early may see stale L1 / read-only
-    // (ld.global.nc) lines of buffers its predecessor is still writing (observed as wrong results
-    // inside CUDA graphs); measured gain was only ~2 %.  CBINFER_PDL=1 enables it for experiments.
-    const char* e = getenv("CBINFER_PDL");
-    cached = (e && e[0] == '1') ? 1 : 0;
-  }
-  return cached != 0;
-}
-
 static inline unsigned grid_for(long long total, int threads, int per_sm = 8) {
   long long blocks = (total + threads - 1) / threads;
   long long cap = (long long)sm_count() * per_sm;
@@ -64,7 +51,6 @@ static inline unsigned grid_for(long long total, int threads, int per_sm = 8) {
 }  // namespace cb
 
 using namespace cb;
-static_assert(cb::kDtRows == cb::TL_H && cb::TL_W == 8, "dilate_tiles_kernel lists 8 x 16 tiles, four per bitmap word");
 
 #define CB_DISPATCH_DTYPE(dtype, ...)                                               \
   switch (dtype) {                                                                  \
@@ -136,11 +122,8 @@ size_t cb_tile_ws_bytes(int B, int H, int W) { return cb::tile_ws_words(B, H, W)
 
 static int dilate_compact_impl(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits, int8_t* dil_map,
                       int32_t* idx, int32_t* count, void* ws, void* tile_ws, int B, int H, int W, int kHHalf,
-                      int kWHalf, int clear_raw, int no_list = 0, const cb::PrefetchHints* hints = nullptr) {
+                      int kWHalf, int clear_raw, int no_list = 0) {
   CB_CHECK_ARG(raw_bits && (idx || no_list) && count && ws, "dilate_compact: null pointer");
-  cb::PrefetchHints ph;
-  memset(&ph, 0, sizeof(ph));
-  if (hints) ph = *hints;
   CB_CHECK_ARG(raw_bits != dil_bits, "dilate_compact: dil_bits must not alias raw_bits");
   CB_CHECK_ARG(kHHalf >= 0 && kWHalf >= 0 && kWHalf <= 31, "dilate_compact: kWHalf must be <= 31");
   CB_CHECK_ARG((long long)B * H * W < (1ll << 31), "dilate_compact: more than 2^31 pixels");
@@ -153,46 +136,15 @@ static int dilate_compact_impl(void* stream, const uint32_t* raw_bits, uint32_t*
   }
   CB_CHECK_ARG(nwords < (1ll << 31), "dilate_compact: bitmap too large");
   const int ntiles = (int)((nwords + kCompactTile - 1) / kCompactTile);
-  cb::launch_pdl(ph.n ? dilate_compact_kernel<true> : dilate_compact_kernel<false>, ntiles, kCompactThreads, 0, s,
+  cb::launch(dilate_compact_kernel, ntiles, kCompactThreads, 0, s,
                                                           raw_bits, dil_bits, dil_map, idx, count,
                                                           ws, B, H, W, (W + 31) / 32, kHHalf,
                                                           kWHalf, (int)nwords, ntiles, 0, 0,
                                                           clear_raw ? const_cast<uint32_t*>(raw_bits) : nullptr,
                                                           (int32_t*)tile_ws, cb::tile_grid_y(H), cb::tile_grid_xp(W),
-                                                          (int)compact_coop(), no_list, ph);
+                                                          (int)compact_coop(), no_list);
   CB_CHECK_LAUNCH("dilate_compact");
   return 0;
-}
-
-int cb_dilate_compact_hinted(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits, int8_t* dil_map,
-                             int32_t* idx, int32_t* count, void* ws, void* tile_ws, int B, int H, int W,
-                             int kHHalf, int kWHalf, int clear_raw, int no_list, int n_hints,
-                             const void* const* hint_base, const int* hint_row_bytes, const int* hint_shift,
-                             const int* hint_h, const int* hint_w) {
-  CB_CHECK_ARG(n_hints >= 0 && n_hints <= cb::kMaxHints, "dilate_compact_hinted: at most %d hints", cb::kMaxHints);
-  CB_CHECK_ARG(n_hints == 0 || (hint_base && hint_row_bytes && hint_shift && hint_h && hint_w),
-               "dilate_compact_hinted: null hint array");
-  CB_CHECK_ARG(!no_list || (tile_ws && dil_bits), "dilate_compact_hinted: no_list needs tile_ws and dil_bits");
-  cb::PrefetchHints ph;
-  memset(&ph, 0, sizeof(ph));
-  for (int i = 0; i < n_hints; ++i) {
-    CB_CHECK_ARG(hint_shift[i] == 0 || hint_shift[i] == 1, "dilate_compact_hinted: shift must be 0 or 1");
-    CB_CHECK_ARG(hint_base[i] && ((uintptr_t)hint_base[i] % 16) == 0 && hint_row_bytes[i] > 0 &&
-                     (hint_row_bytes[i] % 16) == 0 && hint_h[i] > 0 && hint_w[i] > 0,
-                 "dilate_compact_hinted: hint rows must be 16-byte aligned multiples of 16 bytes");
-    // (a hint never reaches beyond its map: rows are clipped to hint_h x hint_w in the kernel)
-    CB_CHECK_ARG((long long)hint_row_bytes[i] * 32 < (1ll << 31), "dilate_compact_hinted: row too large");
-    ph.base[ph.n] = (const char*)hint_base[i];
-    ph.row_bytes[ph.n] = hint_row_bytes[i];
-    ph.shift[ph.n] = hint_shift[i];
-    ph.tH[ph.n] = hint_h[i];
-    ph.tW[ph.n] = hint_w[i];
-    ++ph.n;
-  }
-  if (tile_ws && (long long)cb_bitmap_words(B, H, W) == 0)
-    cudaMemsetAsync((int32_t*)tile_ws + 1, 0, sizeof(int32_t), (cudaStream_t)stream);
-  return dilate_compact_impl(stream, raw_bits, dil_bits, dil_map, idx, count, ws, tile_ws, B, H, W, kHHalf,
-                             kWHalf, clear_raw, no_list, &ph);
 }
 
 int cb_dilate_compact(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits, int8_t* dil_map,
@@ -215,26 +167,6 @@ int cb_dilate_tiles(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits, 
                     void* tile_ws, int B, int H, int W, int kHHalf, int kWHalf, int clear_raw) {
   CB_CHECK_ARG(tile_ws && dil_bits, "dilate_tiles: null pointer");
   if ((long long)cb_bitmap_words(B, H, W) == 0) cudaMemsetAsync((int32_t*)tile_ws + 1, 0, sizeof(int32_t), (cudaStream_t)stream);
-  // CBINFER_DILATE_TILES=1: dilate_tiles_kernel (one block per tile row, one packed atomic per block).
-  // Faster alone (L1 bitmap of the bench: 4.7 vs 5.7 us back to back) but the whole step measured 1.5 %
-  // SLOWER with it on two boxes (0.193 vs 0.190 ms), so dilate_compact_kernel's tile mode stays the default.
-  static const bool lean = [] {
-    const char* e = getenv("CBINFER_DILATE_TILES");
-    return e && e[0] == '1';
-  }();
-  const int ty = cb::tile_grid_y(H), xp = cb::tile_grid_xp(W);
-  if (lean && (long long)cb_bitmap_words(B, H, W) > 0 && cb::dilate_tiles_ok(B, H, W, kHHalf, ty, xp) &&
-      kWHalf <= 31 && kHHalf >= 0 && kWHalf >= 0 && ((uintptr_t)ws % 8) == 0) {
-    CB_CHECK_ARG(raw_bits && count && ws && raw_bits != dil_bits, "dilate_tiles: bad pointers");
-    const int Wd = (W + 31) / 32;
-    // the packed counter is the first 8 bytes of the compaction workspace (CompactHeader.reserved/done,
-    // both zero at rest, so the two kernels can share one workspace)
-    cb::launch_pdl(dilate_tiles_kernel, dim3((unsigned)(B * ty)), dim3(kDtThreads), cb::dilate_tiles_smem(Wd, kHHalf),
-                   (cudaStream_t)stream, raw_bits, dil_bits, count, (unsigned long long*)ws, B, H, W, Wd, kHHalf,
-                   kWHalf, clear_raw ? const_cast<uint32_t*>(raw_bits) : nullptr, (int32_t*)tile_ws, ty, xp);
-    CB_CHECK_LAUNCH("dilate_tiles");
-    return 0;
-  }
   return dilate_compact_impl(stream, raw_bits, dil_bits, nullptr, nullptr, count, ws, tile_ws, B, H, W,
                              kHHalf, kWHalf, clear_raw, 1);
 }
@@ -252,10 +184,10 @@ int cb_pool_compact(void* stream, const uint32_t* in_bits, uint32_t* out_bits, i
   }
   CB_CHECK_ARG(nwords < (1ll << 31), "pool_compact: bitmap too large");
   const int ntiles = (int)((nwords + kCompactTile - 1) / kCompactTile);
-  cb::launch_pdl(dilate_compact_kernel<false>, ntiles, kCompactThreads, 0, s, in_bits, out_bits, nullptr, idx, count, ws,
+  cb::launch(dilate_compact_kernel, ntiles, kCompactThreads, 0, s, in_bits, out_bits, nullptr, idx, count, ws,
                                                           B, oH, oW, (oW + 31) / 32, 0, 0,
                                                           (int)nwords, ntiles, H, (W + 31) / 32, nullptr,
-                                                          nullptr, 0, 0, (int)compact_coop(), 0, cb::PrefetchHints{});
+                                                          nullptr, 0, 0, (int)compact_coop(), 0);
   CB_CHECK_LAUNCH("pool_compact");
   return 0;
 }
@@ -311,7 +243,7 @@ int cb_map_to_bits(void* stream, const int8_t* map, uint32_t* bits, int B, int H
   const long long nwords = (long long)cb_bitmap_words(B, H, W);
   if (nwords == 0) return 0;
   const long long blocks = (nwords + 7) / 8;
-  cb::launch_pdl(map_to_bits_kernel, (unsigned)blocks, 256, 0, (cudaStream_t)stream, map, bits, H, W,
+  cb::launch(map_to_bits_kernel, (unsigned)blocks, 256, 0, (cudaStream_t)stream, map, bits, H, W,
                                                                         (W + 31) / 32, nwords);
   CB_CHECK_LAUNCH("map_to_bits");
   return 0;
@@ -334,7 +266,7 @@ int cb_pack_weights(void* stream, int dtype, int gemm, const void* weight, void*
   if (gemm == CB_GEMM_SIMT_F32) {
     const int CoutP = (Cout + 3) / 4 * 4;
     const long long total = (long long)kH * kW * Cp * CoutP;
-    CB_DISPATCH_DTYPE(dtype, (cb::launch_pdl(pack_weights_simt_kernel<T>, grid_for(total, 256), 256, 0, s, 
+    CB_DISPATCH_DTYPE(dtype, (cb::launch(pack_weights_simt_kernel<T>, grid_for(total, 256), 256, 0, s, 
                                  (const T*)weight, (float*)packed, Cout, Cin, kH, kW, Cp, CoutP)));
     CB_CHECK_LAUNCH("pack_weights");
     return 0;
@@ -364,7 +296,7 @@ static int conv_update_impl(const cb::RowMask& mk, void* stream, int dtype, int 
   if (gemm == CB_GEMM_SIMT_F32) {
     const int CoutP = (Cout + 3) / 4 * 4;
     const unsigned grid = (unsigned)(sm_count() * 4);
-    CB_DISPATCH_DTYPE(dtype, (cb::launch_pdl(conv_simt_kernel<T>, grid, SM_THREADS, 0, s, 
+    CB_DISPATCH_DTYPE(dtype, (cb::launch(conv_simt_kernel<T>, grid, SM_THREADS, 0, s, 
                                  (const T*)state, pitch_in, idx, count, (const float*)packed_w, bias,
                                  (T*)out, pitch_out, H, W, Cout, CoutP, kH, kW, relu)));
     CB_CHECK_LAUNCH("conv_update(simt)");
@@ -416,11 +348,7 @@ int cb_conv_tiled_supported(int dtype, int gemm, int B, int H, int W, int Cin, i
 static int conv_update_tiled_impl(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
                          int pitch_in, const void* tile_ws, const uint32_t* dil_bits,
                          const void* packed_w, const float* bias, void* out, int pitch_out, int B,
-                         int H, int W, int Cin, int Cout, int kH, int kW, int relu, const cb::PoolFuse& pf,
-                         const cb::TileSelf* self = nullptr) {
-  cb::TileSelf sf;
-  memset(&sf, 0, sizeof(sf));
-  if (self) sf = *self;
+                         int H, int W, int Cin, int Cout, int kH, int kW, int relu, const cb::PoolFuse& pf) {
   CB_CHECK_ARG(state && tile_ws && dil_bits && packed_w && bias && out, "conv_update_tiled: null pointer");
   CB_CHECK_ARG(gemm != CB_GEMM_SIMT_F32, "conv_update_tiled: tensor-core modes only");
   const int want_pitch = gemm == CB_GEMM_TC_BF16X3 ? cb::pitch16_of(Cin) : cb_channel_pitch(dtype, Cin);
@@ -431,7 +359,7 @@ static int conv_update_tiled_impl(void* stream, int dtype, int gemm, const void*
   if (B == 0 || H == 0 || W == 0) return 0;
   return cb::umma_conv_update_tiled((cudaStream_t)stream, dtype, gemm, state, state_lo, pitch_in,
                                     (const int32_t*)tile_ws, dil_bits, packed_w, bias, out, pitch_out,
-                                    B, H, W, Cout, kH, kW, relu, pf, sf);
+                                    B, H, W, Cout, kH, kW, relu, pf);
 }
 
 int cb_conv_update_tiled(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
@@ -468,7 +396,7 @@ static int tiled_pool_impl(void* stream, int dtype, int gemm, const void* state,
                               void* pool_out, long long o_sb, long long o_sy, int o_pitch, int oH, int oW,
                               void* next_state, long long n_sb, long long n_sy, int n_pitch, int aux_mode,
                               void* aux_hi, void* aux_lo, uint32_t* next_raw_bits, float threshold,
-                              int update_mode, const cb::TileSelf* self) {
+                              int update_mode) {
   CB_CHECK_ARG(pool_out && next_state && next_raw_bits, "conv_update_tiled_pool: null pointer");
   CB_CHECK_ARG(update_mode == CB_UPDATE_NONE || update_mode == CB_UPDATE_CHANGED || update_mode == CB_UPDATE_ALL,
                "conv_update_tiled_pool: bad update_mode %d", update_mode);
@@ -488,7 +416,7 @@ static int tiled_pool_impl(void* stream, int dtype, int gemm, const void* state,
   CB_DISPATCH_DTYPE(dtype, rc = cb::make_aux<T>(pf.aux, aux_mode, aux_hi, aux_lo, next_state, Cout));
   if (rc) return rc;
   return conv_update_tiled_impl(stream, dtype, gemm, state, state_lo, pitch_in, tile_ws, dil_bits, packed_w,
-                                bias, out, pitch_out, B, H, W, Cin, Cout, kH, kW, relu, pf, self);
+                                bias, out, pitch_out, B, H, W, Cin, Cout, kH, kW, relu, pf);
 }
 
 int cb_conv_update_tiled_pool(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
@@ -502,53 +430,7 @@ int cb_conv_update_tiled_pool(void* stream, int dtype, int gemm, const void* sta
   return tiled_pool_impl(stream, dtype, gemm, state, state_lo, pitch_in, tile_ws, dil_bits, packed_w, bias, out,
                          pitch_out, B, H, W, Cin, Cout, kH, kW, relu, pool_out, o_sb, o_sy, o_pitch, oH, oW,
                          next_state, n_sb, n_sy, n_pitch, aux_mode, aux_hi, aux_lo, next_raw_bits, threshold,
-                         update_mode, nullptr);
-}
-
-int cb_conv_tiled_self_supported(int B, int H, int W, int kH, int kW) {
-  // one warp lane per raw row of a 16-row tile's window (16 + 2*kHHalf <= 32), funnel shifts up to 31;
-  // the barrier word carries the tile count in 20 bits
-  return kH >= 1 && kW >= 1 && (kH & 1) && (kW & 1) && (kH - 1) / 2 <= 8 && (kW - 1) / 2 <= 31 &&
-                 B >= 0 && H >= 0 && W >= 0 && (long long)B * H * W < (1ll << 31) &&
-                 (long long)B * cb::tile_grid_y(H) * cb::tile_grid_xp(W) < (1ll << 20)
-             ? 1 : 0;
-}
-
-int cb_conv_update_tiled_self(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
-                              int pitch_in, void* tile_ws, uint32_t* dil_bits,
-                              const void* packed_w, const float* bias, void* out, int pitch_out, int B,
-                              int H, int W, int Cin, int Cout, int kH, int kW, int relu,
-                              void* pool_out, long long o_sb, long long o_sy, int o_pitch, int oH, int oW,
-                              void* next_state, long long n_sb, long long n_sy, int n_pitch, int aux_mode,
-                              void* aux_hi, void* aux_lo, uint32_t* next_raw_bits, float threshold,
-                              int update_mode, const uint32_t* raw_bits, int32_t* count, void* ws,
-                              int clear_raw) {
-  CB_CHECK_ARG(raw_bits && count && ws && dil_bits && tile_ws, "conv_update_tiled_self: null pointer");
-  CB_CHECK_ARG(raw_bits != dil_bits, "conv_update_tiled_self: dil_bits must not alias raw_bits");
-  CB_CHECK_ARG(cb_conv_tiled_self_supported(B, H, W, kH, kW),
-               "conv_update_tiled_self: filter %dx%d / map %dx%dx%d not supported", kH, kW, B, H, W);
-  if (B == 0 || H == 0 || W == 0) {
-    cudaMemsetAsync(count, 0, sizeof(int32_t), (cudaStream_t)stream);
-    cudaMemsetAsync((int32_t*)tile_ws + 1, 0, sizeof(int32_t), (cudaStream_t)stream);
-    CB_CHECK_LAUNCH("conv_update_tiled_self(memset)");
-    return 0;
-  }
-  cb::TileSelf sf;
-  sf.raw = raw_bits;
-  sf.dil = dil_bits;
-  sf.clear = clear_raw ? const_cast<uint32_t*>(raw_bits) : nullptr;
-  sf.count = count;
-  sf.acc_pix = &reinterpret_cast<cb::CompactHeader*>(ws)->reserved;
-  if (!pool_out) {
-    cb::PoolFuse pf;
-    memset(&pf, 0, sizeof(pf));
-    return conv_update_tiled_impl(stream, dtype, gemm, state, state_lo, pitch_in, tile_ws, dil_bits, packed_w,
-                                  bias, out, pitch_out, B, H, W, Cin, Cout, kH, kW, relu, pf, &sf);
-  }
-  return tiled_pool_impl(stream, dtype, gemm, state, state_lo, pitch_in, tile_ws, dil_bits, packed_w, bias, out,
-                         pitch_out, B, H, W, Cin, Cout, kH, kW, relu, pool_out, o_sb, o_sy, o_pitch, oH, oW,
-                         next_state, n_sb, n_sy, n_pitch, aux_mode, aux_hi, aux_lo, next_raw_bits, threshold,
-                         update_mode, &sf);
+                         update_mode);
 }
 
 int cb_conv_update_masked(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
@@ -619,11 +501,11 @@ int cb_maxpool2x2(void* stream, int dtype, const void* x, long long x_sb, long l
     int glog = 0;
     while ((1 << glog) < cpp && glog < 5) ++glog;
     glog = cb::glog_tuned(glog);
-    CB_DISPATCH_DTYPE(dtype, (cb::launch_pdl(maxpool2x2_vec_kernel<T, VEC>, grid, 256, 0, (cudaStream_t)stream, 
+    CB_DISPATCH_DTYPE(dtype, (cb::launch(maxpool2x2_vec_kernel<T, VEC>, grid, 256, 0, (cudaStream_t)stream, 
                                  (const T*)x, x_sb, x_sy, (int)x_sx, idx, count, dil_bits, (T*)out,
                                  o_sb, o_sy, (int)o_sx, cpp, glog, H, W, oH, oW)));
   } else {
-    CB_DISPATCH_DTYPE(dtype, (cb::launch_pdl(maxpool2x2_kernel<T>, grid, 256, 0, (cudaStream_t)stream, 
+    CB_DISPATCH_DTYPE(dtype, (cb::launch(maxpool2x2_kernel<T>, grid, 256, 0, (cudaStream_t)stream, 
                                  (const T*)x, x_sb, x_sc, x_sy, x_sx, idx, count, dil_bits, (T*)out,
                                  o_sb, o_sc, o_sy, o_sx, C, H, W, oH, oW)));
   }
@@ -677,7 +559,7 @@ int cb_maxpool2x2_detect(void* stream, int dtype, const void* x, long long x_sb,
   CB_DISPATCH_DTYPE(dtype, {                                                                      \
     AuxPlanes aux;                                                                                \
     if (int rc = make_aux<T>(aux, aux_mode, aux_hi, aux_lo, next_state, C)) return rc;            \
-    cb::launch_pdl(maxpool2x2_detect_kernel<T, VEC, U_>, grid, 256, 0, s, (const T*)x, x_sb,     \
+    cb::launch(maxpool2x2_detect_kernel<T, VEC, U_>, grid, 256, 0, s, (const T*)x, x_sb,         \
                    x_sy, x_pitch, idx, count, dil_bits, (T*)out, o_sb, o_sy, o_pitch, cpp, glog, \
                    H, W, oH, oW, (T*)next_state, n_sb, n_sy, n_pitch, aux, next_raw_bits,         \
                    thr_cast<T>(threshold));                                                       \
@@ -698,7 +580,7 @@ int cb_gen_xmatrix(void* stream, int dtype, void* columns, const void* input, co
   if (n <= 0) return 0;
   CB_CHECK_ARG(columns && input && idx, "gen_xmatrix: null pointer");
   const long long total = (long long)n * C * kH * kW;
-  CB_DISPATCH_DTYPE(dtype, (cb::launch_pdl(gen_xmatrix_kernel<T>, grid_for(total, 256, 16), 256, 0, (cudaStream_t)stream, 
+  CB_DISPATCH_DTYPE(dtype, (cb::launch(gen_xmatrix_kernel<T>, grid_for(total, 256, 16), 256, 0, (cudaStream_t)stream, 
                                (T*)columns, (const T*)input, idx, kW, kH, C, W, H, n)));
   CB_CHECK_LAUNCH("gen_xmatrix");
   return 0;
@@ -710,7 +592,7 @@ int cb_matrix_mult(void* stream, int dtype, const void* X, const void* weight, c
   CB_CHECK_ARG(X && weight && bias && Y, "matrix_mult: null pointer");
   dim3 grid((Cout + 31) / 32, (n + 31) / 32);
   CB_CHECK_ARG(grid.y < 65536, "matrix_mult: n too large for the staged op");
-  CB_DISPATCH_DTYPE(dtype, (cb::launch_pdl(matrix_mult_kernel<T>, grid, 256, 0, (cudaStream_t)stream, 
+  CB_DISPATCH_DTYPE(dtype, (cb::launch(matrix_mult_kernel<T>, grid, 256, 0, (cudaStream_t)stream, 
                                (const T*)X, (const T*)weight, (const T*)bias, (T*)Y, n, K, Cout)));
   CB_CHECK_LAUNCH("matrix_mult");
   return 0;
@@ -721,7 +603,7 @@ int cb_update_output(void* stream, int dtype, const void* Yt, void* output, cons
   if (n <= 0) return 0;
   CB_CHECK_ARG(Yt && output && idx, "update_output: null pointer");
   const long long total = (long long)n * Cout;
-  CB_DISPATCH_DTYPE(dtype, (cb::launch_pdl(update_output_kernel<T>, grid_for(total, 256, 16), 256, 0, (cudaStream_t)stream, 
+  CB_DISPATCH_DTYPE(dtype, (cb::launch(update_output_kernel<T>, grid_for(total, 256, 16), 256, 0, (cudaStream_t)stream, 
                                (const T*)Yt, (T*)output, idx, numOutputPixel, n, Cout, relu)));
   CB_CHECK_LAUNCH("update_output");
   return 0;
@@ -735,7 +617,7 @@ int cb_fg_update(void* stream, const float* x, float* prev, const float* weight,
   cudaMemsetAsync(count, 0, sizeof(int32_t), s);
   const long long total = (long long)B * Cin * H * W;
   if (total == 0) return 0;
-  cb::launch_pdl(fg_update_kernel, grid_for((total + 31) / 32 * 32, 256, 8), 256, 0, s, x, prev, weight, out, count, B, Cin,
+  cb::launch(fg_update_kernel, grid_for((total + 31) / 32 * 32, 256, 8), 256, 0, s, x, prev, weight, out, count, B, Cin,
                                                              Cout, H, W, kH, kW, threshold);
   CB_CHECK_LAUNCH("fg_update");
   return 0;
@@ -775,11 +657,11 @@ int cb_resize_bicubic_u8(void* stream, const uint8_t* src, long long s_y, long l
   char* w = (char*)ws;
   uint8_t* tmp = (uint8_t*)(w + p.off_tmp);                    // [sH, dW, C] interleaved
   cudaStream_t s = (cudaStream_t)stream;
-  cb::launch_pdl(cb::resize_pass_u8_kernel<1>, dim3((unsigned)((dW + 255) / 256), (unsigned)sH), dim3(256), 0, s, src,
+  cb::launch(cb::resize_pass_u8_kernel<1>, dim3((unsigned)((dW + 255) / 256), (unsigned)sH), dim3(256), 0, s, src,
                  s_y, s_x, s_c, tmp, (long long)dW * C, (long long)C, 1ll, sH, dW, C,
                  (const int32_t*)(w + p.off_bx), (const int32_t*)(w + p.off_kx), p.ksize_x);
   CB_CHECK_LAUNCH("resize_bicubic_u8(horizontal)");
-  cb::launch_pdl(cb::resize_pass_u8_kernel<0>, dim3((unsigned)((dW + 255) / 256), (unsigned)dH), dim3(256), 0, s,
+  cb::launch(cb::resize_pass_u8_kernel<0>, dim3((unsigned)((dW + 255) / 256), (unsigned)dH), dim3(256), 0, s,
                  (const uint8_t*)tmp, (long long)dW * C, (long long)C, 1ll, dst, d_y, d_x, d_c, dH, dW, C,
                  (const int32_t*)(w + p.off_by), (const int32_t*)(w + p.off_ky), p.ksize_y);
   CB_CHECK_LAUNCH("resize_bicubic_u8(vertical)");
@@ -791,7 +673,7 @@ int cb_resize_bilinear_u8(void* stream, const uint8_t* src, long long s_y, long 
                           float divisor, float cval, float clip_lo, float clip_hi) {
   CB_CHECK_ARG(src && dst && sH > 0 && sW > 0 && dH > 0 && dW > 0 && C >= 1 && divisor != 0.f,
                "resize_bilinear_u8: bad arguments");
-  cb::launch_pdl(cb::resize_bilinear_kernel, dim3((unsigned)((dW + 255) / 256), (unsigned)dH), dim3(256), 0,
+  cb::launch(cb::resize_bilinear_kernel, dim3((unsigned)((dW + 255) / 256), (unsigned)dH), dim3(256), 0,
                  (cudaStream_t)stream, src, s_y, s_x, s_c, sH, sW, dst, d_y, d_x, d_c, dH, dW, C, (double)divisor,
                  (double)cval, (double)clip_lo, (double)clip_hi);
   CB_CHECK_LAUNCH("resize_bilinear_u8");

@@ -26,20 +26,6 @@ int fail(int code, const char* fmt, ...);
   } while (0)
 
 int sm_count();
-bool pdl_enabled();
-
-// Programmatic dependent launch: every kernel of this library starts with pdl_prologue() --
-// "my dependents may be scheduled" + "wait until the grids I depend on have completed and their
-// writes are visible" -- and is launched with programmatic stream serialisation, so the next
-// kernel of the stream is already resident when its predecessor drains (no launch gap between the
-// ~20 dependent kernels of a frame; also inside CUDA graphs).  Experimental, enabled only with
-// CBINFER_PDL=1 (see pdl_enabled()); without the launch attribute both instructions are no-ops.
-__device__ __forceinline__ void pdl_prologue() {
-#ifndef CB_PDL_LATE          // -DCB_PDL_LATE: no early trigger (dependents are released when this grid's CTAs exit)
-  asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-  asm volatile("griddepcontrol.wait;" ::: "memory");
-}
 
 // log2 of the lanes that share one pixel in the candidate-detection / pooling kernels.  One lane
 // per 16-byte chunk would be the obvious choice; two chunks per lane halves the number of warps
@@ -65,16 +51,11 @@ inline void launch_cluster(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t
   cfg.blockDim = block;
   cfg.dynamicSmemBytes = smem;
   cfg.stream = s;
-  cudaLaunchAttribute attr[3];
+  cudaLaunchAttribute attr[2];
   unsigned na = 0;
   if (cooperative) {
     attr[na].id = cudaLaunchAttributeCooperative;
     attr[na].val.cooperative = 1;
-    ++na;
-  }
-  if (pdl_enabled()) {
-    attr[na].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-    attr[na].val.programmaticStreamSerializationAllowed = 1;
     ++na;
   }
   if (cluster_x > 1) {                         // thread-block cluster (cluster_x, 1, 1)
@@ -90,8 +71,8 @@ inline void launch_cluster(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t
 }
 
 template <typename... KArgs, typename... Args>
-inline void launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s,
-                       Args&&... args) {
+inline void launch(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s,
+                   Args&&... args) {
   launch_cluster(kern, grid, block, smem, s, 1u, 0, static_cast<Args&&>(args)...);
 }
 

@@ -92,62 +92,18 @@ __device__ __forceinline__ unsigned pooled_word(const uint32_t* __restrict__ raw
   return d;
 }
 
-// L2 prefetch hints (extension, no reference counterpart).  The kernels that consume a change set a
-// few launches later read rows they have not touched for a frame (the next layer's state at the
-// rewritten pixels: cold in L2, a chain of dependent DRAM round trips inside a latency-bound kernel).
-// The dilation is the first kernel to know WHICH pixels those are, so it asks L2 for them while the
-// contraction in between keeps the tensor cores busy: per dilated word, one cp.async.bulk.prefetch.L2
-// per run of set bits and target (pixel-major maps: a run of pixels is one contiguous byte range).
-// shift = 1: the target has the 2x2-pooled resolution (issued from even rows).  Hints only -- no
-// architectural state changes, results are bit-identical with and without them.
-constexpr int kMaxHints = 3;
-struct PrefetchHints {
-  const char* base[kMaxHints];
-  int row_bytes[kMaxHints], shift[kMaxHints], tH[kMaxHints], tW[kMaxHints];
-  int n;
-};
-
-__device__ __forceinline__ void prefetch_l2_bulk(const void* p, unsigned bytes) {
-  asm volatile("cp.async.bulk.prefetch.L2.global [%0], %1;" ::"l"(p), "r"(bytes) : "memory");
-}
-
-__device__ __forceinline__ void prefetch_hinted_rows(const PrefetchHints& hints, unsigned d, int b, int y, int j) {
-#pragma unroll
-  for (int h = 0; h < kMaxHints; ++h) {        // (constant indices: the parameter struct stays in constant memory)
-    if (h >= hints.n) break;
-    const int sh = hints.shift[h];
-    if (sh && (y & 1)) continue;
-    const int yy = y >> sh, tH = hints.tH[h], tW = hints.tW[h], rb = hints.row_bytes[h];
-    if (yy >= tH) continue;
-    const char* row = hints.base[h] + (long long)(b * tH + yy) * tW * rb;
-    unsigned dd = d;
-    while (dd) {
-      const int x0 = __ffs(dd) - 1;
-      const unsigned inv = ~(dd >> x0);
-      const int len = inv ? __ffs(inv) - 1 : 32 - x0;        // run of set bits x0 .. x0 + len - 1
-      const int xa = (j * 32 + x0) >> sh;
-      int xb = (j * 32 + x0 + len - 1) >> sh;
-      if (xb >= tW) xb = tW - 1;
-      if (xa <= xb) prefetch_l2_bulk(row + (long long)xa * rb, (unsigned)((xb - xa + 1) * rb));
-      dd = x0 + len >= 32 ? 0u : dd & (0xffffffffu << (x0 + len));
-    }
-  }
-}
-
 // List mode: tiles are taken by ticket (atomicAdd on the header's `ticket`), not by blockIdx -- every
 // predecessor of a running tile then holds an earlier ticket, i.e. is running or finished, whatever
 // order the hardware dispatches blocks in, so the look-back cannot starve (as in CUB's single-pass
 // scan).  Tile-only mode has no scan across tiles and keeps blockIdx, and so do grids small enough to
 // be resident as a whole.
-template <bool HINTS>
 __global__ void __launch_bounds__(kCompactThreads)
 dilate_compact_kernel(const uint32_t* __restrict__ raw, uint32_t* __restrict__ dil_bits,
                       int8_t* __restrict__ dil_map, int32_t* __restrict__ idx,
                       int32_t* __restrict__ count, void* ws, int B, int H, int W, int Wd, int kh,
                       int kw, int nwords, int ntiles, int pool_hin, int pool_wdin,
                       uint32_t* __restrict__ clear_bits, int32_t* __restrict__ tile_ws, int tile_ty,
-                      int tile_xp, int coop, int no_list, const PrefetchHints hints) {
-  pdl_prologue();
+                      int tile_xp, int coop, int no_list) {
   CompactHeader* hdr = reinterpret_cast<CompactHeader*>(ws);
   volatile unsigned long long* tstate =
       reinterpret_cast<volatile unsigned long long*>(reinterpret_cast<char*>(ws) + sizeof(CompactHeader));
@@ -203,7 +159,6 @@ dilate_compact_kernel(const uint32_t* __restrict__ raw, uint32_t* __restrict__ d
       d[i] = pool_hin ? pooled_word(raw, r / H, y, j, pool_hin, pool_wdin, W)
                       : dilated_word(win, win0, r, y, j, H, W, Wd, kh, kw);
       if (dil_bits) dil_bits[w] = d[i];
-      if (HINTS && d[i]) prefetch_hinted_rows(hints, d[i], r / H, y, j);
     }
     if (tile_ws) {
       // dirty 8 x 16 output tiles for the tiled contraction (conv_tile.cuh): a word covers four
@@ -444,188 +399,8 @@ __device__ __forceinline__ void block_dilate_compact(uint32_t* __restrict__ raw,
     for (int i = tid; i < nwords; i += nthr) raw[i] = 0u;
 }
 
-// ------------------------------------------------------------------------------------------------
-// dilate_tiles_kernel -- dilation + dirty-tile list + change count, for consumers that walk tiles
-// (cb_dilate_tiles; no ordered index list, hence no scan across blocks).
-//
-// One block per (image, tile row) = 16 map rows x Wd bitmap words: the raw rows it can touch
-// (16 + 2*kh, zero-padded by one word on each side) are staged in shared memory with one round of
-// independent loads; a thread computes a dilated word from shared memory, stores it and ORs it into
-// its column's accumulator; the column accumulators are the tile flags (a word covers four 8-pixel
-// tiles), so every tile has exactly ONE owner thread -- no stamps, no exchange atomics.  ONE 64-bit
-// atomicAdd per block carries (blocks done | tiles appended | changed pixels): its return value is
-// both the block's append position and the "am I last" test, and the last block publishes the totals
-// from it without reading anything back.  Two dependent global round trips per block (stage, atomic)
-// instead of five in dilate_compact_kernel's tile mode.
-// Clearing the raw bitmap (candidate-path layers): a block zeroes the rows only it reads right after
-// staging them; the rows shared with the neighbouring tile rows are left to the last block.
-//   sync word layout: [63:51] blocks done | [50:31] tiles | [30:0] changed pixels   (0 at rest)
-// ------------------------------------------------------------------------------------------------
-constexpr int kDtThreads = 256;
-constexpr int kDtRows = 16;                                   // = TL_H of conv_tile.cuh
-
-__host__ __device__ inline size_t dilate_tiles_smem(int Wd, int kh) {
-  return ((size_t)(kDtRows + 2 * kh) * (Wd + 2) + Wd) * sizeof(uint32_t);
-}
-// limits of the packed counter; beyond them cb_dilate_tiles keeps dilate_compact_kernel
-__host__ __device__ inline bool dilate_tiles_ok(int B, int H, int W, int kh, int tile_ty, int tile_xp) {
-  const int Wd = (W + 31) / 32;
-  return kh <= kDtRows / 2 && (long long)B * tile_ty < 8192 && (long long)B * tile_ty * tile_xp < (1ll << 20) &&
-         dilate_tiles_smem(Wd, kh) <= 48 * 1024;
-}
-
-__global__ void __launch_bounds__(kDtThreads)
-dilate_tiles_kernel(const uint32_t* __restrict__ raw, uint32_t* __restrict__ dil_bits,
-                    int32_t* __restrict__ count, unsigned long long* __restrict__ sync, int B, int H,
-                    int W, int Wd, int kh, int kw, uint32_t* __restrict__ clear_bits,
-                    int32_t* __restrict__ tile_ws, int tile_ty, int tile_xp) {
-  pdl_prologue();
-  extern __shared__ uint32_t dt_smem[];
-  const int WS = Wd + 2, NR = kDtRows + 2 * kh;
-  uint32_t* s_raw = dt_smem;                                  // [NR][WS], column 0 and WS-1 are zero
-  uint32_t* s_col = dt_smem + NR * WS;                        // [Wd] OR of the block's dilated words
-  __shared__ int s_warp[kDtThreads / 32], s_cnt[kDtThreads / 32];
-  __shared__ unsigned long long s_old;
-  __shared__ int s_ntl;
-  const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-  const int b = blockIdx.x / tile_ty, ty = blockIdx.x - b * tile_ty;
-  const int y0 = ty * kDtRows;
-  const uint32_t* rimg = raw + (long long)b * H * Wd;
-
-  // ---- stage rows y0-kh .. y0+15+kh (zero outside the image) ---------------------------------
-  for (int i = tid; i < NR * WS; i += kDtThreads) {
-    const int r = i / WS, c = i - r * WS;
-    const int y = y0 - kh + r, j = c - 1;
-    s_raw[i] = (y >= 0 && y < H && j >= 0 && j < Wd) ? __ldg(rimg + (long long)y * Wd + j) : 0u;
-  }
-  for (int i = tid; i < Wd; i += kDtThreads) s_col[i] = 0u;
-  __syncthreads();
-  if (clear_bits) {                                           // rows nobody else reads: mine to clear
-    uint32_t* cimg = clear_bits + (long long)b * H * Wd;
-    const int lo = ty == 0 ? 0 : kh, hi = ty == tile_ty - 1 ? kDtRows : kDtRows - kh;
-    for (int i = tid; i < (hi - lo) * Wd; i += kDtThreads) {
-      const int y = y0 + lo + i / Wd;
-      if (y < H) cimg[(long long)y * Wd + i % Wd] = 0u;
-    }
-  }
-
-  // ---- dilated words ---------------------------------------------------------------------------
-  int cnt = 0;
-  uint32_t* dimg = dil_bits + (long long)b * H * Wd;
-  for (int i = tid; i < kDtRows * Wd; i += kDtThreads) {
-    const int r = i / Wd, j = i - r * Wd;
-    const int y = y0 + r;
-    if (y >= H) break;
-    unsigned vp = 0, vc = 0, vn = 0;
-    const uint32_t* p = s_raw + r * WS + j;                   // row y-kh, column j-1
-    for (int q = 0; q <= 2 * kh; ++q, p += WS) {
-      vp |= p[0];
-      vc |= p[1];
-      vn |= p[2];
-    }
-    unsigned d = vc;
-    for (int dx = 1; dx <= kw; ++dx) {
-      d |= (vc << dx) | (vp >> (32 - dx));
-      d |= (vc >> dx) | (vn << (32 - dx));
-    }
-    if (j == Wd - 1 && (W & 31)) d &= (1u << (W & 31)) - 1u;
-    dimg[(long long)y * Wd + j] = d;
-    if (d) {
-      atomicOr(&s_col[j], d);
-      cnt += __popc(d);
-    }
-  }
-  __syncthreads();
-
-  // ---- tiles of this block: thread j owns the four tiles of column word j --------------------------
-  // (maps wider than 32 * kDtThreads pixels take several rounds of columns)
-  unsigned flags = 0;
-  int mine = 0;
-  for (int c0 = 0; c0 < Wd; c0 += kDtThreads) {
-    const int j = c0 + tid;
-    unsigned f = 0;
-    if (j < Wd) {
-      const unsigned v = s_col[j];
-#pragma unroll
-      for (int q = 0; q < 4; ++q)
-        if ((v >> (8 * q)) & 0xffu) f |= 1u << q;
-    }
-    if (c0 == 0) flags = f;                                   // first round is kept in registers
-    mine += __popc(f);
-  }
-  // block totals: tiles (prefix needed) and changed pixels
-  int incl = mine;
-#pragma unroll
-  for (int o = 1; o < 32; o <<= 1) {
-    const int v = __shfl_up_sync(0xffffffffu, incl, o);
-    if (lane >= o) incl += v;
-  }
-  int csum = cnt;
-#pragma unroll
-  for (int o = 16; o > 0; o >>= 1) csum += __shfl_xor_sync(0xffffffffu, csum, o);
-  if (lane == 31) s_warp[wid] = incl;
-  if (lane == 0) s_cnt[wid] = csum;
-  __syncthreads();
-  int woff = 0, ntl_blk = 0, cnt_blk = 0;
-#pragma unroll
-  for (int q = 0; q < kDtThreads / 32; ++q) {
-    if (q < wid) woff += s_warp[q];
-    ntl_blk += s_warp[q];
-    cnt_blk += s_cnt[q];
-  }
-  const unsigned nblocks = (unsigned)B * tile_ty;
-  if (tid == 0) {
-    __threadfence();                                          // (clears and dil_bits precede the count)
-    s_old = atomicAdd(sync, (1ull << 51) | ((unsigned long long)ntl_blk << 31) | (unsigned long long)cnt_blk);
-  }
-  __syncthreads();
-  const unsigned long long old = s_old;
-  const int base = (int)((old >> 31) & 0xFFFFFull);
-  const bool last = (unsigned)(old >> 51) == nblocks - 1u;
-  {
-    int32_t* list = tile_ws + 4 + B * tile_ty * tile_xp;
-    int pos = base + woff + incl - mine;
-    const int t0 = (b * tile_ty + ty) * tile_xp;
-    for (int c0 = 0; c0 < Wd; c0 += kDtThreads) {
-      const int j = c0 + tid;
-      unsigned f = flags;
-      if (c0 > 0) {
-        f = 0;
-        if (j < Wd) {
-          const unsigned v = s_col[j];
-#pragma unroll
-          for (int q = 0; q < 4; ++q)
-            if ((v >> (8 * q)) & 0xffu) f |= 1u << q;
-        }
-      }
-#pragma unroll
-      for (int q = 0; q < 4; ++q)
-        if ((f >> q) & 1u) list[pos++] = t0 + 4 * j + q;
-    }
-  }
-  if (last) {
-    if (tid == 0) {
-      tile_ws[1] = base + ntl_blk;
-      *count = (int32_t)(old & 0x7FFFFFFFull) + cnt_blk;
-      *sync = 0ull;
-    }
-    if (clear_bits && kh > 0) {                               // the rows two tile rows share
-      const int slots = (int)nblocks * 2 * kh;                // (image, tile row) x (top kh rows, bottom kh rows)
-      for (int i = tid; i < slots * Wd; i += kDtThreads) {    // (32-bit: < the bitmap's word count)
-        const int row = i / Wd, j = i - row * Wd;
-        const int blk = row / (2 * kh), q = row - blk * 2 * kh;
-        const int bb = blk / tile_ty, tt = blk - bb * tile_ty;
-        if ((q < kh && tt == 0) || (q >= kh && tt == tile_ty - 1)) continue;   // cleared by their owner
-        const int y = tt * kDtRows + (q < kh ? q : kDtRows - 2 * kh + q);
-        if (y < H) clear_bits[((long long)bb * H + y) * Wd + j] = 0u;
-      }
-    }
-  }
-}
-
 __global__ void map_to_bits_kernel(const int8_t* __restrict__ map, uint32_t* __restrict__ bits,
                                    int H, int W, int Wd, long long nwords) {
-  pdl_prologue();
   const int lane = threadIdx.x & 31;
   const long long w = (long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
   if (w >= nwords) return;

@@ -39,7 +39,6 @@ conv_simt_kernel(const T* __restrict__ state, int Cp, const int32_t* __restrict_
                  const int32_t* __restrict__ count, const float* __restrict__ Wp,
                  const float* __restrict__ bias, T* __restrict__ out, int Op, int H, int W,
                  int Cout, int CoutP, int kH, int kW, int relu) {
-  pdl_prologue();
   __shared__ __align__(16) float As[SM_BM][SM_BK + SM_APAD];
   __shared__ __align__(16) float Bs[SM_BK][SM_BN];
   __shared__ int s_pix[SM_BM];               // pixel index or -1
@@ -147,7 +146,6 @@ conv_simt_kernel(const T* __restrict__ state, int Cp, const int32_t* __restrict_
 template <typename T>
 __global__ void pack_weights_simt_kernel(const T* __restrict__ w, float* __restrict__ Wp, int Cout,
                                          int Cin, int kH, int kW, int Cp, int CoutP) {
-  pdl_prologue();
   const long long total = (long long)kH * kW * Cp * CoutP;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
        i += (long long)gridDim.x * blockDim.x) {

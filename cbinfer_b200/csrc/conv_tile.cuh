@@ -101,138 +101,6 @@ struct PoolFuse {
   int update;                    // CB_UPDATE_*
 };
 
-// Optional self-listing prologue (cb_conv_update_tiled_self): the kernel derives the dilated bitmap,
-// the dirty-tile list and the change count from the RAW change bitmap itself -- the job of
-// cb_dilate_tiles (reference: the scatter-dilate of changeDetection_kernel, cbconv2d_cg_backend.cu:62-72)
-// -- so a tile-path layer needs no dilation launch at all.  One warp per (image, tile row, bitmap word):
-// lane l loads the three raw words of row y0 - kh + l (one round of independent loads), dilates them
-// horizontally with funnel shifts; the vertical OR over 2kh + 1 rows is a chain of shuffles; lanes 0..15
-// then hold the 16 dilated words of the item: stored, counted, and folded into four tile flags with
-// ballots (a word covers four 8-pixel tiles); one atomicAdd per warp appends its dirty tiles.  A grid
-// barrier (sense-reversing, all CTAs co-resident: cooperative launch) separates the listing from the
-// contraction; the last CTA to arrive publishes the totals where cb_dilate_tiles would have left them
-// (tile_ws[1], *count) and resets the accumulators, so the workspaces stay interchangeable between the
-// two paths.  raw == nullptr: off.
-struct TileSelf {
-  const uint32_t* raw;           // raw change bitmap of this layer
-  uint32_t* dil;                 // dilated bitmap (output; the kernel's dil_bits)
-  uint32_t* clear;               // raw bitmap to zero once every CTA has consumed it, or nullptr
-  int32_t* count;                // *count = number of dilated pixels
-  unsigned* acc_pix;             // CompactHeader.reserved of the compaction workspace (0 at rest)
-};
-
-// returns the number of dirty tiles (the barrier's release word carries it: no extra load)
-// `scratch`: 40 words of shared memory (the kernel's dynamic buffer, not yet in use: static shared
-// memory would push the kernel past the 227 KB it reserves)
-__device__ __forceinline__ int tile_self_list(const TileSelf& sf, int32_t* tws, int B, int H, int W, int Wd,
-                                              int TY, int TXp, int kh, int kw, int* scratch) {
-  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5, nwarps = blockDim.x >> 5;
-  const int NI = B * TY * Wd;
-  int32_t* list = tws + 4 + B * TY * TXp;
-  unsigned* s_flags = reinterpret_cast<unsigned*>(scratch);  // [16]
-  int* s_pix = scratch + 16;                                 // [16]
-  int& s_base = scratch[32];
-  int& s_ntl = scratch[33];
-  // barrier word tws[3] = generation << 20 | dirty tiles of the last launch; read up front (it cannot
-  // advance before this CTA arrives), needed only at the end
-  volatile unsigned* gen = reinterpret_cast<volatile unsigned*>(tws + 3);
-  unsigned g0 = 0;
-  if (tid == 0) g0 = *gen >> 20;
-  int pix_cta = 0;                                           // thread 0 only
-  // a CTA takes nwarps consecutive items per round (neighbouring words of a tile row: the dirty ones
-  // cluster), and appends the round's tiles with ONE atomicAdd -- same-address returning atomics are
-  // serialised by the L2 (one per warp: 400 of them on the 640x480 layer, measured +10 us)
-  for (int item0 = blockIdx.x * nwarps; item0 < NI; item0 += gridDim.x * nwarps) {
-    const int item = item0 + warp;
-    const bool have = item < NI;
-    const int wx = have ? item % Wd : 0, r = have ? item / Wd : 0;
-    const int ty = r % TY, b = r / TY;
-    const int y0 = ty * TL_H, y = y0 - kh + lane;
-    unsigned vp = 0, vc = 0, vn = 0;
-    if (have && lane < TL_H + 2 * kh && y >= 0 && y < H) {
-      const uint32_t* row = sf.raw + ((long long)b * H + y) * Wd + wx;
-      vc = __ldcg(row);
-      if (wx > 0) vp = __ldcg(row - 1);
-      if (wx + 1 < Wd) vn = __ldcg(row + 1);
-    }
-    unsigned h = vc;
-    for (int dx = 1; dx <= kw; ++dx) {
-      h |= (vc << dx) | (vp >> (32 - dx));
-      h |= (vc >> dx) | (vn << (32 - dx));
-    }
-    if (wx == Wd - 1 && (W & 31)) h &= (1u << (W & 31)) - 1u;
-    unsigned v = 0;
-    for (int d = 0; d <= 2 * kh; ++d) v |= __shfl_down_sync(0xffffffffu, h, d);   // rows y0+l-kh .. y0+l+kh
-    const bool rowok = have && lane < TL_H && y0 + lane < H;
-    if (!rowok) v = 0u;
-    if (rowok) __stcg(sf.dil + ((long long)b * H + y0 + lane) * Wd + wx, v);
-    int pix = __popc(v);
-#pragma unroll
-    for (int o = 16; o > 0; o >>= 1) pix += __shfl_xor_sync(0xffffffffu, pix, o);
-    unsigned flags = 0;
-#pragma unroll
-    for (int q = 0; q < 4; ++q)
-      if (__ballot_sync(0xffffffffu, ((v >> (8 * q)) & 0xffu) != 0u)) flags |= 1u << q;
-    if (lane == 0) {
-      s_flags[warp] = flags;
-      s_pix[warp] = pix;
-    }
-    __syncthreads();
-    if (tid == 0) {
-      int nt = 0;
-      for (int q = 0; q < nwarps; ++q) {
-        nt += __popc(s_flags[q]);
-        pix_cta += s_pix[q];
-      }
-      s_base = nt ? atomicAdd(tws, nt) : 0;
-    }
-    __syncthreads();
-    if (flags && lane < 4 && ((flags >> lane) & 1u)) {
-      int pos = s_base + __popc(flags & ((1u << lane) - 1u));
-      for (int q = 0; q < warp; ++q) pos += __popc(s_flags[q]);
-      __stcg(list + pos, (b * TY + ty) * TXp + 4 * wx + lane);
-    }
-  }
-  // ---- grid barrier: tws[2] arrivals, tws[3] generation | tiles --------------------------------------
-  __syncthreads();
-  if (tid == 0) {
-    if (pix_cta) atomicAdd(sf.acc_pix, (unsigned)pix_cta);
-    __threadfence();
-    const unsigned prev = atomicAdd(reinterpret_cast<unsigned*>(tws + 2), 1u);
-    unsigned word;
-    if (prev == gridDim.x - 1u) {                            // everybody has listed and counted
-      volatile int32_t* vt = tws;
-      const int ntl = vt[0];
-      vt[1] = ntl;
-      vt[0] = 0;
-      *sf.count = (int32_t)*reinterpret_cast<volatile unsigned*>(sf.acc_pix);
-      *reinterpret_cast<volatile unsigned*>(sf.acc_pix) = 0u;
-      vt[2] = 0;
-      word = (((g0 + 1u) & 0xfffu) << 20) | (unsigned)ntl;
-      __threadfence();
-      *gen = word;
-    } else {
-      const long long t0 = clock64();
-      while (((word = *gen) >> 20) == g0) {
-        __nanosleep(64);
-        if (clock64() - t0 > 4000000000ll) __trap();         // a CTA of the grid never arrived
-      }
-    }
-    __threadfence();
-    s_ntl = (int)(word & 0xfffffu);
-  }
-  __syncthreads();
-  if (sf.clear) {                                            // every CTA has read its raw windows
-    for (int item = blockIdx.x * nwarps + warp; item < NI; item += gridDim.x * nwarps) {
-      const int wx = item % Wd, r = item / Wd;
-      const int ty = r % TY, b = r / TY;
-      const int y = ty * TL_H + lane;
-      if (lane < TL_H && y < H) sf.clear[((long long)b * H + y) * Wd + wx] = 0u;
-    }
-  }
-  return s_ntl;
-}
-
 __device__ __forceinline__ void tma_load_4d(uint32_t dst, const CUtensorMap* map, int c0, int c1,
                                             int c2, int c3, uint64_t* bar) {
   asm volatile(
@@ -258,8 +126,7 @@ __global__ void __launch_bounds__(128 + um_epi(BN), BN <= 16 ? 4 : BN <= 64 ? 2 
 conv_tile_kernel(const __grid_constant__ CUtensorMap amap_hi, const __grid_constant__ CUtensorMap amap_lo,
                  const __grid_constant__ CUtensorMap wmap, int32_t* tile_ws,
                  const uint32_t* dil_bits, const float* __restrict__ bias,
-                 TO* __restrict__ out, const TileGeom g, const PoolFuse pf, const TileSelf sf) {
-  pdl_prologue();
+                 TO* __restrict__ out, const TileGeom g, const PoolFuse pf) {
 #ifdef CB_TILE_TRACE
   const long long trace_t0 = clock64();
   if (threadIdx.x == 0) {
@@ -283,59 +150,22 @@ conv_tile_kernel(const __grid_constant__ CUtensorMap amap_hi, const __grid_const
   constexpr int ACC_COLS = MERGE ? 2 * BN : BN;                // TMEM columns of one accumulator
   constexpr int TMEM_COLS = tile_tmem_cols(SPLIT3, BN);
   constexpr int EPI = um_epi(BN);
-  // self-listing mode: dilation + tile list + count first, then a grid barrier (tile_self_list)
-  const bool self = sf.raw != nullptr;
-  int ntl_self = 0;
-  TileCtrl* const ctrl0 =
-      reinterpret_cast<TileCtrl*>(smem + g.nhalo * (NSPLIT * g.nblk * g.plane_bytes) + g.nb * B_STAGE);
-  if (self) {
-    // TMEM first: the hardware starts the next CTA of a TMEM-using kernel on an SM only once the running one
-    // has relinquished its allocation permit (CTA k of an SM enters ~0.9 us after CTA k-1, r02_tile_residency.txt)
-    // -- a CTA that waited in the grid barrier BEFORE allocating kept its SM's other CTAs from ever starting
-    if ((threadIdx.x >> 5) == 2) {
-      asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
-                       smem_u32(&ctrl0->tmem_base)),
-                   "r"((uint32_t)TMEM_COLS)
-                   : "memory");
-      asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    ntl_self = tile_self_list(sf, tile_ws, g.B, g.H, g.W, g.Wd, g.TY, g.TXp, (g.kH - 1) / 2, (g.kW - 1) / 2,
-                              reinterpret_cast<int*>(smem));
-  }
-  // dirty tiles (cb_dilate_compact_tiles, or the prologue above: written by other CTAs of this grid,
-  // hence L2 loads); the shuffle makes the value uniform for the compiler
-  const int ntl = __shfl_sync(0xffffffffu, self ? ntl_self : __ldcg(tile_ws + 1), 0);
+  // dirty tiles (cb_dilate_compact_tiles: written by another grid, hence L2 loads); the shuffle makes
+  // the value uniform for the compiler
+  const int ntl = __shfl_sync(0xffffffffu, __ldcg(tile_ws + 1), 0);
   const int ntiles_n = g.CoutPad / BN;
   const long long total = (long long)ntl * ntiles_n;
-  if ((long long)blockIdx.x >= total) {                      // CTA-uniform, before any barrier / alloc ...
-    if (self) {                                              // ... except the self-listing mode's early allocation
-      tc_fence_before();
-      __syncthreads();
-      tc_fence_after();
-      if ((threadIdx.x >> 5) == 2)
-        asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(ctrl0->tmem_base),
-                     "r"((uint32_t)TMEM_COLS)
-                     : "memory");
-    }
-    return;
-  }
+  if ((long long)blockIdx.x >= total) return;                // CTA-uniform, before any barrier / alloc
   if (smem_u32(smem) & 1023u) __trap();
   const int tid = threadIdx.x, lane = tid & 31;
   const int warp = __shfl_sync(0xffffffffu, tid >> 5, 0);    // provably warp-uniform role index
   const int NT = g.B * g.TY * g.TXp;
   const int32_t* tiles = tile_ws + 4 + NT;
-  // EXPERIMENT (CBINFER_TILE_SCRAMBLE=1): walk the tile list in a pseudo-random order (x 7919 mod n), so
-  // that the tiles in flight at any time are spread over the maps instead of being neighbours
-  const bool scramble = (g.relu & 4) && (ntl % 7919) != 0;
-  auto tile_at = [&](long long w) {
-    const int ti = (int)(w / ntiles_n);
-    return __ldcg(tiles + (scramble ? (int)(((long long)ti * 7919ll) % ntl) : ti));
-  };
+  auto tile_at = [&](long long w) { return __ldcg(tiles + (int)(w / ntiles_n)); };
   const int halo_stage = NSPLIT * g.nblk * g.plane_bytes;
   uint8_t* bring = smem + g.nhalo * halo_stage;
   TileCtrl* ctrl = reinterpret_cast<TileCtrl*>(bring + g.nb * B_STAGE);
-  const bool fake = g.relu & 2;                              // TIMING EXPERIMENT ONLY (CBINFER_TILE_FAKE=1)
-  const bool resident = (ntiles_n == 1 && g.num_kb <= g.nb) || fake;
+  const bool resident = ntiles_n == 1 && g.num_kb <= g.nb;
   const int ph = (g.kH - 1) / 2, pw = (g.kW - 1) / 2;
 
   if (tid == 0) {
@@ -353,7 +183,7 @@ conv_tile_kernel(const __grid_constant__ CUtensorMap amap_hi, const __grid_const
     }
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
   }
-  if (warp == 2 && !self) {
+  if (warp == 2) {
     asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(
                      smem_u32(&ctrl->tmem_base)),
                  "r"((uint32_t)TMEM_COLS)
@@ -382,7 +212,7 @@ conv_tile_kernel(const __grid_constant__ CUtensorMap amap_hi, const __grid_const
     for (long long w = blockIdx.x; w < total; w += gridDim.x, ++it) {
       if (resident && it > 0) break;
       const int nt = (int)(w % ntiles_n);
-      for (int kb = 0; kb < (fake && num_kb > nb ? nb : num_kb); ++kb) {
+      for (int kb = 0; kb < num_kb; ++kb) {
         if (!resident) mbar_wait(&ctrl->b_empty[stage], phase ^ 1u);
         if (leader) {
           const uint32_t b_hi = smem_u32(bring + stage * B_STAGE);
@@ -755,8 +585,6 @@ inline TilePlan tile_plan(int es, bool split3, int bn, int Cp, int B, int H, int
   g.plane_bytes = (g.HWX * g.HWY * g.pix_row + 1023) / 1024 * 1024;
   g.layout = g.pix_row == 16 ? 0 : g.pix_row == 32 ? 6 : g.pix_row == 64 ? 4 : 2;
   g.Cout = Cout; g.CoutPad = CoutPad; g.Op = Op; g.relu = relu ? 1 : 0;
-  if (getenv("CBINFER_TILE_FAKE")) g.relu |= 2;
-  if (getenv("CBINFER_TILE_SCRAMBLE")) g.relu |= 4;
   if ((long long)g.HWX * g.pix_row >= (1 << 18)) return p;
   const int b_stage = nsplit * bn * UM_ROW_BYTES;
   const int tmem_cols = tile_tmem_cols(split3, bn);
@@ -824,7 +652,7 @@ inline CUtensorMapDataType tmap_dtype() {
 template <typename T, typename TO, bool SPLIT3, int BN>
 int launch_conv_tile(cudaStream_t s, const void* state, const void* state_lo, const int32_t* tile_ws,
                      const uint32_t* dil_bits, const void* packed, const float* bias, void* out,
-                     const TilePlan& plan, const PoolFuse& pf, const TileSelf& sf) {
+                     const TilePlan& plan, const PoolFuse& pf) {
   const TileGeom& g = plan.g;
   auto enc = tensor_map_encoder();
   if (!enc) return fail(3, "conv_update_tiled: cuTensorMapEncodeTiled unavailable");
@@ -870,35 +698,10 @@ int launch_conv_tile(cudaStream_t s, const void* state, const void* state_lo, co
   // (the plan counts shared memory and TMEM columns; the register side is pinned by the kernel's
   //  __launch_bounds__: 4 CTAs per SM for N <= 16, 2 for N <= 64)
   long long grid = (long long)sm_count() * plan.occ;
-  if (sf.raw) {
-    // the self-listing prologue ends in a grid barrier: every CTA must be resident (cooperative launch),
-    // so the grid follows the occupancy the runtime reports for this kernel, not the plan's estimate
-    static thread_local int occ_dev = -1, occ_smem = -1, occ_act = 0;
-    if (occ_dev != dev || occ_smem != plan.smem_bytes) {
-      occ_act = 0;
-      cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ_act, kern, 128 + um_epi(BN), (size_t)plan.smem_bytes);
-      occ_dev = dev;
-      occ_smem = plan.smem_bytes;
-    }
-    if (occ_act < 1) return fail(3, "conv_update_tiled_self: kernel cannot be resident");
-    // CBINFER_SELF_COOP=0 (experiment; needs a GPU no other grid is running on): plain launch of the plan's
-    // grid -- the CTAs do become co-resident once the TMEM allocation precedes the barrier, but the runtime
-    // will not vouch for it (it counts ONE block per SM for kernels that allocate TMEM)
-    static const bool plan_grid = [] {
-      const char* e = getenv("CBINFER_SELF_COOP");
-      return e && e[0] == '0';
-    }();
-    if (!plan_grid && grid > (long long)sm_count() * occ_act) grid = (long long)sm_count() * occ_act;
-  }
   if (grid > max_items) grid = max_items;
   if (grid < 1) grid = 1;
-  static const bool coop_self = [] {
-    const char* e = getenv("CBINFER_SELF_COOP");             // tuning knob: 0 = plain launch of the same (resident) grid
-    return !(e && e[0] == '0');
-  }();
-  cb::launch_cluster(kern, dim3((unsigned)grid), dim3(128 + um_epi(BN)), (size_t)plan.smem_bytes, s, 1u,
-                     (sf.raw && coop_self) ? 1 : 0, amap[0], amap[1], wmap, const_cast<int32_t*>(tile_ws), dil_bits, bias,
-                     (TO*)out, g, pf, sf);
+  cb::launch(kern, dim3((unsigned)grid), dim3(128 + um_epi(BN)), (size_t)plan.smem_bytes, s, amap[0], amap[1],
+             wmap, const_cast<int32_t*>(tile_ws), dil_bits, bias, (TO*)out, g, pf);
   CB_CHECK_LAUNCH("conv_update_tiled");
   return 0;
 }
@@ -929,7 +732,7 @@ inline int umma_conv_update_tiled(cudaStream_t s, int dtype, int gemm, const voi
                                   const void* state_lo, int Cp, const int32_t* tile_ws,
                                   const uint32_t* dil_bits, const void* packed, const float* bias,
                                   void* out, int Op, int B, int H, int W, int Cout, int kH, int kW,
-                                  int relu, const PoolFuse& pf, const TileSelf& sf) {
+                                  int relu, const PoolFuse& pf) {
   TilePlan plan;
   umma_tile_plan(plan, dtype, gemm, Cp, B, H, W, Cout, Op, kH, kW, relu);
   CB_CHECK_ARG(plan.ok, "conv_update_tiled: layer shape not supported by the tile path");
@@ -942,11 +745,11 @@ inline int umma_conv_update_tiled(cudaStream_t s, int dtype, int gemm, const voi
   CB_CHECK_ARG(!pf.out || tile_pool_ok(gemm, Cout), "conv_update_tiled: fused pooling needs Cout <= 64, a multiple of 16");
 #define CB_TBN(T_, TO_, S3_)                                                                       \
   switch (bn) {                                                                                    \
-    case 16: return launch_conv_tile<T_, TO_, S3_, 16>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf, sf);   \
-    case 32: return launch_conv_tile<T_, TO_, S3_, 32>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf, sf);   \
-    case 64: return launch_conv_tile<T_, TO_, S3_, 64>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf, sf);   \
-    case 128: return launch_conv_tile<T_, TO_, S3_, 128>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf, sf); \
-    case 256: return launch_conv_tile<T_, TO_, S3_, 256>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf, sf); \
+    case 16: return launch_conv_tile<T_, TO_, S3_, 16>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf);   \
+    case 32: return launch_conv_tile<T_, TO_, S3_, 32>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf);   \
+    case 64: return launch_conv_tile<T_, TO_, S3_, 64>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf);   \
+    case 128: return launch_conv_tile<T_, TO_, S3_, 128>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf); \
+    case 256: return launch_conv_tile<T_, TO_, S3_, 256>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf); \
     default: return fail(2, "conv_update_tiled: unsupported N tile %d", bn);                      \
   }
   if (bf16x3) { CB_TBN(__nv_bfloat16, float, true) }

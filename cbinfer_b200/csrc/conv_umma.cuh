@@ -356,7 +356,6 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap wmap, const T* __restrict__
                  const float* __restrict__ bias, TO* __restrict__ out, int Op, int H, int W,
                  int Cout, int CoutPad, int kH, int kW, int Kp, int relu, int sel_lo, int sel_hi,
                  uint32_t* __restrict__ sk_ws, const RowMask mk) {
-  pdl_prologue();
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   using C = UmmaCfg<T, SPLIT3, BN, DEEP>;
   constexpr int UM_EPI = um_epi(BN), UM_THREADS = um_threads(BN);
@@ -855,7 +854,6 @@ template <typename T, typename TP>
 __global__ void pack_weights_umma_kernel(const T* __restrict__ w, TP* __restrict__ packed, int Cout,
                                          int Cin, int kH, int kW, int Cp, int CoutPad, int KpPad,
                                          int split3) {
-  pdl_prologue();
   const long long plane = (long long)CoutPad * KpPad;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < plane;
        i += (long long)gridDim.x * blockDim.x) {
@@ -924,19 +922,19 @@ inline int umma_pack_weights(cudaStream_t s, int dtype, int gemm, const void* we
   switch (dtype) {
     case CB_F32:
       if (gemm == CB_GEMM_TC_BF16X3)
-        cb::launch_pdl(pack_weights_umma_kernel<float, __nv_bfloat16>, (unsigned)blocks, 256, 0, s, 
+        cb::launch(pack_weights_umma_kernel<float, __nv_bfloat16>, (unsigned)blocks, 256, 0, s, 
             (const float*)weight, (__nv_bfloat16*)packed, Cout, Cin, kH, kW, Cp, CoutPad, KpPad, 2);
       else
-        cb::launch_pdl(pack_weights_umma_kernel<float, float>, (unsigned)blocks, 256, 0, s, 
+        cb::launch(pack_weights_umma_kernel<float, float>, (unsigned)blocks, 256, 0, s, 
             (const float*)weight, (float*)packed, Cout, Cin, kH, kW, Cp, CoutPad, KpPad,
             gemm == CB_GEMM_TC_3X ? 1 : 0);
       break;
     case CB_F16:
-      cb::launch_pdl(pack_weights_umma_kernel<__half, __half>, (unsigned)blocks, 256, 0, s, 
+      cb::launch(pack_weights_umma_kernel<__half, __half>, (unsigned)blocks, 256, 0, s, 
           (const __half*)weight, (__half*)packed, Cout, Cin, kH, kW, Cp, CoutPad, KpPad, 0);
       break;
     case CB_BF16:
-      cb::launch_pdl(pack_weights_umma_kernel<__nv_bfloat16, __nv_bfloat16>, (unsigned)blocks, 256, 0, s, 
+      cb::launch(pack_weights_umma_kernel<__nv_bfloat16, __nv_bfloat16>, (unsigned)blocks, 256, 0, s, 
           (const __nv_bfloat16*)weight, (__nv_bfloat16*)packed, Cout, Cin, kH, kW, Cp, CoutPad,
           KpPad, 0);
       break;
@@ -1062,12 +1060,8 @@ int launch_conv_umma(cudaStream_t s, int dtype, const void* state, const void* s
   grid *= ks;
   // stream-K CTAs wait for each other's partial tiles: cooperative launch = all of them resident, also
   // next to another stream-K grid on a concurrent stream (PoseModel.parallelBranches)
-  static const bool coop_sk = [] {
-    const char* e = getenv("CBINFER_SK_COOP");               // tuning knob: 0 = plain launch
-    return !(e && e[0] == '0');
-  }();
   cb::launch_cluster(kern, (unsigned)grid, um_threads(BN), (size_t)smem_bytes, s, (unsigned)ks,
-                     (sk_ws && coop_sk) ? 1 : 0, map, (const T*)state, (const T*)state_lo, Cp,
+                     sk_ws ? 1 : 0, map, (const T*)state, (const T*)state_lo, Cp,
                                                         idx, count, bias,
                                                         (TO*)out, Op, H, W, Cout, CoutPad, kH, kW,
                                                         Kp, relu, sel_lo, sel_hi, sk_ws, mk);
@@ -1098,13 +1092,6 @@ int dispatch_bn(int bn, cudaStream_t s, int dtype, const void* state, const void
   }
 #undef CB_BN
 }
-
-// conv_pair.cuh: the same contraction on CTA pairs (cta_group::2), for wide layers with many changed pixels
-inline bool pair_supported(int es, int Cp, int CoutPad, int kH, int kW);
-template <typename T, typename TO, bool SPLIT3>
-int launch_conv_pair(cudaStream_t s, const void* state, const void* state_lo, int Cp, const int32_t* idx,
-                     const int32_t* count, const void* packed, const float* bias, void* out, int Op, int H, int W,
-                     int Cout, int CoutPad, int kH, int kW, int relu, int sel_lo, int sel_hi);
 
 inline int umma_conv_update(cudaStream_t s, int dtype, int gemm, const void* state,
                             const void* state_lo, int Cp, const int32_t* idx, const int32_t* count, const void* packed,
@@ -1191,29 +1178,6 @@ inline int umma_conv_update(cudaStream_t s, int dtype, int gemm, const void* sta
     const int rc = run_t(std::true_type{}, bn_small, 0, m_switch, ksplit);
     if (rc) return rc;
     return run_t(std::false_type{}, bn, m_switch, 0x7fffffff);
-  }
-  // Opt-in (CBINFER_PAIR_MIN=n, read per call): wide layers (N tile 256, 16-bit operands) run on CTA pairs
-  // (conv_pair.cuh: tcgen05.mma.cta_group::2, M = 256 per instruction, each CTA loads half of the weight tile)
-  // from n M tiles on; the index-list kernel keeps the smaller counts; both are launched, the count decides on
-  // the device.  Bit-identical results.  OFF by default: measured on the 64 -> 256 7x7 layer it buys 1-5 % from
-  // 20 % change on and loses 10-25 % below (no stream-K, an extra launch) -- profiles/r02_experiments.md.
-  const char* pm_env = getenv("CBINFER_PAIR_MIN");
-  const int pair_min = pm_env ? atoi(pm_env) : 0;
-  const int es_op = umma_operand_es(dtype, gemm);
-  const long long max_mtiles = (P + UM_BM - 1) / UM_BM;
-  if (pair_min > 0 && bn == 256 && !mk.bits && !(relu & 2) && (bf16x3 || dtype == CB_F16 || dtype == CB_BF16) &&
-      pair_supported(es_op, Cp, CoutPad, kH, kW) && max_mtiles >= pair_min && sms >= 2) {
-    const int rc = run_t(std::false_type{}, bn, 0, pair_min);
-    if (rc) return rc;
-    if (bf16x3)
-      return launch_conv_pair<__nv_bfloat16, float, true>(s, state, state_lo, Cp, idx, count, packed, bias, out, Op, H,
-                                                          W, Cout, CoutPad, kH, kW, relu, pair_min, 0x7fffffff);
-    if (dtype == CB_F16)
-      return launch_conv_pair<__half, __half, false>(s, state, state_lo, Cp, idx, count, packed, bias, out, Op, H, W,
-                                                     Cout, CoutPad, kH, kW, relu, pair_min, 0x7fffffff);
-    return launch_conv_pair<__nv_bfloat16, __nv_bfloat16, false>(s, state, state_lo, Cp, idx, count, packed, bias, out,
-                                                                 Op, H, W, Cout, CoutPad, kH, kW, relu, pair_min,
-                                                                 0x7fffffff);
   }
   return run_t(std::false_type{}, bn, 0, 0x7fffffff);
 }

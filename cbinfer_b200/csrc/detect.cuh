@@ -109,7 +109,6 @@ detect_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int x
                   T* __restrict__ st, long long s_sb, long long s_sy, int sp, AuxPlanes aux,
                   uint32_t* __restrict__ bits, int B, int H, int W, int C, int Wd, T thr,
                   unsigned cpv_magic, int wlog) {
-  pdl_prologue();
   __shared__ unsigned s_word[kDetWarps];
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int wpw = 1 << wlog;
@@ -212,7 +211,6 @@ detect_narrow_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, lo
                      long long x_sx, T* __restrict__ st, long long s_sb, long long s_sy,
                      AuxPlanes aux, uint32_t* __restrict__ bits, int B, int H, int W, int C,
                      int Wd, T thr) {
-  pdl_prologue();
   const int lane = threadIdx.x & 31;
   // 32-bit index math (the host checks words < 2^31): two 64-bit divisions per warp were most of this
   // kernel's instructions (ncu: 173 warp instructions per 32 pixels, SM 54 % busy on an HBM-bound scan)
@@ -323,7 +321,6 @@ detect_planar_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, lo
                      T* __restrict__ st, long long s_sb, long long s_sy, int sp, AuxPlanes aux,
                      uint32_t* __restrict__ bits, int B, int H, int W, int C, int Wd, T thr,
                      unsigned cpv_magic, int cps, int nw) {
-  pdl_prologue();
   extern __shared__ __align__(16) unsigned char dp_smem[];
   uint4* xs = reinterpret_cast<uint4*>(dp_smem);                 // [nw*32][cps]
   __shared__ unsigned s_word[kPlanarMaxWords];
@@ -389,7 +386,6 @@ detect_generic_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, l
                       long long x_sx, T* __restrict__ st, long long s_sb, long long s_sc,
                       long long s_sy, long long s_sx, AuxPlanes aux,
                       uint32_t* __restrict__ bits, int B, int H, int W, int C, int Wd, T thr) {
-  pdl_prologue();
   const int lane = threadIdx.x & 31;
   // 32-bit index math (the host checks words < 2^31): two 64-bit divisions per warp were most of this
   // kernel's instructions (ncu: 173 warp instructions per 32 pixels, SM 54 % busy on an HBM-bound scan)
@@ -430,7 +426,6 @@ detect_u8_kernel(const uint8_t* __restrict__ x, long long x_sb, long long x_sc, 
                  long long x_sx, float* __restrict__ st, long long s_sb, long long s_sy,
                  AuxPlanes aux, uint32_t* __restrict__ bits, int B, int H, int W, int C, int Wd,
                  float divisor, float bias, float thr) {
-  pdl_prologue();
   // the 256 possible normalised values, computed once per block with the IEEE division and addition the
   // host would use (bit-identical by construction): a table lookup per channel instead of a division
   __shared__ float lut[256];
@@ -533,27 +528,27 @@ int launch_detect(cudaStream_t stream, const void* x, long long x_sb, long long 
 #define CB_DET(U_)                                                                             \
   if (vec_ok) {                                                                                \
     if (cpv >= 4)                                                                              \
-      cb::launch_pdl(detect_vec_kernel<T, VEC, U_, 4>, grid, block, 0, stream,                             \
+      cb::launch(detect_vec_kernel<T, VEC, U_, 4>, grid, block, 0, stream,                                 \
           (const T*)x, x_sb, x_sy, (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, bits,  \
           B, H, W, C, Wd, thr, magic, wlog);                                                   \
     else                                                                                       \
-      cb::launch_pdl(detect_vec_kernel<T, VEC, U_, 2>, grid, block, 0, stream,                             \
+      cb::launch(detect_vec_kernel<T, VEC, U_, 2>, grid, block, 0, stream,                                 \
           (const T*)x, x_sb, x_sy, (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, bits,  \
           B, H, W, C, Wd, thr, magic, wlog);                                                   \
   } else if (narrow_ok) {                                                                      \
-    cb::launch_pdl(detect_narrow_kernel<T, VEC, U_>, grid, block, 0, stream,                               \
+    cb::launch(detect_narrow_kernel<T, VEC, U_>, grid, block, 0, stream,                                   \
         (const T*)x, x_sb, x_sc, x_sy, x_sx, (T*)state, s_sb, s_sy, aux, bits, B, H, W, C,  \
         Wd, thr);                                                                              \
   } else if (planar_ok) {                                                                      \
     if (planar_smem > 48 * 1024)                                                               \
       cudaFuncSetAttribute(detect_planar_kernel<T, VEC, U_>,                                   \
                            cudaFuncAttributeMaxDynamicSharedMemorySize, (int)planar_smem);     \
-    cb::launch_pdl(detect_planar_kernel<T, VEC, U_>, dim3((unsigned)((words + planar_nw - 1) / planar_nw)), \
+    cb::launch(detect_planar_kernel<T, VEC, U_>, dim3((unsigned)((words + planar_nw - 1) / planar_nw)),     \
         block, planar_smem, stream,                                                            \
         (const T*)x, x_sb, x_sc, x_sy, (T*)state, s_sb, s_sy, (int)s_sx, aux, bits, B, H, W, C, \
         Wd, thr, magic, cps, planar_nw);                                                       \
   } else {                                                                                     \
-    cb::launch_pdl(detect_generic_kernel<T, U_>, grid, block, 0, stream,                                   \
+    cb::launch(detect_generic_kernel<T, U_>, grid, block, 0, stream,                                       \
         (const T*)x, x_sb, x_sc, x_sy, x_sx, (T*)state, s_sb, s_sc, s_sy, s_sx, aux, bits,  \
         B, H, W, C, Wd, thr);                                                                  \
   }
@@ -586,7 +581,7 @@ inline int launch_detect_u8(cudaStream_t stream, const void* x, long long x_sb, 
   const long long blocks = (words + 7) / 8;
   CB_CHECK_ARG(blocks < (1ll << 31), "change_detect_u8: image too large");
 #define CB_DET8(U_)                                                                              \
-  cb::launch_pdl(detect_u8_kernel<U_>, dim3((unsigned)blocks), dim3(256), 0, stream,            \
+  cb::launch(detect_u8_kernel<U_>, dim3((unsigned)blocks), dim3(256), 0, stream,                \
                  (const uint8_t*)x, x_sb, x_sc, x_sy, x_sx, (float*)state, s_sb, s_sy, aux, bits, \
                  B, H, W, C, Wd, divisor, bias, threshold);
   switch (update) {
@@ -626,7 +621,6 @@ detect_sparse_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy
                          AuxPlanes aux, const int32_t* __restrict__ cand,
                          const int32_t* __restrict__ ncand, uint32_t* __restrict__ bits, int H,
                          int W, int C, int Wd, T thr, int glog, FusedCompact fc) {
-  pdl_prologue();
   const int n = *ncand;
   const int lane = threadIdx.x & 31;
   const int G = 1 << glog, ppw = 32 >> glog;
@@ -697,7 +691,6 @@ detect_sparse_generic_kernel(const T* __restrict__ x, long long x_sb, long long 
                              long long s_sc, long long s_sy, long long s_sx, AuxPlanes aux,
                              const int32_t* __restrict__ cand, const int32_t* __restrict__ ncand,
                              uint32_t* __restrict__ bits, int H, int W, int C, int Wd, T thr) {
-  pdl_prologue();
   const int n = *ncand;
   const int P = H * W;
   for (long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x; j < n;
@@ -759,15 +752,15 @@ int launch_detect_sparse(cudaStream_t stream, const void* x, long long x_sb, lon
   FusedCompact fc = fuse ? *fuse : FusedCompact{nullptr, nullptr, nullptr, nullptr, 0, 0, 0, 0};
 #define CB_DETS(U_)                                                                              \
   if (vec_ok && fuse)                                                                            \
-    cb::launch_pdl(detect_sparse_vec_kernel<T, VEC, U_, true>, grid, 256, 0, stream,                         \
+    cb::launch(detect_sparse_vec_kernel<T, VEC, U_, true>, grid, 256, 0, stream,                             \
         (const T*)x, x_sb, x_sy, (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand,      \
         ncand, bits, H, W, C, Wd, thr, glog, fc);                                                \
   else if (vec_ok)                                                                               \
-    cb::launch_pdl(detect_sparse_vec_kernel<T, VEC, U_, false>, grid, 256, 0, stream,                        \
+    cb::launch(detect_sparse_vec_kernel<T, VEC, U_, false>, grid, 256, 0, stream,                            \
         (const T*)x, x_sb, x_sy, (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand,      \
         ncand, bits, H, W, C, Wd, thr, glog, fc);                                                \
   else                                                                                           \
-    cb::launch_pdl(detect_sparse_generic_kernel<T, U_>, grid, 256, 0, stream,                                \
+    cb::launch(detect_sparse_generic_kernel<T, U_>, grid, 256, 0, stream,                                    \
         (const T*)x, x_sb, x_sc, x_sy, x_sx, (T*)state, s_sb, s_sc, s_sy, s_sx, aux, cand,    \
         ncand, bits, H, W, C, Wd, thr);
   switch (update) {
@@ -802,7 +795,6 @@ detect_compact_sparse_kernel(const T* __restrict__ x, long long x_sb, long long 
                              int32_t* __restrict__ count, uint32_t* __restrict__ bits,
                              unsigned* __restrict__ ws, int H, int W, int C, int Wd, T thr,
                              int glog) {
-  pdl_prologue();
   const int n = *ncand;
   uint8_t* flags = reinterpret_cast<uint8_t*>(ws + 4);
   const int lane = threadIdx.x & 31;
@@ -933,7 +925,7 @@ int launch_detect_compact_sparse(cudaStream_t stream, const void* x, long long x
   const int Wd = (W + 31) / 32;
   const T thr = thr_cast<T>(threshold);
 #define CB_DCS(U_)                                                                                 \
-  cb::launch_pdl(detect_compact_sparse_kernel<T, VEC, U_>, grid, 256, 0, stream, (const T*)x,     \
+  cb::launch(detect_compact_sparse_kernel<T, VEC, U_>, grid, 256, 0, stream, (const T*)x,         \
                  x_sb, x_sy, (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand, ncand, idx,   \
                  count, bits, (unsigned*)ws, H, W, C, Wd, thr, glog);
   switch (update) {

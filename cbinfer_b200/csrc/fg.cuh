@@ -16,7 +16,6 @@ __global__ void __launch_bounds__(256)
 fg_update_kernel(const float* __restrict__ x, float* __restrict__ prev,
                  const float* __restrict__ w, float* __restrict__ out, int32_t* __restrict__ count,
                  int B, int Cin, int Cout, int H, int W, int kH, int kW, float thr) {
-  pdl_prologue();
   const int lane = threadIdx.x & 31;
   const long long total = (long long)B * Cin * H * W;
   const long long nwarps = (long long)gridDim.x * (blockDim.x >> 5);
@@ -80,7 +79,6 @@ fg_detect_kernel(const float* __restrict__ x, long long x_sb, long long x_sc, lo
                  __nv_bfloat16* __restrict__ dhi, __nv_bfloat16* __restrict__ dlo, int pitch16,
                  uint32_t* __restrict__ bits, int32_t* __restrict__ count, int B, int H, int W, int C,
                  int Wd, float thr, unsigned cpv_magic, int cps, int nw) {
-  pdl_prologue();
   extern __shared__ __align__(16) unsigned char fg_smem[];
   uint4* xs = reinterpret_cast<uint4*>(fg_smem);                 // [nw*32][cps]
   __shared__ unsigned s_word[kPlanarMaxWords];
@@ -163,7 +161,7 @@ inline int launch_fg_detect(cudaStream_t s, const float* x, long long x_sb, long
   const unsigned magic = cpv > 1 ? (unsigned)((0x100000000ull + cpv - 1) / cpv) : 0u;
   auto kern = xpm ? fg_detect_kernel<1> : fg_detect_kernel<0>;
   if (smem > 48 * 1024) cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  launch_pdl(kern, dim3((unsigned)((words + nw - 1) / nw)), dim3(256), smem, s, x, x_sb, x_sc, x_sy, x_sx, prev,
+  launch(kern, dim3((unsigned)((words + nw - 1) / nw)), dim3(256), smem, s, x, x_sb, x_sc, x_sy, x_sx, prev,
              p_sb, p_sy, pp, (__nv_bfloat16*)dhi, (__nv_bfloat16*)dlo, pitch16_of(C), bits, count, B, H, W, C,
              Wd, thr, magic, cps, nw);
   CB_CHECK_LAUNCH("fg_detect");

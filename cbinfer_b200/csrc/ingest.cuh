@@ -102,7 +102,6 @@ __global__ void __launch_bounds__(256)
 resize_pass_u8_kernel(const uint8_t* __restrict__ src, long long s_y, long long s_x, long long s_c,
                       uint8_t* __restrict__ dst, long long d_y, long long d_x, long long d_c, int oH, int oW,
                       int C, const int32_t* __restrict__ bounds, const int32_t* __restrict__ kk, int ksize) {
-  pdl_prologue();
   const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
   if (x >= oW || y >= oH) return;
   const int o = AXIS == 1 ? x : y;
@@ -129,7 +128,6 @@ __global__ void __launch_bounds__(256)
 resize_bilinear_kernel(const uint8_t* __restrict__ src, long long s_y, long long s_x, long long s_c, int sH,
                        int sW, float* __restrict__ dst, long long d_y, long long d_x, long long d_c, int oH,
                        int oW, int C, double divisor, double cval, double clip_lo, double clip_hi) {
-  pdl_prologue();
   const int x = blockIdx.x * blockDim.x + threadIdx.x, y = blockIdx.y;
   if (x >= oW || y >= oH) return;
   const double r = ((double)sH / oH) * (y + 0.5) - 0.5, c = ((double)sW / oW) * (x + 0.5) - 0.5;

@@ -36,7 +36,6 @@ maxpool2x2_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, long 
                   const int32_t* __restrict__ count, const uint32_t* __restrict__ bits,
                   T* __restrict__ out, long long o_sb, long long o_sc, long long o_sy,
                   long long o_sx, int C, int H, int W, int oH, int oW) {
-  pdl_prologue();
   const int n = *count;
   const int lane = threadIdx.x & 31;
   const int P = H * W, Wd = (W + 31) >> 5;
@@ -84,7 +83,6 @@ maxpool2x2_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, i
                       const int32_t* __restrict__ idx, const int32_t* __restrict__ count,
                       const uint32_t* __restrict__ bits, T* __restrict__ out, long long o_sb,
                       long long o_sy, int op, int cpp, int glog, int H, int W, int oH, int oW) {
-  pdl_prologue();
   const int n = *count;
   const int lane = threadIdx.x & 31;
   const int G = 1 << glog, ppw = 32 >> glog;                // lanes per pixel, pixels per warp
@@ -155,7 +153,6 @@ maxpool2x2_detect_kernel(const T* __restrict__ x, long long x_sb, long long x_sy
                          long long o_sy, int op, int cpp, int glog, int H, int W, int oH, int oW,
                          T* __restrict__ nst, long long n_sb, long long n_sy, int np, AuxPlanes aux,
                          uint32_t* __restrict__ nbits, T thr) {
-  pdl_prologue();
   const int n = *count;
   const int lane = threadIdx.x & 31;
   const int G = 1 << glog, ppw = 32 >> glog;

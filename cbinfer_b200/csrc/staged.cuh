@@ -12,7 +12,6 @@ template <typename T>
 __global__ void gen_xmatrix_kernel(T* __restrict__ cols, const T* __restrict__ in,
                                    const int32_t* __restrict__ idx, int kW, int kH, int C, int W,
                                    int H, int n) {
-  pdl_prologue();
   const long long K = (long long)C * kH * kW;
   const long long total = K * n;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
@@ -38,7 +37,6 @@ template <typename T>
 __global__ void __launch_bounds__(256)
 matrix_mult_kernel(const T* __restrict__ X, const T* __restrict__ Wt, const T* __restrict__ bias,
                    T* __restrict__ Y, int n, int K, int Cout) {
-  pdl_prologue();
   __shared__ float Xs[32][33], Ws[32][33];
   const int tx = threadIdx.x & 15, ty = threadIdx.x >> 4;
   const int m0 = blockIdx.y * 32, n0 = blockIdx.x * 32;
@@ -74,7 +72,6 @@ template <typename T>
 __global__ void update_output_kernel(const T* __restrict__ Yt, T* __restrict__ out,
                                      const int32_t* __restrict__ idx, int HW, int n, int Cout,
                                      int relu) {
-  pdl_prologue();
   const long long total = (long long)n * Cout;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
        i += (long long)gridDim.x * blockDim.x) {

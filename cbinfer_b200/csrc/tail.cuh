@@ -62,7 +62,6 @@ template <int N1>
 __global__ void __launch_bounds__(TAIL_THREADS)
 tail_kernel(const __grid_constant__ CUtensorMap w1map, const __grid_constant__ CUtensorMap w2map,
             const TailArgs a) {
-  pdl_prologue();
   extern __shared__ __align__(1024) uint8_t smem[];
   constexpr int A_KB = TAIL_ROWS * UM_ROW_BYTES;             // one K block of an A plane: 16 KB
   const int tid = threadIdx.x, lane = tid & 31;
@@ -395,7 +394,7 @@ inline int tail_update(cudaStream_t s, const TailArgs& a, const void* packed1, c
         return fail(3, "tail_update: cannot reserve shared memory");                                \
       adev = dev;                                                                                    \
     }                                                                                                \
-    cb::launch_pdl(tail_kernel<N_>, dim3(grid), dim3(TAIL_THREADS), smem, s, m1, m2, a);             \
+    cb::launch(tail_kernel<N_>, dim3(grid), dim3(TAIL_THREADS), smem, s, m1, m2, a);                 \
   }
   switch (N1) {
     case 16: CB_TAIL(16) break;

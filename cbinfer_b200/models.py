@@ -72,22 +72,6 @@ def enableCandidateDetection(m, fusePool=True, maskedConv=True):
             if type(b) is CBConv2d and type(c) is CBConv2d and b.maskedConv and c.maskedConv \
                     and not c.propChangeIndexes:
                 b._fusedTail = [c]
-        # L2 prefetch hints: a layer's dilation knows which pixels the next CB layer(s) will threshold one
-        # contraction later and asks L2 for their state rows (CBConv2d._hints, cb_dilate_compact_hinted)
-        for i, a in enumerate(kids):
-            if type(a) is not CBConv2d or a.finegrained:
-                continue
-            j, sh = i + 1, 0
-            if j < len(kids) and type(kids[j]) is CBPoolMax2d:
-                j, sh = j + 1, 1
-            tg = []
-            while j < len(kids) and type(kids[j]) is CBConv2d and kids[j].candidateDetect \
-                    and not kids[j].finegrained and len(tg) < 2:
-                tg.append((kids[j], sh))
-                if tuple(kids[j].kernel_size) != (1, 1):
-                    break                      # beyond a k x k layer the change set is a different one
-                j += 1
-            a._prefetchNext = tg
     return m
 
 

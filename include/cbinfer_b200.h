@@ -134,21 +134,6 @@ int cb_dilate_compact_tiles(void* stream, const uint32_t* raw_bits, uint32_t* di
 int cb_dilate_tiles(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits, int32_t* count, void* ws,
                     void* tile_ws, int B, int H, int W, int kHHalf, int kWHalf, int clear_raw);
 
-/* cb_dilate_compact / _tiles / cb_dilate_tiles (tile_ws may be NULL; no_list != 0 = cb_dilate_tiles, idx
- * may then be NULL) that additionally asks L2 for rows the kernels a few launches later will read at the
- * changed pixels -- typically the next layer's previous-input state, cold since the last time those
- * pixels changed: for every dilated pixel (b, y, x) and hint i the bytes
- *   hint_base[i] + (((b * hint_h[i] + (y >> s)) * hint_w[i] + (x >> s)) * hint_row_bytes[i],  s = hint_shift[i]
- * (hint_row_bytes of them; s = 1: a map at the 2x2-pooled resolution) are prefetched with
- * cp.async.bulk.prefetch.L2, one instruction per run of pixels.  Pure hints: every output is
- * bit-identical to the unhinted call.  hint_base and hint_row_bytes must be multiples of 16; at most
- * 3 hints.  No reference counterpart (the reference re-scans whole maps, conv2d.py:222-232). */
-int cb_dilate_compact_hinted(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits, int8_t* dil_map,
-                             int32_t* idx, int32_t* count, void* ws, void* tile_ws, int B, int H, int W,
-                             int kHHalf, int kWHalf, int clear_raw, int no_list, int n_hints,
-                             const void* const* hint_base, const int* hint_row_bytes, const int* hint_shift,
-                             const int* hint_h, const int* hint_w);
-
 /* ---- candidate ("sparse") detection ---------------------------------------------------------
  * Same per-pixel test and state maintenance as cb_change_detect, evaluated only at the
  * `*n_candidates` pixels listed in `candidates` (indices b*H*W + y*W + x, any order); raw_bits is
@@ -265,26 +250,6 @@ int cb_conv_update_tiled_pool(void* stream, int dtype, int gemm, const void* sta
                               void* next_state, long long n_sb, long long n_sy, int n_pitch, int aux_mode,
                               void* aux_hi, void* aux_lo, uint32_t* next_raw_bits, float threshold,
                               int update_mode);
-
-/* cb_dilate_tiles + cb_conv_update_tiled[_pool] in ONE launch: the contraction kernel first derives the
- * dilated bitmap (dil_bits, output), the dirty-tile list (tile_ws) and *count from the RAW change bitmap
- * itself -- the scatter-dilate of changeDetection_kernel, cbconv2d_cg_backend.cu:62-72, one warp per 16-row
- * tile-row word -- then crosses a grid barrier (cooperative launch) and walks the tiles; raw_bits is zeroed
- * afterwards when clear_raw != 0.  ws = the layer's cb_compact_ws_bytes() workspace (its header carries the
- * pixel accumulator), tile_ws = cb_tile_ws_bytes(); both are left as cb_dilate_tiles leaves them, so the two
- * paths can alternate on the same buffers.  pool_out == NULL: no pooling fusion (the pooling arguments are
- * then ignored).  Bit-identical to the two-launch sequence.  Needs (kH - 1) / 2 <= 8 and fewer than 2^20
- * tiles (cb_conv_tiled_self_supported). */
-int cb_conv_tiled_self_supported(int B, int H, int W, int kH, int kW);
-int cb_conv_update_tiled_self(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
-                              int pitch_in, void* tile_ws, uint32_t* dil_bits,
-                              const void* packed_w, const float* bias, void* out, int pitch_out, int B,
-                              int H, int W, int Cin, int Cout, int kH, int kW, int relu,
-                              void* pool_out, long long o_sb, long long o_sy, int o_pitch, int oH, int oW,
-                              void* next_state, long long n_sb, long long n_sy, int n_pitch, int aux_mode,
-                              void* aux_hi, void* aux_lo, uint32_t* next_raw_bits, float threshold,
-                              int update_mode, const uint32_t* raw_bits, int32_t* count, void* ws,
-                              int clear_raw);
 
 /* cb_conv_update over a SUPERSET index list: a listed pixel is processed only if its bit is set in
  * `mask_bits` (a raw change bitmap, e.g. what cb_change_detect_sparse just wrote for a 1x1 layer

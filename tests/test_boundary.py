@@ -186,11 +186,9 @@ def test_compat_shim_exports_the_reference_symbols():
             assert getattr(lib, sname) is not None
 
 
-def test_ingest_and_hint_helpers_on_the_host():
-    """host-side pieces of this session's additions (no GPU compute): workspace sizing of the resizer, the
-    self-listing support query, the hint table's filtering and the wiring of the prefetch targets."""
-    import cbinfer_b200 as cb
-    from cbinfer_b200 import _lib, conv2d_cg as cg, models
+def test_resize_workspace_sizing_on_the_host():
+    """host-side sizing of the resizer's workspace (no GPU compute)."""
+    from cbinfer_b200 import _lib
     C = _lib.C
     # resize workspace: tables for both axes + the horizontally resized 8-bit intermediate
     ws = C.cb_resize_ws_bytes(720, 1280, 368, 654, 3)
@@ -198,21 +196,3 @@ def test_ingest_and_hint_helpers_on_the_host():
     kx = math.ceil(2.0 * 1280 / 654) * 2 + 1                                   # Pillow: ceil(support * scale) * 2 + 1
     assert ws >= 32 + 8 * 654 + 4 * 654 * kx + 8 * 368 + 720 * 654 * 3 and ws % 16 == 0
     assert C.cb_resize_ws_bytes(0, 10, 10, 10, 3) == 0
-    # self-listing: one warp lane per row of a 16-row tile's window (kHHalf <= 8), fewer than 2^20 tiles
-    assert C.cb_conv_tiled_self_supported(8, 480, 640, 7, 7) == 1
-    assert C.cb_conv_tiled_self_supported(8, 480, 640, 19, 7) == 0
-    assert C.cb_conv_tiled_self_supported(8, 480, 640, 4, 7) == 0
-    assert C.cb_conv_tiled_self_supported(512, 2160, 3840, 7, 7) == 0
-    # hint table: contiguous, 16-byte aligned pixel-major maps only, at most three
-    ok = torch.zeros(2, 6, 8, 4)
-    h = cg.PrefetchHints([(ok, 0), (ok[..., :3], 0), (torch.zeros(2, 6, 8, 3), 1), (None, 0), (ok, 1), (ok, 0), (ok, 1)])
-    assert h.n == 3 and [s for _, s in h.targets] == [0, 1, 0]
-    assert list(h.row_bytes)[:3] == [16, 16, 16] and list(h.h)[:3] == [6, 6, 6] and list(h.w)[:3] == [8, 8, 8]
-    assert cg.PrefetchHints([]).n == 0
-    # wiring: a layer's dilation hints the state of the CB layers that will threshold its pixels next
-    base = models.sceneLabelingBaseline()
-    m = models.sceneLabelingCBinfer(base, candidateDetect=True)
-    convs = [c for c in m.modules() if type(c) is cb.CBConv2d]
-    nxt = [[(convs.index(t), sh) for t, sh in c._prefetchNext] for c in convs]
-    assert nxt == [[(1, 1)], [(2, 1)], [(3, 0), (4, 0)], [(4, 0)], []]
-    assert all(c._hints(1, 8, 8, torch.device("cpu")) is None for c in convs)           # opt-in knob is off

@@ -158,52 +158,6 @@ def test_detect_dilate_compact(cbm, orc, dt, layout, case):
         assert int(s["count"].item()) == n
 
 
-@pytest.mark.parametrize("case", [(1, 15, 20, 3, 3), (2, 33, 65, 7, 7), (3, 40, 300, 5, 3), (8, 120, 160, 7, 7)])
-def test_hinted_dilation_is_bit_identical(cbm, case):
-    """cb_dilate_compact_hinted (L2 prefetch hints for the next layers' state rows, same resolution and
-    2x2-pooled, odd sizes, rows of 16 B .. 1 KB) returns exactly what the unhinted calls return -- bitmap,
-    ascending list, count, tile list -- in list mode and in tiles-only mode, and leaves the hinted maps
-    untouched."""
-    cg = cbm["cg"]
-    B, H, W, kH, kW = case
-    g = torch.Generator().manual_seed(sum(case))
-    raw_map = (torch.rand(B, H, W, generator=g) < 0.02).to(torch.int8).cuda()
-    raw_map[:, H // 3:H // 3 + 5, W // 4:W // 4 + 9] = 1
-    tg_same = torch.randn(B, H, W, 256, device="cuda")
-    tg_pool = torch.randn(B, (H + 1) // 2, (W + 1) // 2, 4, device="cuda")
-    tg_half = torch.randn(B, H // 2, W // 2, 64, device="cuda").to(torch.bfloat16)
-    keep = [t.clone() for t in (tg_same, tg_pool, tg_half)]
-    hints = cg.PrefetchHints([(tg_same, 0), (tg_pool, 1), (tg_half, 1)])
-    assert hints.n == 3
-    outs = []
-    for h in (None, hints):
-        s = cg.alloc_scratch((B, H, W), "cuda")
-        tws = cg.alloc_tile_ws((B, H, W), "cuda")
-        s["raw_bits"].copy_(cg._map_to_bits(raw_map)[0])
-        cg.dilate_compact(s["raw_bits"], (B, H, W), (kH, kW), s["idx"], s["count"], s["ws"],
-                          dil_bits=s["dil_bits"], tile_ws=tws, hints=h)
-        n = int(s["count"].item())
-        ntl = int(tws[1].item())
-        NT = (tws.numel() - 4) // 2
-        rec = [n, s["idx"][:n].clone(), s["dil_bits"].clone(), ntl, tws[4 + NT:4 + NT + ntl].sort().values.clone()]
-        s2 = cg.alloc_scratch((B, H, W), "cuda")
-        tws2 = cg.alloc_tile_ws((B, H, W), "cuda")
-        s2["raw_bits"].copy_(s["raw_bits"])
-        cg.dilate_tiles(s2["raw_bits"], (B, H, W), (kH, kW), s2["count"], s2["ws"], s2["dil_bits"], tws2,
-                        clear_raw=True, hints=h)
-        ntl2 = int(tws2[1].item())
-        rec += [int(s2["count"].item()), s2["dil_bits"].clone(), ntl2,
-                tws2[4 + NT:4 + NT + ntl2].sort().values.clone(), s2["raw_bits"].clone()]
-        outs.append(rec)
-    torch.cuda.synchronize()
-    assert outs[0][0] > 0 and outs[0][0] == outs[0][5] and outs[0][3] == outs[0][7]
-    for a, b in zip(*outs):
-        assert (a == b) if isinstance(a, int) else torch.equal(a, b)
-    assert int(outs[1][9].abs().sum().item()) == 0                            # clear_raw honoured
-    for t, k in zip((tg_same, tg_pool, tg_half), keep):
-        assert torch.equal(t, k)
-
-
 def test_detect_update_all_and_special_values(cbm, orc):
     cg, lib = cbm["cg"], cbm["lib"]
     x = torch.zeros(1, 1, 2, 4, device="cuda")
@@ -479,51 +433,6 @@ def test_conv_update_masked_superset_list(cbm, mode, dt):
             torch.cuda.synchronize()
             outs.append(out.clone())
         assert torch.equal(outs[0], outs[1])
-
-
-@pytest.mark.parametrize("case", [("bf16x3", "f32", 2, 64, 256, 80, 96, 3, 0.9, True), ("bf16x3", "f32", 1, 64, 256, 120, 160, 7, 0.55, True),
-                                  ("tc", "bf16", 2, 64, 256, 72, 80, 3, 1.0, False), ("tc", "f16", 1, 128, 512, 90, 100, 3, 0.8, True),
-                                  ("bf16x3", "f32", 1, 32, 200, 96, 96, 5, 0.75, False)])
-def test_conv_update_cta_pair_kernel_equals_index_list_kernel(cbm, case, monkeypatch):
-    """wide layers with many changed pixels run on CTA pairs (tcgen05.mma.cta_group::2, conv_pair.cuh): the
-    same products in the same K order as the index-list kernel, so the two must agree BIT FOR BIT
-    (CBINFER_PAIR_MIN=0 keeps the index-list kernel; odd tile counts, ragged Cout, two N tiles included);
-    both within the contraction tolerance of the dense convolution."""
-    cg, cb, lib = cbm["cg"], cbm["cb"], cbm["lib"]
-    mode, dt, B, Cin, Cout, H, W, k, frac, relu = case
-    tdt, gemm = TORCH_DT[dt], cb.CBConv2d.GEMM_MODES[mode]
-    g = torch.Generator().manual_seed(Cin + H)
-    state, sbuf = cg.pixel_major((B, Cin, H, W), tdt, "cuda", 0)
-    state.copy_((torch.rand(B, Cin, H, W, generator=g) - 0.5).to(tdt))
-    w = ((torch.rand(Cout, Cin, k, k, generator=g) - 0.5) * 2 * (Cin * k * k) ** -0.5).to(tdt).cuda()
-    bias = (torch.rand(Cout, generator=g) - 0.5).cuda()
-    idx = torch.nonzero(torch.rand(B * H * W, generator=g) < frac).view(-1).int().cuda()
-    n = idx.numel()
-    assert n > 1000
-    ci = cg.ChangeIndexes.from_tensor(idx, (B, H, W))
-    packed = cg.pack_weights(w, gemm)
-    planes = cg.bf16_planes(sbuf, Cin) if gemm == lib.GEMM_TC_BF16X3 else None
-    outs = []
-    for pair_min in ("0", "1"):          # (no stream-K workspace: whole K ranges per CTA on both sides)
-        monkeypatch.setenv("CBINFER_PAIR_MIN", pair_min)
-        out, obuf = cg.pixel_major((B, Cout, H, W), tdt, "cuda", 0)
-        out.fill_(2.0)
-        for _ in range(2):
-            cg.conv_update(sbuf, ci, packed, bias, obuf, Cin, Cout, (k, k), relu, gemm, planes16=planes)
-        torch.cuda.synchronize()
-        outs.append(out.clone())
-    assert torch.equal(outs[0], outs[1])
-    ref = F.conv2d(state.double(), w.double(), bias.double(), padding=k // 2).float()      # (fp64: no TF32 in the reference)
-    if relu:
-        ref = F.relu(ref)
-    m = torch.zeros(B * H * W, dtype=torch.bool, device="cuda")
-    m[idx.long()] = True
-    tm = m.view(B, 1, H, W).expand(B, Cout, H, W)
-    scale = float(ref.abs().max()) + 1e-30
-    tol = {"f32": 1e-4, "bf16": 1e-2, "f16": 2e-3}[dt]
-    assert float((outs[1].float()[tm] - ref[tm]).abs().max()) / scale <= tol
-    if not bool(tm.all()):
-        assert float((outs[1].float()[~tm] - 2.0).abs().max()) == 0.0
 
 
 def test_conv_update_zero_changes_is_noop(cbm):

@@ -265,27 +265,6 @@ def test_fused_pool_in_tile_epilogue_is_bit_identical(cbm, dt, feedback, monkeyp
                                           ((1, 40, 40), 5, 0.0), ((2, 33, 65), 17, 0.01), ((1, 50, 300), 19, 0.01),
                                           ((8, 240, 320), 7, 0.05), ((1, 7, 9000), 3, 0.05), ((2, 31, 70), 1, 0.2)])
 def test_dilate_tiles_equals_dilate_compact(cbm, shape, k, frac):
-    _dilate_tiles_check(cbm, shape, k, frac)
-
-
-def test_lean_dilate_tiles_kernel_subprocess():
-    """the opt-in one-block-per-tile-row kernel (CBINFER_DILATE_TILES=1, read once per process) gives the
-    same bitmap, count, tile set and cleared raw bitmap: the same checks in a child process"""
-    import os, subprocess, sys
-    repo = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    code = ("import sys; sys.path.insert(0, %r)\n"
-            "from tests import test_gpu_tiles as t\n"
-            "from cbinfer_b200 import conv2d_cg as cg, _lib\n"
-            "for shape, k, frac in (((2, 97, 131), 7, 0.02), ((1, 480, 640), 7, 0.3), ((3, 16, 8), 3, 1.0),\n"
-            "                       ((2, 33, 65), 17, 0.01), ((8, 240, 320), 7, 0.05), ((1, 7, 9000), 3, 0.05)):\n"
-            "    t._dilate_tiles_check(dict(cg=cg, lib=_lib), shape, k, frac)\n"
-            "print('lean ok')\n" % repo)
-    p = subprocess.run([sys.executable, "-c", code], env=dict(os.environ, CBINFER_DILATE_TILES="1"),
-                       capture_output=True, text=True, timeout=600)
-    assert p.returncode == 0 and "lean ok" in p.stdout, p.stdout[-2000:] + p.stderr[-2000:]
-
-
-def _dilate_tiles_check(cbm, shape, k, frac):
     """cb_dilate_tiles (no ordered list) yields the same dilated bitmap, change count and tile set as
     cb_dilate_compact_tiles; the list compacted on demand from the bitmap equals the eager one."""
     cg = cbm["cg"]
@@ -309,8 +288,7 @@ def _dilate_tiles_check(cbm, shape, k, frac):
     lazy = cg.ChangeIndexes(s2["idx"], s2["count"], shape, bits=s2["dil_bits"], ws=s2["ws"], listed=False)
     assert len(lazy) == n
     assert torch.equal(lazy.tensor(), s1["idx"][:n])
-    # clear_raw: same results, and the raw bitmap comes back zeroed (own rows by each block, the rows two
-    # tile rows share by the last block); the workspace is left clean for either kernel
+    # clear_raw: same results, and the raw bitmap comes back zeroed; the workspace is left clean
     rb = raw_bits.clone()
     cg.dilate_tiles(rb, shape, (k, k), s2["count"], s2["ws"], s2["dil_bits"], t2, clear_raw=True)
     assert int(s2["count"]) == n and torch.equal(s1["dil_bits"], s2["dil_bits"]) and int(t2[1]) == int(t1[1])
@@ -371,112 +349,3 @@ def test_fused_tail_is_bit_identical(cbm, feedback, monkeypatch):
         # and against the dense model at the end (thresholded, so only loosely)
         ref = net(frames[-1])
         assert float((runs[0][-1]["out"] - ref).abs().max()) <= 0.2 * float(ref.abs().max()) + 0.05
-
-
-SELF_CASES = [  # mode, dt, B, Cin, Cout, H, W, k, kind, frac
-    ("bf16x3", "f32", 2, 3, 16, 48, 64, 7, "block", 0.10),
-    ("bf16x3", "f32", 8, 16, 64, 120, 160, 7, "block", 0.05),
-    ("bf16x3", "f32", 3, 16, 64, 37, 53, 7, "iid", 0.01),
-    ("tc", "bf16", 2, 64, 64, 46, 46, 3, "block", 0.30),
-    ("tc", "f16", 1, 16, 19, 31, 9, 5, "iid", 0.10),          # W < 32, ragged Cout
-    ("tc", "bf16", 1, 8, 32, 45, 100, 17, "iid", 0.002),      # widest supported window (16 + 2*8 rows)
-    ("bf16x3", "f32", 1, 16, 64, 40, 40, 7, "iid", 0.00),     # nothing changed
-    ("bf16x3", "f32", 2, 16, 64, 33, 70, 7, "iid", 1.00),     # everything changed
-]
-
-
-@pytest.mark.parametrize("case", SELF_CASES)
-def test_self_listing_tile_contraction_is_bit_identical(cbm, case):
-    """cb_conv_update_tiled_self (the tile contraction dilates the raw bitmap, lists its tiles and counts
-    the pixels itself, then crosses a grid barrier) == cb_dilate_tiles + cb_conv_update_tiled: output map,
-    dilated bitmap, count, tile set, cleared raw bitmap; the two paths alternate on the same workspaces."""
-    mode, dt, B, Cin, Cout, H, W, k, kind, frac = case
-    cg, lib, cb = cbm["cg"], cbm["lib"], cbm["cb"]
-    tdt, gemm = TORCH_DT[dt], cb.CBConv2d.GEMM_MODES[mode]
-    assert cg.tiled_supported(tdt, gemm, (B, H, W), Cin, Cout, (k, k)) >= 1
-    assert lib.C.cb_conv_tiled_self_supported(B, H, W, k, k) == 1 and lib.C.cb_conv_tiled_self_supported(B, H, W, 19, 3) == 0
-    gen = torch.Generator().manual_seed(B + 3 * H + W)
-    state, sbuf = cg.pixel_major((B, Cin, H, W), tdt, "cuda", 0)
-    state.copy_((torch.rand(B, Cin, H, W, generator=gen) - 0.5).to(tdt))
-    w = ((torch.rand(Cout, Cin, k, k, generator=gen) - 0.5) * 2 * (Cin * k * k) ** -0.5).to(tdt).cuda()
-    bias = (torch.rand(Cout, generator=gen) - 0.5).float().cuda()
-    packed = cg.pack_weights(w, gemm)
-    shape = (B, H, W)
-    s = cg.alloc_scratch(shape, "cuda")
-    tile_ws = cg.alloc_tile_ws(shape, "cuda")
-    NT = (tile_ws.numel() - 4) // 2
-    recs = []
-    for rep, path in enumerate(("two", "self", "two", "self", "self")):
-        raw = _change_mask(B, H, W, kind, frac, torch.Generator().manual_seed(100 + rep // 2)).to(torch.int8).cuda()
-        s["raw_bits"].copy_(cg._map_to_bits(raw)[0])
-        out, obuf = cg.pixel_major((B, Cout, H, W), tdt, "cuda", 0)
-        out.fill_(2.0)
-        s["dil_bits"].fill_(-1)                    # stale bits of an earlier frame must not survive
-        if path == "two":
-            cg.dilate_tiles(s["raw_bits"], shape, (k, k), s["count"], s["ws"], s["dil_bits"], tile_ws, clear_raw=True)
-            cg.conv_update_tiled(sbuf, tile_ws, s["dil_bits"], packed, bias, obuf, Cin, Cout, (k, k), True, gemm)
-        else:
-            cg.conv_update_tiled(sbuf, tile_ws, s["dil_bits"], packed, bias, obuf, Cin, Cout, (k, k), True, gemm,
-                                 self_list=dict(raw_bits=s["raw_bits"], count=s["count"], ws=s["ws"], clear_raw=True))
-        torch.cuda.synchronize()
-        ntl = int(tile_ws[1])
-        assert int(tile_ws[0]) == 0 and int(tile_ws[2]) == 0        # append counter / barrier arrivals at rest
-        assert int(s["raw_bits"].abs().sum()) == 0                    # clear_raw
-        recs.append((path, rep // 2, obuf.clone(), s["dil_bits"].clone(), int(s["count"]), ntl,
-                     tile_ws[4 + NT:4 + NT + ntl].sort().values.clone()))
-    by = {}
-    for path, frame, *rest in recs:
-        by.setdefault(frame, []).append(rest)
-    for frame, lst in by.items():
-        for other in lst[1:]:
-            for a, b in zip(lst[0], other):
-                assert (a == b) if isinstance(a, int) else torch.equal(a, b), frame
-    if frac > 0:
-        assert recs[0][4] > 0 and recs[0][5] > 0
-
-
-@pytest.mark.parametrize("dt,feedback", [("f32", True), ("f32", False), ("bf16", True)])
-def test_self_listing_in_the_model_is_bit_identical(cbm, dt, feedback, monkeypatch):
-    """conv -> pool -> conv -> pool -> conv on the candidate path with and without CBINFER_SELF_TILES: every
-    output, count, dilated bitmap, state and pooled map of every frame is bit-identical, the raw bitmaps are
-    left clear, and on-demand index lists (lastChangeIndexes) agree."""
-    import torch.nn as nn
-    cb = cbm["cb"]
-    from cbinfer_b200 import models, video
-    tdt = TORCH_DT[dt]
-    torch.manual_seed(11)
-    base = nn.Sequential(nn.Conv2d(3, 16, 7, padding=3), nn.ReLU(), nn.MaxPool2d(2, 2),
-                         nn.Conv2d(16, 64, 7, padding=3), nn.ReLU(), nn.MaxPool2d(2, 2),
-                         nn.Conv2d(64, 32, 3, padding=1)).cuda().to(tdt).eval()
-    frames = [f.cuda().to(tdt) for f in video.sequence(3, 100, 136, 7, 0.08, "block", seed=5)]
-    frames.insert(4, frames[3].clone())            # an unchanged frame
-    runs = []
-    for flag in ("1", "0"):
-        monkeypatch.setenv("CBINFER_SELF_TILES", flag)     # (opt-in knob; "0" = the two-launch default)
-        m = cb.convertPools(cb.convert(base, threshold=0.04))
-        for c in m.modules():
-            if type(c) is cb.CBConv2d:
-                c.feedbackLoop = feedback
-            if type(c) is cb.CBPoolMax2d:
-                c.cloneOutput = False
-        models.enableCandidateDetection(m)
-        outs = []
-        for f in frames:
-            o = m(f)
-            torch.cuda.synchronize()
-            convs = [c for c in m.modules() if type(c) is cb.CBConv2d]
-            pools = [c for c in m.modules() if type(c) is cb.CBPoolMax2d]
-            outs.append(dict(out=o.clone(), counts=[int(c._scratch["count"]) for c in convs],
-                             dil=[c._scratch["dil_bits"].clone() for c in convs],
-                             raw=[c._scratch["raw_bits"].clone() for c in convs[1:]],
-                             states=[c.prevInput.clone() for c in convs],
-                             pooled=[p.outputState.clone() for p in pools],
-                             lists=[c.lastChangeIndexes().clone() for c in convs[:2]]))
-        runs.append(outs)
-    for t, (a, b) in enumerate(zip(*runs)):
-        assert a["counts"] == b["counts"], t
-        assert torch.equal(a["out"], b["out"]), t
-        for k in ("dil", "raw", "states", "pooled", "lists"):
-            for x, y in zip(a[k], b[k]):
-                assert torch.equal(x, y), (t, k)
-    assert sum(runs[0][-1]["counts"]) > 0 and len(runs[0][-1]["lists"][0]) == runs[0][-1]["counts"][0]

@@ -55,7 +55,7 @@ bits, _ = cg._map_to_bits(m)
 s = cg.alloc_scratch(shape, dev)
 tw = cg.alloc_tile_ws(shape, dev)
 for _ in range(2):
-    cg.dilate_tiles(bits, shape, (7, 7), s["count"], s["ws"], s["dil_bits"], tw)            # dilate_tiles_kernel
+    cg.dilate_tiles(bits, shape, (7, 7), s["count"], s["ws"], s["dil_bits"], tw)            # dilate_compact_kernel, tiles only
     cg.dilate_compact(bits, shape, (7, 7), s["idx"], s["count"], s["ws"], dil_bits=s["dil_bits"])  # dilate_compact_kernel
 
 # scene layer 2 sizes: 8 x 16ch x 480x640 conv output -> pool -> 240x320 state; ~135k changed pixels

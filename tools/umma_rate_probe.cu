@@ -20,7 +20,6 @@ namespace cb {
 thread_local char g_err[512] = "";
 int fail(int code, const char* fmt, ...) { (void)fmt; return code; }
 int sm_count() { return 148; }
-bool pdl_enabled() { return false; }
 }  // namespace cb
 using namespace cb;
 
