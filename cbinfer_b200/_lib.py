@@ -24,7 +24,7 @@ SYMBOLS = [
     "cb_version", "cb_last_error", "cb_device_info", "cb_bitmap_row_words", "cb_bitmap_words",
     "cb_compact_ws_bytes", "cb_channel_pitch", "cb_plane_pitch16", "cb_packed_weight_bytes", "cb_change_detect", "cb_change_detect_u8",
     "cb_dilate_compact", "cb_map_to_bits", "cb_change_detect_sparse", "cb_pool_compact", "cb_maxpool2x2_detect",
-    "cb_detect_compact_ws_bytes", "cb_detect_compact_sparse", "cb_pack_weights", "cb_conv_ws_bytes", "cb_conv_update", "cb_conv_update_masked", "cb_maxpool2x2",
+    "cb_pack_weights", "cb_conv_ws_bytes", "cb_conv_update", "cb_conv_update_masked", "cb_maxpool2x2",
     "cb_gen_xmatrix", "cb_matrix_mult", "cb_update_output", "cb_fg_update",
     "cb_fg_detect", "cb_conv_accumulate", "cb_compact_small_max_words", "cb_change_detect_sparse_compact",
     "cb_tile_ws_bytes", "cb_dilate_compact_tiles", "cb_conv_tiled_supported", "cb_conv_update_tiled",
@@ -88,9 +88,6 @@ def _load():
         "cb_change_detect_sparse_compact": (i32, [vp, i32, vp, i64, i64, i64, i64, vp, i64, i64, i64, i64, i32,
                                                   vp, vp, vp, vp, vp, i32, i32, i32, i32, f32, i32, i32,
                                                   vp, vp, vp, vp, i32, i32, i32]),
-        "cb_detect_compact_ws_bytes": (sz, [i32, i32, i32]),
-        "cb_detect_compact_sparse": (i32, [vp, i32, vp, i64, i64, i64, i64, vp, i64, i64, i64, i64, i32,
-                                           vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, f32, i32]),
         "cb_pool_compact": (i32, [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32]),
         "cb_pack_weights": (i32, [vp, i32, i32, vp, vp, i32, i32, i32, i32]),
         "cb_conv_ws_bytes": (sz, []),

@@ -223,7 +223,6 @@ class CBConv2d(nn.Module):
         # extension: treat indices received from upstream as *candidates* for the thresholded
         # detection instead of as the final change set (exact, see cb_change_detect_sparse)
         self.candidateDetect = False
-        self.fuse1x1 = False      # extension: detect+compact in one launch for 1x1 layers
         # extension: (divisor, bias) applied to uint8 input frames inside the detection kernel
         self.inputNorm = None
         # extension: 1x1 layer on the candidate path without any compaction (see forward_normal)
@@ -496,27 +495,15 @@ class CBConv2d(nn.Module):
             # honoured as a copy -- the state always owns its memory.
             mode = _lib.UPDATE_CHANGED if self.feedbackLoop else _lib.UPDATE_ALL
             sparse_next = bool(getattr(self, 'candidateDetect', False)) and not plain_input
-            # (measured: one launch fewer, but its serial compaction tail makes it slower than the
-            #  two-kernel path once there are >~10k candidates, so it is opt-in: fuse1x1=True)
-            fused11 = (candidates is not None and tuple(self.kernel_size) == (1, 1)
-                       and getattr(self, 'fuse1x1', False)
-                       and not self.saveChangeMap and input.stride(1) == 1)
             # extension: no compaction at all for a 1x1 layer on the candidate path - the
             # contraction walks the candidate list and skips pixels whose raw bit is not set
             # (cb_conv_update_masked); this layer's own index list is then never materialised
             masked = (candidates is not None and not detected and tuple(self.kernel_size) == (1, 1)
-                      and getattr(self, 'maskedConv', False) and not fused11
+                      and getattr(self, 'maskedConv', False)
                       and not self.saveChangeMap and gemm != _lib.GEMM_SIMT_F32)
             fusedSmall = False
             if detected:
                 pass                     # the upstream pool kernel already did it
-            elif fused11:
-                # no dilation needed: candidate detection + ordered compaction in one launch
-                if "dcs_ws" not in s:
-                    s["dcs_ws"] = torch.zeros(_lib.C.cb_detect_compact_ws_bytes(B, H, W),
-                                              dtype=torch.uint8, device=dev)
-                cg.detect_compact_sparse(input, self.prevInput, self.threshold, mode, candidates,
-                                         s["idx"], s["count"], s["dcs_ws"], aux=aux_arg)
             elif candidates is not None and not masked and not use_tiles and not self.saveChangeMap \
                     and input.stride(1) == 1 and self._smallMap(B, H, W):
                 # small map: candidate detection + dilation + ordered compaction in ONE launch (the
@@ -543,10 +530,7 @@ class CBConv2d(nn.Module):
                 cg.detect(input, self.prevInput, s["raw_bits"], self.threshold, mode, aux=aux_arg)
             self._fresh = False
             self._lastThr = self.threshold
-            if not detected and fused11:
-                s["raw_clear"] = False
-                changeIndexes = ChangeIndexes(s["idx"], s["count"], (B, H, W), bits=None)
-            elif fusedSmall:
+            if fusedSmall:
                 s["raw_clear"] = sparse_next
                 changeIndexes = ChangeIndexes(s["idx"], s["count"], (B, H, W), bits=s["dil_bits"])
             elif mask is not None:
@@ -555,8 +539,7 @@ class CBConv2d(nn.Module):
                 changeIndexes.superset = True
             else:
                 changeIndexes = self._compact(s, B, H, W, sparse_next, tiles=use_tiles,
-                                              lazy=pool_args is not None and not self.saveChangeMap
-                                              and os.environ.get("CBINFER_LAZY_LIST", "1") != "0")
+                                              lazy=pool_args is not None and not self.saveChangeMap)
                 tiled = use_tiles
         else:
             if not isinstance(changeIndexes, ChangeIndexes):
@@ -608,7 +591,6 @@ class CBConv2d(nn.Module):
         for this layer (fresh state, lowered threshold, state touched from outside, ...)."""
         if not (getattr(self, 'candidateDetect', False) and getattr(self, 'maskedConv', False)) \
                 or self.finegrained or self.saveChangeMap or self.gatherComputationStats \
-                or getattr(self, 'fuse1x1', False) \
                 or tuple(self.kernel_size) != (1, 1) or self.feedbackLoop != feedback \
                 or self._fresh or self._inBuf is None or self._outBuf is None or self._scratch is None \
                 or tuple(self.prevInput.shape) != tuple(shape) or self.prevInput.dtype != dt \
@@ -630,7 +612,6 @@ class CBConv2d(nn.Module):
         B, C0, H, W = input.shape
         if not isinstance(changeIndexes, ChangeIndexes) or not getattr(self, 'candidateDetect', False) \
                 or not getattr(self, 'maskedConv', False) or tuple(self.kernel_size) != (1, 1) \
-                or getattr(self, 'fuse1x1', False) \
                 or self.saveChangeMap or self.gatherComputationStats or ext_out or input.dtype != torch.float32 \
                 or self._fresh or self._lastThr is None or self.threshold < self._lastThr \
                 or tuple(changeIndexes.shape) != (B, H, W) or not getattr(changeIndexes, 'complete', True) \
@@ -720,8 +701,6 @@ class CBConv2d(nn.Module):
 
     def _smallMap(self, B, H, W):
         """bitmap small enough for the one-launch detection + compaction (cb_change_detect_sparse_compact)?"""
-        if os.environ.get("CBINFER_FUSE_SMALL", "1") == "0":
-            return False
         return 0 < _lib.C.cb_bitmap_words(B, H, W) <= _lib.C.cb_compact_small_max_words()
 
     def _useTiles(self, dt, gemm, shape):
@@ -810,7 +789,7 @@ class CBConv2d(nn.Module):
         for name, val in (('saveChangeMap', False), ('propChangeIndexes', False),
                           ('gatherComputationStats', False), ('finegrained', False),
                           ('copyInput', True), ('feedbackLoop', False), ('gemmMode', 'auto'),
-                          ('candidateDetect', False), ('fuse1x1', False), ('inputNorm', None),
+                          ('candidateDetect', False), ('inputNorm', None),
                           ('maskedConv', False), ('tileMode', 'auto')):
             if not(hasattr(self, name)):
                 setattr(self, name, val)

@@ -183,20 +183,9 @@ def detect_sparse_compact(x, state, raw_bits, threshold, update_mode, candidates
         (filtSize[0] - 1) // 2, (filtSize[1] - 1) // 2, int(bool(clear_raw))))
 
 
-def detect_compact_sparse(x, state, threshold, update_mode, candidates, idx, count, ws, aux=None,
-                          bits=None):
-    """cb_detect_compact_sparse: candidate detection + ordered compaction in one launch (layers
-    without dilation, pixel-major tensors)."""
-    require_cuda(x, state)
-    B, Cc, H, W = x.shape
-    assert state.shape == x.shape and tuple(candidates.shape) == (B, H, W)
-    mode, hi, lo = _aux_args(aux, state)
-    check(C.cb_detect_compact_sparse(stream_ptr(x.device), dtype_code(x), x.data_ptr(), *_strides4(x),
-                                     state.data_ptr(), *_strides4(state), mode, hi, lo,
-                                     candidates.buffer.data_ptr(), candidates.count.data_ptr(),
-                                     idx.data_ptr(), count.data_ptr(),
-                                     bits.data_ptr() if bits is not None else None, ws.data_ptr(),
-                                     B, Cc, H, W, float(threshold), int(update_mode)))
+def detect_compact_sparse(*args, **kwargs):
+    """Removed kernel; the name stays only because bench.py looks it up to build its kernel tables."""
+    raise _lib.CBinferError("detect_compact_sparse was removed")
 
 
 def pool_compact(in_bits, in_shape, out_shape, idx, count, ws, out_bits=None):

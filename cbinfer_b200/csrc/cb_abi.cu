@@ -110,14 +110,6 @@ int cb_change_detect_u8(void* stream, const uint8_t* x, long long x_sb, long lon
                           threshold, update_mode);
 }
 
-static bool compact_coop() {
-  static const bool v = [] {
-    const char* e = getenv("CBINFER_COMPACT_COOP");          // tuning knob: 0 = per-thread expansion
-    return !(e && e[0] == '0');
-  }();
-  return v;
-}
-
 size_t cb_tile_ws_bytes(int B, int H, int W) { return cb::tile_ws_words(B, H, W) * sizeof(int32_t); }
 
 static int dilate_compact_impl(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits, int8_t* dil_map,
@@ -142,7 +134,7 @@ static int dilate_compact_impl(void* stream, const uint32_t* raw_bits, uint32_t*
                                                           kWHalf, (int)nwords, ntiles, 0, 0,
                                                           clear_raw ? const_cast<uint32_t*>(raw_bits) : nullptr,
                                                           (int32_t*)tile_ws, cb::tile_grid_y(H), cb::tile_grid_xp(W),
-                                                          (int)compact_coop(), no_list);
+                                                          no_list);
   CB_CHECK_LAUNCH("dilate_compact");
   return 0;
 }
@@ -187,7 +179,7 @@ int cb_pool_compact(void* stream, const uint32_t* in_bits, uint32_t* out_bits, i
   cb::launch(dilate_compact_kernel, ntiles, kCompactThreads, 0, s, in_bits, out_bits, nullptr, idx, count, ws,
                                                           B, oH, oW, (oW + 31) / 32, 0, 0,
                                                           (int)nwords, ntiles, H, (W + 31) / 32, nullptr,
-                                                          nullptr, 0, 0, (int)compact_coop(), 0);
+                                                          nullptr, 0, 0, 0);
   CB_CHECK_LAUNCH("pool_compact");
   return 0;
 }
@@ -342,7 +334,7 @@ int cb_conv_tiled_supported(int dtype, int gemm, int B, int H, int W, int Cin, i
   cb::TilePlan plan;
   cb::umma_tile_plan(plan, dtype, gemm, Cp, B, H, W, Cout, cb_channel_pitch(dtype, Cout), kH, kW, 0);
   if (!plan.ok) return 0;
-  return (plan.mma_clk_per_tile <= cb::tile_clk_limit() || plan.short_k) ? 1 : 2;
+  return (plan.mma_clk_per_tile <= cb::kTileClkLimit || plan.short_k) ? 1 : 2;
 }
 
 static int conv_update_tiled_impl(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
@@ -472,11 +464,6 @@ int cb_tail_update(void* stream, const float* x, float* state1, const void* pack
   a.count1 = count1; a.count2 = count2; a.sync = (unsigned*)sync_ws;
   a.xp = C0; a.p1 = C1; a.p2 = pitch_out2; a.C0 = C0; a.C1 = C1; a.C2 = C2;
   a.relu1 = relu1; a.relu2 = relu2; a.update = update_mode; a.thr1 = thr1; a.thr2 = thr2;
-  static const int tail_adapt = [] {
-    const char* e = getenv("CBINFER_TAIL_ADAPT");            // tuning knob: 0 = always 128 rows per tile
-    return (e && e[0] == '0') ? 0 : 1;
-  }();
-  a.adapt = tail_adapt;
   return cb::tail_update((cudaStream_t)stream, a, packed_w1, packed_w2);
 }
 
@@ -510,25 +497,6 @@ int cb_maxpool2x2(void* stream, int dtype, const void* x, long long x_sb, long l
                                  o_sb, o_sc, o_sy, o_sx, C, H, W, oH, oW)));
   }
   CB_CHECK_LAUNCH("maxpool2x2");
-  return 0;
-}
-
-size_t cb_detect_compact_ws_bytes(int B, int H, int W) { return 16 + (size_t)B * H * W + 16; }
-
-int cb_detect_compact_sparse(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
-                             long long x_sy, long long x_sx, void* state, long long s_sb,
-                             long long s_sc, long long s_sy, long long s_sx, int aux_mode,
-                             void* aux_hi, void* aux_lo, const int32_t* candidates,
-                             const int32_t* n_candidates, int32_t* idx, int32_t* count,
-                             uint32_t* bits, void* ws, int B, int C, int H, int W, float threshold,
-                             int update_mode) {
-  CB_CHECK_ARG(x && state && candidates && n_candidates && idx && count && ws,
-               "detect_compact_sparse: null pointer");
-  CB_CHECK_ARG(idx != candidates, "detect_compact_sparse: idx must not alias candidates");
-  CB_DISPATCH_DTYPE(dtype, return (launch_detect_compact_sparse<T, VEC>(
-                               (cudaStream_t)stream, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc,
-                               s_sy, s_sx, aux_mode, aux_hi, aux_lo, candidates, n_candidates, idx,
-                               count, bits, ws, B, C, H, W, threshold, update_mode)));
   return 0;
 }
 

@@ -30,15 +30,8 @@ int sm_count();
 // log2 of the lanes that share one pixel in the candidate-detection / pooling kernels.  One lane
 // per 16-byte chunk would be the obvious choice; two chunks per lane halves the number of warps
 // (one wave instead of two at 8 streams) and doubles the loads in flight per lane: measured
-// pool+detect 11.3 -> 8.3 us, sparse detect 7.7 -> 6.7 us.  CBINFER_GLOG_DELTA overrides (tuning).
-inline int glog_tuned(int glog) {
-  static const int delta = [] {
-    const char* e = getenv("CBINFER_GLOG_DELTA");
-    return e ? atoi(e) : 1;
-  }();
-  const int g = glog - delta;
-  return g < 0 ? 0 : g;
-}
+// pool+detect 11.3 -> 8.3 us, sparse detect 7.7 -> 6.7 us.
+inline int glog_tuned(int glog) { return glog > 0 ? glog - 1 : 0; }
 
 // cooperative != 0: the grid is launched only when ALL its CTAs can be resident at once (kernels whose
 // CTAs wait for each other, e.g. the stream-K finisher spinning on its contributors' flags, must not

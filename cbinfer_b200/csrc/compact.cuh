@@ -103,7 +103,7 @@ dilate_compact_kernel(const uint32_t* __restrict__ raw, uint32_t* __restrict__ d
                       int32_t* __restrict__ count, void* ws, int B, int H, int W, int Wd, int kh,
                       int kw, int nwords, int ntiles, int pool_hin, int pool_wdin,
                       uint32_t* __restrict__ clear_bits, int32_t* __restrict__ tile_ws, int tile_ty,
-                      int tile_xp, int coop, int no_list) {
+                      int tile_xp, int no_list) {
   CompactHeader* hdr = reinterpret_cast<CompactHeader*>(ws);
   volatile unsigned long long* tstate =
       reinterpret_cast<volatile unsigned long long*>(reinterpret_cast<char*>(ws) + sizeof(CompactHeader));
@@ -247,7 +247,7 @@ dilate_compact_kernel(const uint32_t* __restrict__ raw, uint32_t* __restrict__ d
 
   // ---- expand set bits to ascending pixel indices ------------------------------------------
   int o = s_base + s_warp[wid] + (incl - cnt);
-  if (coop && kCompactWPT == 1 && !dil_map) {
+  if (kCompactWPT == 1 && !dil_map) {
     // warp-cooperative expansion: the warp walks its non-empty words; lane i writes bit i of the
     // current word at its rank -> the 32 stores of a dense word are one coalesced 128-byte line
     // (per-thread expansion writes 32 lines per instruction when a block of pixels changed)

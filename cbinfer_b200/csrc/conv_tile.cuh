@@ -606,16 +606,6 @@ inline TilePlan tile_plan(int es, bool split3, int bn, int Cp, int B, int H, int
   }
   if (!g.nhalo) return p;
   if (nb > TL_MAXB) nb = TL_MAXB;
-  static const int force_occ = [] {
-    const char* e = getenv("CBINFER_TILE_OCC");              // tuning knob: 1 = one CTA per SM
-    return e ? atoi(e) : 0;
-  }();
-  if (force_occ == 1 && occ == 2) {
-    occ = 1;
-    nb = (budget1 - fixed) / b_stage;
-    if (nb > TL_MAXB) nb = TL_MAXB;
-    if (one_ntile && g.num_kb <= nb) nb = g.num_kb;
-  }
   if (occ == 2) {
     // small layers (e.g. the RGB input layer: 50 KB, 64 TMEM columns): up to four CTAs per SM -- their
     // instructions are issue-bound, more issuing warps keep the tensor pipe busier
@@ -623,7 +613,6 @@ inline TilePlan tile_plan(int es, bool split3, int bn, int Cp, int B, int H, int
     if (o > 512 / tmem_cols) o = 512 / tmem_cols;
     if (o > 4) o = 4;
     if (bn > 16 && o > 2) o = 2;                             // register side: __launch_bounds__ of the kernel
-    if (force_occ > 1 && o > force_occ) o = force_occ;
     if (o > occ) occ = o;
   }
   g.nb = nb;
@@ -708,13 +697,7 @@ int launch_conv_tile(cudaStream_t s, const void* state, const void* state_lo, co
 
 // policy threshold: tiles whose tensor work is at most this many cycles (denser layers keep the
 // index-list kernel, whose M tiles hold changed pixels only)
-inline long long tile_clk_limit() {
-  static const long long v = [] {
-    const char* e = getenv("CBINFER_TILE_CLK");
-    return e ? atoll(e) : 12000ll;
-  }();
-  return v;
-}
+constexpr long long kTileClkLimit = 12000;
 
 // fused pooling: one epilogue warp per TMEM lane quarter owns all channels of its pixels
 inline bool tile_pool_ok(int gemm, int Cout) { return Cout <= 64 && (Cout % 16) == 0 && umma_bn(gemm, Cout) == umma_cout_pad(gemm, Cout); }

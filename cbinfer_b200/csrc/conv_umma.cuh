@@ -1156,13 +1156,8 @@ inline int umma_conv_update(cudaStream_t s, int dtype, int gemm, const void* sta
     int m_switch = (2 * sms / 3) / (CoutPad / bn);
     // ... or much earlier when stream-K can spread few coarse tiles over all SMs (a tile cut into
     // <= ~4 K ranges keeps the finisher's partial sums cheap): measured cross-over ~sms/4 tiles
-    static const int sk_switch_div = [] {
-      const char* e = getenv("CBINFER_SK_SWITCH");           // tuning knob: 0 = old rule
-      return e ? atoi(e) : 4;
-    }();
-    if (ws && ws_bytes > (size_t)UM_SK_FLAG_BYTES && sk_switch_div > 0 && CoutPad == bn &&
-        m_switch > sms / sk_switch_div)
-      m_switch = sms / sk_switch_div;
+    if (ws && ws_bytes > (size_t)UM_SK_FLAG_BYTES && CoutPad == bn && m_switch > sms / 4)
+      m_switch = sms / 4;
     if (m_switch < 1) m_switch = 1;
     // split-K over thread-block clusters: few tiles x long K (small maps, big filters) would
     // otherwise leave most SMs idle and each busy SM limited by its own L2 ingest rate

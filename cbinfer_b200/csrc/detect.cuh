@@ -366,13 +366,6 @@ detect_planar_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, lo
 
 // words per block of the planar kernels: every warp gets >= 2 (word, chunk) pairs, within 64 KB
 inline int planar_words_per_block(int cpv, int cps) {
-  static const int forced = [] {
-    const char* e = getenv("CBINFER_PLANAR_NW");               // tuning knob: 1, 2, 4 or 8
-    return e ? atoi(e) : 0;
-  }();
-  if (forced > 0 && forced <= kPlanarMaxWords && (forced & (forced - 1)) == 0 &&
-      (size_t)forced * 32 * cps * 16 <= 96 * 1024)
-    return forced;
   // measured (tools/planar_bench.py, L2 flushed): 4 (word, chunk) pairs per warp, at most 4 words --
   // C=64 fp32 153 -> 135 us at nw=2, bf16 100 -> 94 us at nw=4; 8 words lose again (fewer, fatter blocks)
   int nw = 1;
@@ -771,171 +764,6 @@ int launch_detect_sparse(cudaStream_t stream, const void* x, long long x_sb, lon
   }
 #undef CB_DETS
   CB_CHECK_LAUNCH("change_detect_sparse");
-  return 0;
-}
-
-}  // namespace cb
-
-namespace cb {
-
-// ------------------------------------------------------------------------------------------------
-// Candidate detection fused with ordered compaction, for layers whose change set needs no dilation
-// (1x1 kernels): one launch instead of memset + sparse detection + dilate/compact.
-//   phase 1 (all blocks): per candidate, threshold + state maintenance, flag byte per candidate;
-//   phase 2 (the last block to finish): ordered compaction of the flagged candidates -> idx, count
-//           (and, optionally, their bits in a pre-cleared bitmap).
-// ws: [0] = blocks-done counter (left at 0), then one flag byte per candidate.
-// ------------------------------------------------------------------------------------------------
-template <typename T, int VEC, int UPDATE>
-__global__ void __launch_bounds__(256)
-detect_compact_sparse_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int xp,
-                             T* __restrict__ st, long long s_sb, long long s_sy, int sp,
-                             AuxPlanes aux, const int32_t* __restrict__ cand,
-                             const int32_t* __restrict__ ncand, int32_t* __restrict__ idx,
-                             int32_t* __restrict__ count, uint32_t* __restrict__ bits,
-                             unsigned* __restrict__ ws, int H, int W, int C, int Wd, T thr,
-                             int glog) {
-  const int n = *ncand;
-  uint8_t* flags = reinterpret_cast<uint8_t*>(ws + 4);
-  const int lane = threadIdx.x & 31;
-  const int G = 1 << glog, ppw = 32 >> glog;
-  const int sub = lane >> glog, gl = lane & (G - 1);
-  const unsigned gmask = (G == 32 ? 0xffffffffu : ((1u << G) - 1u)) << (sub * G);
-  const int P = H * W;
-  const int cpv = (C + VEC - 1) / VEC, tail = C % VEC;
-  const long long nwarps = (long long)gridDim.x * (blockDim.x >> 5);
-  for (long long j0 = ((long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * ppw;
-       j0 < n; j0 += nwarps * ppw) {
-    const long long j = j0 + sub;
-    const bool have = j < n;
-    int b = 0, y = 0, xx = 0, gpix = 0;
-    if (have) {
-      gpix = cand[j];
-      b = gpix / P;
-      const int p = gpix - b * P;
-      y = p / W;
-      xx = p - y * W;
-    }
-    const T* xb = x + b * x_sb + y * x_sy + (long long)xx * xp;
-    T* sb = st + b * s_sb + y * s_sy + (long long)xx * sp;
-    bool f = false;
-    if (have) {
-      for (int cc = gl; cc < cpv; cc += G) {
-        uint4 xv = ld16(xb + cc * VEC);
-        const uint4 sv = ld16(sb + cc * VEC);
-        if (tail && cc == cpv - 1) xv = merge_tail<T, VEC>(xv, sv, tail);
-        f |= Chunk<T>::changed(sv, xv, thr);
-        if (UPDATE == CB_UPDATE_ALL) store_state<T>(sb + cc * VEC, xv, aux, gpix, cc * VEC);
-      }
-    }
-    const bool chg = (__ballot_sync(0xffffffffu, f) & gmask) != 0u;
-    if (have) {
-      if (gl == 0) flags[j] = chg ? 1 : 0;
-      if (chg && UPDATE == CB_UPDATE_CHANGED) {
-        for (int cc = gl; cc < cpv; cc += G) {
-          uint4 xv = ld16(xb + cc * VEC);
-          if (tail && cc == cpv - 1) xv = merge_tail<T, VEC>(xv, ld16(sb + cc * VEC), tail);
-          store_state<T>(sb + cc * VEC, xv, aux, gpix, cc * VEC);
-        }
-      }
-    }
-  }
-  // ---- the last block compacts ---------------------------------------------------------------
-  __shared__ unsigned s_last;
-  __shared__ int s_wsum[8];
-  __shared__ int s_run;
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) {
-    const unsigned prev = atomicAdd(ws, 1u);
-    s_last = prev == gridDim.x - 1;
-    if (s_last) ws[0] = 0;
-    s_run = 0;
-  }
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-  const int wid = threadIdx.x >> 5;
-  for (int base = 0; base < n; base += 256 * 8) {          // 8 candidates per thread per round
-    const int j0 = base + threadIdx.x * 8;
-    unsigned m = 0;
-#pragma unroll
-    for (int e = 0; e < 8; ++e)
-      if (j0 + e < n && reinterpret_cast<volatile uint8_t*>(flags)[j0 + e]) m |= 1u << e;
-    const int cnt = __popc(m);
-    int incl = cnt;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int v = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= o) incl += v;
-    }
-    if (lane == 31) s_wsum[wid] = incl;
-    __syncthreads();
-    int woff = 0, total = 0;
-#pragma unroll
-    for (int q = 0; q < 8; ++q) {
-      const int v = s_wsum[q];
-      if (q < wid) woff += v;
-      total += v;
-    }
-    int o = s_run + woff + incl - cnt;
-#pragma unroll
-    for (int e = 0; e < 8; ++e)
-      if (m & (1u << e)) {
-        const int pix = cand[j0 + e];
-        idx[o++] = pix;
-        if (bits) {
-          const int b = pix / P, p = pix - b * P;
-          const int y = p / W, xx = p - y * W;
-          atomicOr(bits + ((long long)b * H + y) * Wd + (xx >> 5), 1u << (xx & 31));
-        }
-      }
-    __syncthreads();
-    if (threadIdx.x == 0) s_run += total;
-    __syncthreads();
-  }
-  if (threadIdx.x == 0) *count = s_run;
-}
-
-template <typename T, int VEC>
-int launch_detect_compact_sparse(cudaStream_t stream, const void* x, long long x_sb, long long x_sc,
-                                 long long x_sy, long long x_sx, void* state, long long s_sb,
-                                 long long s_sc, long long s_sy, long long s_sx, int aux_mode,
-                                 void* aux_hi, void* aux_lo, const int32_t* cand,
-                                 const int32_t* ncand, int32_t* idx, int32_t* count, uint32_t* bits,
-                                 void* ws, int B, int C, int H, int W, float threshold, int update) {
-  const size_t es = sizeof(T);
-  AuxPlanes aux;
-  if (int rc = make_aux<T>(aux, aux_mode, aux_hi, aux_lo, state, C)) return rc;
-  const bool vec_ok = x_sc == 1 && s_sc == 1 && (x_sx % VEC) == 0 && (s_sx % VEC) == 0 &&
-                      x_sx >= C && s_sx >= C && ((x_sy * es) % 16) == 0 && ((s_sy * es) % 16) == 0 &&
-                      ((x_sb * es) % 16) == 0 && ((s_sb * es) % 16) == 0 &&
-                      ((uintptr_t)x % 16) == 0 && ((uintptr_t)state % 16) == 0 &&
-                      x_sx < (1ll << 30) && s_sx < (1ll << 30);
-  CB_CHECK_ARG(vec_ok, "detect_compact_sparse: needs pixel-major, 16-byte aligned x and state");
-  if ((long long)B * H * W == 0) {
-    cudaMemsetAsync(count, 0, sizeof(int32_t), stream);
-    return 0;
-  }
-  const int cpv = (C + VEC - 1) / VEC;
-  int glog = 0;
-  while ((1 << glog) < cpv && glog < 5) ++glog;
-  glog = cb::glog_tuned(glog);
-  const unsigned grid = (unsigned)(sm_count() * 8);
-  const int Wd = (W + 31) / 32;
-  const T thr = thr_cast<T>(threshold);
-#define CB_DCS(U_)                                                                                 \
-  cb::launch(detect_compact_sparse_kernel<T, VEC, U_>, grid, 256, 0, stream, (const T*)x,         \
-                 x_sb, x_sy, (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand, ncand, idx,   \
-                 count, bits, (unsigned*)ws, H, W, C, Wd, thr, glog);
-  switch (update) {
-    case CB_UPDATE_NONE: CB_DCS(CB_UPDATE_NONE) break;
-    case CB_UPDATE_CHANGED: CB_DCS(CB_UPDATE_CHANGED) break;
-    case CB_UPDATE_ALL: CB_DCS(CB_UPDATE_ALL) break;
-    default: return fail(2, "detect_compact_sparse: bad update_mode %d", update);
-  }
-#undef CB_DCS
-  CB_CHECK_LAUNCH("detect_compact_sparse");
   return 0;
 }
 

@@ -42,7 +42,6 @@ struct TailArgs {
   int C0, C1, C2;                // channels: in, mid, out
   int relu1, relu2, update;      // update: CB_UPDATE_CHANGED (feedback) or CB_UPDATE_ALL
   float thr1, thr2;
-  int adapt;                     // 1: fewer rows per tile when the candidates do not fill a wave (below)
 };
 
 struct TailCtrl {
@@ -73,7 +72,7 @@ tail_kernel(const __grid_constant__ CUtensorMap w1map, const __grid_constant__ C
   // phases shrink with the rows, while the MMAs are negligible: 14 275 candidates on 148 CTAs = 138 tiles of
   // 104 rows instead of 112 of 128 on 112 CTAs.  Per-row results do not depend on the tile's other rows.
   int rpt = TAIL_ROWS;
-  if (a.adapt && n < (int)gridDim.x * TAIL_ROWS) {
+  if (n < (int)gridDim.x * TAIL_ROWS) {
     rpt = (((n + (int)gridDim.x - 1) / (int)gridDim.x) + 7) & ~7;
     rpt = rpt < 8 ? 8 : rpt > TAIL_ROWS ? TAIL_ROWS : rpt;
   }

@@ -165,20 +165,6 @@ int cb_change_detect_sparse_compact(void* stream, int dtype, const void* x, long
                                     uint32_t* dil_bits, int32_t* idx, int32_t* count, void* sync_ws,
                                     int kHHalf, int kWHalf, int clear_raw);
 
-/* cb_change_detect_sparse + ordered compaction in ONE launch, for layers whose change set needs no
- * dilation (1x1 kernels): idx[0..n) = the candidates that exceed the threshold, in candidate
- * order, *count = n; state / planes maintained as usual; `bits` (optional, pre-cleared) receives
- * their bits.  Pixel-major x and state only.  ws: cb_detect_compact_ws_bytes() bytes, zeroed once
- * at allocation, private to the stream. */
-size_t cb_detect_compact_ws_bytes(int B, int H, int W);
-int cb_detect_compact_sparse(void* stream, int dtype,
-                             const void* x, long long x_sb, long long x_sc, long long x_sy, long long x_sx,
-                             void* state, long long s_sb, long long s_sc, long long s_sy, long long s_sx,
-                             int aux_mode, void* aux_hi, void* aux_lo,
-                             const int32_t* candidates, const int32_t* n_candidates, int32_t* idx,
-                             int32_t* count, uint32_t* bits, void* ws, int B, int C, int H, int W,
-                             float threshold, int update_mode);
-
 /* 2x2/stride-2 pooled view of a change bitmap, compacted: out bit (yo,xo) = OR of the input bits
  * of window (yo,xo); writes out_bits (optional), idx[0..n) ascending at pooled resolution
  * [B,oH,oW] and *count.  Hands change candidates across a CBPoolMax2d (the reference forwards the

@@ -27,6 +27,18 @@ def test_library_exports_every_declared_symbol():
     assert _lib.C.cb_version() >= 100
 
 
+def test_library_and_module_read_only_the_kept_environment_variables():
+    """A setting measured worse is removed, not kept behind a variable (DESIGN.md §6 says why each
+    of these stays)."""
+    pkg = os.path.join(REPO, "cbinfer_b200")
+    files = [os.path.join(pkg, f) for f in os.listdir(pkg) if f.endswith(".py")]
+    files += [os.path.join(pkg, "csrc", f) for f in os.listdir(os.path.join(pkg, "csrc"))]
+    names = set()
+    for f in files:
+        names |= set(re.findall(r"CBINFER_[A-Z0-9_]+", open(f).read()))
+    assert names == {"CBINFER_" + n for n in ("LIB", "STREAMK", "KSPLIT", "TILES", "FUSE_POOL", "FUSE_TAIL")}
+
+
 def test_size_helpers():
     from cbinfer_b200._lib import C
     assert C.cb_bitmap_row_words(640) == 20 and C.cb_bitmap_row_words(46) == 2

@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """One conv_update shape in isolation (default: scene L3 at 8 streams, ~5 % change): CUDA-event
-timing over graph replays; small enough to wrap in ncu.  Env knobs: CBINFER_M2, CBINFER_STREAMK."""
+timing over graph replays; small enough to wrap in ncu.  Env knob: CBINFER_STREAMK."""
 import argparse, os, sys
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
@@ -53,8 +53,8 @@ def main():
     torch.cuda.synchronize()
     us = e0.elapsed_time(e1) * 1e3 / a.rep
     flops = 2.0 * sel.numel() * Cin * k * k * Cout
-    print("shape %s n=%d %s/%s ws=%s M2=%s SK=%s: %.2f us  %.1f TFLOP/s (algorithmic)" % (
-        a.shape, sel.numel(), a.dtype, a.gemm, ws is not None, os.environ.get("CBINFER_M2", "1"),
+    print("shape %s n=%d %s/%s ws=%s SK=%s: %.2f us  %.1f TFLOP/s (algorithmic)" % (
+        a.shape, sel.numel(), a.dtype, a.gemm, ws is not None,
         os.environ.get("CBINFER_STREAMK", "1"), us, flops / us * 1e-6))
 
 

@@ -1,7 +1,7 @@
 #!/bin/bash
 # A/B of one environment knob on one box, same minute: quick parity subset, then the bench value and the
 # in-step kernel times with the knob off / on, alternating.   usage: tools/gpu_ab.sh KNOB [off_value] [on_value]
-KNOB=${1:-CBINFER_COMPACT_COOP}; OFF=${2:-0}; ON=${3:-1}
+KNOB=${1:-CBINFER_FUSE_TAIL}; OFF=${2:-0}; ON=${3:-1}
 mkdir -p gpurun_out
 cd "$(dirname "$0")/.."
 PYT="python -m pytest -q --tb=short -p no:cacheprovider --timeout 600 -x"

@@ -27,7 +27,7 @@ so = B.SceneStep(model, frames[0], frames[1])
 plain = [so.capture_slot(f) for f in frames]
 
 names = ("detect", "detect_u8", "detect_sparse", "dilate_compact", "dilate_tiles", "pool_compact", "conv_update",
-         "conv_update_tiled", "tail_update", "maxPool2d", "maxPool2d_detect", "detect_compact_sparse")
+         "conv_update_tiled", "tail_update", "maxPool2d", "maxPool2d_detect")
 orig = {n: getattr(cg, n) for n in names}
 log = None
 

@@ -9,7 +9,7 @@ import cbinfer_b200 as cb
 from cbinfer_b200 import models, video, conv2d_cg as cg
 
 OPS = ("detect", "detect_sparse", "dilate_compact", "pool_compact", "conv_update", "maxPool2d",
-       "maxPool2d_detect", "detect_compact_sparse")
+       "maxPool2d_detect")
 
 
 def main():

@@ -35,6 +35,5 @@ for (B, C, H, W) in ((8, 64, 368, 368), (8, 16, 240, 320), (8, 512, 46, 46)):
         nbytes = 2 * x0.numel() * x0.element_size()
         t_pl = timeit(lambda: cg.detect(x1, st, s["raw_bits"], 0.5, _lib.UPDATE_NONE))
         t_pm = timeit(lambda: cg.detect(xp, st, s["raw_bits"], 0.5, _lib.UPDATE_NONE))
-        print("C=%d %dx%d %s: planar x %.1f us (%.2f TB/s)   pixel-major x %.1f us (%.2f TB/s)   nw=%s" % (
-            C, H, W, str(dt).split(".")[-1], t_pl, nbytes / t_pl / 1e6, t_pm, nbytes / t_pm / 1e6,
-            os.environ.get("CBINFER_PLANAR_NW", "auto")), flush=True)
+        print("C=%d %dx%d %s: planar x %.1f us (%.2f TB/s)   pixel-major x %.1f us (%.2f TB/s)" % (
+            C, H, W, str(dt).split(".")[-1], t_pl, nbytes / t_pl / 1e6, t_pm, nbytes / t_pm / 1e6), flush=True)
