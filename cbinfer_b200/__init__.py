@@ -121,7 +121,7 @@ def shareWorkspace(net):
     for m in net.modules():
         if type(m) == CBConv2d:
             if holder is None:
-                holder = m._workspace_holder()
+                holder = m._wsHolder
             m._wsHolder = holder
     return net
 

@@ -16,6 +16,7 @@ What is different underneath (B200-first, not a translation):
   * batch > 1 = independent video streams (the reference is batch 1);
   * CUDA only: the reference's CPU branches (conv2d.py:225-227,244-245,252-253) do not exist.
 """
+import functools
 import os
 
 import torch
@@ -50,6 +51,12 @@ class TailDone(object):
         self.candidates = candidates
 
 
+@functools.lru_cache(maxsize=None)
+def _tiles_ok(dt, gemm, shape, Cin, Cout, filtSize, mode):
+    sup = cg.tiled_supported(dt, gemm, shape, Cin, Cout, filtSize)
+    return sup >= 1 if mode == 'on' else sup == 1
+
+
 def _parse_input(inp):
     """tensor, or ('changeIndexes', tensor, indices) from an upstream CB layer (conv2d.py:180-187)."""
     if type(inp) == tuple:
@@ -71,9 +78,14 @@ class CBPoolMax2d(nn.Module):
         self.propPooledIndexes = False  # extension: hand pooled-resolution change candidates on
         self._fusedNext = []            # extension: [downstream CBConv2d] whose detection is fused in
         self.cloneOutput = True   # reference returns outputState.clone() (conv2d.py:73)
+        self._outVersion = None   # outputState._version as the kernels last left it
         self.register_buffer('outputState', torch.empty(0))
-        self._stateBuf = None
         self.clearMemory()
+
+    def __setstate__(self, state):
+        # pickles of older versions may lack the version record: the state counts as touched
+        super(CBPoolMax2d, self).__setstate__(state)
+        self.__dict__.setdefault('_outVersion', None)
 
     def clearMemory(self):
         self.outputState = self.outputState.new_empty(0)
@@ -81,33 +93,34 @@ class CBPoolMax2d(nn.Module):
         self._scratch = None
 
     def getStateTensors(self):
-        return [self.outputState] if hasattr(self, 'outputState') else []
+        return [self.outputState]
 
     def _pooled_size(self, h, w):
         if self.ceil_mode:
             return (h - 1) // 2 + 1, (w - 1) // 2 + 1
         return h // 2, w // 2
 
+    def _stateAllocated(self, input_shape, dtype, device):
+        """outputState is the pixel-major pooled map the kernels own for an input of `input_shape`
+        (see CBConv2d._stateAllocated)."""
+        B, nc, h, w = input_shape
+        st = self.outputState
+        return self._stateBuf is not None and tuple(st.shape) == (B, nc) + self._pooled_size(h, w) \
+            and st.dtype == dtype and st.device == device and st.data_ptr() == self._stateBuf.data_ptr()
+
+    def _stateTouched(self):
+        """outputState written from outside the kernels since this pool last ran?"""
+        return self._outVersion != self.outputState._version
+
     def _fusedPoolTarget(self, input_shape, dtype, device):
         """What an upstream CBConv2d on the tile path needs to pool inside its own epilogue and run the
         next layer's detection there (cb_conv_update_tiled_pool), or None when this pool's state is
         not allocated yet / was touched from outside, or the next layer's candidate-detection
         conditions do not hold (then the ordinary path runs and sets everything up)."""
-        nxt = self._fusedNext[0] if getattr(self, '_fusedNext', None) else None
-        if nxt is None or self._stateBuf is None:
+        if not self._fusedNext or not self._stateAllocated(input_shape, dtype, device) or self._stateTouched():
             return None
-        B, nc, h, w = input_shape
-        oh, ow = self._pooled_size(h, w)
-        st = self.outputState
-        if list(st.shape) != [B, nc, oh, ow] or st.dtype != dtype or st.device != device \
-                or st.data_ptr() != self._stateBuf.data_ptr() \
-                or getattr(self, '_outVersion', None) != st._version:
-            return None
-        tgt = nxt._fusedDetectTarget(tuple(st.shape), dtype, device)
-        if tgt is None:
-            return None
-        return dict(out=st, next_state=tgt['state'], next_raw_bits=tgt['raw_bits'],
-                    threshold=tgt['threshold'], mode=tgt['mode'], aux=tgt['aux'])
+        tgt = self._fusedNext[0]._fusedDetectTarget(tuple(self.outputState.shape), dtype, device)
+        return None if tgt is None else dict(tgt, out=self.outputState)
 
     def forward(self, inp):
         assert(type(inp) == tuple and inp[0] == 'changeIndexes')
@@ -115,23 +128,25 @@ class CBPoolMax2d(nn.Module):
         changeIndexes = inp[2]
         assert input.dim() == 4
         _lib.require_cuda(input)
+        nxt = self._fusedNext[0] if self._fusedNext else None
         if getattr(changeIndexes, 'pooledBy', None) is self:
             # the producing CBConv2d already pooled its tiles and ran the next layer's detection
             # inside its epilogue (cb_conv_update_tiled_pool)
             changeIndexes.pooledBy = None
-            output = self.outputState.clone() if self.cloneOutput else self.outputState
-            return 'changeIndexes', output, DetectionDone(self._fusedNext[0])
+            handOn = DetectionDone(nxt)
+        else:
+            handOn = self._pool(input, changeIndexes, nxt)
+        output = self.outputState.clone() if self.cloneOutput else self.outputState
+        return output if handOn is None else ('changeIndexes', output, handOn)
+
+    def _pool(self, input, changeIndexes, nxt):
+        """Pool the touched windows; returns what the output tuple hands on, or None (plain output)."""
         B, nc, h, w = input.shape
+        oh, ow = self._pooled_size(h, w)
         if not isinstance(changeIndexes, ChangeIndexes):
             assert(changeIndexes.dim() == 1)
             changeIndexes = ChangeIndexes.from_tensor(changeIndexes, (B, h, w))
-        if self.ceil_mode:
-            oh, ow = (h - 1) // 2 + 1, (w - 1) // 2 + 1
-        else:
-            oh, ow = h // 2, w // 2
-        if list(self.outputState.shape) != [B, nc, oh, ow] or self.outputState.dtype != input.dtype \
-                or self.outputState.device != input.device or self._stateBuf is None \
-                or self.outputState.data_ptr() != self._stateBuf.data_ptr():
+        if not self._stateAllocated(input.shape, input.dtype, input.device):
             # deviation (stated): the reference allocates only once a non-empty index list arrives
             # (conv2d.py:53-62); deciding that needs a host sync, so the state is allocated up front.
             self.outputState, self._stateBuf = cg.pixel_major((B, nc, oh, ow), input.dtype,
@@ -139,23 +154,19 @@ class CBPoolMax2d(nn.Module):
             self._scratch = None
         # candidates handed downstream are complete only if neither the producer's output nor this
         # pool's state was written from outside the kernels (see CBConv2d.forward_normal)
-        complete = getattr(changeIndexes, 'complete', True) and \
-            getattr(self, '_outVersion', None) == self.outputState._version
+        complete = changeIndexes.complete and not self._stateTouched()
         self._outVersion = self.outputState._version
-        nxt = self._fusedNext[0] if getattr(self, '_fusedNext', None) else None
         tgt = None
         if nxt is not None and complete and changeIndexes.bits is not None and input.stride(1) == 1:
-            tgt = nxt._fusedDetectTarget(tuple(self.outputState.shape), input.dtype, input.device)
+            tgt = nxt._fusedDetectTarget((B, nc, oh, ow), input.dtype, input.device)
         if tgt is not None:
             # pooling + the next layer's detection in one kernel (cb_maxpool2x2_detect)
-            cg.maxPool2d_detect(input, self.outputState, changeIndexes, tgt['state'], tgt['raw_bits'],
+            cg.maxPool2d_detect(input, self.outputState, changeIndexes, tgt['next_state'], tgt['next_raw_bits'],
                                 tgt['threshold'], tgt['mode'], aux=tgt['aux'])
-            output = self.outputState.clone() if self.cloneOutput else self.outputState
-            return 'changeIndexes', output, DetectionDone(nxt)
+            nxt._recordDetection()
+            return DetectionDone(nxt)
         cg.maxPool2d(input, self.outputState, changeIndexes, self.kernel_size, self.stride)
-
-        output = self.outputState.clone() if self.cloneOutput else self.outputState
-        if getattr(self, 'propPooledIndexes', False) and changeIndexes.bits is not None:
+        if self.propPooledIndexes and changeIndexes.bits is not None:
             # extension (no reference counterpart): change candidates at the pooled resolution for
             # a downstream CBConv2d with candidateDetect=True
             if self._scratch is None:
@@ -165,12 +176,11 @@ class CBPoolMax2d(nn.Module):
                             out_bits=s["dil_bits"])
             pooled = ChangeIndexes(s["idx"], s["count"], (B, oh, ow), bits=s["dil_bits"])
             pooled.complete = complete
-            return 'changeIndexes', output, pooled
+            return pooled
         if self.propChangeIndexes:
             # reference behaviour: the *input-resolution* indices are forwarded (conv2d.py:75-76)
-            return 'changeIndexes', output, changeIndexes
-        else:
-            return output
+            return changeIndexes
+        return None
 
     def __repr__(self):
         s = ('{name} (k={kernel_size}, s={stride}, ceil_mode={ceil_mode}')
@@ -207,31 +217,49 @@ class CBConv2d(nn.Module):
         self.bias = m.bias
 
         self.threshold = threshold
+        self._setDefaultValues()
 
+        # neighbours whose work runs inside this layer's kernels (models.enableCandidateDetection):
+        # [CBPoolMax2d] pooled in the tile epilogue, [CBConv2d] whose frame cb_tail_update runs too
+        self._fusedPool = None
+        self._fusedTail = None
+        self._inVersion = None    # prevInput._version / prevOutput._version as the kernels last left them
+        self._outVersion = None
+        self._wsHolder = cg.ConvWorkspace()    # shared per model by pycbinfer.convert()
         self.register_buffer('prevInput', self.weight.data.new_empty(0))
         self.register_buffer('prevOutput', self.weight.data.new_empty(0))
         self.clearMemory()
 
-        self.withReLU = False
-        self.saveChangeMap = False
-        self.propChangeIndexes = False
-        self.gatherComputationStats = False
-        self.finegrained = False
-        self.copyInput = True
-        self.feedbackLoop = False
-        self.gemmMode = 'auto'
-        # extension: treat indices received from upstream as *candidates* for the thresholded
-        # detection instead of as the final change set (exact, see cb_change_detect_sparse)
-        self.candidateDetect = False
-        # extension: (divisor, bias) applied to uint8 input frames inside the detection kernel
-        self.inputNorm = None
-        # extension: 1x1 layer on the candidate path without any compaction (see forward_normal)
-        self.maskedConv = False
-        # extension: contraction over dirty 8x16 output tiles (TMA-staged halo, implicit im2col)
-        # instead of the per-pixel gather: 'auto' = where the library recommends it
-        # (cb_conv_tiled_supported == 1; CBINFER_TILES=0 disables), 'on' = wherever supported, 'off'
-        self.tileMode = 'auto'
-        self._wsHolder = cg.ConvWorkspace()    # shared per model by pycbinfer.convert()
+    def _setDefaultValues(self):
+        """The public flags and their defaults; sets those missing (pickles of older versions)."""
+        for name, val in (('withReLU', False), ('saveChangeMap', False), ('propChangeIndexes', False),
+                          ('gatherComputationStats', False), ('finegrained', False),
+                          ('copyInput', True), ('feedbackLoop', False), ('gemmMode', 'auto'),
+                          # extension: treat indices received from upstream as *candidates* for the
+                          # thresholded detection instead of as the final change set (exact, see
+                          # cb_change_detect_sparse)
+                          ('candidateDetect', False),
+                          # extension: (divisor, bias) applied to uint8 input frames inside the
+                          # detection kernel
+                          ('inputNorm', None),
+                          # extension: 1x1 layer on the candidate path without any compaction (see
+                          # forward_normal)
+                          ('maskedConv', False),
+                          # extension: contraction over dirty 8x16 output tiles (TMA-staged halo,
+                          # implicit im2col) instead of the per-pixel gather: 'auto' = where the
+                          # library recommends it (cb_conv_tiled_supported == 1; CBINFER_TILES=0
+                          # disables), 'on' = wherever supported, 'off'
+                          ('tileMode', 'auto')):
+            if not(hasattr(self, name)):
+                setattr(self, name, val)
+
+    def __setstate__(self, state):
+        # pickles of older versions lack what was added since: flags take their defaults, there are
+        # no fused neighbours, and without a version record the state counts as touched
+        super(CBConv2d, self).__setstate__(state)
+        self._setDefaultValues()
+        for name in ('_fusedPool', '_fusedTail', '_inVersion', '_outVersion'):
+            self.__dict__.setdefault(name, None)
 
     # ---- state ---------------------------------------------------------------------------
     def clearMemory(self):
@@ -247,65 +275,90 @@ class CBConv2d(nn.Module):
         self._lastThr = None
         self._lastChanges = None
         self.changeMap = None
-        if getattr(self, '_wsHolder', None) is not None:
-            self._wsHolder.clear()
-        if hasattr(self, 'compStats'):
-            self.compStats = None
+        self.compStats = None
+        self._wsHolder.clear()
 
     def getStateTensors(self):
-        state = []
-        if hasattr(self, 'prevInput'):
-            state += [self.prevInput]
-        if hasattr(self, 'prevOutput'):
-            state += [self.prevOutput]
-        return state
+        return [self.prevInput, self.prevOutput]
+
+    def _stateAllocated(self, shape, dtype, device):
+        """Rule 1, first half: are prevInput / prevOutput the state the kernels own for an input of
+        `shape`, allocated for it and still aliasing _inBuf / _outBuf?  (model.half() / .to() on a
+        warm model replace the registered buffers with tensors that do not.)  Else: reallocate."""
+        B, _, H, W = shape
+        for t, buf, want in ((self.prevInput, self._inBuf, tuple(shape)),
+                             (self.prevOutput, self._outBuf, (B, self.out_channels, H, W))):
+            if buf is None or tuple(t.shape) != want or t.dtype != dtype or t.device != device \
+                    or t.data_ptr() != buf.data_ptr():
+                return False
+        return True
+
+    def _stateTouched(self):
+        """Rule 1, second half: (prevInput, prevOutput) written from outside the kernels since this
+        layer last ran?  The reference's eval scripts snapshot and restore getStateTensors() with
+        copy_ (poseDetection/eval03.py:87-95): torch bumps the tensor version, the kernels do not."""
+        return self._inVersion != self.prevInput._version, self._outVersion != self.prevOutput._version
+
+    def _candidatesExact(self, shape, dtype, device):
+        """Rule 2: may this frame threshold only the candidate pixels (cb_change_detect_sparse)?  Exact
+        while the state is the kernels' own, untouched, not fresh, and the threshold not lowered:
+        every other pixel then still lies within the threshold of the state."""
+        return self.candidateDetect and not self.finegrained and not self._fresh \
+            and self._lastThr is not None and self.threshold >= self._lastThr \
+            and self._stateAllocated(shape, dtype, device) and not any(self._stateTouched())
+
+    def _recordDetection(self):
+        """This layer's detection ran with its threshold (here or inside an upstream kernel)."""
+        self._fresh = False
+        self._lastThr = self.threshold
+        self._inVersion = self.prevInput._version
+
+    def _frameDone(self, changes, handOn):
+        """Record the versions the kernels left and the frame's change list; return the output."""
+        self._inVersion = self.prevInput._version
+        self._outVersion = self.prevOutput._version
+        self._lastChanges = changes
+        if handOn is None:
+            return self.prevOutput
+        return 'changeIndexes', self.prevOutput, handOn
 
     def _gemm(self, dtype):
-        mode = getattr(self, 'gemmMode', 'auto')
-        if mode == 'auto':
+        if self.gemmMode == 'auto':
             return _lib.GEMM_TC_BF16X3 if dtype == torch.float32 else _lib.GEMM_TC
-        g = self.GEMM_MODES[mode]
+        g = self.GEMM_MODES[self.gemmMode]
         if g in (_lib.GEMM_TC_3X, _lib.GEMM_TC_BF16X3) and dtype != torch.float32:
             g = _lib.GEMM_TC
         return g
 
     def _aux(self, gemm):
-        """Auxiliary operand planes of prevInput for the 3x modes (kept in step by the detection
-        kernel); (re)built from prevInput when the mode changes or after a plain copy."""
+        """Auxiliary operand planes of prevInput for the 3x modes, in the ops' `aux` format (kept in
+        step by the detection kernel); (re)built from prevInput when the mode changes or after a
+        plain copy."""
         want = {_lib.GEMM_TC_3X: 'tf32', _lib.GEMM_TC_BF16X3: 'bf16'}.get(gemm) \
             if self.prevInput.dtype == torch.float32 else None
         if want is None:
             self._auxPlanes = None
         elif self._auxPlanes is None or self._auxPlanes[0] != want:
             if want == 'tf32':
-                view, buf = cg.pixel_major(self.prevInput.shape, torch.float32, self.prevInput.device, 0)
+                lo, _ = cg.pixel_major(self.prevInput.shape, torch.float32, self.prevInput.device, 0)
                 fin = torch.isfinite(self.prevInput)
-                view.copy_(torch.where(fin, cg.tf32_lo(torch.where(fin, self.prevInput, 0)), 0))
-                self._auxPlanes = ('tf32', view, buf)
+                lo.copy_(torch.where(fin, cg.tf32_lo(torch.where(fin, self.prevInput, 0)), 0))
+                self._auxPlanes = ('tf32', lo)
             else:
-                hi, lo = cg.bf16_planes(torch.nan_to_num(self._inBuf, posinf=0.0, neginf=0.0),
-                                        self.in_channels)
-                self._auxPlanes = ('bf16', hi, lo)
+                self._auxPlanes = ('bf16',) + cg.bf16_planes(
+                    torch.nan_to_num(self._inBuf, posinf=0.0, neginf=0.0), self.in_channels)
         return self._auxPlanes
 
     def _fusedDetectTarget(self, shape, dtype, device):
         """What an upstream CBPoolMax2d needs to run this layer's detection inside its own kernel,
-        or None when the exactness conditions of candidate detection do not hold (fresh state,
-        lowered threshold, different shape) or the layer is not on the candidate path."""
-        if not getattr(self, 'candidateDetect', False) or self.finegrained or self._fresh \
-                or self._inBuf is None or tuple(self.prevInput.shape) != tuple(shape) \
-                or self.prevInput.dtype != dtype or self._lastThr is None \
-                or getattr(self, '_inVersion', None) != self.prevInput._version \
-                or self.threshold < self._lastThr or self._scratch is None \
-                or not self._scratch.get("raw_clear", False):
+        or None when candidate detection is not exact for this layer this frame."""
+        if not self._candidatesExact(shape, dtype, device) or not self._scratch.get("raw_clear", False):
             return None
         gemm, _, _ = self._weights(dtype, device)
-        aux = self._aux(gemm)
-        self._lastThr = self.threshold
-        return dict(state=self.prevInput, raw_bits=self._scratch["raw_bits"],
+        return dict(next_state=self.prevInput, next_raw_bits=self._scratch["raw_bits"],
                     threshold=self.threshold,
                     mode=_lib.UPDATE_CHANGED if self.feedbackLoop else _lib.UPDATE_ALL,
-                    aux=None if aux is None else (aux[:2] if aux[0] == 'tf32' else aux))
+                    aux=self._aux(gemm))
 
     def _weights(self, dtype, device):
         gemm = self._gemm(dtype)
@@ -329,7 +382,7 @@ class CBConv2d(nn.Module):
         _lib.require_cuda(input)
         if input.dtype != torch.float32:
             raise _lib.CBinferError("the fine-grained path is fp32 only (as in the reference)")
-        if getattr(self, 'gemmMode', 'auto') == 'simt':
+        if self.gemmMode == 'simt':
             return self._forward_fg_planar(input.contiguous())
         B, _, H, W = input.shape
         dev = input.device
@@ -339,11 +392,8 @@ class CBConv2d(nn.Module):
         if self._packed is None or self._packed[0] != key:
             self._packed = (key, cg.pack_weights(self.weight.detach().to(device=dev, dtype=torch.float32), gemm),
                             None)
-        fresh = self.prevInput.size() != input.size() or self._inBuf is None or self._outBuf is None \
-            or self.prevInput.device != dev or self.prevInput.data_ptr() != self._inBuf.data_ptr() \
-            or tuple(self.prevOutput.size()) != outpSize or self.prevOutput.data_ptr() != self._outBuf.data_ptr() \
-            or self._auxPlanes is None or self._auxPlanes[0] != 'fg'
-        if fresh:
+        if not self._stateAllocated(input.shape, torch.float32, dev) \
+                or self._auxPlanes is None or self._auxPlanes[0] != 'fg':
             self.prevOutput, self._outBuf = cg.pixel_major(outpSize, torch.float32, dev, 0)
             self.prevOutput.copy_(F.conv2d(input, self.weight.detach(),
                                            padding=tuple(s // 2 for s in self.weight.size()[2:]),
@@ -351,20 +401,21 @@ class CBConv2d(nn.Module):
             self.prevInput, self._inBuf = cg.pixel_major(input.shape, torch.float32, dev, 0)
             self.prevInput.copy_(input)
             p16 = _lib.C.cb_plane_pitch16(self.in_channels)
-            self._auxPlanes = ('fg', torch.zeros(B, H, W, p16, dtype=torch.bfloat16, device=dev),
-                               torch.zeros(B, H, W, p16, dtype=torch.bfloat16, device=dev))
+            # the thresholded delta planes (hi, lo) of the last frame
+            self._auxPlanes = ('fg', (torch.zeros(B, H, W, p16, dtype=torch.bfloat16, device=dev),
+                                      torch.zeros(B, H, W, p16, dtype=torch.bfloat16, device=dev)))
             self._scratch = cg.alloc_scratch((B, H, W), dev)
             self._scratch["nvalues"] = torch.zeros(1, dtype=torch.int32, device=dev)
         else:
             s = self._scratch
-            planes = self._auxPlanes[1:]
+            _, planes = self._auxPlanes
             cg.fg_detect(input, self.prevInput, self._inBuf, planes, s["raw_bits"], self.threshold,
                          count=s["nvalues"])
             cg.dilate_compact(s["raw_bits"], (B, H, W), self.kernel_size, s["idx"], s["count"], s["ws"],
                               dil_bits=s["dil_bits"])
             changes = ChangeIndexes(s["idx"], s["count"], (B, H, W), bits=s["dil_bits"])
             cg.conv_accumulate(planes, changes, self._packed[1], self._outBuf, self.in_channels,
-                               self.out_channels, self.kernel_size, gemm, ws=self._workspace(dev))
+                               self.out_channels, self.kernel_size, gemm, ws=self._wsHolder.get(dev))
             self._lastChanges = changes
         # the reference updates a clone (:169), so outputs handed out earlier stay as they were
         return F.relu(self.prevOutput) if self.withReLU else self.prevOutput.clone()
@@ -394,8 +445,7 @@ class CBConv2d(nn.Module):
         assert(input.size(-3) == self.in_channels)
         # a layer fed with plain frames re-scans them densely every frame, which rewrites every word of
         # its raw bitmap: nothing ever ORs bits into it, so its compaction need not zero it afterwards
-        plain_input = changeIndexes is None or (isinstance(changeIndexes, DetectionDone)
-                                                and getattr(changeIndexes, 'dense', False))
+        plain_input = changeIndexes is None or (isinstance(changeIndexes, DetectionDone) and changeIndexes.dense)
         _lib.require_cuda(input)
         B, _, H, W = input.shape
         dev, dt = input.device, input.dtype
@@ -403,7 +453,7 @@ class CBConv2d(nn.Module):
         # value = u8 / divisor + bias with inputNorm = (divisor, bias); the layer computes in fp32
         u8norm = None
         if dt == torch.uint8:
-            u8norm = getattr(self, 'inputNorm', None)
+            u8norm = self.inputNorm
             if u8norm is None:
                 raise _lib.CBinferError("uint8 input needs CBConv2d.inputNorm = (divisor, bias), e.g. "
                                         "(255.0, 0.0) for the scene reader's frame/255")
@@ -413,31 +463,19 @@ class CBConv2d(nn.Module):
                 u8norm = None
             dt = torch.float32
 
-        # (model.half() / .to(device) on a warm model replace the registered buffers with fresh
-        #  tensors that no longer alias the pixel-major storage: treat that as a reset)
-        outpSize = (B, self.out_channels, H, W)
-        need_out = tuple(self.prevOutput.size()) != outpSize or self.prevOutput.dtype != dt \
-            or self._outBuf is None or self.prevOutput.device != dev \
-            or self.prevOutput.data_ptr() != self._outBuf.data_ptr()
-        need_in = need_out or self.prevInput.size() != input.size() or self.prevInput.dtype != dt \
-            or self._inBuf is None or self.prevInput.device != dev \
-            or self.prevInput.data_ptr() != self._inBuf.data_ptr()
-        if need_in:       # (a fresh output map needs every pixel recomputed: the input state goes too)
-            self.prevInput, self._inBuf = cg.pixel_major(input.shape, dt, dev, _INF)   # :192-194
+        if not self._stateAllocated(input.shape, dt, dev):
+            # a fresh output map needs every pixel recomputed: the input state goes too
+            self.prevInput, self._inBuf = cg.pixel_major(input.shape, dt, dev, _INF)                 # :192-194
+            self.prevOutput, self._outBuf = cg.pixel_major((B, self.out_channels, H, W), dt, dev, _INF)  # :195-199
             self._auxPlanes = None
             self._scratch = None
             self._fresh = True
-        if need_out:
-            self.prevOutput, self._outBuf = cg.pixel_major(outpSize, dt, dev, _INF)    # :195-199
-        # State tensors written from outside this module's kernels (the reference's eval scripts
-        # snapshot and restore getStateTensors() with copy_, poseDetection/eval03.py:87-95): torch
-        # bumps the tensor version, our kernels do not.  A touched prevInput is treated as fresh
-        # (dense scan, operand planes rebuilt); a touched prevOutput makes this frame's index list
-        # an incomplete candidate set for the next layer.
-        if getattr(self, '_inVersion', None) != self.prevInput._version:
+        # a touched prevInput is treated as fresh (dense scan, operand planes rebuilt); a touched
+        # prevOutput makes this frame's index list an incomplete candidate set for the next layer
+        in_touched, ext_out = self._stateTouched()
+        if in_touched:
             self._fresh = True
             self._auxPlanes = None
-        ext_out = getattr(self, '_outVersion', None) != self.prevOutput._version
         if self._scratch is None:
             self._scratch = cg.alloc_scratch((B, H, W), dev, want_map=self.saveChangeMap)
         if self.saveChangeMap and "dil_map" not in self._scratch:
@@ -451,93 +489,48 @@ class CBConv2d(nn.Module):
         if isinstance(changeIndexes, TailDone):
             # the upstream 1x1 layer's kernel already did this layer's frame (cb_tail_update)
             assert changeIndexes.owner is self
-            self._lastChanges = changeIndexes.candidates
-            self._inVersion = self.prevInput._version
-            self._outVersion = self.prevOutput._version
-            if self.propChangeIndexes:
-                return 'changeIndexes', self.prevOutput, changeIndexes.candidates
-            return self.prevOutput
-        tail = self._tryTail(input, changeIndexes, gemm, packed, bias32, s, outpSize, ext_out)
+            cand = changeIndexes.candidates
+            return self._frameDone(cand, cand if self.propChangeIndexes else None)
+        tail = self._tryTail(input, changeIndexes, gemm, packed, bias32)
         if tail is not None:
             return tail
         aux = self._aux(gemm)
-        aux_arg = None if aux is None else (aux[:2] if aux[0] == 'tf32' else aux)
 
-        candidates = None
-        mask = None
-        tiled = False             # this frame's contraction walks the dirty-tile list
         use_tiles = self._useTiles(dt, gemm, (B, H, W))
         # a directly following CBPoolMax2d (+ the detection of the layer after it) rides along in the
         # tile kernel's epilogue when everything is warmed up (cb_conv_update_tiled_pool); nobody
         # then needs this layer's ordered index list, so it is only compacted on demand
         pool_args = None
-        fp = getattr(self, '_fusedPool', None)
-        if use_tiles and fp and self.propChangeIndexes and not ext_out \
+        if use_tiles and self._fusedPool and self.propChangeIndexes and not ext_out \
                 and os.environ.get("CBINFER_FUSE_POOL", "1") != "0" \
                 and _lib.C.cb_conv_tiled_pool_supported(_lib.dtype_code(dt), gemm, self.out_channels):
-            pool_args = fp[0]._fusedPoolTarget(outpSize, dt, dev)
+            pool_args = self._fusedPool[0]._fusedPoolTarget((B, self.out_channels, H, W), dt, dev)
         detected = isinstance(changeIndexes, DetectionDone)
         if detected:
             assert changeIndexes.owner is self
             changeIndexes = None
-        if changeIndexes is not None and getattr(self, 'candidateDetect', False):
+        candidates = None
+        if changeIndexes is not None and self.candidateDetect:
             candidates, changeIndexes = changeIndexes, None
             if not isinstance(candidates, ChangeIndexes):
                 candidates = ChangeIndexes.from_tensor(candidates.detach(), (B, H, W))
-            if self._fresh or self._lastThr is None or self.threshold < self._lastThr \
-                    or tuple(candidates.shape) != (B, H, W) or not getattr(candidates, 'complete', True):
-                candidates = None          # exactness conditions not met: full scan
+            if tuple(candidates.shape) != (B, H, W) or not candidates.complete \
+                    or not self._candidatesExact(input.shape, dt, dev):
+                candidates = None          # not exact: full scan
 
+        mask = None
+        tiled = False             # this frame's contraction walks the dirty-tile list
         if changeIndexes is None:
             # reference: detect (feedback updates prevInput at changed pixels, :222-224), nonzero
             # (:232), then prevInput.copy_(input) when not in feedback mode (:234-238).  Here the
             # copy is part of the detection pass; copyInput=False (alias the input as state) is
             # honoured as a copy -- the state always owns its memory.
             mode = _lib.UPDATE_CHANGED if self.feedbackLoop else _lib.UPDATE_ALL
-            sparse_next = bool(getattr(self, 'candidateDetect', False)) and not plain_input
-            # extension: no compaction at all for a 1x1 layer on the candidate path - the
-            # contraction walks the candidate list and skips pixels whose raw bit is not set
-            # (cb_conv_update_masked); this layer's own index list is then never materialised
-            masked = (candidates is not None and not detected and tuple(self.kernel_size) == (1, 1)
-                      and getattr(self, 'maskedConv', False)
-                      and not self.saveChangeMap and gemm != _lib.GEMM_SIMT_F32)
-            fusedSmall = False
-            if detected:
-                pass                     # the upstream pool kernel already did it
-            elif candidates is not None and not masked and not use_tiles and not self.saveChangeMap \
-                    and input.stride(1) == 1 and self._smallMap(B, H, W):
-                # small map: candidate detection + dilation + ordered compaction in ONE launch (the
-                # last block of the detection kernel compacts), cb_change_detect_sparse_compact
-                if "sdc_sync" not in s:
-                    s["sdc_sync"] = torch.zeros(1, dtype=torch.int32, device=dev)
-                cg.detect_sparse_compact(input, self.prevInput, s["raw_bits"], self.threshold, mode, candidates,
-                                         self.kernel_size, s["idx"], s["count"], s["sdc_sync"], aux=aux_arg,
-                                         bits_are_clear=s.get("raw_clear", False), dil_bits=s["dil_bits"],
-                                         clear_raw=sparse_next)
-                fusedSmall = True
-            elif candidates is not None:
-                cg.detect_sparse(input, self.prevInput, s["raw_bits"], self.threshold, mode,
-                                 candidates, aux=aux_arg,
-                                 bits_are_clear=s.get("raw_clear", False))
-                if masked:
-                    if "mask_sync" not in s:
-                        s["mask_sync"] = torch.zeros(2, dtype=torch.int32, device=dev)
-                    mask = dict(bits=s["raw_bits"], clear=True, count=s["count"], sync=s["mask_sync"])
-            elif u8norm is not None:
-                cg.detect_u8(input, self.prevInput, s["raw_bits"], self.threshold, mode,
-                             u8norm[0], u8norm[1], aux=aux_arg)
-            else:
-                cg.detect(input, self.prevInput, s["raw_bits"], self.threshold, mode, aux=aux_arg)
-            self._fresh = False
-            self._lastThr = self.threshold
-            if fusedSmall:
-                s["raw_clear"] = sparse_next
-                changeIndexes = ChangeIndexes(s["idx"], s["count"], (B, H, W), bits=s["dil_bits"])
-            elif mask is not None:
-                s["raw_clear"] = True                # the masked contraction clears the bitmap
-                changeIndexes = ChangeIndexes(candidates.buffer, candidates.count, (B, H, W), bits=None)
-                changeIndexes.superset = True
-            else:
+            sparse_next = self.candidateDetect and not plain_input
+            if not detected:     # (else the upstream pool kernel already did it)
+                changeIndexes, mask = self._detect(input, candidates, u8norm, mode, aux, gemm, use_tiles,
+                                                   sparse_next)
+            if changeIndexes is None:
                 changeIndexes = self._compact(s, B, H, W, sparse_next, tiles=use_tiles,
                                               lazy=pool_args is not None and not self.saveChangeMap)
                 tiled = use_tiles
@@ -556,68 +549,90 @@ class CBConv2d(nn.Module):
                 aux = self._aux(gemm)
             # (with feedbackLoop the reference never refreshes prevInput here either, :220,234)
 
-        lo_buf = aux[2] if aux is not None and aux[0] == 'tf32' else None
-        planes16 = aux[1:] if aux is not None and aux[0] == 'bf16' else None
         if tiled:
             # spatially clustered change sets: contraction over the dirty 8x16 tiles (TMA-staged
             # halo, implicit im2col through the UMMA descriptors), rows masked by the dilated bitmap
             cg.conv_update_tiled(self._inBuf, s["tile_ws"], s["dil_bits"], packed, bias32, self._outBuf,
                                  self.in_channels, self.out_channels, self.kernel_size, self.withReLU,
-                                 gemm, lo_buf=lo_buf, planes16=planes16, pool=pool_args)  # :242-251
+                                 gemm, aux=aux, pool=pool_args)                             # :242-251
             if pool_args is not None:
-                changeIndexes.pooledBy = fp[0]
+                changeIndexes.pooledBy = self._fusedPool[0]
+                self._fusedPool[0]._fusedNext[0]._recordDetection()
         else:
             cg.conv_update(self._inBuf, changeIndexes, packed, bias32, self._outBuf, self.in_channels,
                            self.out_channels, self.kernel_size, self.withReLU, gemm,
-                           lo_buf=lo_buf, planes16=planes16,
-                           ws=self._workspace(dev), mask=mask)                         # :242-251
-        self._inVersion = self.prevInput._version
-        self._outVersion = self.prevOutput._version
-        self._lastChanges = changeIndexes
-        if ext_out and isinstance(changeIndexes, ChangeIndexes):
-            changeIndexes.complete = False
-        elif isinstance(changeIndexes, ChangeIndexes):
-            changeIndexes.complete = True
+                           aux=aux, ws=self._wsHolder.get(dev), mask=mask)                 # :242-251
+        if isinstance(changeIndexes, ChangeIndexes):
+            changeIndexes.complete = not ext_out
+        return self._frameDone(changeIndexes, changeIndexes if self.propChangeIndexes else None)
 
-        if self.propChangeIndexes:
-            return 'changeIndexes', self.prevOutput, changeIndexes
+    def _detect(self, input, candidates, u8norm, mode, aux, gemm, use_tiles, sparse_next):
+        """Dense scan, or the test of the `candidates` only.  Returns (change list if the launch
+        built one, mask of the masked contraction), each or both None."""
+        B, _, H, W = input.shape
+        s = self._scratch
+        # extension: no compaction at all for a 1x1 layer on the candidate path - the
+        # contraction walks the candidate list and skips pixels whose raw bit is not set
+        # (cb_conv_update_masked); this layer's own index list is then never materialised
+        masked = (candidates is not None and tuple(self.kernel_size) == (1, 1) and self.maskedConv
+                  and not self.saveChangeMap and gemm != _lib.GEMM_SIMT_F32)
+        changes = mask = None
+        if candidates is not None and not masked and not use_tiles and not self.saveChangeMap \
+                and input.stride(1) == 1 and self._smallMap(B, H, W):
+            # small map: candidate detection + dilation + ordered compaction in ONE launch (the
+            # last block of the detection kernel compacts), cb_change_detect_sparse_compact
+            if "sdc_sync" not in s:
+                s["sdc_sync"] = torch.zeros(1, dtype=torch.int32, device=input.device)
+            cg.detect_sparse_compact(input, self.prevInput, s["raw_bits"], self.threshold, mode, candidates,
+                                     self.kernel_size, s["idx"], s["count"], s["sdc_sync"], aux=aux,
+                                     bits_are_clear=s.get("raw_clear", False), dil_bits=s["dil_bits"],
+                                     clear_raw=sparse_next)
+            s["raw_clear"] = sparse_next
+            changes = ChangeIndexes(s["idx"], s["count"], (B, H, W), bits=s["dil_bits"])
+        elif candidates is not None:
+            cg.detect_sparse(input, self.prevInput, s["raw_bits"], self.threshold, mode,
+                             candidates, aux=aux,
+                             bits_are_clear=s.get("raw_clear", False))
+            if masked:
+                if "mask_sync" not in s:
+                    s["mask_sync"] = torch.zeros(2, dtype=torch.int32, device=input.device)
+                mask = dict(bits=s["raw_bits"], clear=True, count=s["count"], sync=s["mask_sync"])
+                s["raw_clear"] = True                # the masked contraction clears the bitmap
+                changes = ChangeIndexes(candidates.buffer, candidates.count, (B, H, W), bits=None)
+                changes.superset = True
+        elif u8norm is not None:
+            cg.detect_u8(input, self.prevInput, s["raw_bits"], self.threshold, mode,
+                         u8norm[0], u8norm[1], aux=aux)
         else:
-            return self.prevOutput
+            cg.detect(input, self.prevInput, s["raw_bits"], self.threshold, mode, aux=aux)
+        self._recordDetection()
+        return changes, mask
 
     # ---- two chained 1x1 layers in one launch (extension) ------------------------------------------
+    def _tailReady(self, shape, dtype, device):
+        """May this masked 1x1 layer's frame run inside cb_tail_update?"""
+        return self.maskedConv and tuple(self.kernel_size) == (1, 1) and not self.saveChangeMap \
+            and not self.gatherComputationStats and self._candidatesExact(shape, dtype, device) \
+            and self._scratch.get("raw_clear", False)
+
     def _tailTarget(self, shape, dt, dev, feedback):
         """What the 1x1 layer feeding this one needs to run this layer's frame inside its own kernel
-        (cb_tail_update), or None while the exactness conditions of candidate detection do not hold
-        for this layer (fresh state, lowered threshold, state touched from outside, ...)."""
-        if not (getattr(self, 'candidateDetect', False) and getattr(self, 'maskedConv', False)) \
-                or self.finegrained or self.saveChangeMap or self.gatherComputationStats \
-                or tuple(self.kernel_size) != (1, 1) or self.feedbackLoop != feedback \
-                or self._fresh or self._inBuf is None or self._outBuf is None or self._scratch is None \
-                or tuple(self.prevInput.shape) != tuple(shape) or self.prevInput.dtype != dt \
-                or self.prevInput.device != dev or self._lastThr is None or self.threshold < self._lastThr \
-                or getattr(self, '_inVersion', None) != self.prevInput._version \
-                or getattr(self, '_outVersion', None) != self.prevOutput._version \
-                or self.prevInput.data_ptr() != self._inBuf.data_ptr() \
-                or self.prevOutput.data_ptr() != self._outBuf.data_ptr() \
-                or not self._scratch.get("raw_clear", False):
+        (cb_tail_update), or None when that does not apply to this layer this frame."""
+        if self.feedbackLoop != feedback or not self._tailReady(shape, dt, dev):
             return None
         gemm, packed, bias32 = self._weights(dt, dev)
         return dict(gemm=gemm, packed=packed, bias=bias32, state=self._inBuf, out=self._outBuf,
                     thr=self.threshold, relu=self.withReLU, count=self._scratch["count"])
 
-    def _tryTail(self, input, changeIndexes, gemm, packed, bias32, s, outpSize, ext_out):
-        ft = getattr(self, '_fusedTail', None)
-        if not ft or os.environ.get("CBINFER_FUSE_TAIL", "1") == "0":
+    def _tryTail(self, input, changeIndexes, gemm, packed, bias32):
+        if not self._fusedTail or os.environ.get("CBINFER_FUSE_TAIL", "1") == "0" \
+                or not isinstance(changeIndexes, ChangeIndexes) or input.dtype != torch.float32:
             return None
         B, C0, H, W = input.shape
-        if not isinstance(changeIndexes, ChangeIndexes) or not getattr(self, 'candidateDetect', False) \
-                or not getattr(self, 'maskedConv', False) or tuple(self.kernel_size) != (1, 1) \
-                or self.saveChangeMap or self.gatherComputationStats or ext_out or input.dtype != torch.float32 \
-                or self._fresh or self._lastThr is None or self.threshold < self._lastThr \
-                or tuple(changeIndexes.shape) != (B, H, W) or not getattr(changeIndexes, 'complete', True) \
-                or not s.get("raw_clear", False):
+        if tuple(changeIndexes.shape) != (B, H, W) or not changeIndexes.complete \
+                or not self._tailReady(input.shape, input.dtype, input.device):
             return None
-        nxt = ft[0]
+        nxt = self._fusedTail[0]
         C1, C2 = self.out_channels, nxt.out_channels
         if not _lib.C.cb_tail_supported(_lib.dtype_code(input.dtype), gemm, C0, C1, C2):
             return None
@@ -625,9 +640,10 @@ class CBConv2d(nn.Module):
         if input.stride() != (H * W * C0, 1, W * C0, C0) or self._inBuf.shape[3] != C0 \
                 or self._outBuf.shape[3] != C1:
             return None
-        tgt = nxt._tailTarget(outpSize, input.dtype, input.device, self.feedbackLoop)
+        tgt = nxt._tailTarget((B, C1, H, W), input.dtype, input.device, self.feedbackLoop)
         if tgt is None or tgt['gemm'] != gemm:
             return None
+        s = self._scratch
         if "tail_sync" not in s:
             s["tail_sync"] = torch.zeros(4, dtype=torch.int32, device=input.device)
         x_buf = input.permute(0, 2, 3, 1)
@@ -639,32 +655,21 @@ class CBConv2d(nn.Module):
         # the kernel splits its operands on the fly: the layers' operand planes are stale now
         self._auxPlanes = None
         nxt._auxPlanes = None
-        self._lastThr = self.threshold
-        nxt._lastThr = nxt.threshold
-        self._inVersion = self.prevInput._version
-        self._outVersion = self.prevOutput._version
+        self._recordDetection()
+        nxt._recordDetection()
         sup = ChangeIndexes(changeIndexes._buffer, changeIndexes.count, (B, H, W), bits=changeIndexes.bits,
                             ws=changeIndexes._ws, listed=changeIndexes.listed)
         sup.superset = True
-        self._lastChanges = sup
-        return 'changeIndexes', self.prevOutput, TailDone(nxt, sup)
+        return self._frameDone(sup, TailDone(nxt, sup))
 
     def lastChangeIndexes(self):
         """This frame's change indexes as an int32 tensor (ascending b*H*W + y*W + x): what the
         reference hands on as ``changeIndexes`` (conv2d.py:256-257).  The list of a layer on the
         tile path is compacted only now, on demand."""
-        ci = getattr(self, '_lastChanges', None)
+        ci = self._lastChanges
         if ci is None:
             raise _lib.CBinferError("no frame processed yet")
         return ci.tensor() if isinstance(ci, ChangeIndexes) else ci
-
-    def _workspace_holder(self):
-        if getattr(self, '_wsHolder', None) is None:
-            self._wsHolder = cg.ConvWorkspace()
-        return self._wsHolder
-
-    def _workspace(self, dev):
-        return self._workspace_holder().get(dev)
 
     def detectInput(self, input):
         """Run only this layer's (dense) change detection on `input` and return the tuple that makes
@@ -674,29 +679,24 @@ class CBConv2d(nn.Module):
         tensor.  Needs a warmed-up layer (state allocated by an ordinary forward of this shape)."""
         input = input.detach()
         _lib.require_cuda(input)
-        B, _, H, W = input.shape
         dt = torch.float32 if input.dtype == torch.uint8 else input.dtype
-        if self._inBuf is None or self._scratch is None or self.prevInput.size() != input.size() \
-                or self.prevInput.dtype != dt or self.finegrained or self.gatherComputationStats:
+        if self.finegrained or self.gatherComputationStats \
+                or not self._stateAllocated(input.shape, dt, input.device):
             raise _lib.CBinferError("detectInput: run one ordinary forward of this input shape first")
-        if getattr(self, '_inVersion', None) != self.prevInput._version:
-            self._fresh = True
-            self._auxPlanes = None
+        if self._stateTouched()[0]:
+            self._auxPlanes = None       # rebuilt from the touched state; the scan below is dense anyway
         gemm, _, _ = self._weights(dt, input.device)
         aux = self._aux(gemm)
-        aux_arg = None if aux is None else (aux[:2] if aux[0] == 'tf32' else aux)
         mode = _lib.UPDATE_CHANGED if self.feedbackLoop else _lib.UPDATE_ALL
         if input.dtype == torch.uint8:
-            norm = getattr(self, 'inputNorm', None)
+            norm = self.inputNorm
             if norm is None or self.in_channels > 4:
                 raise _lib.CBinferError("detectInput: uint8 input needs inputNorm and <= 4 channels")
             cg.detect_u8(input, self.prevInput, self._scratch["raw_bits"], self.threshold, mode,
-                         norm[0], norm[1], aux=aux_arg)
+                         norm[0], norm[1], aux=aux)
         else:
-            cg.detect(input, self.prevInput, self._scratch["raw_bits"], self.threshold, mode, aux=aux_arg)
-        self._fresh = False
-        self._lastThr = self.threshold
-        self._inVersion = self.prevInput._version
+            cg.detect(input, self.prevInput, self._scratch["raw_bits"], self.threshold, mode, aux=aux)
+        self._recordDetection()
         return 'changeIndexes', input, DetectionDone(self, dense=True)
 
     def _smallMap(self, B, H, W):
@@ -705,15 +705,10 @@ class CBConv2d(nn.Module):
 
     def _useTiles(self, dt, gemm, shape):
         """tile path for this layer / shape?  (tileMode 'auto': where the library recommends it)"""
-        mode = getattr(self, 'tileMode', 'auto')
-        if mode == 'off' or os.environ.get("CBINFER_TILES", "1") == "0" or gemm == _lib.GEMM_SIMT_F32:
+        if self.tileMode == 'off' or os.environ.get("CBINFER_TILES", "1") == "0" or gemm == _lib.GEMM_SIMT_F32:
             return False
-        key = (dt, gemm, tuple(shape), mode)
-        cache = self.__dict__.setdefault('_tileOk', {})
-        if key not in cache:
-            sup = cg.tiled_supported(dt, gemm, shape, self.in_channels, self.out_channels, self.kernel_size)
-            cache[key] = sup >= 1 if mode == 'on' else sup == 1
-        return cache[key]
+        return _tiles_ok(dt, gemm, tuple(shape), self.in_channels, self.out_channels, tuple(self.kernel_size),
+                         self.tileMode)
 
     def _selfTiles(self, B, H, W):
         """Always False: no kernel lists its own tiles.  bench.py reads it to count launches."""
@@ -757,7 +752,6 @@ class CBConv2d(nn.Module):
         )
 
     def forward(self, inp):
-        self._setDefaultValues()
         with torch.no_grad():
             if self.finegrained:
                 assert(self.feedbackLoop == False)
@@ -766,7 +760,6 @@ class CBConv2d(nn.Module):
                 return self.forward_normal(inp)
 
     def __repr__(self):
-        self._setDefaultValues()
         s = ('{name} (th={threshold}, {in_channels}->{out_channels}, k={kernel_size}'
              ', s={stride}, copyInput={copyInput}')
         if self.padding != (0,) * len(self.padding):
@@ -784,12 +777,3 @@ class CBConv2d(nn.Module):
         s += ', propChgIdxs={propChangeIndexes}'
         s += ')'
         return s.format(name=self.__class__.__name__, **self.__dict__)
-
-    def _setDefaultValues(self):
-        for name, val in (('saveChangeMap', False), ('propChangeIndexes', False),
-                          ('gatherComputationStats', False), ('finegrained', False),
-                          ('copyInput', True), ('feedbackLoop', False), ('gemmMode', 'auto'),
-                          ('candidateDetect', False), ('inputNorm', None),
-                          ('maskedConv', False), ('tileMode', 'auto')):
-            if not(hasattr(self, name)):
-                setattr(self, name, val)

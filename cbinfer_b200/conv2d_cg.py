@@ -318,22 +318,29 @@ class ConvWorkspace(object):
         self.buf = None
 
 
-def conv_update(state_buf, changes, packed_w, bias_f32, out_buf, Cin, Cout, filtSize, relu, gemm,
-                lo_buf=None, planes16=None, ws=None, mask=None):
-    """cb_conv_update on pixel-major buffers [B,H,W,pitch].  GEMM_TC_3X (fp32) consumes the tf32
-    remainder plane `lo_buf`, GEMM_TC_BF16X3 the bf16 hi/lo planes `planes16`; both are derived
-    on the fly when the caller does not maintain them (cb_change_detect can)."""
-    B, H, W, Cp = state_buf.shape
-    assert out_buf.shape[:3] == state_buf.shape[:3]
-    src, src_lo, pitch = state_buf, lo_buf, Cp
+def _conv_operands(state_buf, Cin, gemm, aux):
+    """(source, remainder plane or None, pitch) the contraction reads: the bf16 hi/lo planes for
+    GEMM_TC_BF16X3, else the state with, for GEMM_TC_3X on fp32 data, its tf32 remainder plane.
+    `aux` holds the planes in the format of :func:`_aux_args`; without it they are derived from
+    the state on the fly."""
     if gemm == _lib.GEMM_TC_BF16X3:
         assert state_buf.dtype == torch.float32
-        if planes16 is None:
-            planes16 = bf16_planes(state_buf, Cin)
-        src, src_lo = planes16
-        pitch = src.shape[3]
-    elif gemm == _lib.GEMM_TC_3X and state_buf.dtype == torch.float32 and lo_buf is None:
-        src_lo = tf32_lo(state_buf)
+        _, hi, lo = aux if aux is not None else ('bf16',) + bf16_planes(state_buf, Cin)
+        return hi, lo, hi.shape[3]
+    lo = None
+    if gemm == _lib.GEMM_TC_3X and state_buf.dtype == torch.float32:
+        lo = aux[1] if aux is not None else tf32_lo(state_buf)
+    return state_buf, lo, state_buf.shape[3]
+
+
+def conv_update(state_buf, changes, packed_w, bias_f32, out_buf, Cin, Cout, filtSize, relu, gemm,
+                aux=None, ws=None, mask=None):
+    """cb_conv_update on pixel-major buffers [B,H,W,pitch].  GEMM_TC_3X (fp32) consumes the tf32
+    remainder plane, GEMM_TC_BF16X3 the bf16 hi/lo planes, passed as `aux` (see _aux_args: what
+    cb_change_detect keeps in step) or derived on the fly."""
+    B, H, W, _ = state_buf.shape
+    assert out_buf.shape[:3] == state_buf.shape[:3]
+    src, src_lo, pitch = _conv_operands(state_buf, Cin, gemm, aux)
     if mask is not None:
         # `changes` is a superset list; mask = dict(bits=raw bitmap, clear=bool, count=int32[1] out,
         # sync=int32[2] zeroed once): only pixels whose bit is set are processed (cb_conv_update_masked)
@@ -389,21 +396,13 @@ def conv_accumulate(planes16, changes, packed_w, out_buf, Cin, Cout, filtSize, g
 
 
 def conv_update_tiled(state_buf, tile_ws, dil_bits, packed_w, bias_f32, out_buf, Cin, Cout, filtSize,
-                      relu, gemm, lo_buf=None, planes16=None, pool=None):
+                      relu, gemm, aux=None, pool=None):
     """cb_conv_update_tiled on pixel-major buffers: the contraction over the dirty 8x16 tiles listed
     in `tile_ws` (TMA-staged halo tiles, implicit im2col), writing the pixels set in `dil_bits`.
     Operand conventions as :func:`conv_update`."""
-    B, H, W, Cp = state_buf.shape
+    B, H, W, _ = state_buf.shape
     assert out_buf.shape[:3] == state_buf.shape[:3]
-    src, src_lo, pitch = state_buf, lo_buf, Cp
-    if gemm == _lib.GEMM_TC_BF16X3:
-        assert state_buf.dtype == torch.float32
-        if planes16 is None:
-            planes16 = bf16_planes(state_buf, Cin)
-        src, src_lo = planes16
-        pitch = src.shape[3]
-    elif gemm == _lib.GEMM_TC_3X and state_buf.dtype == torch.float32 and lo_buf is None:
-        src_lo = tf32_lo(state_buf)
+    src, src_lo, pitch = _conv_operands(state_buf, Cin, gemm, aux)
     if pool is not None:
         # pool = dict(out=pooled map view, next_state=view, next_raw_bits, threshold, mode, aux): the
         # epilogue also re-pools the touched 2x2 windows and runs the next layer's detection on them

@@ -156,6 +156,23 @@ def test_hierarchical_tuner_and_pickle_roundtrip(tmp_path):
     assert repr(back) == repr(pose)
 
 
+def test_pickle_of_an_older_version_gets_the_attributes_added_since(tmp_path):
+    """a module pickled before a flag or a piece of private state existed loads with the flag's
+    default, no fused neighbours and no version record (its state counts as written from outside)."""
+    import cbinfer_b200 as cb
+    conv = cb.CBConv2d(nn.Conv2d(3, 4, 3, padding=1), 0.1)
+    pool = cb.CBPoolMax2d(nn.MaxPool2d(2, 2))
+    for name in ('candidateDetect', 'tileMode', '_fusedPool', '_fusedTail', '_inVersion', '_outVersion'):
+        del conv.__dict__[name]
+    del pool.__dict__['_outVersion']
+    path = str(tmp_path / "old.net")
+    torch.save(nn.Sequential(conv, pool), path)
+    conv, pool = torch.load(path, weights_only=False)
+    assert conv.candidateDetect is False and conv.tileMode == 'auto'
+    assert conv._fusedPool is None and conv._fusedTail is None
+    assert conv._inVersion is None and conv._outVersion is None and pool._outVersion is None
+
+
 def test_bench_reference_arm_is_product_free():
     """bench.py's reference arm rebuilds the dense model and the synthetic video in plain torch
     (it must not load libcbinfer_sm100.so): both must equal the package's builders bit for bit, and

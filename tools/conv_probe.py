@@ -31,11 +31,11 @@ def main():
     sel = torch.cat([torch.arange(per, dtype=torch.int32) + b * H * W + (H // 3) * W for b in range(B)]).cuda()
     ci = cg.ChangeIndexes.from_tensor(sel, (B, H, W))
     packed = cg.pack_weights(w, gemm)
-    planes = cg.bf16_planes(sbuf, Cin) if gemm == _lib.GEMM_TC_BF16X3 else None
+    planes = ('bf16',) + cg.bf16_planes(sbuf, Cin) if gemm == _lib.GEMM_TC_BF16X3 else None
     ws = None if a.no_ws else torch.zeros(_lib.C.cb_conv_ws_bytes(), dtype=torch.uint8, device="cuda")
 
     def run():
-        cg.conv_update(sbuf, ci, packed, bias, obuf, Cin, Cout, (k, k), True, gemm, planes16=planes, ws=ws)
+        cg.conv_update(sbuf, ci, packed, bias, obuf, Cin, Cout, (k, k), True, gemm, aux=planes, ws=ws)
 
     for _ in range(3):
         run()

@@ -42,18 +42,18 @@ def one(B, Cin, Cout, H, W, k, rate, mode, dt, kind="block"):
     s = cg.alloc_scratch(shape, "cuda")
     tws = cg.alloc_tile_ws(shape, "cuda")
     packed = cg.pack_weights(w, gemm)
-    planes = cg.bf16_planes(sbuf, Cin) if gemm == _lib.GEMM_TC_BF16X3 else None
+    planes = ('bf16',) + cg.bf16_planes(sbuf, Cin) if gemm == _lib.GEMM_TC_BF16X3 else None
     ws = torch.zeros(_lib.C.cb_conv_ws_bytes(), dtype=torch.uint8, device="cuda")
     cg.dilate_compact(raw_bits, shape, (k, k), s["idx"], s["count"], s["ws"], dil_bits=s["dil_bits"], tile_ws=tws)
     ci = cg.ChangeIndexes(s["idx"], s["count"], shape, bits=s["dil_bits"])
     n, ntl = int(s["count"]), int(tws[1])
     t_dc = timed(lambda: cg.dilate_compact(raw_bits, shape, (k, k), s["idx"], s["count"], s["ws"], dil_bits=s["dil_bits"], tile_ws=tws))
     t_dc0 = timed(lambda: cg.dilate_compact(raw_bits, shape, (k, k), s["idx"], s["count"], s["ws"], dil_bits=s["dil_bits"]))
-    t_g = timed(lambda: cg.conv_update(sbuf, ci, packed, bias, obuf, Cin, Cout, (k, k), True, gemm, planes16=planes, ws=ws))
+    t_g = timed(lambda: cg.conv_update(sbuf, ci, packed, bias, obuf, Cin, Cout, (k, k), True, gemm, aux=planes, ws=ws))
     sup = cg.tiled_supported(dt, gemm, shape, Cin, Cout, (k, k))
     t_t = float("nan")
     if sup:
-        t_t = timed(lambda: cg.conv_update_tiled(sbuf, tws, s["dil_bits"], packed, bias, obuf, Cin, Cout, (k, k), True, gemm, planes16=planes))
+        t_t = timed(lambda: cg.conv_update_tiled(sbuf, tws, s["dil_bits"], packed, bias, obuf, Cin, Cout, (k, k), True, gemm, aux=planes))
     fl = 2.0 * n * Cin * k * k * Cout
     print("B%d %3d->%-3d %4dx%-4d k%d %s %.0f%% %s: n=%d tiles=%d (eff %.2f) | compact %.2f us (+tiles %.2f) | gather %.2f us | tiled %.2f us (%.1f TFLOP/s alg, sup=%d)"
           % (B, Cin, Cout, H, W, k, kind, rate * 100, mode, n, ntl, n / max(ntl * 128, 1), t_dc0, t_dc, t_g, t_t, fl / t_t * 1e-6, sup), flush=True)

@@ -32,7 +32,7 @@ def run(B, Cin, Cout, H, W, k, rate, cold, pool=False):
     s = cg.alloc_scratch(shape, "cuda")
     tws = cg.alloc_tile_ws(shape, "cuda")
     packed = cg.pack_weights(w, gemm)
-    planes = cg.bf16_planes(sbuf, Cin)
+    planes = ('bf16',) + cg.bf16_planes(sbuf, Cin)
     cg.dilate_compact(raw_bits, shape, (k, k), s["idx"], s["count"], s["ws"], dil_bits=s["dil_bits"], tile_ws=tws)
     ntl = int(tws[1])
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
@@ -45,7 +45,7 @@ def run(B, Cin, Cout, H, W, k, rate, cold, pool=False):
         pargs = dict(out=pv, next_state=nv, next_raw_bits=s2["raw_bits"], threshold=0.05, mode=_lib.UPDATE_CHANGED,
                      aux=('bf16', nh, nl))
     for _ in range(3):
-        cg.conv_update_tiled(sbuf, tws, s["dil_bits"], packed, bias, obuf, Cin, Cout, (k, k), True, gemm, planes16=planes,
+        cg.conv_update_tiled(sbuf, tws, s["dil_bits"], packed, bias, obuf, Cin, Cout, (k, k), True, gemm, aux=planes,
                              pool=pargs)
     torch.cuda.synchronize()
     buf = (ctypes.c_longlong * (2048 * 32))()
@@ -55,7 +55,7 @@ def run(B, Cin, Cout, H, W, k, rate, cold, pool=False):
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    cg.conv_update_tiled(sbuf, tws, s["dil_bits"], packed, bias, obuf, Cin, Cout, (k, k), True, gemm, planes16=planes,
+    cg.conv_update_tiled(sbuf, tws, s["dil_bits"], packed, bias, obuf, Cin, Cout, (k, k), True, gemm, aux=planes,
                          pool=pargs)
     e1.record()
     torch.cuda.synchronize()
