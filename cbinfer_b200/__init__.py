@@ -9,13 +9,15 @@ return types; the per-frame work runs in ``libcbinfer_sm100.so`` (include/cbinfe
 import torch
 import torch.nn as nn
 
+from . import conv2d_cg as _cg
+from ._lib import CBinferError
 from .conv2d import CBConv2d
 from .conv2d import CBPoolMax2d
 from .conv2d_cg import ChangeIndexes
 
 __all__ = ['CBConv2d', 'CBPoolMax2d', 'ChangeIndexes', 'subsitute', 'convertRecur', 'mergeReLURecur',
            'propChangeIndexesOf1x1', 'clearMemory', 'getStateTensors', 'convert',
-           'tuneThresholdParameters', 'convertPools', 'shareWorkspace']
+           'tuneThresholdParameters', 'convertPools', 'shareWorkspace', 'resetStreams']
 
 verbose = False
 
@@ -107,6 +109,48 @@ def clearMemory(net):
     """drop the per-layer state of every CB layer (reference __init__.py:79-82)"""
     for layer in _cb_layers(net):
         layer.clearMemory()
+
+
+def resetStreams(net, streams):
+    """Start a new sequence in some streams of a batched model, in place: every CB layer under `net`
+    gets those streams' slices of its state set to what a cleared model starts from (+inf state,
+    zero operand planes).  Their next frame is then computed exactly as by a freshly cleared model,
+    while the other streams stay on the candidate path with their own change sets; nothing is freed,
+    so captured CUDA graphs stay valid (DESIGN.md section 3.12).
+
+    `net` must be the whole model the caller runs per frame: the argument needs every CB layer to
+    start over together.  The first layer then sees every pixel of a reset stream change, and each
+    layer after it receives all of them as candidates from the layer before; a layer left out would
+    keep its state for those streams and, being on the candidate path, would never test the pixels
+    its upstream neighbour does not hand on.
+
+    `streams`: an iterable of stream indices (the mask is built on the host and copied with an
+    ordinary asynchronous copy), or a bool / uint8 CUDA tensor [B] read on the device, which makes
+    the call capturable in a CUDA graph.  Work is enqueued on the current stream.  A model that has
+    not run yet has nothing to reset.  Fine-grained layers with state are not supported."""
+    if isinstance(streams, torch.Tensor) and not streams.is_cuda:
+        raise CBinferError("resetStreams: the stream mask must be a CUDA tensor (got one on %s)" % streams.device)
+    segments = [seg for layer in _cb_layers(net) for seg in layer._resetSegments()]
+    if not segments:
+        return
+    counts = set(buf.shape[0] for buf, _, _ in segments)
+    if len(counts) != 1:
+        raise CBinferError("resetStreams: the layers hold state of different batch sizes %s" % sorted(counts))
+    B = counts.pop()
+    dev = segments[0][0].device
+    if isinstance(streams, torch.Tensor):
+        mask = streams
+        if mask.dim() != 1 or mask.numel() != B:
+            raise CBinferError("resetStreams: a mask of shape %s for %d streams" % (tuple(mask.shape), B))
+    else:
+        idx = [int(i) for i in streams]
+        bad = [i for i in idx if not 0 <= i < B]
+        if bad:
+            raise CBinferError("resetStreams: stream indices %s out of range for %d streams" % (bad, B))
+        host = torch.zeros(B, dtype=torch.uint8)
+        host[idx] = 1
+        mask = host.to(dev, non_blocking=True)
+    _cg.reset_streams(segments, mask)
 
 
 def getStateTensors(net):

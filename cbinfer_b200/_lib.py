@@ -16,6 +16,7 @@ F32, F16, BF16 = 0, 1, 2
 UPDATE_NONE, UPDATE_CHANGED, UPDATE_ALL = 0, 1, 2
 GEMM_SIMT_F32, GEMM_TC, GEMM_TC_3X, GEMM_TC_BF16X3 = 0, 1, 2, 3
 AUX_NONE, AUX_TF32_LO, AUX_BF16_PAIR = 0, 1, 2
+RESET_FILL_ZERO, RESET_FILL_INF = 0, 1
 
 _DTYPES = {torch.float32: F32, torch.float16: F16, torch.bfloat16: BF16}
 
@@ -29,9 +30,15 @@ SYMBOLS = [
     "cb_fg_detect", "cb_conv_accumulate", "cb_compact_small_max_words", "cb_change_detect_sparse_compact",
     "cb_tile_ws_bytes", "cb_dilate_compact_tiles", "cb_conv_tiled_supported", "cb_conv_update_tiled",
     "cb_conv_tiled_pool_supported", "cb_conv_update_tiled_pool", "cb_dilate_tiles",
-    "cb_tail_supported", "cb_tail_update",
+    "cb_tail_supported", "cb_tail_update", "cb_reset_streams",
     "cb_resize_ws_bytes", "cb_resize_bicubic_u8_init", "cb_resize_bicubic_u8", "cb_resize_bilinear_u8",
 ]
+
+
+class ResetSegment(ctypes.Structure):
+    """cb_reset_segment: one pixel-major buffer whose per-stream slices cb_reset_streams rewrites."""
+    _fields_ = [("base", ctypes.c_void_p), ("pixels", ctypes.c_longlong), ("pitch_bytes", ctypes.c_int),
+                ("channel_bytes", ctypes.c_int), ("dtype", ctypes.c_int), ("fill", ctypes.c_int)]
 
 
 def _load():
@@ -71,6 +78,7 @@ def _load():
         "cb_tail_supported": (i32, [i32] * 5),
         "cb_tail_update": (i32, [vp, vp, vp, vp, vp, vp, i32, f32, vp, vp, vp, vp, i32, i32, f32, vp, vp, i32, i32, i32,
                                  i32, vp, vp, vp]),
+        "cb_reset_streams": (i32, [vp, vp, i32, ctypes.POINTER(ResetSegment), i32]),
         "cb_dilate_tiles": (i32, [vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32]),
         "cb_conv_tiled_pool_supported": (i32, [i32, i32, i32]),
         "cb_conv_update_tiled_pool": (i32, [vp, i32, i32, vp, vp, i32, vp, vp, vp, vp, vp, i32, i32, i32, i32,

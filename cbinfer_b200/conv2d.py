@@ -95,6 +95,12 @@ class CBPoolMax2d(nn.Module):
     def getStateTensors(self):
         return [self.outputState]
 
+    def _resetSegments(self):
+        """The pooled map as a cg.reset_streams segment (+inf), if allocated."""
+        if self._stateBuf is None:
+            return []
+        return [(self._stateBuf, self.outputState.shape[1], _INF)]
+
     def _pooled_size(self, h, w):
         if self.ceil_mode:
             return (h - 1) // 2 + 1, (w - 1) // 2 + 1
@@ -280,6 +286,22 @@ class CBConv2d(nn.Module):
 
     def getStateTensors(self):
         return [self.prevInput, self.prevOutput]
+
+    def _resetSegments(self):
+        """The pixel-major state as cg.reset_streams segments: prevInput / prevOutput (+inf) and the
+        operand planes of prevInput (0, what _aux builds from a +inf state), where allocated."""
+        if (self.finegrained and self.prevInput.numel() > 0) or \
+                (self._auxPlanes is not None and self._auxPlanes[0] == 'fg'):
+            raise _lib.CBinferError("resetStreams: a fine-grained layer's first frame is a dense convolution "
+                                    "of the whole batch; it cannot start one stream over")
+        if self._inBuf is None:
+            return []
+        segs = [(self._inBuf, self.in_channels, _INF), (self._outBuf, self.out_channels, _INF)]
+        if self._auxPlanes is not None and self._auxPlanes[0] == 'tf32':
+            segs.append((self._auxPlanes[1].permute(0, 2, 3, 1), self.in_channels, 0))
+        elif self._auxPlanes is not None and self._auxPlanes[0] == 'bf16':
+            segs += [(plane, self.in_channels, 0) for plane in self._auxPlanes[1:]]
+        return segs
 
     def _stateAllocated(self, shape, dtype, device):
         """Rule 1, first half: are prevInput / prevOutput the state the kernels own for an input of

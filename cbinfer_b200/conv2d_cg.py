@@ -440,6 +440,33 @@ def tail_update(x_buf, state1_buf, packed1, bias1, out1_buf, relu1, thr1, state2
                            int(update_mode), count1.data_ptr(), count2.data_ptr(), sync.data_ptr()))
 
 
+def reset_streams(segments, mask):
+    """cb_reset_streams: for every stream b with ``mask[b] != 0`` rewrite stream b's slice of each
+    segment.  A segment is ``(buf, channels, fill)``: ``buf`` a pixel-major [B,H,W,*] tensor whose
+    pixel stride (``buf.stride(2)``) is the pitch and whose first ``channels`` channels are real;
+    those are set to ``fill`` (``inf`` or 0), the pad channels up to the pitch to 0.  ``mask`` is a
+    bool / uint8 CUDA tensor [B]; it is read on the device, so the call can be captured in a graph."""
+    require_cuda(mask)
+    if mask.dim() != 1 or mask.dtype not in (torch.bool, torch.uint8) or not mask.is_contiguous():
+        raise _lib.CBinferError("reset_streams: the mask must be a contiguous bool or uint8 tensor [B]")
+    B = mask.numel()
+    segs = (_lib.ResetSegment * max(len(segments), 1))()
+    for i, (buf, channels, fill) in enumerate(segments):
+        require_cuda(buf)
+        Bb, H, W, _ = buf.shape
+        pitch = buf.stride(2)
+        if Bb != B or buf.device != mask.device:
+            raise _lib.CBinferError("reset_streams: a buffer of %d streams on %s, a mask of %d on %s"
+                                    % (Bb, buf.device, B, mask.device))
+        assert buf.stride(3) == 1 and buf.stride(1) == W * pitch and buf.stride(0) == H * W * pitch \
+            and channels <= pitch, "pixel-major buffers only"
+        es = buf.element_size()
+        segs[i] = _lib.ResetSegment(buf.data_ptr(), H * W, pitch * es, channels * es, dtype_code(buf),
+                                    _lib.RESET_FILL_INF if fill != 0 else _lib.RESET_FILL_ZERO)
+    with torch.cuda.device(mask.device):
+        check(C.cb_reset_streams(stream_ptr(mask.device), mask.data_ptr(), B, segs, len(segments)))
+
+
 def pixel_major(shape, dtype, device, fill):
     """Allocate a [B,C,H,W]-shaped *view* over a pixel-major [B,H,W,pitch] buffer whose pitch is
     C rounded up to 16 bytes.  Real channels are set to `fill`, pad channels to 0 (they meet zero

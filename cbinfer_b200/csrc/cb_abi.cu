@@ -14,6 +14,7 @@
 #include "ingest.cuh"
 #include "fg.cuh"
 #include "pool.cuh"
+#include "reset.cuh"
 #include "staged.cuh"
 #include "tail.cuh"
 
@@ -540,6 +541,62 @@ int cb_maxpool2x2_detect(void* stream, int dtype, const void* x, long long x_sb,
   }
 #undef CB_MPD
   CB_CHECK_LAUNCH("maxpool2x2_detect");
+  return 0;
+}
+
+int cb_reset_streams(void* stream, const uint8_t* mask, int B, const cb_reset_segment* segments,
+                     int n_segments) {
+  CB_CHECK_ARG(B > 0 && B <= 65535, "reset_streams: B = %d out of [1, 65535]", B);
+  CB_CHECK_ARG(n_segments >= 0, "reset_streams: negative segment count %d", n_segments);
+  CB_CHECK_ARG(mask && (n_segments == 0 || segments), "reset_streams: null pointer");
+  for (int i = 0; i < n_segments; ++i) {
+    const cb_reset_segment& g = segments[i];
+    CB_CHECK_ARG(g.dtype == CB_F32 || g.dtype == CB_F16 || g.dtype == CB_BF16,
+                 "reset_streams: segment %d: bad dtype %d", i, g.dtype);
+    const int es = cb::esize(g.dtype);
+    CB_CHECK_ARG(g.fill == CB_RESET_FILL_ZERO || g.fill == CB_RESET_FILL_INF,
+                 "reset_streams: segment %d: bad fill %d", i, g.fill);
+    CB_CHECK_ARG(g.pixels >= 0 && g.pitch_bytes > 0 && g.pitch_bytes % es == 0,
+                 "reset_streams: segment %d: pixels %lld, pitch %d bytes", i, g.pixels, g.pitch_bytes);
+    CB_CHECK_ARG(g.channel_bytes >= 0 && g.channel_bytes % es == 0 && g.channel_bytes <= g.pitch_bytes,
+                 "reset_streams: segment %d: %d channel bytes in a %d-byte pitch", i, g.channel_bytes,
+                 g.pitch_bytes);
+    CB_CHECK_ARG(g.pixels <= (1ll << 62) / g.pitch_bytes / B, "reset_streams: segment %d too large", i);
+    CB_CHECK_ARG(g.pixels == 0 || (g.base && (uintptr_t)g.base % es == 0),
+                 "reset_streams: segment %d: base not aligned to its %d-byte elements", i, es);
+  }
+  static const unsigned kInf[3] = {0x7f800000u, 0x7c00u, 0x7f80u};      // fp32, fp16, bf16
+  cb::ResetBatch rb;
+  rb.n = 0;
+  rb.cta0[0] = 0;
+  for (int i = 0; i <= n_segments; ++i) {
+    const bool more = i < n_segments;
+    long long slice = 0, ctas = 0;
+    if (more) {
+      slice = segments[i].pixels * segments[i].pitch_bytes;
+      ctas = (slice + cb::kResetChunksPerCta * 16 - 1) / (cb::kResetChunksPerCta * 16);
+      if (ctas == 0) continue;                                            // empty segment
+    }
+    // launch what is collected when the batch is full, the grid would grow past 2^31 - 1, or at the end
+    if (rb.n > 0 && (!more || rb.n == cb::kResetMaxSegs || rb.cta0[rb.n] + ctas > 0x7fffffffll)) {
+      cb::launch(reset_streams_kernel, dim3(rb.cta0[rb.n], (unsigned)B), dim3(cb::kResetThreads), 0,
+                 (cudaStream_t)stream, rb, mask);
+      CB_CHECK_LAUNCH("reset_streams");
+      rb.n = 0;
+    }
+    if (!more) break;
+    CB_CHECK_ARG(ctas <= 0x7fffffffll, "reset_streams: segment %d too large for one grid", i);
+    const cb_reset_segment& g = segments[i];
+    cb::ResetSeg& s = rb.seg[rb.n];
+    s.base = (char*)g.base;
+    s.slice = slice;
+    s.fill = g.fill == CB_RESET_FILL_INF ? kInf[g.dtype] : 0u;
+    s.pitch = g.pitch_bytes;
+    s.chan = g.channel_bytes;
+    s.es = cb::esize(g.dtype);
+    rb.cta0[rb.n + 1] = rb.cta0[rb.n] + (unsigned)ctas;
+    ++rb.n;
+  }
   return 0;
 }
 

@@ -91,6 +91,14 @@ class FramePipeline(object):
             self.out_done[s].record(self.d2h)
         return s
 
+    def reset(self, streams):
+        """Start a new sequence in `streams` (see cbinfer_b200.resetStreams): enqueued on the compute
+        stream, so it applies from the next `submit`ted frame on; frames already submitted are
+        computed without it.  The captured graphs stay valid."""
+        from . import resetStreams
+        with torch.cuda.stream(self.compute):
+            resetStreams(self.model, streams)
+
     def wait(self, slot):
         self.out_done[slot].synchronize()
         return self.out_host[slot]

@@ -296,6 +296,32 @@ int cb_maxpool2x2_detect(void* stream, int dtype, const void* x, long long x_sb,
                          long long n_sb, long long n_sy, int n_pitch, int aux_mode, void* aux_hi,
                          void* aux_lo, uint32_t* next_raw_bits, float threshold, int update_mode);
 
+/* ---- per-stream state reset -----------------------------------------------------------------
+ * Starts a new sequence in some streams of a batch without touching the others: for every b with
+ * mask[b] != 0 (mask: uint8[B] in device memory, read on the device), stream b's slice of every
+ * segment is rewritten.  A segment is one pixel-major buffer [B, pixels, pitch_bytes]: stream b's
+ * slice is the `pixels * pitch_bytes` bytes at base + b * pixels * pitch_bytes.  In each pixel the
+ * first channel_bytes bytes (the real channels) are set to +inf of the segment's dtype
+ * (CB_RESET_FILL_INF) or to 0 (CB_RESET_FILL_ZERO); the pad channels behind them are set to 0.
+ * A model whose every layer's state (previous input, previous output, pooled map: +inf; operand
+ * planes: 0) is reset this way computes the reset streams' next frame exactly like a freshly
+ * cleared model (DESIGN.md section 3.12).  One launch for up to 96 segments (more are split over
+ * several launches); no host synchronisation, capturable in a CUDA graph.  base must be aligned to
+ * the element size, pitch_bytes and channel_bytes multiples of it, channel_bytes <= pitch_bytes.
+ * No reference counterpart (the reference is batch 1 and frees all state, conv2d.py:147-148). */
+#define CB_RESET_FILL_ZERO 0
+#define CB_RESET_FILL_INF 1
+typedef struct cb_reset_segment {
+  void* base;              /* stream 0's slice                                              */
+  long long pixels;        /* pixels per stream (H * W)                                     */
+  int pitch_bytes;         /* bytes per pixel                                               */
+  int channel_bytes;       /* bytes of real channels per pixel                              */
+  int dtype;               /* CB_F32 / CB_F16 / CB_BF16: element size and the +inf written  */
+  int fill;                /* CB_RESET_FILL_INF or CB_RESET_FILL_ZERO                       */
+} cb_reset_segment;
+int cb_reset_streams(void* stream, const uint8_t* mask, int B, const cb_reset_segment* segments,
+                     int n_segments);
+
 /* ---- staged (unfused) ops in the reference's planar layout --------------------------------
  * 1:1 replacements used by the op-level wrappers and parity tests. n is a host count here,
  * exactly as in the reference signatures. */
