@@ -486,12 +486,10 @@ int cb_maxpool2x2(void* stream, int dtype, const void* x, long long x_sb, long l
                       (x_sx == C || (C + vec - 1) / vec * vec == x_sx);
   if (vec_ok) {
     const int cpp = (int)(x_sx / vec);
-    int glog = 0;
-    while ((1 << glog) < cpp && glog < 5) ++glog;
-    glog = cb::glog_tuned(glog);
-    CB_DISPATCH_DTYPE(dtype, (cb::launch(maxpool2x2_vec_kernel<T, VEC>, grid, 256, 0, (cudaStream_t)stream, 
-                                 (const T*)x, x_sb, x_sy, (int)x_sx, idx, count, dil_bits, (T*)out,
-                                 o_sb, o_sy, (int)o_sx, cpp, glog, H, W, oH, oW)));
+    CB_DISPATCH_DTYPE(dtype, (cb::launch(maxpool2x2_detect_kernel<T, VEC, CB_UPDATE_NONE, false>, grid, 256, 0,
+                                         (cudaStream_t)stream, (const T*)x, x_sb, x_sy, (int)x_sx, idx, count,
+                                         dil_bits, (T*)out, o_sb, o_sy, (int)o_sx, cpp, cb::group_log2(cpp), H, W,
+                                         oH, oW, nullptr, 0ll, 0ll, 0, AuxPlanes{}, nullptr, T{})));
   } else {
     CB_DISPATCH_DTYPE(dtype, (cb::launch(maxpool2x2_kernel<T>, grid, 256, 0, (cudaStream_t)stream, 
                                  (const T*)x, x_sb, x_sc, x_sy, x_sx, idx, count, dil_bits, (T*)out,
@@ -519,29 +517,20 @@ int cb_maxpool2x2_detect(void* stream, int dtype, const void* x, long long x_sb,
                   ((uintptr_t)out % 16) == 0 && ((uintptr_t)next_state % 16) == 0;
   CB_CHECK_ARG(ok, "maxpool2x2_detect: needs pixel-major, 16-byte aligned tensors of equal pitch");
   const int cpp = x_pitch / vec;
-  int glog = 0;
-  while ((1 << glog) < cpp && glog < 5) ++glog;
-  glog = cb::glog_tuned(glog);
+  const int glog = cb::group_log2(cpp);
   const unsigned grid = (unsigned)(sm_count() * 16);
   cudaStream_t s = (cudaStream_t)stream;
-#define CB_MPD(U_)                                                                                \
-  CB_DISPATCH_DTYPE(dtype, {                                                                      \
-    AuxPlanes aux;                                                                                \
-    if (int rc = make_aux<T>(aux, aux_mode, aux_hi, aux_lo, next_state, C)) return rc;            \
-    cb::launch(maxpool2x2_detect_kernel<T, VEC, U_>, grid, 256, 0, s, (const T*)x, x_sb,         \
-                   x_sy, x_pitch, idx, count, dil_bits, (T*)out, o_sb, o_sy, o_pitch, cpp, glog, \
-                   H, W, oH, oW, (T*)next_state, n_sb, n_sy, n_pitch, aux, next_raw_bits,         \
-                   thr_cast<T>(threshold));                                                       \
-  })
-  switch (update_mode) {
-    case CB_UPDATE_NONE: CB_MPD(CB_UPDATE_NONE); break;
-    case CB_UPDATE_CHANGED: CB_MPD(CB_UPDATE_CHANGED); break;
-    case CB_UPDATE_ALL: CB_MPD(CB_UPDATE_ALL); break;
-    default: return cb::fail(2, "maxpool2x2_detect: bad update_mode %d", update_mode);
-  }
-#undef CB_MPD
-  CB_CHECK_LAUNCH("maxpool2x2_detect");
-  return 0;
+  return dispatch_update(update_mode, "maxpool2x2_detect", [&](auto U) {
+    CB_DISPATCH_DTYPE(dtype, {
+      AuxPlanes aux;
+      if (int rc = make_aux<T>(aux, aux_mode, aux_hi, aux_lo, next_state, C)) return rc;
+      cb::launch(maxpool2x2_detect_kernel<T, VEC, U>, grid, 256, 0, s, (const T*)x, x_sb, x_sy, x_pitch, idx,
+                 count, dil_bits, (T*)out, o_sb, o_sy, o_pitch, cpp, glog, H, W, oH, oW, (T*)next_state, n_sb,
+                 n_sy, n_pitch, aux, next_raw_bits, thr_cast<T>(threshold));
+    })
+    CB_CHECK_LAUNCH("maxpool2x2_detect");
+    return 0;
+  });
 }
 
 int cb_reset_streams(void* stream, const uint8_t* mask, int B, const cb_reset_segment* segments,

@@ -6,6 +6,8 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include <type_traits>
+
 #include "../../include/cbinfer_b200.h"
 
 namespace cb {
@@ -27,11 +29,27 @@ int fail(int code, const char* fmt, ...);
 
 int sm_count();
 
-// log2 of the lanes that share one pixel in the candidate-detection / pooling kernels.  One lane
-// per 16-byte chunk would be the obvious choice; two chunks per lane halves the number of warps
-// (one wave instead of two at 8 streams) and doubles the loads in flight per lane: measured
-// pool+detect 11.3 -> 8.3 us, sparse detect 7.7 -> 6.7 us.
-inline int glog_tuned(int glog) { return glog > 0 ? glog - 1 : 0; }
+// log2 of the lanes that share one pixel in the candidate-detection / pooling kernels: one lane per
+// two 16-byte chunks, at most 16 lanes.  One lane per chunk would be the obvious choice; two chunks per
+// lane halves the number of warps (one wave instead of two at 8 streams) and doubles the loads in
+// flight per lane: measured pool+detect 11.3 -> 8.3 us, sparse detect 7.7 -> 6.7 us.
+inline int group_log2(int chunks) {
+  int g = 0;
+  while (g < 4 && (2 << g) < chunks) ++g;
+  return g;
+}
+
+// Calls f(std::integral_constant<int, update>{}), so that the kernels f launches take the update mode
+// as a template argument; an unknown mode fails with "<what>: bad update_mode".
+template <typename F>
+inline int dispatch_update(int update, const char* what, F&& f) {
+  switch (update) {
+    case CB_UPDATE_NONE: return f(std::integral_constant<int, CB_UPDATE_NONE>{});
+    case CB_UPDATE_CHANGED: return f(std::integral_constant<int, CB_UPDATE_CHANGED>{});
+    case CB_UPDATE_ALL: return f(std::integral_constant<int, CB_UPDATE_ALL>{});
+    default: return fail(2, "%s: bad update_mode %d", what, update);
+  }
+}
 
 // cooperative != 0: the grid is launched only when ALL its CTAs can be resident at once (kernels whose
 // CTAs wait for each other, e.g. the stream-K finisher spinning on its contributors' flags, must not
@@ -69,12 +87,7 @@ inline void launch(void (*kern)(KArgs...), dim3 grid, dim3 block, size_t smem, c
   launch_cluster(kern, grid, block, smem, s, 1u, 0, static_cast<Args&&>(args)...);
 }
 
-// ---- dtype traits --------------------------------------------------------------------------
-template <int DT> struct DType;
-template <> struct DType<CB_F32> { using T = float; static constexpr int VEC = 4; };
-template <> struct DType<CB_F16> { using T = __half; static constexpr int VEC = 8; };
-template <> struct DType<CB_BF16> { using T = __nv_bfloat16; static constexpr int VEC = 8; };
-
+// ---- dtype helpers -------------------------------------------------------------------------
 __host__ __device__ inline int esize(int dtype) { return dtype == CB_F32 ? 4 : 2; }
 // channel pitch of the bf16 operand planes of an fp32 layer: a multiple of 16 bytes (an RGB input
 // layer gets 16-byte pixels: the smallest pixel the tiled contraction's shared-memory descriptors

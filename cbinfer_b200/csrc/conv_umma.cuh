@@ -1080,15 +1080,16 @@ int dispatch_bn(int bn, cudaStream_t s, int dtype, const void* state, const void
     return launch_conv_umma<T, TO, SPLIT3, N, DEEP>(s, dtype, state, state_lo, Cp, idx, count, packed, bias, out, \
                                           Op, B, H, W, Cout, CoutPad, kH, kW, relu, sel_lo,   \
                                           sel_hi, ksplit, ws, ws_bytes, mk);
-  if (DEEP) {                                  // the deep variant only exists for N tiles <= 64
+  if constexpr (DEEP) {                        // the deep variant only exists for N tiles <= 64
     switch (bn) {
       CB_BN(16) CB_BN(32) CB_BN(64)
       default: return fail(2, "conv_update: unsupported deep N tile %d", bn);
     }
-  }
-  switch (bn) {
-    CB_BN(16) CB_BN(32) CB_BN(64) CB_BN(128) CB_BN(256)
-    default: return fail(2, "conv_update: unsupported N tile %d", bn);
+  } else {
+    switch (bn) {
+      CB_BN(16) CB_BN(32) CB_BN(64) CB_BN(128) CB_BN(256)
+      default: return fail(2, "conv_update: unsupported N tile %d", bn);
+    }
   }
 #undef CB_BN
 }

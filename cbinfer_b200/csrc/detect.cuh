@@ -99,6 +99,36 @@ __device__ __forceinline__ uint4 ld16_stream(const void* p) { return __ldcs(rein
 
 constexpr int kDetWarps = 8;                   // warps per block
 
+// The bitmap word of this warp in the kernels that give each warp one word (32 pixels of a row):
+// image b, row y and this lane's pixel column xx; false beyond the map.  32-bit index math (the host
+// checks words < 2^31): two 64-bit divisions per warp were most of these kernels' instructions (ncu:
+// 173 warp instructions per 32 pixels, SM 54 % busy on an HBM-bound scan)
+__device__ __forceinline__ bool warp_word(unsigned& warp, int& b, int& y, int& xx, int B, int H, int Wd) {
+  warp = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
+  if (warp >= (unsigned)(B * H * Wd)) return false;
+  const unsigned r = warp / (unsigned)Wd;
+  const int j = (int)(warp - r * (unsigned)Wd);
+  b = (int)(r / (unsigned)H);
+  y = (int)(r - (unsigned)b * (unsigned)H);
+  xx = j * 32 + (threadIdx.x & 31);
+  return true;
+}
+
+// One pixel, any strides, one channel at a time: any channel changed?  The state follows UPDATE.
+template <typename T, int UPDATE>
+__device__ __forceinline__ bool pixel_changed_scalar(const T* xp, long long x_sc, T* sp, long long s_sc,
+                                                     int C, T thr, const AuxPlanes& aux, long long gpix) {
+  bool f = false;
+  for (int c = 0; c < C; ++c) {
+    const T xv = xp[c * x_sc];
+    f |= value_changed(sp[c * s_sc], xv, thr);
+    if (UPDATE == CB_UPDATE_ALL) store_state_scalar(sp + c * s_sc, xv, aux, gpix, c);
+  }
+  if (UPDATE == CB_UPDATE_CHANGED && f)
+    for (int c = 0; c < C; ++c) store_state_scalar(sp + c * s_sc, xp[c * x_sc], aux, gpix, c);
+  return f;
+}
+
 // x: pixel-major, pitch xp (elements); state: pixel-major, pitch sp.  Rows may be strided (sy).
 // U chunk-iterations are batched: all 2*U 16-byte loads of a batch are issued before the first
 // ballot, so every lane keeps 2*U loads in flight (the ballots would otherwise serialise them).
@@ -205,38 +235,51 @@ detect_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int x
 // Generic x (any strides, e.g. the user's planar NCHW frame) against a pixel-major state whose
 // pixel is exactly one 16-byte chunk (C <= 4 fp32 / C <= 8 half): lane = pixel, the state is one
 // vector load/store per pixel and x is read plane by plane (coalesced across lanes).
-template <typename T, int VEC, int UPDATE>
+// S = uint8_t: frame ingest (decoder / camera output, any strides: HWC interleaved or planar) into a
+// fp32 state.  The normalisation of the reference's readers -- frame/255
+// (sceneLabeling/videoSequenceReader.py:65), frame/256 - 0.5 (openPose/PoseDetector.py:72) -- is
+// applied on the fly with IEEE division and addition, so the result is bit-identical to detecting on
+// the host-normalised fp32 frame, at a quarter of the host->device bytes.  Otherwise divisor and bias
+// are unused.
+template <typename T, int VEC, int UPDATE, typename S = T>
 __global__ void __launch_bounds__(256)
-detect_narrow_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, long long x_sy,
+detect_narrow_kernel(const S* __restrict__ x, long long x_sb, long long x_sc, long long x_sy,
                      long long x_sx, T* __restrict__ st, long long s_sb, long long s_sy,
                      AuxPlanes aux, uint32_t* __restrict__ bits, int B, int H, int W, int C,
-                     int Wd, T thr) {
-  const int lane = threadIdx.x & 31;
-  // 32-bit index math (the host checks words < 2^31): two 64-bit divisions per warp were most of this
-  // kernel's instructions (ncu: 173 warp instructions per 32 pixels, SM 54 % busy on an HBM-bound scan)
-  const unsigned warp = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  if (warp >= (unsigned)(B * H * Wd)) return;
-  const unsigned r = warp / (unsigned)Wd;
-  const int j = (int)(warp - r * (unsigned)Wd);
-  const int b = (int)(r / (unsigned)H);
-  const int y = (int)(r - (unsigned)b * (unsigned)H);
-  const int xx = j * 32 + lane;
+                     int Wd, T thr, float divisor, float bias) {
+  constexpr bool kU8 = std::is_same<S, uint8_t>::value;
+  const float* lut = nullptr;
+  if constexpr (kU8) {
+    // the 256 possible normalised values, computed once per block with the IEEE division and addition
+    // the host would use (bit-identical by construction): a table lookup per channel instead of a
+    // division.  Every thread takes part before any warp leaves.
+    __shared__ float s_lut[256];
+    s_lut[threadIdx.x] = __fadd_rn(__fdiv_rn((float)threadIdx.x, divisor), bias);
+    __syncthreads();
+    lut = s_lut;
+  }
+  unsigned warp;
+  int b, y, xx;
+  if (!warp_word(warp, b, y, xx, B, H, Wd)) return;
   bool f = false;
   if (xx < W) {
-    const T* xp = x + b * x_sb + y * x_sy + xx * x_sx;
+    const S* xp = x + b * x_sb + y * x_sy + xx * x_sx;
     T* sp = st + b * s_sb + y * s_sy + (long long)xx * VEC;
-    uint4 sv = ld16_stream(sp);
+    const uint4 sv = ld16_stream(sp);
     uint4 nv = sv;                             // pad lanes keep the state's (zero) value
     T* ne = reinterpret_cast<T*>(&nv);
 #pragma unroll
-    for (int c = 0; c < VEC; ++c)
-      if (c < C) ne[c] = ld_stream(xp + c * x_sc);
+    for (int c = 0; c < VEC; ++c) {
+      if (c >= C) continue;
+      if constexpr (kU8) ne[c] = lut[__ldcs(xp + c * x_sc)];
+      else ne[c] = ld_stream(xp + c * x_sc);
+    }
     f = Chunk<T>::changed(sv, nv, thr);
     if (UPDATE == CB_UPDATE_ALL || (UPDATE == CB_UPDATE_CHANGED && f))
       store_state<T>(sp, nv, aux, ((long long)b * H + y) * W + xx, 0);
   }
   const unsigned word = __ballot_sync(0xffffffffu, f);
-  if (lane == 0) bits[warp] = word;
+  if ((threadIdx.x & 31) == 0) bits[warp] = word;
 }
 
 // Planar x (NCHW: the pixels of a row are contiguous, any channel stride -- what a dense layer or the
@@ -379,77 +422,14 @@ detect_generic_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, l
                       long long x_sx, T* __restrict__ st, long long s_sb, long long s_sc,
                       long long s_sy, long long s_sx, AuxPlanes aux,
                       uint32_t* __restrict__ bits, int B, int H, int W, int C, int Wd, T thr) {
-  const int lane = threadIdx.x & 31;
-  // 32-bit index math (the host checks words < 2^31): two 64-bit divisions per warp were most of this
-  // kernel's instructions (ncu: 173 warp instructions per 32 pixels, SM 54 % busy on an HBM-bound scan)
-  const unsigned warp = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  if (warp >= (unsigned)(B * H * Wd)) return;
-  const unsigned r = warp / (unsigned)Wd;
-  const int j = (int)(warp - r * (unsigned)Wd);
-  const int b = (int)(r / (unsigned)H);
-  const int y = (int)(r - (unsigned)b * (unsigned)H);
-  const int xx = j * 32 + lane;
-  bool f = false;
-  const T* xp = x + b * x_sb + y * x_sy + xx * x_sx;
-  T* sp = st + b * s_sb + y * s_sy + xx * s_sx;
-  const long long gpix = ((long long)b * H + y) * W + xx;
-  if (xx < W) {
-    for (int c = 0; c < C; ++c) {
-      const T xv = xp[c * x_sc];
-      const T sv = sp[c * s_sc];
-      f |= value_changed(sv, xv, thr);
-      if (UPDATE == CB_UPDATE_ALL) store_state_scalar(sp + c * s_sc, xv, aux, gpix, c);
-    }
-    if (UPDATE == CB_UPDATE_CHANGED && f)
-      for (int c = 0; c < C; ++c) store_state_scalar(sp + c * s_sc, xp[c * x_sc], aux, gpix, c);
-  }
+  unsigned warp;
+  int b, y, xx;
+  if (!warp_word(warp, b, y, xx, B, H, Wd)) return;
+  const bool f = xx < W && pixel_changed_scalar<T, UPDATE>(x + b * x_sb + y * x_sy + xx * x_sx, x_sc,
+                                                            st + b * s_sb + y * s_sy + xx * s_sx, s_sc, C,
+                                                            thr, aux, ((long long)b * H + y) * W + xx);
   const unsigned word = __ballot_sync(0xffffffffu, f);
-  if (lane == 0) bits[warp] = word;
-}
-
-// uint8 frame ingest (decoder / camera output, any strides: HWC interleaved or planar) against a
-// pixel-major fp32 state whose pixel is one 16-byte chunk (C <= 4).  The normalisation of the
-// reference's readers -- frame/255 (sceneLabeling/videoSequenceReader.py:65), frame/256 - 0.5
-// (openPose/PoseDetector.py:72) -- is applied on the fly with IEEE division and addition, so the
-// result is bit-identical to detecting on the host-normalised fp32 frame, at a quarter of the
-// host->device bytes.
-template <int UPDATE>
-__global__ void __launch_bounds__(256)
-detect_u8_kernel(const uint8_t* __restrict__ x, long long x_sb, long long x_sc, long long x_sy,
-                 long long x_sx, float* __restrict__ st, long long s_sb, long long s_sy,
-                 AuxPlanes aux, uint32_t* __restrict__ bits, int B, int H, int W, int C, int Wd,
-                 float divisor, float bias, float thr) {
-  // the 256 possible normalised values, computed once per block with the IEEE division and addition the
-  // host would use (bit-identical by construction): a table lookup per channel instead of a division
-  __shared__ float lut[256];
-  lut[threadIdx.x] = __fadd_rn(__fdiv_rn((float)threadIdx.x, divisor), bias);
-  __syncthreads();
-  const int lane = threadIdx.x & 31;
-  // 32-bit index math (the host checks words < 2^31): two 64-bit divisions per warp were most of this
-  // kernel's instructions (ncu: 173 warp instructions per 32 pixels, SM 54 % busy on an HBM-bound scan)
-  const unsigned warp = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-  if (warp >= (unsigned)(B * H * Wd)) return;
-  const unsigned r = warp / (unsigned)Wd;
-  const int j = (int)(warp - r * (unsigned)Wd);
-  const int b = (int)(r / (unsigned)H);
-  const int y = (int)(r - (unsigned)b * (unsigned)H);
-  const int xx = j * 32 + lane;
-  bool f = false;
-  if (xx < W) {
-    const uint8_t* xp = x + b * x_sb + y * x_sy + xx * x_sx;
-    float* sp = st + b * s_sb + y * s_sy + (long long)xx * 4;
-    const uint4 sv = ld16_stream(sp);
-    uint4 nv = sv;                             // pad lanes keep the state's (zero) value
-    float* ne = reinterpret_cast<float*>(&nv);
-#pragma unroll
-    for (int c = 0; c < 4; ++c)
-      if (c < C) ne[c] = lut[__ldcs(xp + c * x_sc)];
-    f = Chunk<float>::changed(sv, nv, thr);
-    if (UPDATE == CB_UPDATE_ALL || (UPDATE == CB_UPDATE_CHANGED && f))
-      store_state<float>(sp, nv, aux, ((long long)b * H + y) * W + xx, 0);
-  }
-  const unsigned word = __ballot_sync(0xffffffffu, f);
-  if (lane == 0) bits[warp] = word;
+  if ((threadIdx.x & 31) == 0) bits[warp] = word;
 }
 
 template <typename T> __host__ __device__ inline T thr_cast(float t);
@@ -482,6 +462,19 @@ inline int make_aux(AuxPlanes& aux, int aux_mode, void* aux_hi, void* aux_lo, co
   return 0;
 }
 
+// x and the state pixel-major: channel-contiguous pixels of whole 16-byte chunks, 16-byte aligned
+// (the vector kernels)
+template <typename T, int VEC>
+inline bool pixel_major_ok(const void* x, long long x_sb, long long x_sc, long long x_sy, long long x_sx,
+                           const void* state, long long s_sb, long long s_sc, long long s_sy, long long s_sx,
+                           int C) {
+  const size_t es = sizeof(T);
+  return x_sc == 1 && s_sc == 1 && (x_sx % VEC) == 0 && (s_sx % VEC) == 0 && x_sx >= C && s_sx >= C &&
+         ((x_sy * es) % 16) == 0 && ((s_sy * es) % 16) == 0 && ((x_sb * es) % 16) == 0 &&
+         ((s_sb * es) % 16) == 0 && ((uintptr_t)x % 16) == 0 && ((uintptr_t)state % 16) == 0 &&
+         x_sx < (1ll << 30) && s_sx < (1ll << 30);
+}
+
 template <typename T, int VEC>
 int launch_detect(cudaStream_t stream, const void* x, long long x_sb, long long x_sc,
                   long long x_sy, long long x_sx, void* state, long long s_sb, long long s_sc,
@@ -494,11 +487,7 @@ int launch_detect(cudaStream_t stream, const void* x, long long x_sb, long long 
   const size_t es = sizeof(T);
   AuxPlanes aux;
   if (int rc = make_aux<T>(aux, aux_mode, aux_hi, aux_lo, state, C)) return rc;
-  const bool vec_ok = x_sc == 1 && s_sc == 1 && (x_sx % VEC) == 0 && (s_sx % VEC) == 0 &&
-                      x_sx >= C && s_sx >= C && ((x_sy * es) % 16) == 0 && ((s_sy * es) % 16) == 0 &&
-                      ((x_sb * es) % 16) == 0 && ((s_sb * es) % 16) == 0 &&
-                      ((uintptr_t)x % 16) == 0 && ((uintptr_t)state % 16) == 0 &&
-                      x_sx < (1ll << 30) && s_sx < (1ll << 30);
+  const bool vec_ok = pixel_major_ok<T, VEC>(x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy, s_sx, C);
   const bool narrow_ok = !vec_ok && s_sc == 1 && s_sx == VEC && C <= VEC &&
                          ((s_sy * es) % 16) == 0 && ((s_sb * es) % 16) == 0 &&
                          ((uintptr_t)state % 16) == 0;
@@ -518,42 +507,31 @@ int launch_detect(cudaStream_t stream, const void* x, long long x_sb, long long 
   const long long blocks = vec_ok ? vec_blocks : (words + 7) / 8;
   CB_CHECK_ARG(blocks < (1ll << 31) && words < (1ll << 31), "change_detect: image too large");
   dim3 grid((unsigned)blocks), block(256);
-#define CB_DET(U_)                                                                             \
-  if (vec_ok) {                                                                                \
-    if (cpv >= 4)                                                                              \
-      cb::launch(detect_vec_kernel<T, VEC, U_, 4>, grid, block, 0, stream,                                 \
-          (const T*)x, x_sb, x_sy, (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, bits,  \
-          B, H, W, C, Wd, thr, magic, wlog);                                                   \
-    else                                                                                       \
-      cb::launch(detect_vec_kernel<T, VEC, U_, 2>, grid, block, 0, stream,                                 \
-          (const T*)x, x_sb, x_sy, (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, bits,  \
-          B, H, W, C, Wd, thr, magic, wlog);                                                   \
-  } else if (narrow_ok) {                                                                      \
-    cb::launch(detect_narrow_kernel<T, VEC, U_>, grid, block, 0, stream,                                   \
-        (const T*)x, x_sb, x_sc, x_sy, x_sx, (T*)state, s_sb, s_sy, aux, bits, B, H, W, C,  \
-        Wd, thr);                                                                              \
-  } else if (planar_ok) {                                                                      \
-    if (planar_smem > 48 * 1024)                                                               \
-      cudaFuncSetAttribute(detect_planar_kernel<T, VEC, U_>,                                   \
-                           cudaFuncAttributeMaxDynamicSharedMemorySize, (int)planar_smem);     \
-    cb::launch(detect_planar_kernel<T, VEC, U_>, dim3((unsigned)((words + planar_nw - 1) / planar_nw)),     \
-        block, planar_smem, stream,                                                            \
-        (const T*)x, x_sb, x_sc, x_sy, (T*)state, s_sb, s_sy, (int)s_sx, aux, bits, B, H, W, C, \
-        Wd, thr, magic, cps, planar_nw);                                                       \
-  } else {                                                                                     \
-    cb::launch(detect_generic_kernel<T, U_>, grid, block, 0, stream,                                       \
-        (const T*)x, x_sb, x_sc, x_sy, x_sx, (T*)state, s_sb, s_sc, s_sy, s_sx, aux, bits,  \
-        B, H, W, C, Wd, thr);                                                                  \
-  }
-  switch (update) {
-    case CB_UPDATE_NONE: CB_DET(CB_UPDATE_NONE) break;
-    case CB_UPDATE_CHANGED: CB_DET(CB_UPDATE_CHANGED) break;
-    case CB_UPDATE_ALL: CB_DET(CB_UPDATE_ALL) break;
-    default: return fail(2, "change_detect: bad update_mode %d", update);
-  }
-#undef CB_DET
-  CB_CHECK_LAUNCH("change_detect");
-  return 0;
+  return dispatch_update(update, "change_detect", [&](auto U) {
+    if (vec_ok) {
+      if (cpv >= 4)
+        cb::launch(detect_vec_kernel<T, VEC, U, 4>, grid, block, 0, stream, (const T*)x, x_sb, x_sy, (int)x_sx,
+                   (T*)state, s_sb, s_sy, (int)s_sx, aux, bits, B, H, W, C, Wd, thr, magic, wlog);
+      else
+        cb::launch(detect_vec_kernel<T, VEC, U, 2>, grid, block, 0, stream, (const T*)x, x_sb, x_sy, (int)x_sx,
+                   (T*)state, s_sb, s_sy, (int)s_sx, aux, bits, B, H, W, C, Wd, thr, magic, wlog);
+    } else if (narrow_ok) {
+      cb::launch(detect_narrow_kernel<T, VEC, U>, grid, block, 0, stream, (const T*)x, x_sb, x_sc, x_sy, x_sx,
+                 (T*)state, s_sb, s_sy, aux, bits, B, H, W, C, Wd, thr, 0.f, 0.f);
+    } else if (planar_ok) {
+      if (planar_smem > 48 * 1024)
+        cudaFuncSetAttribute(detect_planar_kernel<T, VEC, U>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                             (int)planar_smem);
+      cb::launch(detect_planar_kernel<T, VEC, U>, dim3((unsigned)((words + planar_nw - 1) / planar_nw)), block,
+                 planar_smem, stream, (const T*)x, x_sb, x_sc, x_sy, (T*)state, s_sb, s_sy, (int)s_sx, aux, bits,
+                 B, H, W, C, Wd, thr, magic, cps, planar_nw);
+    } else {
+      cb::launch(detect_generic_kernel<T, U>, grid, block, 0, stream, (const T*)x, x_sb, x_sc, x_sy, x_sx,
+                 (T*)state, s_sb, s_sc, s_sy, s_sx, aux, bits, B, H, W, C, Wd, thr);
+    }
+    CB_CHECK_LAUNCH("change_detect");
+    return 0;
+  });
 }
 
 
@@ -573,19 +551,13 @@ inline int launch_detect_u8(cudaStream_t stream, const void* x, long long x_sb, 
   if (int rc = make_aux<float>(aux, aux_mode, aux_hi, aux_lo, state, C)) return rc;
   const long long blocks = (words + 7) / 8;
   CB_CHECK_ARG(blocks < (1ll << 31), "change_detect_u8: image too large");
-#define CB_DET8(U_)                                                                              \
-  cb::launch(detect_u8_kernel<U_>, dim3((unsigned)blocks), dim3(256), 0, stream,                \
-                 (const uint8_t*)x, x_sb, x_sc, x_sy, x_sx, (float*)state, s_sb, s_sy, aux, bits, \
-                 B, H, W, C, Wd, divisor, bias, threshold);
-  switch (update) {
-    case CB_UPDATE_NONE: CB_DET8(CB_UPDATE_NONE) break;
-    case CB_UPDATE_CHANGED: CB_DET8(CB_UPDATE_CHANGED) break;
-    case CB_UPDATE_ALL: CB_DET8(CB_UPDATE_ALL) break;
-    default: return fail(2, "change_detect_u8: bad update_mode %d", update);
-  }
-#undef CB_DET8
-  CB_CHECK_LAUNCH("change_detect_u8");
-  return 0;
+  return dispatch_update(update, "change_detect_u8", [&](auto U) {
+    cb::launch(detect_narrow_kernel<float, 4, U, uint8_t>, dim3((unsigned)blocks), dim3(256), 0, stream,
+               (const uint8_t*)x, x_sb, x_sc, x_sy, x_sx, (float*)state, s_sb, s_sy, aux, bits, B, H, W, C, Wd,
+               threshold, divisor, bias);
+    CB_CHECK_LAUNCH("change_detect_u8");
+    return 0;
+  });
 }
 
 
@@ -693,17 +665,8 @@ detect_sparse_generic_kernel(const T* __restrict__ x, long long x_sb, long long 
     const int y = p / W, xx = p - y * W;
     const T* xp = x + b * x_sb + y * x_sy + xx * x_sx;
     T* sp = st + b * s_sb + y * s_sy + xx * s_sx;
-    bool f = false;
-    for (int c = 0; c < C; ++c) {
-      const T xv = xp[c * x_sc];
-      f |= value_changed(sp[c * s_sc], xv, thr);
-      if (UPDATE == CB_UPDATE_ALL) store_state_scalar(sp + c * s_sc, xv, aux, (long long)pix, c);
-    }
-    if (f) {
+    if (pixel_changed_scalar<T, UPDATE>(xp, x_sc, sp, s_sc, C, thr, aux, (long long)pix))
       atomicOr(bits + ((long long)b * H + y) * Wd + (xx >> 5), 1u << (xx & 31));
-      if (UPDATE == CB_UPDATE_CHANGED)
-        for (int c = 0; c < C; ++c) store_state_scalar(sp + c * s_sc, xp[c * x_sc], aux, (long long)pix, c);
-    }
   }
 }
 
@@ -720,19 +683,11 @@ int launch_detect_sparse(cudaStream_t stream, const void* x, long long x_sb, lon
   if (!bits_are_clear && cudaMemsetAsync(bits, 0, (size_t)words * 4, stream) != cudaSuccess)
     return fail(3, "change_detect_sparse: memset failed");
   const T thr = thr_cast<T>(threshold);
-  const size_t es = sizeof(T);
   AuxPlanes aux;
   if (int rc = make_aux<T>(aux, aux_mode, aux_hi, aux_lo, state, C)) return rc;
-  const bool vec_ok = x_sc == 1 && s_sc == 1 && (x_sx % VEC) == 0 && (s_sx % VEC) == 0 &&
-                      x_sx >= C && s_sx >= C && ((x_sy * es) % 16) == 0 && ((s_sy * es) % 16) == 0 &&
-                      ((x_sb * es) % 16) == 0 && ((s_sb * es) % 16) == 0 &&
-                      ((uintptr_t)x % 16) == 0 && ((uintptr_t)state % 16) == 0 &&
-                      x_sx < (1ll << 30) && s_sx < (1ll << 30);
+  const bool vec_ok = pixel_major_ok<T, VEC>(x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy, s_sx, C);
   unsigned grid = (unsigned)(sm_count() * 16);
-  const int cpv = (C + VEC - 1) / VEC;
-  int glog = 0;
-  while ((1 << glog) < cpv && glog < 5) ++glog;
-  glog = cb::glog_tuned(glog);
+  const int glog = group_log2((C + VEC - 1) / VEC);
   {
     // small maps: no more blocks than there are pixels to look at (every block of the fused variant
     // passes through one atomic)
@@ -743,28 +698,19 @@ int launch_detect_sparse(cudaStream_t stream, const void* x, long long x_sb, lon
   CB_CHECK_ARG(!fuse || (vec_ok && words <= kCompactWin), "change_detect_sparse_compact: needs pixel-major "
                "tensors and a bitmap of at most %d words", kCompactWin);
   FusedCompact fc = fuse ? *fuse : FusedCompact{nullptr, nullptr, nullptr, nullptr, 0, 0, 0, 0};
-#define CB_DETS(U_)                                                                              \
-  if (vec_ok && fuse)                                                                            \
-    cb::launch(detect_sparse_vec_kernel<T, VEC, U_, true>, grid, 256, 0, stream,                             \
-        (const T*)x, x_sb, x_sy, (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand,      \
-        ncand, bits, H, W, C, Wd, thr, glog, fc);                                                \
-  else if (vec_ok)                                                                               \
-    cb::launch(detect_sparse_vec_kernel<T, VEC, U_, false>, grid, 256, 0, stream,                            \
-        (const T*)x, x_sb, x_sy, (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand,      \
-        ncand, bits, H, W, C, Wd, thr, glog, fc);                                                \
-  else                                                                                           \
-    cb::launch(detect_sparse_generic_kernel<T, U_>, grid, 256, 0, stream,                                    \
-        (const T*)x, x_sb, x_sc, x_sy, x_sx, (T*)state, s_sb, s_sc, s_sy, s_sx, aux, cand,    \
-        ncand, bits, H, W, C, Wd, thr);
-  switch (update) {
-    case CB_UPDATE_NONE: CB_DETS(CB_UPDATE_NONE) break;
-    case CB_UPDATE_CHANGED: CB_DETS(CB_UPDATE_CHANGED) break;
-    case CB_UPDATE_ALL: CB_DETS(CB_UPDATE_ALL) break;
-    default: return fail(2, "change_detect_sparse: bad update_mode %d", update);
-  }
-#undef CB_DETS
-  CB_CHECK_LAUNCH("change_detect_sparse");
-  return 0;
+  return dispatch_update(update, "change_detect_sparse", [&](auto U) {
+    if (vec_ok && fuse)
+      cb::launch(detect_sparse_vec_kernel<T, VEC, U, true>, grid, 256, 0, stream, (const T*)x, x_sb, x_sy,
+                 (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand, ncand, bits, H, W, C, Wd, thr, glog, fc);
+    else if (vec_ok)
+      cb::launch(detect_sparse_vec_kernel<T, VEC, U, false>, grid, 256, 0, stream, (const T*)x, x_sb, x_sy,
+                 (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand, ncand, bits, H, W, C, Wd, thr, glog, fc);
+    else
+      cb::launch(detect_sparse_generic_kernel<T, U>, grid, 256, 0, stream, (const T*)x, x_sb, x_sc, x_sy, x_sx,
+                 (T*)state, s_sb, s_sc, s_sy, s_sx, aux, cand, ncand, bits, H, W, C, Wd, thr);
+    CB_CHECK_LAUNCH("change_detect_sparse");
+    return 0;
+  });
 }
 
 }  // namespace cb

@@ -29,6 +29,39 @@ __device__ __forceinline__ __nv_bfloat16 max_keep(__nv_bfloat16 v, __nv_bfloat16
   return __hgt(u, v) ? u : v;
 }
 
+// The first changed pixel of a 2x2 window (in row-major order) owns it: only the owner recomputes the
+// window.  (b, y, xx) is a changed pixel of the dilated bitmap `bits`.
+__device__ __forceinline__ bool window_owner(const uint32_t* bits, int b, int y, int xx, int H, int W, int Wd) {
+  const long long r = (long long)b * H + y;
+  bool owner = true;
+  if (xx & 1) owner = !bit_at(bits, r, Wd, xx - 1);
+  if (owner && (y & 1)) {
+    const int xe = xx & ~1;
+    owner = !bit_at(bits, r - 1, Wd, xe) && !(xe + 1 < W && bit_at(bits, r - 1, Wd, xe + 1));
+  }
+  return owner;
+}
+
+// Element-wise maximum of the four 16-byte chunks of a 2x2 window
+template <typename T, int VEC>
+__device__ __forceinline__ uint4 window_max16(const uint4& v00, const uint4& v01, const uint4& v10, const uint4& v11) {
+  uint4 res;
+  const T* e00 = reinterpret_cast<const T*>(&v00);
+  const T* e01 = reinterpret_cast<const T*>(&v01);
+  const T* e10 = reinterpret_cast<const T*>(&v10);
+  const T* e11 = reinterpret_cast<const T*>(&v11);
+  T* er = reinterpret_cast<T*>(&res);
+#pragma unroll
+  for (int e = 0; e < VEC; ++e) {
+    T v = max_keep(neg_inf<T>(), e00[e]);
+    v = max_keep(v, e01[e]);
+    v = max_keep(v, e10[e]);
+    v = max_keep(v, e11[e]);
+    er[e] = v;
+  }
+  return res;
+}
+
 template <typename T>
 __global__ void __launch_bounds__(256)
 maxpool2x2_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, long long x_sy,
@@ -46,16 +79,7 @@ maxpool2x2_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, long 
     const int y = p / W, xx = p - y * W;
     const int yo = y >> 1, xo = xx >> 1;
     if (yo >= oH || xo >= oW) continue;
-    if (bits) {                                // first changed pixel of the window owns it
-      const long long r = (long long)b * H + y;
-      bool owner = true;
-      if (xx & 1) owner = !bit_at(bits, r, Wd, xx - 1);
-      if (owner && (y & 1)) {
-        const int xe = xx & ~1;
-        owner = !bit_at(bits, r - 1, Wd, xe) && !(xe + 1 < W && bit_at(bits, r - 1, Wd, xe + 1));
-      }
-      if (!owner) continue;
-    }
+    if (bits && !window_owner(bits, b, y, xx, H, W, Wd)) continue;
     const int y0 = yo * 2, x0 = xo * 2;
     const bool hy = y0 + 1 < H, hx = x0 + 1 < W;
     const T* base = x + b * x_sb + y0 * x_sy + x0 * x_sx;
@@ -74,78 +98,18 @@ maxpool2x2_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, long 
   }
 }
 
-// Pixel-major fast path: a group of G lanes (G = power of two >= chunks per pixel, <= 32) owns one
-// changed pixel, so a warp works on 32/G list entries at once with 16-byte loads/stores; the four
-// window pixels are 4 independent vector loads per lane.
-template <typename T, int VEC>
-__global__ void __launch_bounds__(256)
-maxpool2x2_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int xp,
-                      const int32_t* __restrict__ idx, const int32_t* __restrict__ count,
-                      const uint32_t* __restrict__ bits, T* __restrict__ out, long long o_sb,
-                      long long o_sy, int op, int cpp, int glog, int H, int W, int oH, int oW) {
-  const int n = *count;
-  const int lane = threadIdx.x & 31;
-  const int G = 1 << glog, ppw = 32 >> glog;                // lanes per pixel, pixels per warp
-  const int sub = lane >> glog, gl = lane & (G - 1);
-  const int P = H * W, Wd = (W + 31) >> 5;
-  const long long nwarps = (long long)gridDim.x * (blockDim.x >> 5);
-  for (long long j0 = ((long long)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5)) * ppw;
-       j0 < n; j0 += nwarps * ppw) {
-    const long long j = j0 + sub;
-    if (j >= n) continue;
-    const int pix = __ldg(idx + j);
-    const int b = pix / P, p = pix - b * P;
-    const int y = p / W, xx = p - y * W;
-    const int yo = y >> 1, xo = xx >> 1;
-    if (yo >= oH || xo >= oW) continue;
-    if (bits) {                                // first changed pixel of the window owns it
-      const long long r = (long long)b * H + y;
-      bool owner = true;
-      if (xx & 1) owner = !bit_at(bits, r, Wd, xx - 1);
-      if (owner && (y & 1)) {
-        const int xe = xx & ~1;
-        owner = !bit_at(bits, r - 1, Wd, xe) && !(xe + 1 < W && bit_at(bits, r - 1, Wd, xe + 1));
-      }
-      if (!owner) continue;
-    }
-    const int y0 = yo * 2, x0 = xo * 2;
-    const bool hy = y0 + 1 < H, hx = x0 + 1 < W;
-    const T* base = x + b * x_sb + y0 * x_sy + (long long)x0 * xp;
-    T* o = out + b * o_sb + yo * o_sy + (long long)xo * op;
-    for (int cc = gl; cc < cpp; cc += G) {
-      const T* q = base + cc * VEC;
-      uint4 v00 = ldg16(q), v01 = v00, v10 = v00, v11 = v00;
-      if (hx) v01 = ldg16(q + xp);
-      if (hy) {
-        v10 = ldg16(q + x_sy);
-        v11 = hx ? ldg16(q + x_sy + xp) : v10;
-      }
-      uint4 res;
-      const T* e00 = reinterpret_cast<const T*>(&v00);
-      const T* e01 = reinterpret_cast<const T*>(&v01);
-      const T* e10 = reinterpret_cast<const T*>(&v10);
-      const T* e11 = reinterpret_cast<const T*>(&v11);
-      T* er = reinterpret_cast<T*>(&res);
-#pragma unroll
-      for (int e = 0; e < VEC; ++e) {
-        T v = max_keep(neg_inf<T>(), e00[e]);
-        v = max_keep(v, e01[e]);
-        v = max_keep(v, e10[e]);
-        v = max_keep(v, e11[e]);
-        er[e] = v;
-      }
-      st16(o + cc * VEC, res);
-    }
-  }
-}
-
-// Pool + downstream change detection in one pass (pixel-major only): the lane group that
-// recomputes a pooled pixel still holds its new channel values, so it thresholds them against the
-// NEXT layer's previous-input state right away, ORs the change bit into that layer's (pre-cleared)
-// raw bitmap and maintains its state / operand planes.  Replaces three launches of the candidate
-// path (pool, pooled compaction, sparse detection) and is exact for the same reason candidate
-// detection is: only re-pooled pixels can differ from what the next layer saw last frame.
-template <typename T, int VEC, int UPDATE>
+// Pixel-major 2x2 pooling: a group of G lanes (G = 1 << glog, see group_log2) owns one changed pixel,
+// so a warp works on 32/G list entries at once with 16-byte loads/stores; the four window pixels are 4
+// independent vector loads per lane.
+// DETECT: pool + downstream change detection in one pass: the lane group that recomputes a pooled
+// pixel still holds its new channel values, so it thresholds them against the NEXT layer's
+// previous-input state right away, ORs the change bit into that layer's (pre-cleared) raw bitmap and
+// maintains its state / operand planes.  Replaces three launches of the candidate path (pool, pooled
+// compaction, sparse detection) and is exact for the same reason candidate detection is: only
+// re-pooled pixels can differ from what the next layer saw last frame.  Without DETECT the next-layer
+// arguments and UPDATE are unused, and `bits` may be null (then every listed pixel recomputes its
+// window).
+template <typename T, int VEC, int UPDATE, bool DETECT = true>
 __global__ void __launch_bounds__(256)
 maxpool2x2_detect_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int xp,
                          const int32_t* __restrict__ idx, const int32_t* __restrict__ count,
@@ -155,7 +119,7 @@ maxpool2x2_detect_kernel(const T* __restrict__ x, long long x_sb, long long x_sy
                          uint32_t* __restrict__ nbits, T thr) {
   const int n = *count;
   const int lane = threadIdx.x & 31;
-  const int G = 1 << glog, ppw = 32 >> glog;
+  const int G = 1 << glog, ppw = 32 >> glog;                // lanes per pixel, pixels per warp
   const int sub = lane >> glog, gl = lane & (G - 1);
   const unsigned gmask = (G == 32 ? 0xffffffffu : ((1u << G) - 1u)) << (sub * G);
   const int P = H * W, Wd = (W + 31) >> 5, oWd = (oW + 31) >> 5;
@@ -172,16 +136,9 @@ maxpool2x2_detect_kernel(const T* __restrict__ x, long long x_sb, long long x_sy
       const int y = p / W, xx = p - y * W;
       yo = y >> 1;
       xo = xx >> 1;
-      work = yo < oH && xo < oW;
-      if (work) {                              // first changed pixel of the window owns it
-        const long long r = (long long)b * H + y;
-        if (xx & 1) work = !bit_at(bits, r, Wd, xx - 1);
-        if (work && (y & 1)) {
-          const int xe = xx & ~1;
-          work = !bit_at(bits, r - 1, Wd, xe) && !(xe + 1 < W && bit_at(bits, r - 1, Wd, xe + 1));
-        }
-      }
+      work = yo < oH && xo < oW && (!(DETECT || bits) || window_owner(bits, b, y, xx, H, W, Wd));
     }
+    if (!DETECT && !work) continue;            // (lanes with nothing to pool wait at no ballot)
     const int y0 = yo * 2, x0 = xo * 2;
     const bool hy = y0 + 1 < H, hx = x0 + 1 < W;
     const T* base = x + b * x_sb + y0 * x_sy + (long long)x0 * xp;
@@ -198,26 +155,16 @@ maxpool2x2_detect_kernel(const T* __restrict__ x, long long x_sb, long long x_sy
           v10 = ldg16(q + x_sy);
           v11 = hx ? ldg16(q + x_sy + xp) : v10;
         }
-        const uint4 sv = ld16(ns + cc * VEC);
-        uint4 res;
-        const T* e00 = reinterpret_cast<const T*>(&v00);
-        const T* e01 = reinterpret_cast<const T*>(&v01);
-        const T* e10 = reinterpret_cast<const T*>(&v10);
-        const T* e11 = reinterpret_cast<const T*>(&v11);
-        T* er = reinterpret_cast<T*>(&res);
-#pragma unroll
-        for (int e = 0; e < VEC; ++e) {
-          T v = max_keep(neg_inf<T>(), e00[e]);
-          v = max_keep(v, e01[e]);
-          v = max_keep(v, e10[e]);
-          v = max_keep(v, e11[e]);
-          er[e] = v;
-        }
+        const uint4 sv = DETECT ? ld16(ns + cc * VEC) : uint4{};   // in flight with the window loads
+        const uint4 res = window_max16<T, VEC>(v00, v01, v10, v11);
         st16(o + cc * VEC, res);
-        f |= Chunk<T>::changed(sv, res, thr);
-        if (UPDATE == CB_UPDATE_ALL) store_state<T>(ns + cc * VEC, res, aux, opix, cc * VEC);
+        if (DETECT) {
+          f |= Chunk<T>::changed(sv, res, thr);
+          if (UPDATE == CB_UPDATE_ALL) store_state<T>(ns + cc * VEC, res, aux, opix, cc * VEC);
+        }
       }
     }
+    if (!DETECT) continue;
     const bool chg = (__ballot_sync(0xffffffffu, f) & gmask) != 0u;
     if (work && chg) {
       if (gl == 0) atomicOr(nbits + ((long long)b * oH + yo) * oWd + (xo >> 5), 1u << (xo & 31));
