@@ -17,7 +17,8 @@ from .conv2d_cg import ChangeIndexes
 
 __all__ = ['CBConv2d', 'CBPoolMax2d', 'ChangeIndexes', 'subsitute', 'convertRecur', 'mergeReLURecur',
            'propChangeIndexesOf1x1', 'clearMemory', 'getStateTensors', 'convert',
-           'tuneThresholdParameters', 'convertPools', 'shareWorkspace', 'resetStreams']
+           'tuneThresholdParameters', 'convertPools', 'shareWorkspace', 'resetStreams',
+           'setActiveStreams']
 
 verbose = False
 
@@ -151,6 +152,68 @@ def resetStreams(net, streams):
         host[idx] = 1
         mask = host.to(dev, non_blocking=True)
     _cg.reset_streams(segments, mask)
+
+
+def setActiveStreams(net, streams):
+    """Select the streams of a batched model that have a new frame: from the next frame on, a stream
+    that is not active is skipped.  The dense change scan of every plain-input CB layer (the first
+    layer, and layers behind dense modules such as a torch.cat) neither reads its input slice nor
+    writes its state and reports no change for it, so every later kernel leaves it alone too: its
+    state and outputs stay exactly as they were, and its slice of the input frame may hold anything
+    (need not be uploaded).  Layers fed a change set by an upstream CB layer ignore the mask.  With
+    fixed thresholds, the result equals feeding the skipped streams their previous frame again
+    (DESIGN.md section 3.13).
+
+    `streams`: an iterable of active stream indices, a bool / uint8 CUDA tensor [B] (non-zero =
+    active), or None.  The first call allocates one device uint8 [B] mask and hands it to every
+    CBConv2d under `net`; later calls write into that same buffer on the current stream (a host
+    index list is built on the host and copied asynchronously; a tensor is copied on the device, so
+    that call can be captured in a CUDA graph), so graphs captured with the mask read what was last
+    written before each replay.  An index list needs B: from the mask already set or from the
+    layers' state, so the first call on a model that has not run takes a tensor.  None detaches the
+    mask (every stream active again): graphs captured without a mask never see one, and graphs
+    captured with it must not be replayed after detaching.  The mask's length must equal the
+    frames' batch size (checked at forward).  Fine-grained layers and gatherComputationStats are
+    not supported."""
+    convs = [c for c in _cb_layers(net) if type(c) is CBConv2d]
+    for c in convs:
+        if c.finegrained or (c._auxPlanes is not None and c._auxPlanes[0] == 'fg'):
+            raise CBinferError("setActiveStreams: a fine-grained layer's dense scan (cb_fg_detect) cannot "
+                               "skip streams")
+        if c.gatherComputationStats and streams is not None:
+            raise CBinferError("setActiveStreams: gatherComputationStats reads the whole input")
+    if streams is None:
+        for c in convs:
+            c._activeMask = None
+        return
+    buf = next((c._activeMask for c in convs if c._activeMask is not None), None)
+    if isinstance(streams, torch.Tensor):
+        if not streams.is_cuda:
+            raise CBinferError("setActiveStreams: the stream mask must be a CUDA tensor (got one on %s)"
+                               % streams.device)
+        if streams.dim() != 1 or streams.dtype not in (torch.bool, torch.uint8):
+            raise CBinferError("setActiveStreams: the mask must be a bool or uint8 tensor [B], got %s %s"
+                               % (streams.dtype, tuple(streams.shape)))
+        if buf is None or buf.numel() != streams.numel() or buf.device != streams.device:
+            buf = torch.empty(streams.numel(), dtype=torch.uint8, device=streams.device)
+        buf.copy_(streams)
+    else:
+        if buf is None:
+            state = [c._inBuf for c in convs if c._inBuf is not None]
+            if not state:
+                raise CBinferError("setActiveStreams: the model has not run yet, so the number of streams is "
+                                   "unknown; pass a CUDA mask tensor [B]")
+            buf = torch.empty(state[0].shape[0], dtype=torch.uint8, device=state[0].device)
+        B = buf.numel()
+        idx = [int(i) for i in streams]
+        bad = [i for i in idx if not 0 <= i < B]
+        if bad:
+            raise CBinferError("setActiveStreams: stream indices %s out of range for %d streams" % (bad, B))
+        host = torch.zeros(B, dtype=torch.uint8)
+        host[idx] = 1
+        buf.copy_(host, non_blocking=True)
+    for c in convs:
+        c._activeMask = buf
 
 
 def getStateTensors(net):

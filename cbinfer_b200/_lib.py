@@ -24,6 +24,7 @@ _DTYPES = {torch.float32: F32, torch.float16: F16, torch.bfloat16: BF16}
 SYMBOLS = [
     "cb_version", "cb_last_error", "cb_device_info", "cb_bitmap_row_words", "cb_bitmap_words",
     "cb_compact_ws_bytes", "cb_channel_pitch", "cb_plane_pitch16", "cb_packed_weight_bytes", "cb_change_detect", "cb_change_detect_u8",
+    "cb_change_detect_streams", "cb_change_detect_u8_streams",
     "cb_dilate_compact", "cb_map_to_bits", "cb_change_detect_sparse", "cb_pool_compact", "cb_maxpool2x2_detect",
     "cb_pack_weights", "cb_conv_ws_bytes", "cb_conv_update", "cb_conv_update_masked", "cb_maxpool2x2",
     "cb_gen_xmatrix", "cb_matrix_mult", "cb_update_output", "cb_fg_update",
@@ -69,6 +70,10 @@ def _load():
                                    vp, i32, i32, i32, i32, f32, i32]),
         "cb_change_detect_u8": (i32, [vp, vp, i64, i64, i64, i64, vp, i64, i64, i64, i64, i32, vp, vp, vp,
                                       i32, i32, i32, i32, f32, f32, f32, i32]),
+        "cb_change_detect_streams": (i32, [vp, i32, vp, i64, i64, i64, i64, vp, i64, i64, i64, i64, i32, vp, vp,
+                                           vp, i32, i32, i32, i32, f32, i32, vp]),
+        "cb_change_detect_u8_streams": (i32, [vp, vp, i64, i64, i64, i64, vp, i64, i64, i64, i64, i32, vp, vp, vp,
+                                              i32, i32, i32, i32, f32, f32, f32, i32, vp]),
         "cb_dilate_compact": (i32, [vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32]),
         "cb_tile_ws_bytes": (sz, [i32, i32, i32]),
         "cb_dilate_compact_tiles": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, i32, i32, i32, i32, i32, i32]),

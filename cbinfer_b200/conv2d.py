@@ -231,6 +231,7 @@ class CBConv2d(nn.Module):
         self._fusedTail = None
         self._inVersion = None    # prevInput._version / prevOutput._version as the kernels last left them
         self._outVersion = None
+        self._activeMask = None   # active-stream mask (cbinfer_b200.setActiveStreams), None = all
         self._wsHolder = cg.ConvWorkspace()    # shared per model by pycbinfer.convert()
         self.register_buffer('prevInput', self.weight.data.new_empty(0))
         self.register_buffer('prevOutput', self.weight.data.new_empty(0))
@@ -264,7 +265,7 @@ class CBConv2d(nn.Module):
         # no fused neighbours, and without a version record the state counts as touched
         super(CBConv2d, self).__setstate__(state)
         self._setDefaultValues()
-        for name in ('_fusedPool', '_fusedTail', '_inVersion', '_outVersion'):
+        for name in ('_fusedPool', '_fusedTail', '_inVersion', '_outVersion', '_activeMask'):
             self.__dict__.setdefault(name, None)
 
     # ---- state ---------------------------------------------------------------------------
@@ -505,6 +506,9 @@ class CBConv2d(nn.Module):
         s = self._scratch
 
         if self.gatherComputationStats:
+            if self._activeMask is not None:
+                raise _lib.CBinferError("gatherComputationStats reads the whole input: it cannot be combined "
+                                        "with an active-stream mask (setActiveStreams)")
             self._gatherStats(input)
 
         gemm, packed, bias32 = self._weights(dt, dev)
@@ -550,8 +554,11 @@ class CBConv2d(nn.Module):
             mode = _lib.UPDATE_CHANGED if self.feedbackLoop else _lib.UPDATE_ALL
             sparse_next = self.candidateDetect and not plain_input
             if not detected:     # (else the upstream pool kernel already did it)
+                # only the dense scan of a plain input skips inactive streams: a layer fed a change set
+                # must keep its full scans whole (see setActiveStreams)
+                active = self._streamMask(B) if plain_input else None
                 changeIndexes, mask = self._detect(input, candidates, u8norm, mode, aux, gemm, use_tiles,
-                                                   sparse_next)
+                                                   sparse_next, active)
             if changeIndexes is None:
                 changeIndexes = self._compact(s, B, H, W, sparse_next, tiles=use_tiles,
                                               lazy=pool_args is not None and not self.saveChangeMap)
@@ -588,9 +595,10 @@ class CBConv2d(nn.Module):
             changeIndexes.complete = not ext_out
         return self._frameDone(changeIndexes, changeIndexes if self.propChangeIndexes else None)
 
-    def _detect(self, input, candidates, u8norm, mode, aux, gemm, use_tiles, sparse_next):
+    def _detect(self, input, candidates, u8norm, mode, aux, gemm, use_tiles, sparse_next, active=None):
         """Dense scan, or the test of the `candidates` only.  Returns (change list if the launch
-        built one, mask of the masked contraction), each or both None."""
+        built one, mask of the masked contraction), each or both None.  `active`: the active-stream
+        mask the dense scan honours, or None."""
         B, _, H, W = input.shape
         s = self._scratch
         # extension: no compaction at all for a 1x1 layer on the candidate path - the
@@ -624,11 +632,19 @@ class CBConv2d(nn.Module):
                 changes.superset = True
         elif u8norm is not None:
             cg.detect_u8(input, self.prevInput, s["raw_bits"], self.threshold, mode,
-                         u8norm[0], u8norm[1], aux=aux)
+                         u8norm[0], u8norm[1], aux=aux, active=active)
         else:
-            cg.detect(input, self.prevInput, s["raw_bits"], self.threshold, mode, aux=aux)
+            cg.detect(input, self.prevInput, s["raw_bits"], self.threshold, mode, aux=aux, active=active)
         self._recordDetection()
         return changes, mask
+
+    def _streamMask(self, B):
+        """The active-stream mask for a frame of B streams, or None when none is set."""
+        m = self._activeMask
+        if m is not None and m.numel() != B:
+            raise _lib.CBinferError("active-stream mask of %d streams, the frame has %d (setActiveStreams)"
+                                    % (m.numel(), B))
+        return m
 
     # ---- two chained 1x1 layers in one launch (extension) ------------------------------------------
     def _tailReady(self, shape, dtype, device):
@@ -715,9 +731,10 @@ class CBConv2d(nn.Module):
             if norm is None or self.in_channels > 4:
                 raise _lib.CBinferError("detectInput: uint8 input needs inputNorm and <= 4 channels")
             cg.detect_u8(input, self.prevInput, self._scratch["raw_bits"], self.threshold, mode,
-                         norm[0], norm[1], aux=aux)
+                         norm[0], norm[1], aux=aux, active=self._streamMask(input.shape[0]))
         else:
-            cg.detect(input, self.prevInput, self._scratch["raw_bits"], self.threshold, mode, aux=aux)
+            cg.detect(input, self.prevInput, self._scratch["raw_bits"], self.threshold, mode, aux=aux,
+                      active=self._streamMask(input.shape[0]))
         self._recordDetection()
         return 'changeIndexes', input, DetectionDone(self, dense=True)
 
@@ -777,6 +794,8 @@ class CBConv2d(nn.Module):
         with torch.no_grad():
             if self.finegrained:
                 assert(self.feedbackLoop == False)
+                if self._activeMask is not None:
+                    raise _lib.CBinferError("an active-stream mask is not supported on a fine-grained layer")
                 return self.forward_fg(inp)
             else:
                 return self.forward_normal(inp)

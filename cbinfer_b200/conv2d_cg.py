@@ -124,30 +124,49 @@ def _aux_args(aux, state):
     return _lib.AUX_BF16_PAIR, aux[1].data_ptr(), aux[2].data_ptr()
 
 
-def detect(x, state, raw_bits, threshold, update_mode, aux=None):
+def _active_ptr(active, B, device):
+    """Device pointer of an active-stream mask (a contiguous bool / uint8 CUDA tensor [B] on x's
+    device), or None for no mask (every stream active)."""
+    if active is None:
+        return None
+    require_cuda(active)
+    if active.dim() != 1 or active.dtype not in (torch.bool, torch.uint8) or not active.is_contiguous():
+        raise _lib.CBinferError("active-stream mask: a contiguous bool or uint8 tensor [B] is needed, got %s %s"
+                                % (active.dtype, tuple(active.shape)))
+    if active.numel() != B or active.device != device:
+        raise _lib.CBinferError("active-stream mask: %d entries on %s for %d streams on %s"
+                                % (active.numel(), active.device, B, device))
+    return active.data_ptr()
+
+
+def detect(x, state, raw_bits, threshold, update_mode, aux=None, active=None):
     """cb_change_detect: raw (un-dilated) change bitmap of x vs state; updates state and, when
-    given, the auxiliary operand planes `aux` (see _aux_args)."""
+    given, the auxiliary operand planes `aux` (see _aux_args).  `active`: optional bool / uint8
+    CUDA tensor [B], read on the device; a stream with active[b] == 0 is skipped (its bitmap words
+    0, its x not read, its state and planes untouched: cb_change_detect_streams)."""
     require_cuda(x, state, raw_bits)
     B, Cc, H, W = x.shape
     assert state.shape == x.shape and state.dtype == x.dtype
+    act = _active_ptr(active, B, x.device)
     mode, hi, lo = _aux_args(aux, state)
-    check(C.cb_change_detect(stream_ptr(x.device), dtype_code(x), x.data_ptr(), *_strides4(x),
-                             state.data_ptr(), *_strides4(state), mode, hi, lo,
-                             raw_bits.data_ptr(), B, Cc, H, W, float(threshold), int(update_mode)))
+    check(C.cb_change_detect_streams(stream_ptr(x.device), dtype_code(x), x.data_ptr(), *_strides4(x),
+                                     state.data_ptr(), *_strides4(state), mode, hi, lo,
+                                     raw_bits.data_ptr(), B, Cc, H, W, float(threshold), int(update_mode), act))
 
 
-def detect_u8(x, state, raw_bits, threshold, update_mode, divisor, bias, aux=None):
+def detect_u8(x, state, raw_bits, threshold, update_mode, divisor, bias, aux=None, active=None):
     """cb_change_detect_u8: detection on a uint8 frame normalised on the fly as u8/divisor + bias
     (the readers' /255 resp. /256 - 0.5); `state` is the fp32 pixel-major state.  Bit-identical to
-    :func:`detect` on ``x.float() / divisor + bias``."""
+    :func:`detect` on ``x.float() / divisor + bias``.  `active` as in :func:`detect`."""
     require_cuda(x, state, raw_bits)
     B, Cc, H, W = x.shape
     assert x.dtype == torch.uint8 and state.dtype == torch.float32 and state.shape == x.shape
+    act = _active_ptr(active, B, x.device)
     mode, hi, lo = _aux_args(aux, state)
-    check(C.cb_change_detect_u8(stream_ptr(x.device), x.data_ptr(), *_strides4(x),
-                                state.data_ptr(), *_strides4(state), mode, hi, lo,
-                                raw_bits.data_ptr(), B, Cc, H, W, float(divisor), float(bias),
-                                float(threshold), int(update_mode)))
+    check(C.cb_change_detect_u8_streams(stream_ptr(x.device), x.data_ptr(), *_strides4(x),
+                                        state.data_ptr(), *_strides4(state), mode, hi, lo,
+                                        raw_bits.data_ptr(), B, Cc, H, W, float(divisor), float(bias),
+                                        float(threshold), int(update_mode), act))
 
 
 def detect_sparse(x, state, raw_bits, threshold, update_mode, candidates, aux=None,

@@ -85,18 +85,39 @@ int cb_channel_pitch(int dtype, int C) {
   return (C + v - 1) / v * v;
 }
 
-int cb_change_detect(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
-                     long long x_sy, long long x_sx, void* state, long long s_sb, long long s_sc,
-                     long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
-                     uint32_t* raw_bits, int B, int C, int H, int W, float threshold,
-                     int update_mode) {
+int cb_change_detect_streams(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
+                             long long x_sy, long long x_sx, void* state, long long s_sb, long long s_sc,
+                             long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
+                             uint32_t* raw_bits, int B, int C, int H, int W, float threshold,
+                             int update_mode, const uint8_t* active) {
   CB_CHECK_ARG(x && state && raw_bits, "change_detect: null pointer");
   CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect: bad shape");
   CB_DISPATCH_DTYPE(dtype, return (launch_detect<T, VEC>((cudaStream_t)stream, x, x_sb, x_sc, x_sy,
                                                         x_sx, state, s_sb, s_sc, s_sy, s_sx, aux_mode,
                                                         aux_hi, aux_lo, raw_bits, B, C, H, W, threshold,
-                                                        update_mode)));
+                                                        update_mode, active)));
   return 0;
+}
+
+int cb_change_detect(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
+                     long long x_sy, long long x_sx, void* state, long long s_sb, long long s_sc,
+                     long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
+                     uint32_t* raw_bits, int B, int C, int H, int W, float threshold,
+                     int update_mode) {
+  return cb_change_detect_streams(stream, dtype, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy, s_sx,
+                                  aux_mode, aux_hi, aux_lo, raw_bits, B, C, H, W, threshold, update_mode, nullptr);
+}
+
+int cb_change_detect_u8_streams(void* stream, const uint8_t* x, long long x_sb, long long x_sc,
+                                long long x_sy, long long x_sx, float* state, long long s_sb, long long s_sc,
+                                long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
+                                uint32_t* raw_bits, int B, int C, int H, int W, float divisor, float bias,
+                                float threshold, int update_mode, const uint8_t* active) {
+  CB_CHECK_ARG(x && state && raw_bits, "change_detect_u8: null pointer");
+  CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect_u8: bad shape");
+  return launch_detect_u8((cudaStream_t)stream, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy,
+                          s_sx, aux_mode, aux_hi, aux_lo, raw_bits, B, C, H, W, divisor, bias,
+                          threshold, update_mode, active);
 }
 
 int cb_change_detect_u8(void* stream, const uint8_t* x, long long x_sb, long long x_sc,
@@ -104,11 +125,9 @@ int cb_change_detect_u8(void* stream, const uint8_t* x, long long x_sb, long lon
                         long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
                         uint32_t* raw_bits, int B, int C, int H, int W, float divisor, float bias,
                         float threshold, int update_mode) {
-  CB_CHECK_ARG(x && state && raw_bits, "change_detect_u8: null pointer");
-  CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect_u8: bad shape");
-  return launch_detect_u8((cudaStream_t)stream, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy,
-                          s_sx, aux_mode, aux_hi, aux_lo, raw_bits, B, C, H, W, divisor, bias,
-                          threshold, update_mode);
+  return cb_change_detect_u8_streams(stream, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy, s_sx, aux_mode,
+                                     aux_hi, aux_lo, raw_bits, B, C, H, W, divisor, bias, threshold, update_mode,
+                                     nullptr);
 }
 
 size_t cb_tile_ws_bytes(int B, int H, int W) { return cb::tile_ws_words(B, H, W) * sizeof(int32_t); }

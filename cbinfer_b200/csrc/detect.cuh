@@ -11,6 +11,11 @@
 //   * narrow path (any x strides, state pixel = one 16-byte chunk, e.g. the RGB input frame).
 //   * generic path (any strides on both sides).
 // HBM-bound: algorithmic bytes = 2*C*P*s read (+ P/8 bitmap, + feedback writes).
+//
+// Active-stream mask (`active`, uint8 [B] on the device, may be null = every stream): the dense
+// kernels decide per bitmap word (a word never spans two images, rows are padded to whole words).
+// A word of a stream with active[b] == 0 is written as 0 and nothing of that stream's x, state or
+// operand planes is loaded or stored; every block barrier is still reached by all threads.
 #pragma once
 #include "cb_common.cuh"
 #include "compact.cuh"
@@ -138,17 +143,17 @@ __global__ void __launch_bounds__(kDetWarps * 32)
 detect_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int xp,
                   T* __restrict__ st, long long s_sb, long long s_sy, int sp, AuxPlanes aux,
                   uint32_t* __restrict__ bits, int B, int H, int W, int C, int Wd, T thr,
-                  unsigned cpv_magic, int wlog) {
+                  unsigned cpv_magic, int wlog, const uint8_t* __restrict__ active) {
   __shared__ unsigned s_word[kDetWarps];
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int wpw = 1 << wlog;
   const int part = wid & (wpw - 1), slot = wid >> wlog;
   const int word = blockIdx.x * (kDetWarps >> wlog) + slot;      // < 2^31 words (host-checked)
-  const bool active = word < B * H * Wd;
+  const bool inmap = word < B * H * Wd;
   if (wlog > 0) {
     if (threadIdx.x < kDetWarps) s_word[threadIdx.x] = 0u;
     __syncthreads();
-  } else if (!active) {
+  } else if (!inmap) {
     return;
   }
   const int cpv = (C + VEC - 1) / VEC;       // 16-byte chunks per pixel that hold real channels
@@ -160,7 +165,7 @@ detect_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int x
   int nq = 0;
   long long pixbase = 0;
   unsigned wordbits = 0;
-  if (active) {
+  if (inmap) {
     const int j = word % Wd;
     const int r = word / Wd;
     const int y = r % H;
@@ -169,7 +174,7 @@ detect_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int x
     const int npx = min(32, W - x0);
     xb = x + b * x_sb + y * x_sy + (long long)x0 * xp;
     sb = st + b * s_sb + y * s_sy + (long long)x0 * sp;
-    nq = npx * cpv;
+    nq = (active && !__ldg(active + b)) ? 0 : npx * cpv;   // skipped stream: no loads, word 0
     pixbase = ((long long)b * H + y) * W + x0;
 
     bool mychg = false;                      // flag of pixel `lane` (this warp's slice only)
@@ -212,10 +217,10 @@ detect_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int x
     wordbits = __ballot_sync(0xffffffffu, mychg);
   }
   if (wlog > 0) {                              // OR the partial words of the warps sharing a word
-    if (active && lane == 0 && wordbits) atomicOr(&s_word[slot], wordbits);
+    if (inmap && lane == 0 && wordbits) atomicOr(&s_word[slot], wordbits);
     __syncthreads();
     wordbits = s_word[slot];
-    if (!active) return;
+    if (!inmap) return;
   }
   if (part == 0 && lane == 0) bits[word] = wordbits;
 
@@ -246,7 +251,7 @@ __global__ void __launch_bounds__(256)
 detect_narrow_kernel(const S* __restrict__ x, long long x_sb, long long x_sc, long long x_sy,
                      long long x_sx, T* __restrict__ st, long long s_sb, long long s_sy,
                      AuxPlanes aux, uint32_t* __restrict__ bits, int B, int H, int W, int C,
-                     int Wd, T thr, float divisor, float bias) {
+                     int Wd, T thr, float divisor, float bias, const uint8_t* __restrict__ active) {
   constexpr bool kU8 = std::is_same<S, uint8_t>::value;
   const float* lut = nullptr;
   if constexpr (kU8) {
@@ -262,7 +267,7 @@ detect_narrow_kernel(const S* __restrict__ x, long long x_sb, long long x_sc, lo
   int b, y, xx;
   if (!warp_word(warp, b, y, xx, B, H, Wd)) return;
   bool f = false;
-  if (xx < W) {
+  if (xx < W && (!active || __ldg(active + b))) {
     const S* xp = x + b * x_sb + y * x_sy + xx * x_sx;
     T* sp = st + b * s_sb + y * s_sy + (long long)xx * VEC;
     const uint4 sv = ld16_stream(sp);
@@ -296,13 +301,13 @@ detect_narrow_kernel(const S* __restrict__ x, long long x_sb, long long x_sc, lo
 constexpr int kPlanarMaxWords = 8;
 struct PlanarWord {
   long long xoff, soff, pix;     // element offsets of the word's first pixel in x / the state, global pixel index
-  int npx;                       // valid pixels (0: word beyond the map)
+  int npx;                       // valid pixels (0: word beyond the map, -1: word of a skipped stream)
 };
 
 __device__ __forceinline__ void planar_words_setup(PlanarWord* wi, unsigned* s_word, int word0, int nw,
                                                    long long nwords, int H, int W, int Wd, long long x_sb,
                                                    long long x_sy, long long x_sx, long long s_sb,
-                                                   long long s_sy, int sp) {
+                                                   long long s_sy, int sp, const uint8_t* active = nullptr) {
   if (threadIdx.x < (unsigned)nw) {
     const long long word = (long long)word0 + threadIdx.x;
     PlanarWord w = {0, 0, 0, 0};
@@ -312,7 +317,9 @@ __device__ __forceinline__ void planar_words_setup(PlanarWord* wi, unsigned* s_w
       const int y = (int)(r % H);
       const long long b = r / H;
       const int x0 = j * 32;
-      w.npx = min(32, W - x0);
+      // npx = -1: a word of a skipped stream; nothing of it is loaded, tested or stored, but it is
+      // written (as 0), unlike a word beyond the map (npx = 0)
+      w.npx = (active && !__ldg(active + b)) ? -1 : min(32, W - x0);
       w.xoff = b * x_sb + y * x_sy + x0 * x_sx;
       w.soff = b * s_sb + y * s_sy + (long long)x0 * sp;
       w.pix = (b * H + y) * W + x0;
@@ -363,14 +370,14 @@ __global__ void __launch_bounds__(256)
 detect_planar_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, long long x_sy,
                      T* __restrict__ st, long long s_sb, long long s_sy, int sp, AuxPlanes aux,
                      uint32_t* __restrict__ bits, int B, int H, int W, int C, int Wd, T thr,
-                     unsigned cpv_magic, int cps, int nw) {
+                     unsigned cpv_magic, int cps, int nw, const uint8_t* __restrict__ active) {
   extern __shared__ __align__(16) unsigned char dp_smem[];
   uint4* xs = reinterpret_cast<uint4*>(dp_smem);                 // [nw*32][cps]
   __shared__ unsigned s_word[kPlanarMaxWords];
   __shared__ PlanarWord wi[kPlanarMaxWords];
   const long long nwords = (long long)B * H * Wd;
   const int word0 = blockIdx.x * nw;
-  planar_words_setup(wi, s_word, word0, nw, nwords, H, W, Wd, x_sb, x_sy, 1, s_sb, s_sy, sp);
+  planar_words_setup(wi, s_word, word0, nw, nwords, H, W, Wd, x_sb, x_sy, 1, s_sb, s_sy, sp, active);
   const int cpv = (C + VEC - 1) / VEC, tail = C % VEC;
   planar_load_tile<T, VEC>(xs, wi, x, x_sc, 1, nw, cpv, cps, C, cpv_magic);
   __syncthreads();
@@ -392,7 +399,7 @@ detect_planar_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, lo
     planar_flag(s_word, w, m);
   }
   __syncthreads();
-  if (threadIdx.x < (unsigned)nw && wi[threadIdx.x].npx > 0) bits[word0 + threadIdx.x] = s_word[threadIdx.x];
+  if (threadIdx.x < (unsigned)nw && wi[threadIdx.x].npx != 0) bits[word0 + threadIdx.x] = s_word[threadIdx.x];
   if (UPDATE == CB_UPDATE_CHANGED) {              // feedback: accept the new value at changed pixels
     for (int q = threadIdx.x; q < nq; q += 256) {
       const int t = cpv == 1 ? q : (int)__umulhi((unsigned)q, cpv_magic), cc = q - t * cpv;
@@ -421,11 +428,12 @@ __global__ void __launch_bounds__(256)
 detect_generic_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, long long x_sy,
                       long long x_sx, T* __restrict__ st, long long s_sb, long long s_sc,
                       long long s_sy, long long s_sx, AuxPlanes aux,
-                      uint32_t* __restrict__ bits, int B, int H, int W, int C, int Wd, T thr) {
+                      uint32_t* __restrict__ bits, int B, int H, int W, int C, int Wd, T thr,
+                      const uint8_t* __restrict__ active) {
   unsigned warp;
   int b, y, xx;
   if (!warp_word(warp, b, y, xx, B, H, Wd)) return;
-  const bool f = xx < W && pixel_changed_scalar<T, UPDATE>(x + b * x_sb + y * x_sy + xx * x_sx, x_sc,
+  const bool f = xx < W && (!active || __ldg(active + b)) && pixel_changed_scalar<T, UPDATE>(x + b * x_sb + y * x_sy + xx * x_sx, x_sc,
                                                             st + b * s_sb + y * s_sy + xx * s_sx, s_sc, C,
                                                             thr, aux, ((long long)b * H + y) * W + xx);
   const unsigned word = __ballot_sync(0xffffffffu, f);
@@ -479,7 +487,8 @@ template <typename T, int VEC>
 int launch_detect(cudaStream_t stream, const void* x, long long x_sb, long long x_sc,
                   long long x_sy, long long x_sx, void* state, long long s_sb, long long s_sc,
                   long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
-                  uint32_t* bits, int B, int C, int H, int W, float threshold, int update) {
+                  uint32_t* bits, int B, int C, int H, int W, float threshold, int update,
+                  const uint8_t* active) {
   const int Wd = (W + 31) / 32;
   const long long words = (long long)B * H * Wd;
   if (words == 0) return 0;
@@ -511,23 +520,23 @@ int launch_detect(cudaStream_t stream, const void* x, long long x_sb, long long 
     if (vec_ok) {
       if (cpv >= 4)
         cb::launch(detect_vec_kernel<T, VEC, U, 4>, grid, block, 0, stream, (const T*)x, x_sb, x_sy, (int)x_sx,
-                   (T*)state, s_sb, s_sy, (int)s_sx, aux, bits, B, H, W, C, Wd, thr, magic, wlog);
+                   (T*)state, s_sb, s_sy, (int)s_sx, aux, bits, B, H, W, C, Wd, thr, magic, wlog, active);
       else
         cb::launch(detect_vec_kernel<T, VEC, U, 2>, grid, block, 0, stream, (const T*)x, x_sb, x_sy, (int)x_sx,
-                   (T*)state, s_sb, s_sy, (int)s_sx, aux, bits, B, H, W, C, Wd, thr, magic, wlog);
+                   (T*)state, s_sb, s_sy, (int)s_sx, aux, bits, B, H, W, C, Wd, thr, magic, wlog, active);
     } else if (narrow_ok) {
       cb::launch(detect_narrow_kernel<T, VEC, U>, grid, block, 0, stream, (const T*)x, x_sb, x_sc, x_sy, x_sx,
-                 (T*)state, s_sb, s_sy, aux, bits, B, H, W, C, Wd, thr, 0.f, 0.f);
+                 (T*)state, s_sb, s_sy, aux, bits, B, H, W, C, Wd, thr, 0.f, 0.f, active);
     } else if (planar_ok) {
       if (planar_smem > 48 * 1024)
         cudaFuncSetAttribute(detect_planar_kernel<T, VEC, U>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)planar_smem);
       cb::launch(detect_planar_kernel<T, VEC, U>, dim3((unsigned)((words + planar_nw - 1) / planar_nw)), block,
                  planar_smem, stream, (const T*)x, x_sb, x_sc, x_sy, (T*)state, s_sb, s_sy, (int)s_sx, aux, bits,
-                 B, H, W, C, Wd, thr, magic, cps, planar_nw);
+                 B, H, W, C, Wd, thr, magic, cps, planar_nw, active);
     } else {
       cb::launch(detect_generic_kernel<T, U>, grid, block, 0, stream, (const T*)x, x_sb, x_sc, x_sy, x_sx,
-                 (T*)state, s_sb, s_sc, s_sy, s_sx, aux, bits, B, H, W, C, Wd, thr);
+                 (T*)state, s_sb, s_sc, s_sy, s_sx, aux, bits, B, H, W, C, Wd, thr, active);
     }
     CB_CHECK_LAUNCH("change_detect");
     return 0;
@@ -539,7 +548,8 @@ inline int launch_detect_u8(cudaStream_t stream, const void* x, long long x_sb, 
                             long long x_sy, long long x_sx, void* state, long long s_sb,
                             long long s_sc, long long s_sy, long long s_sx, int aux_mode,
                             void* aux_hi, void* aux_lo, uint32_t* bits, int B, int C, int H, int W,
-                            float divisor, float bias, float threshold, int update) {
+                            float divisor, float bias, float threshold, int update,
+                            const uint8_t* active) {
   const int Wd = (W + 31) / 32;
   const long long words = (long long)B * H * Wd;
   if (words == 0) return 0;
@@ -554,7 +564,7 @@ inline int launch_detect_u8(cudaStream_t stream, const void* x, long long x_sb, 
   return dispatch_update(update, "change_detect_u8", [&](auto U) {
     cb::launch(detect_narrow_kernel<float, 4, U, uint8_t>, dim3((unsigned)blocks), dim3(256), 0, stream,
                (const uint8_t*)x, x_sb, x_sc, x_sy, x_sx, (float*)state, s_sb, s_sy, aux, bits, B, H, W, C, Wd,
-               threshold, divisor, bias);
+               threshold, divisor, bias, active);
     CB_CHECK_LAUNCH("change_detect_u8");
     return 0;
   });

@@ -9,6 +9,8 @@ kernels are fast: a 640x480 fp32 frame is 3.7 MB of PCIe traffic.
 """
 import torch
 
+from ._lib import CBinferError
+
 
 class FrameGraph(object):
     """Capture ``model(static_input)`` once; ``replay()`` re-runs it on whatever the caller copied
@@ -36,9 +38,16 @@ class FramePipeline(object):
     """Feed pinned host frames through a converted model with copies overlapped with compute.
 
     depth input slots, each with its own captured graph of the same model (the model's state is
-    shared, so graphs replay strictly in submission order on the compute stream)."""
+    shared, so graphs replay strictly in submission order on the compute stream).
 
-    def __init__(self, model, example_frame, depth=2):
+    activeStreams=True: ``submit(frame, active)`` may name the streams that have a new frame; only
+    their slices cross PCIe and the others are skipped by the model (cbinfer_b200.setActiveStreams).
+    The constructor sets an all-active mask on the model before capturing the graphs, and refuses a
+    model in which a module other than a CB layer reads the input frame directly: the input slot of
+    a skipped stream holds a stale frame, which only the mask-honouring CB layers may be given."""
+
+    def __init__(self, model, example_frame, depth=2, activeStreams=False):
+        from . import CBConv2d, CBPoolMax2d, setActiveStreams
         dev = example_frame.device
         assert dev.type == "cuda"
         self.model = model
@@ -47,10 +56,29 @@ class FramePipeline(object):
         self.h2d = torch.cuda.Stream(dev)
         self.d2h = torch.cuda.Stream(dev)
         self.inputs = [example_frame.clone() for _ in range(depth)]
+        B = example_frame.shape[0]
+        self._mask = None
         cur = torch.cuda.current_stream(dev)
         self.compute.wait_stream(cur)
+        readers, hooks = [], []
+        if activeStreams:
+            def pre_hook(mod, args):
+                if any(isinstance(a, torch.Tensor) and a.data_ptr() == self.inputs[0].data_ptr() for a in args):
+                    readers.append(type(mod).__name__)
+            hooks = [m.register_forward_pre_hook(pre_hook) for m in model.modules()
+                     if not list(m.children()) and type(m) not in (CBConv2d, CBPoolMax2d)]
         with torch.cuda.stream(self.compute), torch.no_grad():
-            probe = model(self.inputs[0])                 # allocates state on first use
+            if activeStreams:
+                setActiveStreams(model, torch.ones(B, dtype=torch.uint8, device=dev))
+                self._mask = next(c._activeMask for c in model.modules() if type(c) is CBConv2d)
+            try:
+                probe = model(self.inputs[0])                 # allocates state on first use
+            finally:
+                for h in hooks:
+                    h.remove()
+            if readers:
+                raise CBinferError("FramePipeline(activeStreams=True): %s read the input frame directly; a "
+                                   "skipped stream's slice of it is stale" % sorted(set(readers)))
             if isinstance(probe, tuple) and probe and probe[0] == 'changeIndexes':
                 probe = probe[1]
             self.graphs = [FrameGraph(model, x, warmup=True) for x in self.inputs]
@@ -65,22 +93,61 @@ class FramePipeline(object):
         self.in_ready = [torch.cuda.Event() for _ in range(depth)]
         self.out_ready = [torch.cuda.Event() for _ in range(depth)]   # device-side result copied
         self.out_done = [torch.cuda.Event() for _ in range(depth)]    # host buffer filled
+        if activeStreams:
+            # per-slot staging of the mask in pinned host and in device memory: it travels with the
+            # slot's frame on the copy stream, and the device mask that every graph reads is written
+            # from it on the compute stream right before the slot's replay (writing the shared
+            # buffer on the copy stream would race with the previous slot's replay)
+            self.mask_host = [torch.ones(B, dtype=torch.uint8).pin_memory() for _ in range(depth)]
+            self.mask_dev = [torch.ones(B, dtype=torch.uint8, device=dev) for _ in range(depth)]
         self.t = 0
         for e in self.in_free + self.out_done:
             e.record(self.compute)
 
-    def submit(self, host_frame):
+    def submit(self, host_frame, active=None):
         """Queue one frame (pinned host tensor); returns the slot whose host result buffer will
-        hold this frame's output once `wait(slot)` returns."""
+        hold this frame's output once `wait(slot)` returns.
+
+        `active` (activeStreams=True only): the indices of the streams that have a new frame, None =
+        all.  Only their slices of `host_frame` are copied (one copy per contiguous run); the other
+        streams are skipped and their rows of the result hold their previous output."""
+        B = self.inputs[0].shape[0]
+        if active is None:
+            keep = [True] * B
+        else:
+            if self._mask is None:
+                raise CBinferError("FramePipeline.submit(active=...) needs FramePipeline(activeStreams=True)")
+            idx = [int(i) for i in active]
+            if any(not 0 <= i < B for i in idx):
+                raise CBinferError("FramePipeline.submit: stream indices %s out of range for %d streams" % (idx, B))
+            keep = [False] * B
+            for i in idx:
+                keep[i] = True
         s = self.t % self.depth
         self.t += 1
+        if self._mask is not None:
+            self.in_ready[s].synchronize()                 # the slot's last upload has read the staging
+            self.mask_host[s].copy_(torch.tensor(keep, dtype=torch.uint8))
         with torch.cuda.stream(self.h2d):
             self.h2d.wait_event(self.in_free[s])
-            self.inputs[s].copy_(host_frame, non_blocking=True)
+            b = 0
+            while b < B:                                   # one copy per contiguous run of active streams
+                if not keep[b]:
+                    b += 1
+                    continue
+                e = b
+                while e < B and keep[e]:
+                    e += 1
+                self.inputs[s][b:e].copy_(host_frame[b:e], non_blocking=True)
+                b = e
+            if self._mask is not None:
+                self.mask_dev[s].copy_(self.mask_host[s], non_blocking=True)
             self.in_ready[s].record(self.h2d)
         with torch.cuda.stream(self.compute):
             self.compute.wait_event(self.in_ready[s])
             self.compute.wait_event(self.out_done[s])      # previous D2H of this slot finished
+            if self._mask is not None:
+                self._mask.copy_(self.mask_dev[s])
             out = self.graphs[s].replay()
             self.in_free[s].record(self.compute)
             self.out_dev[s].copy_(out[0] if self._multi else out)

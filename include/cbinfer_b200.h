@@ -101,6 +101,27 @@ int cb_change_detect_u8(void* stream, const uint8_t* x, long long x_sb, long lon
                         uint32_t* raw_bits, int B, int C, int H, int W, float divisor, float bias,
                         float threshold, int update_mode);
 
+/* ---- active-stream mask ----------------------------------------------------------------------
+ * cb_change_detect / cb_change_detect_u8 with an active-stream mask: active is uint8[B] in device
+ * memory, read on the device (capturable in a CUDA graph), or NULL = every stream (then exactly the
+ * plain entry points, which forward here with NULL).  For a stream b with active[b] == 0 the call
+ * writes b's bitmap words as 0 and neither reads b's slice of x nor reads or writes b's state and
+ * operand planes: b is skipped for this frame, as if it had been fed its previous frame again.  The
+ * other streams are computed exactly as without the mask.  No reference counterpart (the reference
+ * is batch 1; DESIGN.md section 3.13). */
+int cb_change_detect_streams(void* stream, int dtype,
+                             const void* x, long long x_sb, long long x_sc, long long x_sy, long long x_sx,
+                             void* state, long long s_sb, long long s_sc, long long s_sy, long long s_sx,
+                             int aux_mode, void* aux_hi, void* aux_lo, uint32_t* raw_bits, int B, int C,
+                             int H, int W, float threshold, int update_mode,
+                             const uint8_t* active /* [B], device; 0 = skip; NULL = all */);
+int cb_change_detect_u8_streams(void* stream, const uint8_t* x, long long x_sb, long long x_sc,
+                                long long x_sy, long long x_sx, float* state, long long s_sb, long long s_sc,
+                                long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
+                                uint32_t* raw_bits, int B, int C, int H, int W, float divisor, float bias,
+                                float threshold, int update_mode,
+                                const uint8_t* active /* [B], device; 0 = skip; NULL = all */);
+
 /* ---- propagation + compaction -------------------------------------------------------------
  * replaces: the scatter-dilate inside changeDetection_kernel (cbconv2d_cg_backend.cu:62-72),
  *           changePropagation (conv2d_cg.py:15-19 -> cbconv2d_cg_backend.cu:101-136) and
