@@ -32,23 +32,31 @@ _INF = float("inf")
 
 
 class DetectionDone(object):
-    """Marker in the index slot of the ('changeIndexes', x, idx) tuple: the upstream CBPoolMax2d
-    already ran this layer's change detection (fused into its pooling kernel); the layer's raw
-    bitmap, state and operand planes are up to date."""
+    """Marker in the index slot of the ('changeIndexes', x, idx) tuple: the change detection of the
+    CBConv2d `owner` already ran on x -- in CBConv2d.detectInput, or fused into the kernel of an
+    upstream CBPoolMax2d or tile epilogue; its raw bitmap, state and operand planes are up to date.
+    The owner records the detection when it takes the marker."""
 
     def __init__(self, owner, dense=False):
         self.owner = owner
         self.dense = dense        # True: a dense scan wrote every bitmap word (CBConv2d.detectInput)
 
 
-class TailDone(object):
-    """Marker in the index slot of the tuple: the upstream 1x1 CBConv2d already ran this layer's
-    detection AND contraction inside its own kernel (cb_tail_update); this layer's state and output
-    are up to date.  `candidates` is the superset list both layers walked."""
+class FrameDone(object):
+    """Marker in the index slot of the tuple: the frame of `owner` already ran inside an upstream
+    kernel.  For a CBPoolMax2d: the CBConv2d before it pooled in its tile epilogue and ran the
+    detection of the layer after the pool there (cb_conv_update_tiled_pool).  For a CBConv2d: the
+    1x1 layer before it ran its detection and contraction (cb_tail_update); `candidates` is the
+    superset list both layers walked."""
 
-    def __init__(self, owner, candidates):
+    def __init__(self, owner, candidates=None):
         self.owner = owner
         self.candidates = candidates
+
+
+def _checkOwner(marker, module):
+    if marker.owner is not module:      # the work it reports was done for that module, not this one
+        raise _lib.CBinferError("%s got a %s for another module" % (type(module).__name__, type(marker).__name__))
 
 
 @functools.lru_cache(maxsize=None)
@@ -76,16 +84,17 @@ class CBPoolMax2d(nn.Module):
         self.ceil_mode = m.ceil_mode
         self.propChangeIndexes = False
         self.propPooledIndexes = False  # extension: hand pooled-resolution change candidates on
-        self._fusedNext = []            # extension: [downstream CBConv2d] whose detection is fused in
+        self._fusedNext = None          # extension: [downstream CBConv2d] whose detection is fused in
         self.cloneOutput = True   # reference returns outputState.clone() (conv2d.py:73)
         self._outVersion = None   # outputState._version as the kernels last left it
         self.register_buffer('outputState', torch.empty(0))
         self.clearMemory()
 
     def __setstate__(self, state):
-        # pickles of older versions may lack the version record: the state counts as touched
+        # pickles of older versions may lack these: no fused neighbour, and the state counts as touched
         super(CBPoolMax2d, self).__setstate__(state)
-        self.__dict__.setdefault('_outVersion', None)
+        for name in ('_fusedNext', '_outVersion'):
+            self.__dict__.setdefault(name, None)
 
     def clearMemory(self):
         self.outputState = self.outputState.new_empty(0)
@@ -130,18 +139,17 @@ class CBPoolMax2d(nn.Module):
 
     def forward(self, inp):
         assert(type(inp) == tuple and inp[0] == 'changeIndexes')
-        input = inp[1].detach()
-        changeIndexes = inp[2]
+        input, handed = inp[1].detach(), inp[2]
         assert input.dim() == 4
         _lib.require_cuda(input)
         nxt = self._fusedNext[0] if self._fusedNext else None
-        if getattr(changeIndexes, 'pooledBy', None) is self:
-            # the producing CBConv2d already pooled its tiles and ran the next layer's detection
-            # inside its epilogue (cb_conv_update_tiled_pool)
-            changeIndexes.pooledBy = None
+        if isinstance(handed, FrameDone):
+            # the producing CBConv2d already pooled its tiles and ran the next layer's detection inside
+            # its epilogue (cb_conv_update_tiled_pool); that layer records it on taking the DetectionDone
+            _checkOwner(handed, self)
             handOn = DetectionDone(nxt)
         else:
-            handOn = self._pool(input, changeIndexes, nxt)
+            handOn = self._pool(input, handed, nxt)
         output = self.outputState.clone() if self.cloneOutput else self.outputState
         return output if handOn is None else ('changeIndexes', output, handOn)
 
@@ -169,7 +177,6 @@ class CBPoolMax2d(nn.Module):
             # pooling + the next layer's detection in one kernel (cb_maxpool2x2_detect)
             cg.maxPool2d_detect(input, self.outputState, changeIndexes, tgt['next_state'], tgt['next_raw_bits'],
                                 tgt['threshold'], tgt['mode'], aux=tgt['aux'])
-            nxt._recordDetection()
             return DetectionDone(nxt)
         cg.maxPool2d(input, self.outputState, changeIndexes, self.kernel_size, self.stride)
         if self.propPooledIndexes and changeIndexes.bits is not None:
@@ -331,10 +338,10 @@ class CBConv2d(nn.Module):
             and self._stateAllocated(shape, dtype, device) and not any(self._stateTouched())
 
     def _recordDetection(self):
-        """This layer's detection ran with its threshold (here or inside an upstream kernel)."""
+        """This layer's detection ran with its threshold (here or inside an upstream kernel).  The
+        state's version is recorded where a frame ends (_frameDone, detectInput)."""
         self._fresh = False
         self._lastThr = self.threshold
-        self._inVersion = self.prevInput._version
 
     def _frameDone(self, changes, handOn):
         """Record the versions the kernels left and the frame's change list; return the output."""
@@ -463,15 +470,33 @@ class CBConv2d(nn.Module):
 
     # ---- coarse-grained path (conv2d.py:178-259) ---------------------------------------------
     def forward_normal(self, inp):
-        input, changeIndexes = _parse_input(inp)
+        input, handed = _parse_input(inp)
         assert(input.dim() == 4)
         assert(input.size(-3) == self.in_channels)
-        # a layer fed with plain frames re-scans them densely every frame, which rewrites every word of
-        # its raw bitmap: nothing ever ORs bits into it, so its compaction need not zero it afterwards
-        plain_input = changeIndexes is None or (isinstance(changeIndexes, DetectionDone) and changeIndexes.dense)
         _lib.require_cuda(input)
+        # `handed`: nothing (a plain frame), the upstream layer's change list, or a marker that an
+        # upstream kernel already ran part of this frame.  This layer records that work itself: the
+        # upstream module read its state (_fusedDetectTarget, _tailTarget) right before the launch,
+        # nothing since reads _fresh or _lastThr, and kernels bump no tensor versions.
+        if isinstance(handed, (DetectionDone, FrameDone)):
+            _checkOwner(handed, self)
+            self._recordDetection()
+        if isinstance(handed, FrameDone):
+            # cb_tail_update ran this layer's detection and contraction too; it split the operands on
+            # the fly, so this layer's operand planes are stale
+            self._auxPlanes = None
+            return self._frameDone(handed.candidates, handed.candidates if self.propChangeIndexes else None)
         B, _, H, W = input.shape
         dev, dt = input.device, input.dtype
+        detected = isinstance(handed, DetectionDone)
+        upstream = None           # the upstream layer's change list
+        if handed is not None and not detected:
+            assert(handed.dim() == 1)
+            upstream = handed if isinstance(handed, ChangeIndexes) \
+                else ChangeIndexes.from_tensor(handed.detach(), (B, H, W))
+        # a layer fed with plain frames re-scans them densely every frame, which rewrites every word of
+        # its raw bitmap: nothing ever ORs bits into it, so its compaction need not zero it afterwards
+        plain_input = handed is None or (detected and handed.dense)
         # uint8 frames (decoder output) are normalised inside the detection kernel:
         # value = u8 / divisor + bias with inputNorm = (divisor, bias); the layer computes in fp32
         u8norm = None
@@ -480,8 +505,7 @@ class CBConv2d(nn.Module):
             if u8norm is None:
                 raise _lib.CBinferError("uint8 input needs CBConv2d.inputNorm = (divisor, bias), e.g. "
                                         "(255.0, 0.0) for the scene reader's frame/255")
-            if (changeIndexes is not None and not isinstance(changeIndexes, DetectionDone)) \
-                    or self.gatherComputationStats or self.in_channels > 4:
+            if upstream is not None or self.gatherComputationStats or self.in_channels > 4:
                 input = input.float().div(u8norm[0]).add(u8norm[1])     # rare paths: plain fp32
                 u8norm = None
             dt = torch.float32
@@ -512,12 +536,7 @@ class CBConv2d(nn.Module):
             self._gatherStats(input)
 
         gemm, packed, bias32 = self._weights(dt, dev)
-        if isinstance(changeIndexes, TailDone):
-            # the upstream 1x1 layer's kernel already did this layer's frame (cb_tail_update)
-            assert changeIndexes.owner is self
-            cand = changeIndexes.candidates
-            return self._frameDone(cand, cand if self.propChangeIndexes else None)
-        tail = self._tryTail(input, changeIndexes, gemm, packed, bias32)
+        tail = self._tryTail(input, upstream, gemm, packed, bias32)
         if tail is not None:
             return tail
         aux = self._aux(gemm)
@@ -531,47 +550,33 @@ class CBConv2d(nn.Module):
                 and os.environ.get("CBINFER_FUSE_POOL", "1") != "0" \
                 and _lib.C.cb_conv_tiled_pool_supported(_lib.dtype_code(dt), gemm, self.out_channels):
             pool_args = self._fusedPool[0]._fusedPoolTarget((B, self.out_channels, H, W), dt, dev)
-        detected = isinstance(changeIndexes, DetectionDone)
-        if detected:
-            assert changeIndexes.owner is self
-            changeIndexes = None
-        candidates = None
-        if changeIndexes is not None and self.candidateDetect:
-            candidates, changeIndexes = changeIndexes, None
-            if not isinstance(candidates, ChangeIndexes):
-                candidates = ChangeIndexes.from_tensor(candidates.detach(), (B, H, W))
-            if tuple(candidates.shape) != (B, H, W) or not candidates.complete \
-                    or not self._candidatesExact(input.shape, dt, dev):
-                candidates = None          # not exact: full scan
+        # the upstream list as this frame's detection candidates, where that is exact
+        candidates = upstream if self.candidateDetect and upstream is not None \
+            and tuple(upstream.shape) == (B, H, W) and upstream.complete \
+            and self._candidatesExact(input.shape, dt, dev) else None
 
         mask = None
         tiled = False             # this frame's contraction walks the dirty-tile list
-        if changeIndexes is None:
+        if upstream is None or self.candidateDetect:
             # reference: detect (feedback updates prevInput at changed pixels, :222-224), nonzero
             # (:232), then prevInput.copy_(input) when not in feedback mode (:234-238).  Here the
             # copy is part of the detection pass; copyInput=False (alias the input as state) is
             # honoured as a copy -- the state always owns its memory.
-            mode = _lib.UPDATE_CHANGED if self.feedbackLoop else _lib.UPDATE_ALL
             sparse_next = self.candidateDetect and not plain_input
-            if not detected:     # (else the upstream pool kernel already did it)
-                # only the dense scan of a plain input skips inactive streams: a layer fed a change set
-                # must keep its full scans whole (see setActiveStreams)
-                active = self._streamMask(B) if plain_input else None
-                changeIndexes, mask = self._detect(input, candidates, u8norm, mode, aux, gemm, use_tiles,
-                                                   sparse_next, active)
-            if changeIndexes is None:
-                changeIndexes = self._compact(s, B, H, W, sparse_next, tiles=use_tiles,
-                                              lazy=pool_args is not None and not self.saveChangeMap)
+            changes, mask = (None, None) if detected else \
+                self._detect(input, candidates, u8norm, aux, gemm, use_tiles, sparse_next)
+            if changes is None:
+                changes = self._compact(s, B, H, W, sparse_next, tiles=use_tiles,
+                                        lazy=pool_args is not None and not self.saveChangeMap)
                 tiled = use_tiles
         else:
-            if not isinstance(changeIndexes, ChangeIndexes):
-                assert(changeIndexes.dim() == 1)
-                changeIndexes = ChangeIndexes.from_tensor(changeIndexes.detach(), (B, H, W))
-            elif tuple(changeIndexes.shape) != (B, H, W):
+            # the upstream list is this frame's change set (reference behaviour)
+            if tuple(upstream.shape) != (B, H, W):
                 # e.g. a CBPoolMax2d with the reference's propChangeIndexes forwards INPUT-resolution
                 # indices (conv2d.py:75-76): using them here would scatter out of bounds
                 raise _lib.CBinferError("change indexes refer to a %s grid, this layer's map is %s"
-                                        % (tuple(changeIndexes.shape), (B, H, W)))
+                                        % (tuple(upstream.shape), (B, H, W)))
+            changes = upstream
             if not self.feedbackLoop:
                 self.prevInput.copy_(input)                                            # :234-236
                 self._auxPlanes = None
@@ -584,23 +589,24 @@ class CBConv2d(nn.Module):
             cg.conv_update_tiled(self._inBuf, s["tile_ws"], s["dil_bits"], packed, bias32, self._outBuf,
                                  self.in_channels, self.out_channels, self.kernel_size, self.withReLU,
                                  gemm, aux=aux, pool=pool_args)                             # :242-251
-            if pool_args is not None:
-                changeIndexes.pooledBy = self._fusedPool[0]
-                self._fusedPool[0]._fusedNext[0]._recordDetection()
         else:
-            cg.conv_update(self._inBuf, changeIndexes, packed, bias32, self._outBuf, self.in_channels,
+            cg.conv_update(self._inBuf, changes, packed, bias32, self._outBuf, self.in_channels,
                            self.out_channels, self.kernel_size, self.withReLU, gemm,
                            aux=aux, ws=self._wsHolder.get(dev), mask=mask)                 # :242-251
-        if isinstance(changeIndexes, ChangeIndexes):
-            changeIndexes.complete = not ext_out
-        return self._frameDone(changeIndexes, changeIndexes if self.propChangeIndexes else None)
+        changes.complete = not ext_out
+        if tiled and pool_args is not None:
+            return self._frameDone(changes, FrameDone(self._fusedPool[0]))     # the epilogue did its frame
+        return self._frameDone(changes, changes if self.propChangeIndexes else None)
 
-    def _detect(self, input, candidates, u8norm, mode, aux, gemm, use_tiles, sparse_next, active=None):
+    def _detect(self, input, candidates, u8norm, aux, gemm, use_tiles, sparse_next):
         """Dense scan, or the test of the `candidates` only.  Returns (change list if the launch
-        built one, mask of the masked contraction), each or both None.  `active`: the active-stream
-        mask the dense scan honours, or None."""
+        built one, mask of the masked contraction), each or both None.  `sparse_next`: this layer
+        is fed change sets, so its bitmap is left clear for the next candidate test, and a dense scan
+        covers every stream (see setActiveStreams); else the dense scan skips inactive streams."""
         B, _, H, W = input.shape
         s = self._scratch
+        mode = _lib.UPDATE_CHANGED if self.feedbackLoop else _lib.UPDATE_ALL
+        active = None if sparse_next else self._streamMask(B)
         # extension: no compaction at all for a 1x1 layer on the candidate path - the
         # contraction walks the candidate list and skips pixels whose raw bit is not set
         # (cb_conv_update_masked); this layer's own index list is then never materialised
@@ -690,15 +696,13 @@ class CBConv2d(nn.Module):
                        changeIndexes, C0, C1, C2,
                        _lib.UPDATE_CHANGED if self.feedbackLoop else _lib.UPDATE_ALL,
                        s["count"], tgt['count'], s["tail_sync"])
-        # the kernel splits its operands on the fly: the layers' operand planes are stale now
+        # the kernel splits its operands on the fly: this layer's operand planes are stale now
         self._auxPlanes = None
-        nxt._auxPlanes = None
         self._recordDetection()
-        nxt._recordDetection()
         sup = ChangeIndexes(changeIndexes._buffer, changeIndexes.count, (B, H, W), bits=changeIndexes.bits,
                             ws=changeIndexes._ws, listed=changeIndexes.listed)
         sup.superset = True
-        return self._frameDone(sup, TailDone(nxt, sup))
+        return self._frameDone(sup, FrameDone(nxt, sup))
 
     def lastChangeIndexes(self):
         """This frame's change indexes as an int32 tensor (ascending b*H*W + y*W + x): what the
@@ -724,18 +728,13 @@ class CBConv2d(nn.Module):
         if self._stateTouched()[0]:
             self._auxPlanes = None       # rebuilt from the touched state; the scan below is dense anyway
         gemm, _, _ = self._weights(dt, input.device)
-        aux = self._aux(gemm)
-        mode = _lib.UPDATE_CHANGED if self.feedbackLoop else _lib.UPDATE_ALL
+        norm = None
         if input.dtype == torch.uint8:
             norm = self.inputNorm
             if norm is None or self.in_channels > 4:
                 raise _lib.CBinferError("detectInput: uint8 input needs inputNorm and <= 4 channels")
-            cg.detect_u8(input, self.prevInput, self._scratch["raw_bits"], self.threshold, mode,
-                         norm[0], norm[1], aux=aux, active=self._streamMask(input.shape[0]))
-        else:
-            cg.detect(input, self.prevInput, self._scratch["raw_bits"], self.threshold, mode, aux=aux,
-                      active=self._streamMask(input.shape[0]))
-        self._recordDetection()
+        self._detect(input, None, norm, self._aux(gemm), gemm, False, False)
+        self._inVersion = self.prevInput._version
         return 'changeIndexes', input, DetectionDone(self, dense=True)
 
     def _smallMap(self, B, H, W):

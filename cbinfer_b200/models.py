@@ -35,6 +35,11 @@ def enableCandidateDetection(m, fusePool=True, maskedConv=True):
     """B200 extension (no reference counterpart): inside every nn.Sequential, let each CB layer
     hand its change set to a directly following CB layer as detection *candidates*, so that layer
     thresholds only the pixels that were just rewritten instead of re-scanning its whole input.
+    Where the neighbours allow it, one kernel also does a neighbour's part of the frame: a pool runs
+    the next conv's detection and a conv on the tile path pools in its epilogue (``fusePool``), and
+    two trailing masked 1x1 layers run in one launch (``maskedConv``).  The launching module reads
+    the neighbour's state; the neighbour learns of the work from the marker it receives in the
+    ('changeIndexes', x, marker) tuple (DetectionDone / FrameDone) and records it itself.
     Results are identical to the dense scan (tests/test_gpu_modules.py)."""
     import torch.nn as nn
     for seq in [mm for mm in m.modules() if type(mm) is nn.Sequential]:
@@ -54,7 +59,7 @@ def enableCandidateDetection(m, fusePool=True, maskedConv=True):
             # detection of the conv after the pool there), cb_conv_update_tiled_pool
             for a, p, b in zip(kids[:-2], kids[1:-1], kids[2:]):
                 if type(a) is CBConv2d and type(p) is CBPoolMax2d and type(b) is CBConv2d \
-                        and getattr(p, '_fusedNext', None) and not a.finegrained:
+                        and p._fusedNext and not a.finegrained:
                     a._fusedPool = [p]
         if maskedConv:
             # a 1x1 layer fed by a CB conv whose own index list nobody needs as an exact list (it is

@@ -164,12 +164,13 @@ def test_pickle_of_an_older_version_gets_the_attributes_added_since(tmp_path):
     pool = cb.CBPoolMax2d(nn.MaxPool2d(2, 2))
     for name in ('candidateDetect', 'tileMode', '_fusedPool', '_fusedTail', '_inVersion', '_outVersion'):
         del conv.__dict__[name]
-    del pool.__dict__['_outVersion']
+    for name in ('_fusedNext', '_outVersion'):
+        del pool.__dict__[name]
     path = str(tmp_path / "old.net")
     torch.save(nn.Sequential(conv, pool), path)
     conv, pool = torch.load(path, weights_only=False)
     assert conv.candidateDetect is False and conv.tileMode == 'auto'
-    assert conv._fusedPool is None and conv._fusedTail is None
+    assert conv._fusedPool is None and conv._fusedTail is None and pool._fusedNext is None
     assert conv._inVersion is None and conv._outVersion is None and pool._outVersion is None
 
 

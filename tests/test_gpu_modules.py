@@ -757,3 +757,18 @@ def test_change_indexes_of_wrong_grid_are_rejected():
     x = rand_tensor((1, 3, 12, 16), "f32", 1)
     with pytest.raises(_lib.CBinferError):
         conv1(pool(conv0(x)))
+
+
+def test_marker_for_another_module_is_rejected():
+    """A DetectionDone / FrameDone in the tuple tells its owner that an upstream kernel already did
+    part of the owner's frame; any other module taking it would skip work nobody did."""
+    import cbinfer_b200 as cb
+    from cbinfer_b200._lib import CBinferError
+    from cbinfer_b200.conv2d import DetectionDone, FrameDone
+    a, b = (cb.CBConv2d(nn.Conv2d(4, 4, 3, padding=1).cuda(), 0.1) for _ in range(2))
+    pool = cb.CBPoolMax2d(nn.MaxPool2d(2, 2))
+    x = rand_tensor((1, 4, 12, 16), "f32", 1)
+    for module, marker in ((b, DetectionDone(a)), (b, FrameDone(a)), (pool, FrameDone(a))):
+        with pytest.raises(CBinferError):
+            module(('changeIndexes', x, marker))
+    assert b._fresh and b._lastThr is None           # nothing was recorded for b
