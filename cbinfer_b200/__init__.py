@@ -18,7 +18,7 @@ from .conv2d_cg import ChangeIndexes
 __all__ = ['CBConv2d', 'CBPoolMax2d', 'ChangeIndexes', 'subsitute', 'convertRecur', 'mergeReLURecur',
            'propChangeIndexesOf1x1', 'clearMemory', 'getStateTensors', 'convert',
            'tuneThresholdParameters', 'convertPools', 'shareWorkspace', 'resetStreams',
-           'setActiveStreams']
+           'setActiveStreams', 'trackStreamChanges', 'streamChangeCounts']
 
 verbose = False
 
@@ -214,6 +214,60 @@ def setActiveStreams(net, streams):
         buf.copy_(host, non_blocking=True)
     for c in convs:
         c._activeMask = buf
+
+
+def trackStreamChanges(net, enable=True, B=None):
+    """Count, per video stream, the output pixels each CBConv2d under `net` recomputes.  After this,
+    every frame writes ``counts[l, b]``: the number of output pixels of stream b that layer l (in
+    ``net.modules()`` order) recomputed in that frame -- the layer's change count split by stream,
+    written by the kernels that already produce that count, so no launch is added (DESIGN.md section
+    3.14).  A stream skipped by the active-stream mask, or fed its previous frame again, gets 0 in
+    every row; a stream started over by resetStreams gets H*W of each layer on its next frame.  If the
+    last layer's count of stream b is 0, b's output is bit-identical to its previous frame.
+
+    Allocates one device int32 [L, B] buffer (plus the kernels' accumulators) and hands each CBConv2d
+    its row; returns the layers' qualified names in row order.  B comes from the argument or from the
+    layers' state (as setActiveStreams takes it); a frame of another batch size raises at forward.
+    The buffer (streamChangeCounts) is the same tensor every frame, so CUDA graphs captured after this
+    call keep writing it.  enable=False detaches it.  Pools get no row; fine-grained layers on the
+    planar path (gemmMode='simt') are not supported."""
+    named = [(name, c) for name, c in net.named_modules() if type(c) is CBConv2d]
+    convs = [c for _, c in named]
+    if not enable:
+        for c in convs:
+            c._streamRow = None
+        return []
+    for c in convs:
+        if c.finegrained and c.gemmMode == 'simt':
+            raise CBinferError("trackStreamChanges: the planar fine-grained path (gemmMode='simt') does not "
+                               "count changes per stream")
+    state = [c._inBuf for c in convs if c._inBuf is not None]
+    if B is None:
+        if not state:
+            raise CBinferError("trackStreamChanges: the model has not run yet, so the number of streams is "
+                               "unknown; pass B")
+        B = state[0].shape[0]
+    B = int(B)
+    if B < 1:
+        raise CBinferError("trackStreamChanges: B = %d streams" % B)
+    dev = state[0].device if state else next(net.parameters()).device
+    if dev.type != "cuda":
+        raise CBinferError("trackStreamChanges: the model is on %s; the counts live on a CUDA device" % dev)
+    counts = torch.zeros(len(convs), B, dtype=torch.int32, device=dev)
+    acc = torch.zeros(len(convs), B + 1, dtype=torch.int32, device=dev)    # zero at rest (the kernels keep it so)
+    for l, c in enumerate(convs):
+        c._streamRow = (counts, l, acc)
+    return [name for name, _ in named]
+
+
+def streamChangeCounts(net):
+    """The device int32 [L, B] buffer of per-stream change counts of a model set up with
+    trackStreamChanges: row l holds layer l's counts of the last frame.  Always the same tensor; read
+    it after the frame's work (it is written on the stream the frame ran on)."""
+    for c in net.modules():
+        if type(c) is CBConv2d and c._streamRow is not None:
+            return c._streamRow[0]
+    raise CBinferError("streamChangeCounts: the model is not tracked (trackStreamChanges)")
 
 
 def getStateTensors(net):

@@ -33,6 +33,9 @@ SYMBOLS = [
     "cb_conv_tiled_pool_supported", "cb_conv_update_tiled_pool", "cb_dilate_tiles",
     "cb_tail_supported", "cb_tail_update", "cb_reset_streams",
     "cb_resize_ws_bytes", "cb_resize_bicubic_u8_init", "cb_resize_bicubic_u8", "cb_resize_bilinear_u8",
+    "cb_dilate_compact_streams", "cb_dilate_compact_tiles_streams", "cb_dilate_tiles_streams",
+    "cb_change_detect_sparse_compact_streams", "cb_conv_update_masked_streams", "cb_tail_update_streams",
+    "cb_stream_bucket",
 ]
 
 
@@ -122,6 +125,12 @@ def _load():
         "cb_conv_accumulate": (i32, [vp, i32, i32, vp, vp, i32, vp, vp, vp, vp, i32, i32, i32, i32, i32,
                                      i32, i32, i32, vp, sz]),
     }
+    # the *_streams variants: the plain call's arguments + one row of per-stream counts and its accumulator
+    for name in ("cb_dilate_compact", "cb_dilate_compact_tiles", "cb_dilate_tiles", "cb_change_detect_sparse_compact",
+                 "cb_conv_update_masked"):
+        sig[name + "_streams"] = (i32, sig[name][1] + [vp, vp])
+    sig["cb_tail_update_streams"] = (i32, sig["cb_tail_update"][1] + [i32, i32, vp, vp, vp, vp])
+    sig["cb_stream_bucket"] = (i32, [vp, vp, vp, i32, i32, vp, vp])
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
         fn.restype = res

@@ -239,6 +239,9 @@ class CBConv2d(nn.Module):
         self._inVersion = None    # prevInput._version / prevOutput._version as the kernels last left them
         self._outVersion = None
         self._activeMask = None   # active-stream mask (cbinfer_b200.setActiveStreams), None = all
+        # per-stream change counts (cbinfer_b200.trackStreamChanges): (counts int32 [L,B], this layer's
+        # row l, accumulators int32 [L,B+1] zeroed once), or None = not tracked
+        self._streamRow = None
         self._wsHolder = cg.ConvWorkspace()    # shared per model by pycbinfer.convert()
         self.register_buffer('prevInput', self.weight.data.new_empty(0))
         self.register_buffer('prevOutput', self.weight.data.new_empty(0))
@@ -272,7 +275,7 @@ class CBConv2d(nn.Module):
         # no fused neighbours, and without a version record the state counts as touched
         super(CBConv2d, self).__setstate__(state)
         self._setDefaultValues()
-        for name in ('_fusedPool', '_fusedTail', '_inVersion', '_outVersion', '_activeMask'):
+        for name in ('_fusedPool', '_fusedTail', '_inVersion', '_outVersion', '_activeMask', '_streamRow'):
             self.__dict__.setdefault(name, None)
 
     # ---- state ---------------------------------------------------------------------------
@@ -413,8 +416,12 @@ class CBConv2d(nn.Module):
         if input.dtype != torch.float32:
             raise _lib.CBinferError("the fine-grained path is fp32 only (as in the reference)")
         if self.gemmMode == 'simt':
+            if self._streamRow is not None:
+                raise _lib.CBinferError("per-stream change counts are not supported on the planar fine-grained "
+                                        "path (gemmMode='simt')")
             return self._forward_fg_planar(input.contiguous())
         B, _, H, W = input.shape
+        rows = self._streams(B)
         dev = input.device
         outpSize = (B, self.out_channels, H, W)
         gemm = _lib.GEMM_TC_BF16X3
@@ -436,13 +443,15 @@ class CBConv2d(nn.Module):
                                       torch.zeros(B, H, W, p16, dtype=torch.bfloat16, device=dev)))
             self._scratch = cg.alloc_scratch((B, H, W), dev)
             self._scratch["nvalues"] = torch.zeros(1, dtype=torch.int32, device=dev)
+            if rows is not None:
+                rows[0].fill_(H * W)              # the dense first frame computes every output pixel
         else:
             s = self._scratch
             _, planes = self._auxPlanes
             cg.fg_detect(input, self.prevInput, self._inBuf, planes, s["raw_bits"], self.threshold,
                          count=s["nvalues"])
             cg.dilate_compact(s["raw_bits"], (B, H, W), self.kernel_size, s["idx"], s["count"], s["ws"],
-                              dil_bits=s["dil_bits"])
+                              dil_bits=s["dil_bits"], streams=rows)
             changes = ChangeIndexes(s["idx"], s["count"], (B, H, W), bits=s["dil_bits"])
             cg.conv_accumulate(planes, changes, self._packed[1], self._outBuf, self.in_channels,
                                self.out_channels, self.kernel_size, gemm, ws=self._wsHolder.get(dev))
@@ -488,6 +497,7 @@ class CBConv2d(nn.Module):
             return self._frameDone(handed.candidates, handed.candidates if self.propChangeIndexes else None)
         B, _, H, W = input.shape
         dev, dt = input.device, input.dtype
+        rows = self._streams(B)
         detected = isinstance(handed, DetectionDone)
         upstream = None           # the upstream layer's change list
         if handed is not None and not detected:
@@ -577,6 +587,8 @@ class CBConv2d(nn.Module):
                 raise _lib.CBinferError("change indexes refer to a %s grid, this layer's map is %s"
                                         % (tuple(upstream.shape), (B, H, W)))
             changes = upstream
+            if rows is not None:
+                cg.stream_bucket(changes, (B, H, W), rows)
             if not self.feedbackLoop:
                 self.prevInput.copy_(input)                                            # :234-236
                 self._auxPlanes = None
@@ -622,7 +634,7 @@ class CBConv2d(nn.Module):
             cg.detect_sparse_compact(input, self.prevInput, s["raw_bits"], self.threshold, mode, candidates,
                                      self.kernel_size, s["idx"], s["count"], s["sdc_sync"], aux=aux,
                                      bits_are_clear=s.get("raw_clear", False), dil_bits=s["dil_bits"],
-                                     clear_raw=sparse_next)
+                                     clear_raw=sparse_next, streams=self._streams(B))
             s["raw_clear"] = sparse_next
             changes = ChangeIndexes(s["idx"], s["count"], (B, H, W), bits=s["dil_bits"])
         elif candidates is not None:
@@ -632,7 +644,8 @@ class CBConv2d(nn.Module):
             if masked:
                 if "mask_sync" not in s:
                     s["mask_sync"] = torch.zeros(2, dtype=torch.int32, device=input.device)
-                mask = dict(bits=s["raw_bits"], clear=True, count=s["count"], sync=s["mask_sync"])
+                mask = dict(bits=s["raw_bits"], clear=True, count=s["count"], sync=s["mask_sync"],
+                            streams=self._streams(B))
                 s["raw_clear"] = True                # the masked contraction clears the bitmap
                 changes = ChangeIndexes(candidates.buffer, candidates.count, (B, H, W), bits=None)
                 changes.superset = True
@@ -643,6 +656,17 @@ class CBConv2d(nn.Module):
             cg.detect(input, self.prevInput, s["raw_bits"], self.threshold, mode, aux=aux, active=active)
         self._recordDetection()
         return changes, mask
+
+    def _streams(self, B):
+        """This layer's per-stream counts row for a frame of B streams, as (counts int32 [B], accumulator
+        int32 [B+1]), or None when the model is not tracked (cbinfer_b200.trackStreamChanges)."""
+        if self._streamRow is None:
+            return None
+        counts, l, acc = self._streamRow
+        if counts.shape[1] != B:
+            raise _lib.CBinferError("per-stream change counts of %d streams, the frame has %d (trackStreamChanges)"
+                                    % (counts.shape[1], B))
+        return counts[l], acc[l]
 
     def _streamMask(self, B):
         """The active-stream mask for a frame of B streams, or None when none is set."""
@@ -687,6 +711,9 @@ class CBConv2d(nn.Module):
         tgt = nxt._tailTarget((B, C1, H, W), input.dtype, input.device, self.feedbackLoop)
         if tgt is None or tgt['gemm'] != gemm:
             return None
+        rows1, rows2 = self._streams(B), nxt._streams(B)
+        if (rows1 is None) != (rows2 is None):      # one kernel writes both rows or neither
+            return None
         s = self._scratch
         if "tail_sync" not in s:
             s["tail_sync"] = torch.zeros(4, dtype=torch.int32, device=input.device)
@@ -695,7 +722,7 @@ class CBConv2d(nn.Module):
                        tgt['state'], tgt['packed'], tgt['bias'], tgt['out'], tgt['relu'], tgt['thr'],
                        changeIndexes, C0, C1, C2,
                        _lib.UPDATE_CHANGED if self.feedbackLoop else _lib.UPDATE_ALL,
-                       s["count"], tgt['count'], s["tail_sync"])
+                       s["count"], tgt['count'], s["tail_sync"], streams1=rows1, streams2=rows2)
         # the kernel splits its operands on the fly: this layer's operand planes are stale now
         self._auxPlanes = None
         self._recordDetection()
@@ -759,7 +786,7 @@ class CBConv2d(nn.Module):
         if tiles and lazy:
             # tiles + dilated bitmap + count only; the ordered list is compacted if somebody asks
             cg.dilate_tiles(s["raw_bits"], (B, H, W), self.kernel_size, s["count"], s["ws"], s["dil_bits"],
-                            s["tile_ws"], clear_raw=sparse_next)
+                            s["tile_ws"], clear_raw=sparse_next, streams=self._streams(B))
             s["raw_clear"] = sparse_next
             return ChangeIndexes(s["idx"], s["count"], (B, H, W), bits=s["dil_bits"], ws=s["ws"], listed=False)
         dil_map = s.get("dil_map") if self.saveChangeMap else None
@@ -767,7 +794,7 @@ class CBConv2d(nn.Module):
         # consumed, so the next frame's candidate detection needs no memset
         cg.dilate_compact(s["raw_bits"], (B, H, W), self.kernel_size, s["idx"], s["count"],
                           s["ws"], dil_bits=s["dil_bits"], dil_map=dil_map, clear_raw=sparse_next,
-                          tile_ws=s["tile_ws"] if tiles else None)
+                          tile_ws=s["tile_ws"] if tiles else None, streams=self._streams(B))
         s["raw_clear"] = sparse_next
         if self.saveChangeMap:
             self.changeMap = dil_map[0] if B == 1 else dil_map

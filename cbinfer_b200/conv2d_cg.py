@@ -185,21 +185,48 @@ def detect_sparse(x, state, raw_bits, threshold, update_mode, candidates, aux=No
                                     int(update_mode), int(bool(bits_are_clear))))
 
 
+def _streams_args(streams, B):
+    """(stream_counts, stream_acc) pointers of a per-stream counts row: `streams` = (counts, acc), int32 CUDA
+    tensors of at least B (counts) and B (acc) entries, or None = (None, None)."""
+    if streams is None:
+        return None, None
+    counts, acc = streams
+    require_cuda(counts, acc)
+    if counts.dtype != torch.int32 or acc.dtype != torch.int32 or counts.numel() < B or acc.numel() < B \
+            or not counts.is_contiguous() or not acc.is_contiguous():
+        raise _lib.CBinferError("per-stream counts: contiguous int32 tensors of >= %d entries are needed" % B)
+    return counts.data_ptr(), acc.data_ptr()
+
+
+def stream_bucket(changes, shape, streams):
+    """cb_stream_bucket: counts[b] = number of entries of the index list `changes` (a
+    :class:`ChangeIndexes`, any order) in stream b of a [B,H,W] grid; `streams` = (counts int32 [B],
+    accumulator int32 [B+1] zeroed once)."""
+    B, H, W = shape
+    sc, acc = _streams_args(streams, B)
+    if streams[1].numel() < B + 1:
+        raise _lib.CBinferError("stream_bucket: the accumulator needs B + 1 = %d entries" % (B + 1))
+    check(C.cb_stream_bucket(stream_ptr(changes.count.device), changes.buffer.data_ptr(), changes.count.data_ptr(),
+                             B, H * W, sc, acc))
+
+
 def detect_sparse_compact(x, state, raw_bits, threshold, update_mode, candidates, filtSize, idx, count, sync,
-                          aux=None, bits_are_clear=False, dil_bits=None, clear_raw=False):
+                          aux=None, bits_are_clear=False, dil_bits=None, clear_raw=False, streams=None):
     """cb_change_detect_sparse_compact: candidate detection + dilation + ordered compaction in one launch
-    (small maps: at most cb_compact_small_max_words() bitmap words).  `sync` = int32[1], zeroed once."""
+    (small maps: at most cb_compact_small_max_words() bitmap words).  `sync` = int32[1], zeroed once.
+    `streams`: optional (counts int32 [B], accumulator int32 [B] zeroed once): the count split by stream
+    (cb_change_detect_sparse_compact_streams)."""
     require_cuda(x, state, raw_bits)
     B, Cc, H, W = x.shape
     assert state.shape == x.shape and state.dtype == x.dtype
     assert tuple(candidates.shape) == (B, H, W)
     mode, hi, lo = _aux_args(aux, state)
-    check(C.cb_change_detect_sparse_compact(
+    check(C.cb_change_detect_sparse_compact_streams(
         stream_ptr(x.device), dtype_code(x), x.data_ptr(), *_strides4(x), state.data_ptr(), *_strides4(state),
         mode, hi, lo, candidates.buffer.data_ptr(), candidates.count.data_ptr(), raw_bits.data_ptr(), B, Cc, H, W,
         float(threshold), int(update_mode), int(bool(bits_are_clear)),
         dil_bits.data_ptr() if dil_bits is not None else None, idx.data_ptr(), count.data_ptr(), sync.data_ptr(),
-        (filtSize[0] - 1) // 2, (filtSize[1] - 1) // 2, int(bool(clear_raw))))
+        (filtSize[0] - 1) // 2, (filtSize[1] - 1) // 2, int(bool(clear_raw)), *_streams_args(streams, B)))
 
 
 def detect_compact_sparse(*args, **kwargs):
@@ -217,33 +244,37 @@ def pool_compact(in_bits, in_shape, out_shape, idx, count, ws, out_bits=None):
                             idx.data_ptr(), count.data_ptr(), ws.data_ptr(), B, H, W, oH, oW))
 
 
-def dilate_tiles(raw_bits, shape, filtSize, count, ws, dil_bits, tile_ws, clear_raw=False):
-    """cb_dilate_tiles: dilation + dirty-tile list + change count, no ordered index list."""
+def dilate_tiles(raw_bits, shape, filtSize, count, ws, dil_bits, tile_ws, clear_raw=False, streams=None):
+    """cb_dilate_tiles: dilation + dirty-tile list + change count, no ordered index list.  `streams` as in
+    :func:`detect_sparse_compact`."""
     B, H, W = shape
-    check(C.cb_dilate_tiles(stream_ptr(raw_bits.device), raw_bits.data_ptr(), dil_bits.data_ptr(),
-                            count.data_ptr(), ws.data_ptr(), tile_ws.data_ptr(), B, H, W,
-                            (filtSize[0] - 1) // 2, (filtSize[1] - 1) // 2, int(bool(clear_raw))))
+    check(C.cb_dilate_tiles_streams(stream_ptr(raw_bits.device), raw_bits.data_ptr(), dil_bits.data_ptr(),
+                                    count.data_ptr(), ws.data_ptr(), tile_ws.data_ptr(), B, H, W,
+                                    (filtSize[0] - 1) // 2, (filtSize[1] - 1) // 2, int(bool(clear_raw)),
+                                    *_streams_args(streams, B)))
 
 
 def dilate_compact(raw_bits, shape, filtSize, idx, count, ws, dil_bits=None, dil_map=None,
-                   clear_raw=False, tile_ws=None):
+                   clear_raw=False, tile_ws=None, streams=None):
     """cb_dilate_compact: dilation by the filter footprint + ordered compaction.  With `tile_ws`
     (cb_tile_ws_bytes of zeroed int32 device memory) the dirty 8x16 output tiles are listed as well
-    (cb_dilate_compact_tiles), for :func:`conv_update_tiled`."""
+    (cb_dilate_compact_tiles), for :func:`conv_update_tiled`.  `streams` as in
+    :func:`detect_sparse_compact`."""
     B, H, W = shape
+    sc, acc = _streams_args(streams, B)
     if tile_ws is not None:
-        check(C.cb_dilate_compact_tiles(stream_ptr(raw_bits.device), raw_bits.data_ptr(),
-                                        dil_bits.data_ptr() if dil_bits is not None else None,
-                                        dil_map.data_ptr() if dil_map is not None else None,
-                                        idx.data_ptr(), count.data_ptr(), ws.data_ptr(),
-                                        tile_ws.data_ptr(), B, H, W, (filtSize[0] - 1) // 2,
-                                        (filtSize[1] - 1) // 2, int(bool(clear_raw))))
+        check(C.cb_dilate_compact_tiles_streams(stream_ptr(raw_bits.device), raw_bits.data_ptr(),
+                                                dil_bits.data_ptr() if dil_bits is not None else None,
+                                                dil_map.data_ptr() if dil_map is not None else None,
+                                                idx.data_ptr(), count.data_ptr(), ws.data_ptr(),
+                                                tile_ws.data_ptr(), B, H, W, (filtSize[0] - 1) // 2,
+                                                (filtSize[1] - 1) // 2, int(bool(clear_raw)), sc, acc))
         return
-    check(C.cb_dilate_compact(stream_ptr(raw_bits.device), raw_bits.data_ptr(),
-                              dil_bits.data_ptr() if dil_bits is not None else None,
-                              dil_map.data_ptr() if dil_map is not None else None,
-                              idx.data_ptr(), count.data_ptr(), ws.data_ptr(), B, H, W,
-                              (filtSize[0] - 1) // 2, (filtSize[1] - 1) // 2, int(bool(clear_raw))))
+    check(C.cb_dilate_compact_streams(stream_ptr(raw_bits.device), raw_bits.data_ptr(),
+                                      dil_bits.data_ptr() if dil_bits is not None else None,
+                                      dil_map.data_ptr() if dil_map is not None else None,
+                                      idx.data_ptr(), count.data_ptr(), ws.data_ptr(), B, H, W,
+                                      (filtSize[0] - 1) // 2, (filtSize[1] - 1) // 2, int(bool(clear_raw)), sc, acc))
 
 
 def alloc_tile_ws(shape, device):
@@ -362,8 +393,9 @@ def conv_update(state_buf, changes, packed_w, bias_f32, out_buf, Cin, Cout, filt
     src, src_lo, pitch = _conv_operands(state_buf, Cin, gemm, aux)
     if mask is not None:
         # `changes` is a superset list; mask = dict(bits=raw bitmap, clear=bool, count=int32[1] out,
-        # sync=int32[2] zeroed once): only pixels whose bit is set are processed (cb_conv_update_masked)
-        check(C.cb_conv_update_masked(stream_ptr(state_buf.device), dtype_code(state_buf), gemm,
+        # sync=int32[2] zeroed once, optional streams as in detect_sparse_compact): only pixels whose bit
+        # is set are processed (cb_conv_update_masked[_streams])
+        check(C.cb_conv_update_masked_streams(stream_ptr(state_buf.device), dtype_code(state_buf), gemm,
                                       src.data_ptr(), src_lo.data_ptr() if src_lo is not None else None,
                                       pitch, changes.buffer.data_ptr(), changes.count.data_ptr(),
                                       packed_w.data_ptr(), bias_f32.data_ptr(), out_buf.data_ptr(),
@@ -371,7 +403,8 @@ def conv_update(state_buf, changes, packed_w, bias_f32, out_buf, Cin, Cout, filt
                                       int(bool(relu)), ws.data_ptr() if ws is not None else None,
                                       ws.numel() if ws is not None else 0,
                                       mask['bits'].data_ptr(), int(bool(mask.get('clear', False))),
-                                      mask['count'].data_ptr(), mask['sync'].data_ptr()))
+                                      mask['count'].data_ptr(), mask['sync'].data_ptr(),
+                                      *_streams_args(mask.get('streams'), B)))
         return
     check(C.cb_conv_update(stream_ptr(state_buf.device), dtype_code(state_buf), gemm,
                            src.data_ptr(), src_lo.data_ptr() if src_lo is not None else None,
@@ -446,17 +479,22 @@ def conv_update_tiled(state_buf, tile_ws, dil_bits, packed_w, bias_f32, out_buf,
 
 
 def tail_update(x_buf, state1_buf, packed1, bias1, out1_buf, relu1, thr1, state2_buf, packed2, bias2,
-                out2_buf, relu2, thr2, candidates, C0, C1, C2, update_mode, count1, count2, sync):
+                out2_buf, relu2, thr2, candidates, C0, C1, C2, update_mode, count1, count2, sync,
+                streams1=None, streams2=None):
     """cb_tail_update: two chained 1x1 change-based layers (detect, contraction, detect,
-    contraction) for the candidate pixels in one launch; pixel-major fp32 buffers [B,H,W,pitch]."""
+    contraction) for the candidate pixels in one launch; pixel-major fp32 buffers [B,H,W,pitch].
+    `streams1` / `streams2`: optional per-stream counts rows of the two layers, as in
+    :func:`detect_sparse_compact` (both or neither)."""
     assert x_buf.dtype == torch.float32 and x_buf.shape[3] == C0 and state1_buf.shape == x_buf.shape
     assert out1_buf.shape[3] == C1 and state2_buf.shape == out1_buf.shape
-    check(C.cb_tail_update(stream_ptr(x_buf.device), x_buf.data_ptr(), state1_buf.data_ptr(),
+    B, H, W, _ = x_buf.shape
+    check(C.cb_tail_update_streams(stream_ptr(x_buf.device), x_buf.data_ptr(), state1_buf.data_ptr(),
                            packed1.data_ptr(), bias1.data_ptr(), out1_buf.data_ptr(), int(bool(relu1)),
                            float(thr1), state2_buf.data_ptr(), packed2.data_ptr(), bias2.data_ptr(),
                            out2_buf.data_ptr(), out2_buf.shape[3], int(bool(relu2)), float(thr2),
                            candidates.buffer.data_ptr(), candidates.count.data_ptr(), C0, C1, C2,
-                           int(update_mode), count1.data_ptr(), count2.data_ptr(), sync.data_ptr()))
+                           int(update_mode), count1.data_ptr(), count2.data_ptr(), sync.data_ptr(), B, H * W,
+                           *_streams_args(streams1, B), *_streams_args(streams2, B)))
 
 
 def reset_streams(segments, mask):

@@ -132,10 +132,23 @@ int cb_change_detect_u8(void* stream, const uint8_t* x, long long x_sb, long lon
 
 size_t cb_tile_ws_bytes(int B, int H, int W) { return cb::tile_ws_words(B, H, W) * sizeof(int32_t); }
 
+// per-stream counts (the *_streams entry points): an output row needs its own accumulator
+#define CB_CHECK_STREAMS(counts, acc, what)                                                        \
+  CB_CHECK_ARG(!(counts) || ((acc) && (void*)(acc) != (void*)(counts)),                          \
+               what ": stream_counts needs a separate stream_acc")
+
+// a launch that has nothing to scan still writes its row of per-stream counts (zeros)
+static int zero_stream_counts(cudaStream_t s, int32_t* counts, int B, const char* what) {
+  if (counts && B > 0 && cudaMemsetAsync(counts, 0, (size_t)B * sizeof(int32_t), s) != cudaSuccess)
+    return cb::fail(3, "%s: memset of the stream counts failed", what);
+  return 0;
+}
+
 static int dilate_compact_impl(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits, int8_t* dil_map,
                       int32_t* idx, int32_t* count, void* ws, void* tile_ws, int B, int H, int W, int kHHalf,
-                      int kWHalf, int clear_raw, int no_list = 0) {
+                      int kWHalf, int clear_raw, int no_list, int32_t* stream_counts, int32_t* stream_acc) {
   CB_CHECK_ARG(raw_bits && (idx || no_list) && count && ws, "dilate_compact: null pointer");
+  CB_CHECK_STREAMS(stream_counts, stream_acc, "dilate_compact");
   CB_CHECK_ARG(raw_bits != dil_bits, "dilate_compact: dil_bits must not alias raw_bits");
   CB_CHECK_ARG(kHHalf >= 0 && kWHalf >= 0 && kWHalf <= 31, "dilate_compact: kWHalf must be <= 31");
   CB_CHECK_ARG((long long)B * H * W < (1ll << 31), "dilate_compact: more than 2^31 pixels");
@@ -144,43 +157,84 @@ static int dilate_compact_impl(void* stream, const uint32_t* raw_bits, uint32_t*
   if (nwords == 0) {
     cudaMemsetAsync(count, 0, sizeof(int32_t), s);
     CB_CHECK_LAUNCH("dilate_compact(memset)");
-    return 0;
+    return zero_stream_counts(s, stream_counts, B, "dilate_compact");
   }
   CB_CHECK_ARG(nwords < (1ll << 31), "dilate_compact: bitmap too large");
   const int ntiles = (int)((nwords + kCompactTile - 1) / kCompactTile);
-  cb::launch(dilate_compact_kernel, ntiles, kCompactThreads, 0, s,
-                                                          raw_bits, dil_bits, dil_map, idx, count,
-                                                          ws, B, H, W, (W + 31) / 32, kHHalf,
-                                                          kWHalf, (int)nwords, ntiles, 0, 0,
-                                                          clear_raw ? const_cast<uint32_t*>(raw_bits) : nullptr,
-                                                          (int32_t*)tile_ws, cb::tile_grid_y(H), cb::tile_grid_xp(W),
-                                                          no_list);
+  uint32_t* clear = clear_raw ? const_cast<uint32_t*>(raw_bits) : nullptr;
+  if (stream_counts)
+    cb::launch(dilate_compact_kernel<true>, ntiles, kCompactThreads, 0, s, raw_bits, dil_bits, dil_map, idx, count,
+               ws, B, H, W, (W + 31) / 32, kHHalf, kWHalf, (int)nwords, ntiles, 0, 0, clear, (int32_t*)tile_ws,
+               cb::tile_grid_y(H), cb::tile_grid_xp(W), no_list, stream_counts, stream_acc);
+  else
+    cb::launch(dilate_compact_kernel<false>, ntiles, kCompactThreads, 0, s, raw_bits, dil_bits, dil_map, idx, count,
+               ws, B, H, W, (W + 31) / 32, kHHalf, kWHalf, (int)nwords, ntiles, 0, 0, clear, (int32_t*)tile_ws,
+               cb::tile_grid_y(H), cb::tile_grid_xp(W), no_list, nullptr, nullptr);
   CB_CHECK_LAUNCH("dilate_compact");
   return 0;
+}
+
+int cb_dilate_compact_streams(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits, int8_t* dil_map,
+                              int32_t* idx, int32_t* count, void* ws, int B, int H, int W, int kHHalf,
+                              int kWHalf, int clear_raw, int32_t* stream_counts, int32_t* stream_acc) {
+  return dilate_compact_impl(stream, raw_bits, dil_bits, dil_map, idx, count, ws, nullptr, B, H, W,
+                             kHHalf, kWHalf, clear_raw, 0, stream_counts, stream_acc);
 }
 
 int cb_dilate_compact(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits, int8_t* dil_map,
                       int32_t* idx, int32_t* count, void* ws, int B, int H, int W, int kHHalf,
                       int kWHalf, int clear_raw) {
-  return dilate_compact_impl(stream, raw_bits, dil_bits, dil_map, idx, count, ws, nullptr, B, H, W,
-                             kHHalf, kWHalf, clear_raw);
+  return cb_dilate_compact_streams(stream, raw_bits, dil_bits, dil_map, idx, count, ws, B, H, W, kHHalf, kWHalf,
+                                   clear_raw, nullptr, nullptr);
+}
+
+int cb_dilate_compact_tiles_streams(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits,
+                                    int8_t* dil_map, int32_t* idx, int32_t* count, void* ws, void* tile_ws,
+                                    int B, int H, int W, int kHHalf, int kWHalf, int clear_raw,
+                                    int32_t* stream_counts, int32_t* stream_acc) {
+  CB_CHECK_ARG(tile_ws, "dilate_compact_tiles: null tile workspace");
+  CB_CHECK_STREAMS(stream_counts, stream_acc, "dilate_compact_tiles");
+  if ((long long)cb_bitmap_words(B, H, W) == 0) cudaMemsetAsync((int32_t*)tile_ws + 1, 0, sizeof(int32_t), (cudaStream_t)stream);
+  return dilate_compact_impl(stream, raw_bits, dil_bits, dil_map, idx, count, ws, tile_ws, B, H, W,
+                             kHHalf, kWHalf, clear_raw, 0, stream_counts, stream_acc);
 }
 
 int cb_dilate_compact_tiles(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits,
                             int8_t* dil_map, int32_t* idx, int32_t* count, void* ws, void* tile_ws,
                             int B, int H, int W, int kHHalf, int kWHalf, int clear_raw) {
-  CB_CHECK_ARG(tile_ws, "dilate_compact_tiles: null tile workspace");
+  return cb_dilate_compact_tiles_streams(stream, raw_bits, dil_bits, dil_map, idx, count, ws, tile_ws, B, H, W,
+                                         kHHalf, kWHalf, clear_raw, nullptr, nullptr);
+}
+
+int cb_dilate_tiles_streams(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits, int32_t* count, void* ws,
+                            void* tile_ws, int B, int H, int W, int kHHalf, int kWHalf, int clear_raw,
+                            int32_t* stream_counts, int32_t* stream_acc) {
+  CB_CHECK_ARG(tile_ws && dil_bits, "dilate_tiles: null pointer");
+  CB_CHECK_STREAMS(stream_counts, stream_acc, "dilate_tiles");
   if ((long long)cb_bitmap_words(B, H, W) == 0) cudaMemsetAsync((int32_t*)tile_ws + 1, 0, sizeof(int32_t), (cudaStream_t)stream);
-  return dilate_compact_impl(stream, raw_bits, dil_bits, dil_map, idx, count, ws, tile_ws, B, H, W,
-                             kHHalf, kWHalf, clear_raw);
+  return dilate_compact_impl(stream, raw_bits, dil_bits, nullptr, nullptr, count, ws, tile_ws, B, H, W,
+                             kHHalf, kWHalf, clear_raw, 1, stream_counts, stream_acc);
 }
 
 int cb_dilate_tiles(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits, int32_t* count, void* ws,
                     void* tile_ws, int B, int H, int W, int kHHalf, int kWHalf, int clear_raw) {
-  CB_CHECK_ARG(tile_ws && dil_bits, "dilate_tiles: null pointer");
-  if ((long long)cb_bitmap_words(B, H, W) == 0) cudaMemsetAsync((int32_t*)tile_ws + 1, 0, sizeof(int32_t), (cudaStream_t)stream);
-  return dilate_compact_impl(stream, raw_bits, dil_bits, nullptr, nullptr, count, ws, tile_ws, B, H, W,
-                             kHHalf, kWHalf, clear_raw, 1);
+  return cb_dilate_tiles_streams(stream, raw_bits, dil_bits, count, ws, tile_ws, B, H, W, kHHalf, kWHalf,
+                                 clear_raw, nullptr, nullptr);
+}
+
+int cb_stream_bucket(void* stream, const int32_t* idx, const int32_t* count, int B, int hw,
+                     int32_t* stream_counts, int32_t* stream_acc) {
+  CB_CHECK_ARG(idx && count && stream_counts, "stream_bucket: null pointer");
+  CB_CHECK_STREAMS(stream_counts, stream_acc, "stream_bucket");
+  CB_CHECK_ARG(B > 0 && hw >= 0 && (long long)B * hw < (1ll << 31), "stream_bucket: bad shape B = %d, H*W = %d",
+               B, hw);
+  cudaStream_t s = (cudaStream_t)stream;
+  if (hw == 0) return zero_stream_counts(s, stream_counts, B, "stream_bucket");
+  const long long cap = (long long)sm_count() * 4, need = ((long long)B * hw + 255) / 256;
+  const unsigned grid = (unsigned)(need < cap ? need : cap);
+  cb::launch(stream_bucket_kernel, grid, 256, 0, s, idx, count, hw, B, stream_counts, stream_acc);
+  CB_CHECK_LAUNCH("stream_bucket");
+  return 0;
 }
 
 int cb_pool_compact(void* stream, const uint32_t* in_bits, uint32_t* out_bits, int32_t* idx,
@@ -196,10 +250,10 @@ int cb_pool_compact(void* stream, const uint32_t* in_bits, uint32_t* out_bits, i
   }
   CB_CHECK_ARG(nwords < (1ll << 31), "pool_compact: bitmap too large");
   const int ntiles = (int)((nwords + kCompactTile - 1) / kCompactTile);
-  cb::launch(dilate_compact_kernel, ntiles, kCompactThreads, 0, s, in_bits, out_bits, nullptr, idx, count, ws,
+  cb::launch(dilate_compact_kernel<false>, ntiles, kCompactThreads, 0, s, in_bits, out_bits, nullptr, idx, count, ws,
                                                           B, oH, oW, (oW + 31) / 32, 0, 0,
                                                           (int)nwords, ntiles, H, (W + 31) / 32, nullptr,
-                                                          nullptr, 0, 0, 0);
+                                                          nullptr, 0, 0, 0, nullptr, nullptr);
   CB_CHECK_LAUNCH("pool_compact");
   return 0;
 }
@@ -222,6 +276,37 @@ int cb_change_detect_sparse(void* stream, int dtype, const void* x, long long x_
 
 int cb_compact_small_max_words(void) { return cb::kCompactWin; }
 
+int cb_change_detect_sparse_compact_streams(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
+                                            long long x_sy, long long x_sx, void* state, long long s_sb,
+                                            long long s_sc, long long s_sy, long long s_sx, int aux_mode,
+                                            void* aux_hi, void* aux_lo, const int32_t* candidates,
+                                            const int32_t* n_candidates, uint32_t* raw_bits, int B, int C, int H,
+                                            int W, float threshold, int update_mode, int bits_are_clear,
+                                            uint32_t* dil_bits, int32_t* idx, int32_t* count, void* sync_ws,
+                                            int kHHalf, int kWHalf, int clear_raw, int32_t* stream_counts,
+                                            int32_t* stream_acc) {
+  CB_CHECK_ARG(x && state && raw_bits && candidates && n_candidates && idx && count && sync_ws,
+               "change_detect_sparse_compact: null pointer");
+  CB_CHECK_STREAMS(stream_counts, stream_acc, "change_detect_sparse_compact");
+  CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect_sparse_compact: bad shape");
+  CB_CHECK_ARG(kHHalf >= 0 && kWHalf >= 0 && kWHalf <= 31, "change_detect_sparse_compact: kWHalf must be <= 31");
+  CB_CHECK_ARG(raw_bits != dil_bits, "change_detect_sparse_compact: dil_bits must not alias raw_bits");
+  const long long nwords = (long long)cb_bitmap_words(B, H, W);
+  if (nwords == 0) {
+    cudaMemsetAsync(count, 0, sizeof(int32_t), (cudaStream_t)stream);
+    return zero_stream_counts((cudaStream_t)stream, stream_counts, B, "change_detect_sparse_compact");
+  }
+  CB_CHECK_ARG(nwords <= cb::kCompactWin, "change_detect_sparse_compact: bitmap of %lld words > %d", nwords,
+               cb::kCompactWin);
+  cb::FusedCompact fc{dil_bits, idx, count, (unsigned*)sync_ws, kHHalf, kWHalf, (int)nwords, clear_raw,
+                      stream_counts, stream_acc, B};
+  CB_DISPATCH_DTYPE(dtype, return (launch_detect_sparse<T, VEC>(
+                               (cudaStream_t)stream, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc,
+                               s_sy, s_sx, aux_mode, aux_hi, aux_lo, candidates, n_candidates, raw_bits,
+                               B, C, H, W, threshold, update_mode, bits_are_clear, &fc)));
+  return 0;
+}
+
 int cb_change_detect_sparse_compact(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
                                     long long x_sy, long long x_sx, void* state, long long s_sb,
                                     long long s_sc, long long s_sy, long long s_sx, int aux_mode,
@@ -230,24 +315,10 @@ int cb_change_detect_sparse_compact(void* stream, int dtype, const void* x, long
                                     int W, float threshold, int update_mode, int bits_are_clear,
                                     uint32_t* dil_bits, int32_t* idx, int32_t* count, void* sync_ws,
                                     int kHHalf, int kWHalf, int clear_raw) {
-  CB_CHECK_ARG(x && state && raw_bits && candidates && n_candidates && idx && count && sync_ws,
-               "change_detect_sparse_compact: null pointer");
-  CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect_sparse_compact: bad shape");
-  CB_CHECK_ARG(kHHalf >= 0 && kWHalf >= 0 && kWHalf <= 31, "change_detect_sparse_compact: kWHalf must be <= 31");
-  CB_CHECK_ARG(raw_bits != dil_bits, "change_detect_sparse_compact: dil_bits must not alias raw_bits");
-  const long long nwords = (long long)cb_bitmap_words(B, H, W);
-  if (nwords == 0) {
-    cudaMemsetAsync(count, 0, sizeof(int32_t), (cudaStream_t)stream);
-    return 0;
-  }
-  CB_CHECK_ARG(nwords <= cb::kCompactWin, "change_detect_sparse_compact: bitmap of %lld words > %d", nwords,
-               cb::kCompactWin);
-  cb::FusedCompact fc{dil_bits, idx, count, (unsigned*)sync_ws, kHHalf, kWHalf, (int)nwords, clear_raw};
-  CB_DISPATCH_DTYPE(dtype, return (launch_detect_sparse<T, VEC>(
-                               (cudaStream_t)stream, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc,
-                               s_sy, s_sx, aux_mode, aux_hi, aux_lo, candidates, n_candidates, raw_bits,
-                               B, C, H, W, threshold, update_mode, bits_are_clear, &fc)));
-  return 0;
+  return cb_change_detect_sparse_compact_streams(stream, dtype, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy,
+                                                 s_sx, aux_mode, aux_hi, aux_lo, candidates, n_candidates, raw_bits,
+                                                 B, C, H, W, threshold, update_mode, bits_are_clear, dil_bits, idx,
+                                                 count, sync_ws, kHHalf, kWHalf, clear_raw, nullptr, nullptr);
 }
 
 int cb_map_to_bits(void* stream, const int8_t* map, uint32_t* bits, int B, int H, int W) {
@@ -445,33 +516,57 @@ int cb_conv_update_tiled_pool(void* stream, int dtype, int gemm, const void* sta
                          update_mode);
 }
 
-int cb_conv_update_masked(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
-                          int pitch_in, const int32_t* idx, const int32_t* count, const void* packed_w,
-                          const float* bias, void* out, int pitch_out, int B, int H, int W, int Cin,
-                          int Cout, int kH, int kW, int relu, void* ws, size_t ws_bytes,
-                          uint32_t* mask_bits, int clear_mask, int32_t* count_out, void* sync_ws) {
+int cb_conv_update_masked_streams(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
+                                  int pitch_in, const int32_t* idx, const int32_t* count, const void* packed_w,
+                                  const float* bias, void* out, int pitch_out, int B, int H, int W, int Cin,
+                                  int Cout, int kH, int kW, int relu, void* ws, size_t ws_bytes,
+                                  uint32_t* mask_bits, int clear_mask, int32_t* count_out, void* sync_ws,
+                                  int32_t* stream_counts, int32_t* stream_acc) {
   CB_CHECK_ARG(mask_bits && sync_ws, "conv_update_masked: null pointer");
+  CB_CHECK_STREAMS(stream_counts, stream_acc, "conv_update_masked");
+  CB_CHECK_ARG(!stream_counts || gemm != CB_GEMM_SIMT_F32, "conv_update_masked: tensor-core modes only");
   cb::RowMask mk;
   mk.bits = mask_bits;
   mk.clear = clear_mask ? mask_bits : nullptr;
   mk.count_out = count_out;
   mk.sync = (unsigned*)sync_ws;
   mk.nwords = (int)cb_bitmap_words(B, H, W);
+  mk.stream_counts = stream_counts;
+  mk.stream_acc = stream_acc;
+  mk.B = B;
+  if (stream_counts && (H == 0 || W == 0))                // nothing is launched below
+    if (int rc = zero_stream_counts((cudaStream_t)stream, stream_counts, B, "conv_update_masked")) return rc;
   return conv_update_impl(mk, stream, dtype, gemm, state, state_lo, pitch_in, idx, count, packed_w, bias,
                           out, pitch_out, B, H, W, Cin, Cout, kH, kW, relu ? 1 : 0, ws, ws_bytes);
+}
+
+int cb_conv_update_masked(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
+                          int pitch_in, const int32_t* idx, const int32_t* count, const void* packed_w,
+                          const float* bias, void* out, int pitch_out, int B, int H, int W, int Cin,
+                          int Cout, int kH, int kW, int relu, void* ws, size_t ws_bytes,
+                          uint32_t* mask_bits, int clear_mask, int32_t* count_out, void* sync_ws) {
+  return cb_conv_update_masked_streams(stream, dtype, gemm, state, state_lo, pitch_in, idx, count, packed_w, bias,
+                                       out, pitch_out, B, H, W, Cin, Cout, kH, kW, relu, ws, ws_bytes, mask_bits,
+                                       clear_mask, count_out, sync_ws, nullptr, nullptr);
 }
 
 int cb_tail_supported(int dtype, int gemm, int C0, int C1, int C2) {
   return dtype == CB_F32 && gemm == CB_GEMM_TC_BF16X3 && cb::tail_supported(C0, C1, C2) ? 1 : 0;
 }
 
-int cb_tail_update(void* stream, const float* x, float* state1, const void* packed_w1, const float* bias1,
-                   float* out1, int relu1, float thr1, float* state2, const void* packed_w2,
-                   const float* bias2, float* out2, int pitch_out2, int relu2, float thr2,
-                   const int32_t* candidates, const int32_t* n_candidates, int C0, int C1, int C2,
-                   int update_mode, int32_t* count1, int32_t* count2, void* sync_ws) {
+int cb_tail_update_streams(void* stream, const float* x, float* state1, const void* packed_w1, const float* bias1,
+                           float* out1, int relu1, float thr1, float* state2, const void* packed_w2,
+                           const float* bias2, float* out2, int pitch_out2, int relu2, float thr2,
+                           const int32_t* candidates, const int32_t* n_candidates, int C0, int C1, int C2,
+                           int update_mode, int32_t* count1, int32_t* count2, void* sync_ws, int B, int hw,
+                           int32_t* stream_counts1, int32_t* stream_acc1, int32_t* stream_counts2,
+                           int32_t* stream_acc2) {
   CB_CHECK_ARG(x && state1 && packed_w1 && bias1 && out1 && state2 && packed_w2 && bias2 && out2 && candidates &&
                    n_candidates && count1 && count2 && sync_ws, "tail_update: null pointer");
+  CB_CHECK_STREAMS(stream_counts1, stream_acc1, "tail_update");
+  CB_CHECK_STREAMS(stream_counts2, stream_acc2, "tail_update");
+  CB_CHECK_ARG(!stream_counts1 == !stream_counts2, "tail_update: per-stream counts for both layers or neither");
+  CB_CHECK_ARG(!stream_counts1 || (B > 0 && hw > 0), "tail_update: bad shape B = %d, H*W = %d", B, hw);
   CB_CHECK_ARG(update_mode == CB_UPDATE_NONE || update_mode == CB_UPDATE_CHANGED || update_mode == CB_UPDATE_ALL,
                "tail_update: bad update_mode %d", update_mode);
   CB_CHECK_ARG(((uintptr_t)x % 16) == 0 && ((uintptr_t)state1 % 16) == 0 && ((uintptr_t)out1 % 16) == 0 &&
@@ -484,7 +579,19 @@ int cb_tail_update(void* stream, const float* x, float* state1, const void* pack
   a.count1 = count1; a.count2 = count2; a.sync = (unsigned*)sync_ws;
   a.xp = C0; a.p1 = C1; a.p2 = pitch_out2; a.C0 = C0; a.C1 = C1; a.C2 = C2;
   a.relu1 = relu1; a.relu2 = relu2; a.update = update_mode; a.thr1 = thr1; a.thr2 = thr2;
+  a.sc1 = stream_counts1; a.sc2 = stream_counts2; a.acc1 = stream_acc1; a.acc2 = stream_acc2;
+  a.hw = hw; a.B = B;
   return cb::tail_update((cudaStream_t)stream, a, packed_w1, packed_w2);
+}
+
+int cb_tail_update(void* stream, const float* x, float* state1, const void* packed_w1, const float* bias1,
+                   float* out1, int relu1, float thr1, float* state2, const void* packed_w2,
+                   const float* bias2, float* out2, int pitch_out2, int relu2, float thr2,
+                   const int32_t* candidates, const int32_t* n_candidates, int C0, int C1, int C2,
+                   int update_mode, int32_t* count1, int32_t* count2, void* sync_ws) {
+  return cb_tail_update_streams(stream, x, state1, packed_w1, bias1, out1, relu1, thr1, state2, packed_w2, bias2,
+                                out2, pitch_out2, relu2, thr2, candidates, n_candidates, C0, C1, C2, update_mode,
+                                count1, count2, sync_ws, 0, 0, nullptr, nullptr, nullptr, nullptr);
 }
 
 int cb_maxpool2x2(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,

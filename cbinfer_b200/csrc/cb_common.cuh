@@ -175,4 +175,18 @@ __device__ __forceinline__ void st16(void* p, const uint4& v) {
   *reinterpret_cast<uint4*>(p) = v;
 }
 
+// ---- per-stream change counts (cb_*_streams entry points) ----------------------------------
+// Adds `c` to acc[b] for every stream b held by a lane of the warp: one atomic per (warp, stream).
+// Lanes may hold streams in any order; b < 0 marks a lane with nothing to add.  All 32 lanes call.
+__device__ __forceinline__ void stream_add_warp(int b, unsigned c, int32_t* acc) {
+  const unsigned same = __match_any_sync(0xffffffffu, b);
+  const unsigned sum = __reduce_add_sync(same, c);
+  if (b >= 0 && sum && (int)(threadIdx.x & 31) == __ffs(same) - 1) atomicAdd(acc + b, (int)sum);
+}
+// Run by the block that publishes a kernel's total, after every block's additions to `acc`:
+// counts[b] = acc[b], and acc is left zero for the next launch.
+__device__ __forceinline__ void stream_publish(int32_t* acc, int32_t* counts, int B) {
+  for (int b = threadIdx.x; b < B; b += blockDim.x) counts[b] = atomicExch(acc + b, 0);
+}
+
 }  // namespace cb

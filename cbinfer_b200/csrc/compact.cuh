@@ -97,13 +97,17 @@ __device__ __forceinline__ unsigned pooled_word(const uint32_t* __restrict__ raw
 // order the hardware dispatches blocks in, so the look-back cannot starve (as in CUB's single-pass
 // scan).  Tile-only mode has no scan across tiles and keeps blockIdx, and so do grids small enough to
 // be resident as a whole.
+// TRACK: the count is also split by stream: every warp adds its words' popcounts to stream_acc[b]
+// (int32 [B], zero at rest), and the last tile copies it to stream_counts[b] and zeroes it again.
+template <bool TRACK>
 __global__ void __launch_bounds__(kCompactThreads)
 dilate_compact_kernel(const uint32_t* __restrict__ raw, uint32_t* __restrict__ dil_bits,
                       int8_t* __restrict__ dil_map, int32_t* __restrict__ idx,
                       int32_t* __restrict__ count, void* ws, int B, int H, int W, int Wd, int kh,
                       int kw, int nwords, int ntiles, int pool_hin, int pool_wdin,
                       uint32_t* __restrict__ clear_bits, int32_t* __restrict__ tile_ws, int tile_ty,
-                      int tile_xp, int no_list) {
+                      int tile_xp, int no_list, int32_t* __restrict__ stream_counts,
+                      int32_t* __restrict__ stream_acc) {
   CompactHeader* hdr = reinterpret_cast<CompactHeader*>(ws);
   volatile unsigned long long* tstate =
       reinterpret_cast<volatile unsigned long long*>(reinterpret_cast<char*>(ws) + sizeof(CompactHeader));
@@ -184,7 +188,10 @@ dilate_compact_kernel(const uint32_t* __restrict__ raw, uint32_t* __restrict__ d
       tt0[i] = t0;
     }
     cnt += __popc(d[i]);
+    // (a word never spans two streams: rows are padded to whole words)
+    if constexpr (TRACK) stream_add_warp(w < nwords ? w / Wd / H : -1, __popc(d[i]), stream_acc);
   }
+  if constexpr (TRACK) __threadfence();       // my additions precede the block's done-increment
 
   if (no_list) {
     // tiles only (the consumer walks the tile list and masks rows with dil_bits): no ordered index
@@ -343,6 +350,10 @@ dilate_compact_kernel(const uint32_t* __restrict__ raw, uint32_t* __restrict__ d
     if (s_last)
       for (int i = tid; i < nwords; i += kCompactThreads) clear_bits[i] = 0u;
   }
+  if constexpr (TRACK) {
+    __syncthreads();
+    if (s_last) stream_publish(stream_acc, stream_counts, B);
+  }
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -353,11 +364,15 @@ dilate_compact_kernel(const uint32_t* __restrict__ raw, uint32_t* __restrict__ d
 // dependent-launch chain, not by bytes (pose network: 92 layers of <= 4416 bitmap words at batch 1).
 // Same results as dilate_compact_kernel: dilated bitmap, ascending index list, count; optional
 // zeroing of the raw bitmap.  All threads of the block must call it; `s_win` holds kCompactWin words.
+// TRACK: the count split by stream is written to stream_counts[0, B), through stream_acc as in
+// dilate_compact_kernel.
 // ------------------------------------------------------------------------------------------------
+template <bool TRACK>
 __device__ __forceinline__ void block_dilate_compact(uint32_t* __restrict__ raw, uint32_t* __restrict__ dil_bits,
                                                      int32_t* __restrict__ idx, int32_t* __restrict__ count,
                                                      uint32_t* s_win, int* s_warp, int H, int W, int Wd,
-                                                     int kh, int kw, int nwords, bool clear) {
+                                                     int kh, int kw, int nwords, bool clear,
+                                                     int32_t* stream_counts, int32_t* stream_acc, int B) {
   const int tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31, wid = tid >> 5, nwarp = nthr >> 5;
   for (int i = tid; i < nwords; i += nthr) s_win[i] = __ldcg(raw + i);     // (written by other blocks: L2)
   __syncthreads();
@@ -395,8 +410,50 @@ __device__ __forceinline__ void block_dilate_compact(uint32_t* __restrict__ raw,
     }
   }
   if (tid == 0) *count = total;
+  if constexpr (TRACK) {
+    // word k of every thread in one warp-wide step (lanes hold ascending words of few streams)
+    for (int k = 0; k < wpt; ++k) {
+      const int w = w0 + k;
+      const bool have = w < w1;
+      const unsigned d = have ? dilated_word(s_win, 0, w / Wd, (w / Wd) % H, w % Wd, H, W, Wd, kh, kw) : 0u;
+      stream_add_warp(have ? w / Wd / H : -1, __popc(d), stream_acc);
+    }
+    __threadfence();
+    __syncthreads();
+    stream_publish(stream_acc, stream_counts, B);
+  }
   if (clear)
     for (int i = tid; i < nwords; i += nthr) raw[i] = 0u;
+}
+
+// ------------------------------------------------------------------------------------------------
+// stream_bucket_kernel -- per-stream counts of an index list the layer did not build itself (handed on
+// from upstream or by the user; any order): counts[b] = #{ j < *count : idx[j] / hw == b }.  `acc` is
+// int32 [B + 1], zero at rest: the per-stream sums, then the finished-block counter; the last block
+// copies the sums to `counts` and leaves `acc` zero.  Indices outside [0, B*hw) are not counted.
+// ------------------------------------------------------------------------------------------------
+__global__ void __launch_bounds__(256)
+stream_bucket_kernel(const int32_t* __restrict__ idx, const int32_t* __restrict__ count, int hw, int B,
+                     int32_t* __restrict__ counts, int32_t* __restrict__ acc) {
+  __shared__ unsigned s_last;
+  const int n = *count;
+  for (long long j0 = (long long)blockIdx.x * blockDim.x; j0 < n; j0 += (long long)gridDim.x * blockDim.x) {
+    const long long j = j0 + threadIdx.x;
+    int b = -1;
+    if (j < n) {
+      const int v = __ldg(idx + j);
+      if (v >= 0 && v / hw < B) b = v / hw;
+    }
+    stream_add_warp(b, 1u, acc);
+  }
+  __threadfence();
+  __syncthreads();
+  if (threadIdx.x == 0) s_last = atomicAdd(reinterpret_cast<unsigned*>(acc + B), 1u) == gridDim.x - 1u;
+  __syncthreads();
+  if (!s_last) return;
+  __threadfence();
+  stream_publish(acc, counts, B);
+  if (threadIdx.x == 0) acc[B] = 0;
 }
 
 __global__ void map_to_bits_kernel(const int8_t* __restrict__ map, uint32_t* __restrict__ bits,

@@ -318,15 +318,21 @@ __device__ __forceinline__ void st_release_gpu(uint32_t* p, uint32_t v) {
 // compaction between detection and contraction for layers that need no dilation.  The number of
 // processed pixels is written to *count_out; with `clear` the last CTA to finish zeroes the bitmap
 // (ready for the next frame's atomicOr-ing detection).  `sync` = {done counter, count accumulator},
-// zeroed once by the caller, left clean by the kernel.
+// zeroed once by the caller, left clean by the kernel.  With `stream_counts` (the kernel's TRACK
+// variant) the processed pixels are also counted per stream b = pix / (H*W): added to stream_acc
+// (int32 [B], zero at rest), copied to stream_counts and zeroed by the same last CTA.
 struct RowMask {
   const uint32_t* bits;
   uint32_t* clear;
   int32_t* count_out;
   unsigned* sync;
   int nwords;
+  int32_t* stream_counts;
+  int32_t* stream_acc;
+  int B;
 };
 // (s_flag: one word of dynamic shared memory -- the kernel must not own static shared memory)
+template <bool TRACK>
 __device__ __forceinline__ void rowmask_finish(const RowMask& mk, volatile unsigned* s_flag) {
   // every CTA of the selected variant passes here exactly once, after its last read of the bitmap
   __syncthreads();
@@ -342,6 +348,7 @@ __device__ __forceinline__ void rowmask_finish(const RowMask& mk, volatile unsig
     if (mk.count_out) *mk.count_out = (int32_t)atomicExch(mk.sync + 1, 0u);
     mk.sync[0] = 0u;
   }
+  if constexpr (TRACK) stream_publish(mk.stream_acc, mk.stream_counts, mk.B);
   if (mk.clear)
     for (int i = threadIdx.x; i < mk.nwords; i += blockDim.x) mk.clear[i] = 0u;
 }
@@ -349,7 +356,7 @@ __device__ __forceinline__ void rowmask_finish(const RowMask& mk, volatile unsig
 // packed weights: [NSPLIT][CoutPad][KpPad] elements of T (K-major); tensor map dims {KpPad, NSPLIT*CoutPad}
 // T = operand element type in the state planes / shared memory, TO = element type of `out`
 // (TO != T only for 3xBF16: bf16 hi/lo operand planes of an fp32 layer).
-template <typename T, typename TO, bool SPLIT3, int BN, bool DEEP>
+template <typename T, typename TO, bool SPLIT3, int BN, bool DEEP, bool TRACK>
 __global__ void __launch_bounds__(um_threads(BN))
 conv_umma_kernel(const __grid_constant__ CUtensorMap wmap, const T* __restrict__ state,
                  const T* __restrict__ state_lo, int Cp, const int32_t* __restrict__ idx, const int32_t* __restrict__ count,
@@ -380,7 +387,7 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap wmap, const T* __restrict__
   const bool sk = !DEEP && sk_ws != nullptr;              // stream-K (never together with clusters)
   if (!sk && tile0 >= total_tiles) {                      // group-uniform: before any barrier / alloc
     if (KSmax > 1) { cluster_sync_all(); cluster_sync_all(); }   // busy peers still sync twice
-    if (mk.bits) rowmask_finish(mk, reinterpret_cast<volatile unsigned*>(smem_raw));
+    if (mk.bits) rowmask_finish<TRACK>(mk, reinterpret_cast<volatile unsigned*>(smem_raw));
     return;
   }
 
@@ -398,7 +405,7 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap wmap, const T* __restrict__
   const long long sk_grid = sk ? (sk_units < (long long)gridDim.x ? (sk_units > 0 ? sk_units : 1)
                                                                   : (long long)gridDim.x) : 1;
   if (sk && (long long)blockIdx.x >= sk_grid) {            // CTA-uniform: before any barrier / alloc
-    if (mk.bits) rowmask_finish(mk, reinterpret_cast<volatile unsigned*>(smem_raw));
+    if (mk.bits) rowmask_finish<TRACK>(mk, reinterpret_cast<volatile unsigned*>(smem_raw));
     return;
   }
   if (sk)
@@ -501,6 +508,10 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap wmap, const T* __restrict__
         if (mk.bits && kb0 == 0 && tile - mt * ntiles == 0 && krank == 0) {   // once per M tile
           const unsigned m = __ballot_sync(0xffffffffu, pix >= 0);
           if ((tid & 31) == 0 && m) atomicAdd(mk.sync + 1, (unsigned)__popc(m));
+          if constexpr (TRACK) {
+            stream_add_warp(pix >= 0 ? pix / P : -1, 1u, mk.stream_acc);
+            __threadfence();                                // before this CTA's rowmask_finish
+          }
         }
       }
       asm volatile("bar.sync 1, %0;" ::"n"(UM_PRODUCERS) : "memory");   // producers only
@@ -843,7 +854,7 @@ conv_umma_kernel(const __grid_constant__ CUtensorMap wmap, const T* __restrict__
                  "r"((uint32_t)C::TMEM_COLS)
                  : "memory");
   }
-  if (mk.bits) rowmask_finish(mk, &ctrl->pad);
+  if (mk.bits) rowmask_finish<TRACK>(mk, &ctrl->pad);
 }
 
 // ---- weight packing ----------------------------------------------------------------------------
@@ -957,7 +968,7 @@ inline PFN_cuTensorMapEncodeTiled_v12000 tensor_map_encoder() {
   return fn;
 }
 
-template <typename T, typename TO, bool SPLIT3, int BN, bool DEEP>
+template <typename T, typename TO, bool SPLIT3, int BN, bool DEEP, bool TRACK>
 int launch_conv_umma(cudaStream_t s, int dtype, const void* state, const void* state_lo, int Cp,
                      const int32_t* idx,
                      const int32_t* count, const void* packed, const float* bias, void* out,
@@ -982,7 +993,7 @@ int launch_conv_umma(cudaStream_t s, int dtype, const void* state, const void* s
                          CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
                          CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return fail(3, "conv_update: cuTensorMapEncodeTiled failed (%d)", (int)r);
-  auto kern = conv_umma_kernel<T, TO, SPLIT3, BN, DEEP>;
+  auto kern = conv_umma_kernel<T, TO, SPLIT3, BN, DEEP, TRACK>;
   static thread_local int attr_dev = -1;
   int dev = 0;
   cudaGetDevice(&dev);
@@ -1069,7 +1080,7 @@ int launch_conv_umma(cudaStream_t s, int dtype, const void* state, const void* s
   return 0;
 }
 
-template <typename T, typename TO, bool SPLIT3, bool DEEP>
+template <typename T, typename TO, bool SPLIT3, bool DEEP, bool TRACK>
 int dispatch_bn(int bn, cudaStream_t s, int dtype, const void* state, const void* state_lo, int Cp,
                 const int32_t* idx,
                 const int32_t* count, const void* packed, const float* bias, void* out, int Op,
@@ -1077,7 +1088,7 @@ int dispatch_bn(int bn, cudaStream_t s, int dtype, const void* state, const void
                 int sel_hi, int ksplit, void* ws, size_t ws_bytes, const RowMask& mk) {
 #define CB_BN(N)                                                                              \
   case N:                                                                                     \
-    return launch_conv_umma<T, TO, SPLIT3, N, DEEP>(s, dtype, state, state_lo, Cp, idx, count, packed, bias, out, \
+    return launch_conv_umma<T, TO, SPLIT3, N, DEEP, TRACK>(s, dtype, state, state_lo, Cp, idx, count, packed, bias, out, \
                                           Op, B, H, W, Cout, CoutPad, kH, kW, relu, sel_lo,   \
                                           sel_hi, ksplit, ws, ws_bytes, mk);
   if constexpr (DEEP) {                        // the deep variant only exists for N tiles <= 64
@@ -1117,29 +1128,33 @@ inline int umma_conv_update(cudaStream_t s, int dtype, int gemm, const void* sta
   // layers) but give few CTAs when few pixels changed; the count is only known on the device, so
   // when a small change set is plausible (expected tiles at 10 % change < half the SMs) a second,
   // finer tiling is launched as well and each kernel checks the count to see whether it is its turn.
-  auto run_t = [&](auto deep_tag, int tile_n, int lo, int hi, int ksplit = 1) -> int {
-    constexpr bool DP = decltype(deep_tag)::value;
+  auto run_tt = [&](auto deep_tag, auto track_tag, int tile_n, int lo, int hi, int ksplit) -> int {
+    constexpr bool DP = decltype(deep_tag)::value, TR = decltype(track_tag)::value;
     if (bf16x3)
-      return dispatch_bn<__nv_bfloat16, float, true, DP>(tile_n, s, dtype, state, state_lo, Cp, idx,
+      return dispatch_bn<__nv_bfloat16, float, true, DP, TR>(tile_n, s, dtype, state, state_lo, Cp, idx,
                                                          count, packed, bias, out, Op, B, H, W,
                                                          Cout, CoutPad, kH, kW, relu, lo, hi, ksplit, ws, ws_bytes, mk);
     switch (dtype) {
       case CB_F32:
-        return split3 ? dispatch_bn<float, float, true, DP>(tile_n, s, dtype, state, state_lo, Cp, idx, count,
+        return split3 ? dispatch_bn<float, float, true, DP, TR>(tile_n, s, dtype, state, state_lo, Cp, idx, count,
                                                  packed, bias, out, Op, B, H, W, Cout, CoutPad, kH,
                                                  kW, relu, lo, hi, ksplit, ws, ws_bytes, mk)
-                      : dispatch_bn<float, float, false, DP>(tile_n, s, dtype, state, state_lo, Cp, idx, count,
+                      : dispatch_bn<float, float, false, DP, TR>(tile_n, s, dtype, state, state_lo, Cp, idx, count,
                                                   packed, bias, out, Op, B, H, W, Cout, CoutPad,
                                                   kH, kW, relu, lo, hi, ksplit, ws, ws_bytes, mk);
       case CB_F16:
-        return dispatch_bn<__half, __half, false, DP>(tile_n, s, dtype, state, state_lo, Cp, idx, count, packed,
+        return dispatch_bn<__half, __half, false, DP, TR>(tile_n, s, dtype, state, state_lo, Cp, idx, count, packed,
                                           bias, out, Op, B, H, W, Cout, CoutPad, kH, kW, relu, lo, hi, ksplit, ws, ws_bytes, mk);
       case CB_BF16:
-        return dispatch_bn<__nv_bfloat16, __nv_bfloat16, false, DP>(tile_n, s, dtype, state, state_lo, Cp, idx, count,
+        return dispatch_bn<__nv_bfloat16, __nv_bfloat16, false, DP, TR>(tile_n, s, dtype, state, state_lo, Cp, idx, count,
                                                  packed, bias, out, Op, B, H, W, Cout, CoutPad, kH,
                                                  kW, relu, lo, hi, ksplit, ws, ws_bytes, mk);
       default: return fail(2, "conv_update: bad dtype %d", dtype);
     }
+  };
+  auto run_t = [&](auto deep_tag, int tile_n, int lo, int hi, int ksplit = 1) -> int {
+    return mk.stream_counts ? run_tt(deep_tag, std::true_type{}, tile_n, lo, hi, ksplit)
+                            : run_tt(deep_tag, std::false_type{}, tile_n, lo, hi, ksplit);
   };
   const long long P = (long long)B * H * W;
   const int sms = sm_count();

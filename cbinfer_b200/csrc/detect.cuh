@@ -587,9 +587,12 @@ struct FusedCompact {
   int32_t* count;
   unsigned* sync;                // one word, zero at rest: blocks done
   int kh, kw, nwords, clear;
+  int32_t* stream_counts;        // TRACK: the count split by stream (int32 [B]) and its accumulator
+  int32_t* stream_acc;
+  int B;
 };
 
-template <typename T, int VEC, int UPDATE, bool FUSE = false>
+template <typename T, int VEC, int UPDATE, bool FUSE = false, bool TRACK = false>
 __global__ void __launch_bounds__(256)
 detect_sparse_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int xp,
                          T* __restrict__ st, long long s_sb, long long s_sy, int sp,
@@ -654,8 +657,8 @@ detect_sparse_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy
     __syncthreads();
     if (!s_last) return;
     __threadfence();
-    block_dilate_compact(bits, fc.dil_bits, fc.idx, fc.count, s_win, s_warp, H, W, Wd, fc.kh, fc.kw, fc.nwords,
-                         fc.clear != 0);
+    block_dilate_compact<TRACK>(bits, fc.dil_bits, fc.idx, fc.count, s_win, s_warp, H, W, Wd, fc.kh, fc.kw,
+                                fc.nwords, fc.clear != 0, fc.stream_counts, fc.stream_acc, fc.B);
   }
 }
 
@@ -707,9 +710,12 @@ int launch_detect_sparse(cudaStream_t stream, const void* x, long long x_sb, lon
   }
   CB_CHECK_ARG(!fuse || (vec_ok && words <= kCompactWin), "change_detect_sparse_compact: needs pixel-major "
                "tensors and a bitmap of at most %d words", kCompactWin);
-  FusedCompact fc = fuse ? *fuse : FusedCompact{nullptr, nullptr, nullptr, nullptr, 0, 0, 0, 0};
+  FusedCompact fc = fuse ? *fuse : FusedCompact{nullptr, nullptr, nullptr, nullptr, 0, 0, 0, 0, nullptr, nullptr, 0};
   return dispatch_update(update, "change_detect_sparse", [&](auto U) {
-    if (vec_ok && fuse)
+    if (vec_ok && fuse && fc.stream_counts)
+      cb::launch(detect_sparse_vec_kernel<T, VEC, U, true, true>, grid, 256, 0, stream, (const T*)x, x_sb, x_sy,
+                 (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand, ncand, bits, H, W, C, Wd, thr, glog, fc);
+    else if (vec_ok && fuse)
       cb::launch(detect_sparse_vec_kernel<T, VEC, U, true>, grid, 256, 0, stream, (const T*)x, x_sb, x_sy,
                  (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand, ncand, bits, H, W, C, Wd, thr, glog, fc);
     else if (vec_ok)

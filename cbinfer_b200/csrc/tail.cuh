@@ -42,6 +42,10 @@ struct TailArgs {
   int C0, C1, C2;                // channels: in, mid, out
   int relu1, relu2, update;      // update: CB_UPDATE_CHANGED (feedback) or CB_UPDATE_ALL
   float thr1, thr2;
+  // TRACK: count1 / count2 split by stream b = pixel / hw into sc1 / sc2 (int32 [B] each), through the
+  // accumulators acc1 / acc2 (int32 [B] each, zero at rest), which the last CTA copies and zeroes
+  int32_t *sc1, *sc2, *acc1, *acc2;
+  int hw, B;
 };
 
 struct TailCtrl {
@@ -57,7 +61,7 @@ __device__ __forceinline__ uint32_t tail_sw128(int r, int k) {
   return (uint32_t)((r >> 3) * 1024 + (r & 7) * 128 + ((((k & 63) >> 3) ^ (r & 7)) << 4) + (k & 7) * 2);
 }
 
-template <int N1>
+template <int N1, bool TRACK>
 __global__ void __launch_bounds__(TAIL_THREADS)
 tail_kernel(const __grid_constant__ CUtensorMap w1map, const __grid_constant__ CUtensorMap w2map,
             const TailArgs a) {
@@ -89,6 +93,7 @@ tail_kernel(const __grid_constant__ CUtensorMap w1map, const __grid_constant__ C
   TailCtrl* ctrl = reinterpret_cast<TailCtrl*>(w2s + 2 * W2_B);
   auto retire = [&](int c1, int c2) {                        // every CTA passes here exactly once
     if (tid == 0) {
+      if constexpr (TRACK) ctrl->pad = 0u;                   // (all threads: "this CTA publishes")
       if (c1) atomicAdd(a.sync + 1, (unsigned)c1);
       if (c2) atomicAdd(a.sync + 2, (unsigned)c2);
       __threadfence();
@@ -97,6 +102,14 @@ tail_kernel(const __grid_constant__ CUtensorMap w1map, const __grid_constant__ C
         *a.count1 = (int32_t)atomicExch(a.sync + 1, 0u);
         *a.count2 = (int32_t)atomicExch(a.sync + 2, 0u);
         a.sync[0] = 0u;
+        if constexpr (TRACK) ctrl->pad = 1u;
+      }
+    }
+    if constexpr (TRACK) {
+      __syncthreads();
+      if (*reinterpret_cast<volatile uint32_t*>(&ctrl->pad)) {
+        stream_publish(a.acc1, a.sc1, a.B);
+        stream_publish(a.acc2, a.sc2, a.B);
       }
     }
   };
@@ -278,6 +291,11 @@ tail_kernel(const __grid_constant__ CUtensorMap w1map, const __grid_constant__ C
         for (int c = 0; c < a.C1; c += 4) st16(s2 + c, ld16(o1 + c));
       tot1 += pix1 >= 0;
       tot2 += (pix1 >= 0 && f2);
+      if constexpr (TRACK) {
+        stream_add_warp(pix1 >= 0 ? pix1 / a.hw : -1, 1u, a.acc1);
+        stream_add_warp(pix1 >= 0 && f2 ? pix1 / a.hw : -1, 1u, a.acc2);
+        __threadfence();                                     // before this CTA's retire
+      }
       tc_fence_before();
       fence_proxy_async_smem();
     }
@@ -383,22 +401,23 @@ inline int tail_update(cudaStream_t s, const TailArgs& a, const void* packed1, c
   const size_t smem = (size_t)2 * nkb1 * TAIL_ROWS * UM_ROW_BYTES + (size_t)2 * nkb1 * N1 * UM_ROW_BYTES +
                       2 * 16 * UM_ROW_BYTES + sizeof(TailCtrl) + 64;
   const unsigned grid = (unsigned)sm_count();
-#define CB_TAIL(N_)                                                                                  \
+#define CB_TAIL(N_, TR_)                                                                             \
   {                                                                                                  \
     static thread_local int adev = -1;                                                               \
     int dev = 0;                                                                                     \
     cudaGetDevice(&dev);                                                                             \
     if (adev != dev) {                                                                               \
-      if (cudaFuncSetAttribute(tail_kernel<N_>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024) != cudaSuccess) \
+      if (cudaFuncSetAttribute(tail_kernel<N_, TR_>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024) != cudaSuccess) \
         return fail(3, "tail_update: cannot reserve shared memory");                                \
       adev = dev;                                                                                    \
     }                                                                                                \
-    cb::launch(tail_kernel<N_>, dim3(grid), dim3(TAIL_THREADS), smem, s, m1, m2, a);                 \
+    cb::launch(tail_kernel<N_, TR_>, dim3(grid), dim3(TAIL_THREADS), smem, s, m1, m2, a);            \
   }
+  const bool track = a.sc1 != nullptr;
   switch (N1) {
-    case 16: CB_TAIL(16) break;
-    case 32: CB_TAIL(32) break;
-    case 64: CB_TAIL(64) break;
+    case 16: if (track) CB_TAIL(16, true) else CB_TAIL(16, false) break;
+    case 32: if (track) CB_TAIL(32, true) else CB_TAIL(32, false) break;
+    case 64: if (track) CB_TAIL(64, true) else CB_TAIL(64, false) break;
     default: return fail(2, "tail_update: bad mid channel count %d", N1);
   }
 #undef CB_TAIL

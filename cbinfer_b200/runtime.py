@@ -44,10 +44,14 @@ class FramePipeline(object):
     their slices cross PCIe and the others are skipped by the model (cbinfer_b200.setActiveStreams).
     The constructor sets an all-active mask on the model before capturing the graphs, and refuses a
     model in which a module other than a CB layer reads the input frame directly: the input slot of
-    a skipped stream holds a stale frame, which only the mask-honouring CB layers may be given."""
+    a skipped stream holds a stale frame, which only the mask-honouring CB layers may be given.
 
-    def __init__(self, model, example_frame, depth=2, activeStreams=False):
-        from . import CBConv2d, CBPoolMax2d, setActiveStreams
+    trackChanges=True: the model's per-stream change counts (cbinfer_b200.trackStreamChanges, enabled
+    here if it is not yet) travel with each slot's output: ``changeCounts(slot)`` is the int32 [L, B]
+    host copy of the frame's counts, valid after ``wait(slot)``."""
+
+    def __init__(self, model, example_frame, depth=2, activeStreams=False, trackChanges=False):
+        from . import CBConv2d, CBPoolMax2d, setActiveStreams, streamChangeCounts, trackStreamChanges
         dev = example_frame.device
         assert dev.type == "cuda"
         self.model = model
@@ -71,6 +75,8 @@ class FramePipeline(object):
             if activeStreams:
                 setActiveStreams(model, torch.ones(B, dtype=torch.uint8, device=dev))
                 self._mask = next(c._activeMask for c in model.modules() if type(c) is CBConv2d)
+            if trackChanges and not any(type(c) is CBConv2d and c._streamRow is not None for c in model.modules()):
+                trackStreamChanges(model, B=B)
             try:
                 probe = model(self.inputs[0])                 # allocates state on first use
             finally:
@@ -100,6 +106,13 @@ class FramePipeline(object):
             # buffer on the copy stream would race with the previous slot's replay)
             self.mask_host = [torch.ones(B, dtype=torch.uint8).pin_memory() for _ in range(depth)]
             self.mask_dev = [torch.ones(B, dtype=torch.uint8, device=dev) for _ in range(depth)]
+        self._counts = None
+        if trackChanges:
+            # the model's buffer is rewritten by every replay: copied per slot on the compute stream right
+            # after the replay (as the output), then to pinned host memory on the copy stream
+            self._counts = streamChangeCounts(model)
+            self.counts_dev = [torch.empty_like(self._counts) for _ in range(depth)]
+            self.counts_host = [torch.empty(self._counts.shape, dtype=torch.int32).pin_memory() for _ in range(depth)]
         self.t = 0
         for e in self.in_free + self.out_done:
             e.record(self.compute)
@@ -151,10 +164,14 @@ class FramePipeline(object):
             out = self.graphs[s].replay()
             self.in_free[s].record(self.compute)
             self.out_dev[s].copy_(out[0] if self._multi else out)
+            if self._counts is not None:
+                self.counts_dev[s].copy_(self._counts)
             self.out_ready[s].record(self.compute)
         with torch.cuda.stream(self.d2h):
             self.d2h.wait_event(self.out_ready[s])
             self.out_host[s].copy_(self.out_dev[s], non_blocking=True)
+            if self._counts is not None:
+                self.counts_host[s].copy_(self.counts_dev[s], non_blocking=True)
             self.out_done[s].record(self.d2h)
         return s
 
@@ -169,6 +186,13 @@ class FramePipeline(object):
     def wait(self, slot):
         self.out_done[slot].synchronize()
         return self.out_host[slot]
+
+    def changeCounts(self, slot):
+        """The per-stream change counts (int32 [L, B] host tensor, see trackStreamChanges) of the frame
+        last submitted to `slot`; valid after ``wait(slot)``.  Needs FramePipeline(trackChanges=True)."""
+        if self._counts is None:
+            raise CBinferError("FramePipeline.changeCounts needs FramePipeline(trackChanges=True)")
+        return self.counts_host[slot]
 
     def drain(self):
         self.h2d.synchronize()

@@ -292,6 +292,55 @@ int cb_tail_update(void* stream, const float* x, float* state1, const void* pack
                    const int32_t* candidates, const int32_t* n_candidates, int C0, int C1, int C2,
                    int update_mode, int32_t* count1, int32_t* count2, void* sync_ws);
 
+/* ---- per-stream change counts ---------------------------------------------------------------
+ * The *_streams entry points are the calls above plus one row of per-stream counts: on every call
+ * (also one with nothing to do) stream_counts[b], b < B, is set to the part of the call's count that
+ * lies in stream b -- pixel p belongs to stream p / (H*W) -- so the row sums to *count:
+ *   cb_dilate_compact / _tiles / cb_dilate_tiles and cb_change_detect_sparse_compact: dilated pixels;
+ *   cb_conv_update_masked: processed pixels (*count_out; tensor-core modes); cb_tail_update: the pixels
+ *   each layer updated (*count1 -> stream_counts1, *count2 -> stream_counts2, B streams of hw pixels).
+ * The row is written, never added to, so a CUDA graph needs no memset node for it.  stream_acc is the
+ * row's accumulator: int32 [B] of device memory, zeroed once at allocation, private to the row and
+ * left zero by every call; a non-NULL stream_counts needs it.  NULL stream_counts = the plain call
+ * (the entry points above forward here with NULL).
+ * cb_stream_bucket counts an index list the caller did not build with one of these calls (any order,
+ * *count read on the device): stream_counts[b] = #{ j < *count : idx[j] / hw == b }, indices outside
+ * [0, B*hw) not counted; its stream_acc is int32 [B + 1] (the last word counts finished blocks). */
+int cb_dilate_compact_streams(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits, int8_t* dil_map,
+                              int32_t* idx, int32_t* count, void* ws, int B, int H, int W, int kHHalf,
+                              int kWHalf, int clear_raw, int32_t* stream_counts, int32_t* stream_acc);
+int cb_dilate_compact_tiles_streams(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits,
+                                    int8_t* dil_map, int32_t* idx, int32_t* count, void* ws, void* tile_ws,
+                                    int B, int H, int W, int kHHalf, int kWHalf, int clear_raw,
+                                    int32_t* stream_counts, int32_t* stream_acc);
+int cb_dilate_tiles_streams(void* stream, const uint32_t* raw_bits, uint32_t* dil_bits, int32_t* count, void* ws,
+                            void* tile_ws, int B, int H, int W, int kHHalf, int kWHalf, int clear_raw,
+                            int32_t* stream_counts, int32_t* stream_acc);
+int cb_change_detect_sparse_compact_streams(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
+                                            long long x_sy, long long x_sx, void* state, long long s_sb,
+                                            long long s_sc, long long s_sy, long long s_sx, int aux_mode,
+                                            void* aux_hi, void* aux_lo, const int32_t* candidates,
+                                            const int32_t* n_candidates, uint32_t* raw_bits, int B, int C, int H,
+                                            int W, float threshold, int update_mode, int bits_are_clear,
+                                            uint32_t* dil_bits, int32_t* idx, int32_t* count, void* sync_ws,
+                                            int kHHalf, int kWHalf, int clear_raw, int32_t* stream_counts,
+                                            int32_t* stream_acc);
+int cb_conv_update_masked_streams(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
+                                  int pitch_in, const int32_t* idx, const int32_t* count, const void* packed_w,
+                                  const float* bias, void* out, int pitch_out, int B, int H, int W, int Cin,
+                                  int Cout, int kH, int kW, int relu, void* ws, size_t ws_bytes,
+                                  uint32_t* mask_bits, int clear_mask, int32_t* count_out, void* sync_ws,
+                                  int32_t* stream_counts, int32_t* stream_acc);
+int cb_tail_update_streams(void* stream, const float* x, float* state1, const void* packed_w1, const float* bias1,
+                           float* out1, int relu1, float thr1, float* state2, const void* packed_w2,
+                           const float* bias2, float* out2, int pitch_out2, int relu2, float thr2,
+                           const int32_t* candidates, const int32_t* n_candidates, int C0, int C1, int C2,
+                           int update_mode, int32_t* count1, int32_t* count2, void* sync_ws, int B, int hw,
+                           int32_t* stream_counts1, int32_t* stream_acc1, int32_t* stream_counts2,
+                           int32_t* stream_acc2);
+int cb_stream_bucket(void* stream, const int32_t* idx, const int32_t* count, int B, int hw,
+                     int32_t* stream_counts, int32_t* stream_acc);
+
 /* ---- change-based 2x2/stride-2 max pooling ------------------------------------------------
  * replaces: maxPool2d (conv2d_cg.py:33-37 -> cbconv2d_cg_backend.cu:199-240, half :207-250).
  * For every changed input pixel idx[j] (j < *count) recompute the max of its 2x2 window over
