@@ -18,7 +18,8 @@ from .conv2d_cg import ChangeIndexes
 __all__ = ['CBConv2d', 'CBPoolMax2d', 'ChangeIndexes', 'subsitute', 'convertRecur', 'mergeReLURecur',
            'propChangeIndexesOf1x1', 'clearMemory', 'getStateTensors', 'convert',
            'tuneThresholdParameters', 'convertPools', 'shareWorkspace', 'resetStreams',
-           'setActiveStreams', 'trackStreamChanges', 'streamChangeCounts']
+           'setActiveStreams', 'trackStreamChanges', 'streamChangeCounts', 'setStreamThresholds',
+           'streamThresholds']
 
 verbose = False
 
@@ -268,6 +269,108 @@ def streamChangeCounts(net):
         if type(c) is CBConv2d and c._streamRow is not None:
             return c._streamRow[0]
     raise CBinferError("streamChangeCounts: the model is not tracked (trackStreamChanges)")
+
+
+def setStreamThresholds(net, table):
+    """Give each video stream of a batched model its own change thresholds.  `table[l, b]` is the threshold
+    of CBConv2d l (every CBConv2d under `net` in named_modules() order, the row order of
+    trackStreamChanges) for stream b: wherever layer l's change detection runs -- its own kernel, an
+    upstream pool or tile epilogue, the fused tail -- stream b's pixels are tested against it, rounded to
+    the layer's data type as the scalar `threshold` is.  Stream b then computes exactly what the model
+    computes with the scalar thresholds ``table[:, b]`` (DESIGN.md section 3.15).  Returns the layers'
+    qualified names in row order.
+
+    The first call allocates one device fp32 [L, B] table, starting from the threshold each layer's last
+    detection used (its scalar before any frame), and hands every CBConv2d its row; later calls write into it on the current stream, so CUDA graphs
+    captured with the table read the values it holds at each replay.  Raising a value, or writing the same
+    value, takes effect in place.  LOWERING A VALUE RESTARTS THE STREAM when that row belongs to a layer
+    that thresholds only the candidates an upstream layer hands on (candidateDetect, fed a change set in
+    its last frame): pixels that no upstream change touches could now exceed the threshold, and only a
+    full rescan would find them.  The call therefore decides on the device which streams had such a value
+    lowered and resets them as resetStreams does, in the same enqueued work: their next frame is computed
+    as by a freshly cleared model with the new thresholds, and the other streams are not touched.  Layers
+    that scan their input densely every frame (plain input, no candidateDetect) never need this.
+
+    `table`: host values (nested lists, a numpy array or a CPU tensor [L, B]; checked for shape and for
+    NaN and infinite values, then copied asynchronously), or a CUDA fp32 tensor [L, B], copied on the
+    device so that the call can be captured in a CUDA graph; a CUDA table is not checked for its values.
+    B comes from the table attached already, else from the layers' state, else from `table`.  While a
+    table is attached the scalar `threshold` is not read: a frame raises CBinferError if it was assigned
+    since.  None detaches the table: each layer's next eager frame scans densely (the scalar threshold may
+    have been lowered), and graphs captured with the table must not be replayed after detaching.
+    Fine-grained layers and gatherComputationStats are not supported."""
+    named = [(name, c) for name, c in net.named_modules() if type(c) is CBConv2d]
+    convs = [c for _, c in named]
+    if table is None:
+        for c in convs:
+            if c._thrRow is not None:
+                c._thrRow = None
+                c._lastThr = None
+        return []
+    for c in convs:
+        if c.finegrained or (c._auxPlanes is not None and c._auxPlanes[0] == 'fg'):
+            raise CBinferError("setStreamThresholds: fine-grained layers (cb_fg_detect) take one scalar threshold")
+        if c.gatherComputationStats:
+            raise CBinferError("setStreamThresholds: gatherComputationStats thresholds with the scalar threshold")
+    L = len(convs)
+    cur = next((c._thrRow[0] for c in convs if c._thrRow is not None), None)
+    state = [c._inBuf for c in convs if c._inBuf is not None]
+    if cur is not None:
+        B, dev = cur.shape[1], cur.device
+    elif state:
+        B, dev = state[0].shape[0], state[0].device
+    else:
+        B, dev = None, next(net.parameters()).device
+    if isinstance(table, torch.Tensor) and table.is_cuda:
+        if table.dtype != torch.float32 or table.dim() != 2 or table.shape[0] != L \
+                or (B is not None and table.shape[1] != B) or (dev.type == "cuda" and table.device != dev):
+            raise CBinferError("setStreamThresholds: a CUDA fp32 table [%d, %s] on %s is needed, got %s %s on %s"
+                               % (L, B if B is not None else "B", dev, table.dtype, tuple(table.shape), table.device))
+        new, dev = table, table.device
+    else:
+        host = torch.as_tensor(table, dtype=torch.float32)
+        if host.dim() != 2 or host.shape[0] != L or (B is not None and host.shape[1] != B):
+            raise CBinferError("setStreamThresholds: a table [%d, %s] is needed, got %s"
+                               % (L, B if B is not None else "B", tuple(host.shape)))
+        if not bool(torch.isfinite(host).all()):
+            raise CBinferError("setStreamThresholds: the table holds NaN or infinite values")
+        new = None
+    B = new.shape[1] if new is not None else host.shape[1]
+    if B < 1:
+        raise CBinferError("setStreamThresholds: B = %d streams" % B)
+    if dev.type != "cuda":
+        raise CBinferError("setStreamThresholds: the model is on %s; the table lives on a CUDA device" % dev)
+    if new is None:
+        new = host.to(dev, non_blocking=True)
+    if cur is None:
+        # the thresholds the layers' state was built with: the one each layer's last detection used, or
+        # its scalar before any detection (then there is no state the table could make inexact)
+        built = [c._lastThr if c._lastThr is not None else c.threshold for c in convs]
+        cur = torch.tensor([float(t) for t in built], dtype=torch.float32).to(dev).unsqueeze(1) \
+            .repeat(1, B).contiguous()
+        for l, c in enumerate(convs):
+            c._thrRow = (cur, l, c.threshold)
+    # a stream restarts if a layer that tests only the candidates handed to it got a lower value
+    fed = [l for l, c in enumerate(convs) if c.candidateDetect and c._lastPlain is False]
+    segments = [seg for layer in _cb_layers(net) for seg in layer._resetSegments()]
+    lowered = None
+    if fed and segments and new is not cur:
+        lowered = torch.stack([new[l] < cur[l] for l in fed]).any(0)
+    if new is not cur:
+        cur.copy_(new)
+    if lowered is not None:
+        _cg.reset_streams(segments, lowered)
+    return [name for name, _ in named]
+
+
+def streamThresholds(net):
+    """The device fp32 [L, B] table of per-stream thresholds attached by setStreamThresholds: the same tensor
+    until it is detached.  Write it through setStreamThresholds: a value lowered by writing into the tensor
+    directly does not restart the streams that need it."""
+    for c in net.modules():
+        if type(c) is CBConv2d and c._thrRow is not None:
+            return c._thrRow[0]
+    raise CBinferError("streamThresholds: no per-stream thresholds are attached (setStreamThresholds)")
 
 
 def getStateTensors(net):

@@ -36,6 +36,9 @@ SYMBOLS = [
     "cb_dilate_compact_streams", "cb_dilate_compact_tiles_streams", "cb_dilate_tiles_streams",
     "cb_change_detect_sparse_compact_streams", "cb_conv_update_masked_streams", "cb_tail_update_streams",
     "cb_stream_bucket",
+    "cb_change_detect_thr", "cb_change_detect_u8_thr", "cb_change_detect_sparse_thr",
+    "cb_change_detect_sparse_compact_thr", "cb_maxpool2x2_detect_thr", "cb_conv_update_tiled_pool_thr",
+    "cb_tail_update_thr",
 ]
 
 
@@ -131,6 +134,12 @@ def _load():
         sig[name + "_streams"] = (i32, sig[name][1] + [vp, vp])
     sig["cb_tail_update_streams"] = (i32, sig["cb_tail_update"][1] + [i32, i32, vp, vp, vp, vp])
     sig["cb_stream_bucket"] = (i32, [vp, vp, vp, i32, i32, vp, vp])
+    # the *_thr variants: the newest variant's arguments + the per-stream thresholds (one table per layer)
+    for name in ("cb_change_detect_streams", "cb_change_detect_u8_streams", "cb_change_detect_sparse",
+                 "cb_change_detect_sparse_compact_streams", "cb_maxpool2x2_detect", "cb_conv_update_tiled_pool",
+                 "cb_tail_update_streams"):
+        tables = 2 if name == "cb_tail_update_streams" else 1
+        sig[name.replace("_streams", "") + "_thr"] = (i32, sig[name][1] + [vp] * tables)
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
         fn.restype = res

@@ -176,7 +176,7 @@ class CBPoolMax2d(nn.Module):
         if tgt is not None:
             # pooling + the next layer's detection in one kernel (cb_maxpool2x2_detect)
             cg.maxPool2d_detect(input, self.outputState, changeIndexes, tgt['next_state'], tgt['next_raw_bits'],
-                                tgt['threshold'], tgt['mode'], aux=tgt['aux'])
+                                tgt['threshold'], tgt['mode'], aux=tgt['aux'], thr_b=tgt['thr_b'])
             return DetectionDone(nxt)
         cg.maxPool2d(input, self.outputState, changeIndexes, self.kernel_size, self.stride)
         if self.propPooledIndexes and changeIndexes.bits is not None:
@@ -242,6 +242,10 @@ class CBConv2d(nn.Module):
         # per-stream change counts (cbinfer_b200.trackStreamChanges): (counts int32 [L,B], this layer's
         # row l, accumulators int32 [L,B+1] zeroed once), or None = not tracked
         self._streamRow = None
+        # per-stream thresholds (cbinfer_b200.setStreamThresholds): (table fp32 [L,B], this layer's row l, the
+        # scalar threshold when the table was attached), or None = the scalar threshold for every stream
+        self._thrRow = None
+        self._lastPlain = None    # was the last frame's input plain (not a change set)?  None: no frame yet
         self._wsHolder = cg.ConvWorkspace()    # shared per model by pycbinfer.convert()
         self.register_buffer('prevInput', self.weight.data.new_empty(0))
         self.register_buffer('prevOutput', self.weight.data.new_empty(0))
@@ -275,7 +279,8 @@ class CBConv2d(nn.Module):
         # no fused neighbours, and without a version record the state counts as touched
         super(CBConv2d, self).__setstate__(state)
         self._setDefaultValues()
-        for name in ('_fusedPool', '_fusedTail', '_inVersion', '_outVersion', '_activeMask', '_streamRow'):
+        for name in ('_fusedPool', '_fusedTail', '_inVersion', '_outVersion', '_activeMask', '_streamRow', '_thrRow',
+                     '_lastPlain'):
             self.__dict__.setdefault(name, None)
 
     # ---- state ---------------------------------------------------------------------------
@@ -335,9 +340,11 @@ class CBConv2d(nn.Module):
     def _candidatesExact(self, shape, dtype, device):
         """Rule 2: may this frame threshold only the candidate pixels (cb_change_detect_sparse)?  Exact
         while the state is the kernels' own, untouched, not fresh, and the threshold not lowered:
-        every other pixel then still lies within the threshold of the state."""
+        every other pixel then still lies within the threshold of the state.  With per-stream
+        thresholds attached, a stream whose value was lowered is started over by setStreamThresholds
+        itself, so the scalar comparison does not apply."""
         return self.candidateDetect and not self.finegrained and not self._fresh \
-            and self._lastThr is not None and self.threshold >= self._lastThr \
+            and self._lastThr is not None and (self._thrRow is not None or self.threshold >= self._lastThr) \
             and self._stateAllocated(shape, dtype, device) and not any(self._stateTouched())
 
     def _recordDetection(self):
@@ -389,7 +396,7 @@ class CBConv2d(nn.Module):
             return None
         gemm, _, _ = self._weights(dtype, device)
         return dict(next_state=self.prevInput, next_raw_bits=self._scratch["raw_bits"],
-                    threshold=self.threshold,
+                    threshold=self.threshold, thr_b=self._thrB(shape[0]),
                     mode=_lib.UPDATE_CHANGED if self.feedbackLoop else _lib.UPDATE_ALL,
                     aux=self._aux(gemm))
 
@@ -494,10 +501,12 @@ class CBConv2d(nn.Module):
             # cb_tail_update ran this layer's detection and contraction too; it split the operands on
             # the fly, so this layer's operand planes are stale
             self._auxPlanes = None
+            self._lastPlain = False
             return self._frameDone(handed.candidates, handed.candidates if self.propChangeIndexes else None)
         B, _, H, W = input.shape
         dev, dt = input.device, input.dtype
         rows = self._streams(B)
+        self._thrB(B)             # (a table of another batch size raises before any state is touched)
         detected = isinstance(handed, DetectionDone)
         upstream = None           # the upstream layer's change list
         if handed is not None and not detected:
@@ -507,6 +516,7 @@ class CBConv2d(nn.Module):
         # a layer fed with plain frames re-scans them densely every frame, which rewrites every word of
         # its raw bitmap: nothing ever ORs bits into it, so its compaction need not zero it afterwards
         plain_input = handed is None or (detected and handed.dense)
+        self._lastPlain = plain_input
         # uint8 frames (decoder output) are normalised inside the detection kernel:
         # value = u8 / divisor + bias with inputNorm = (divisor, bias); the layer computes in fp32
         u8norm = None
@@ -619,6 +629,7 @@ class CBConv2d(nn.Module):
         s = self._scratch
         mode = _lib.UPDATE_CHANGED if self.feedbackLoop else _lib.UPDATE_ALL
         active = None if sparse_next else self._streamMask(B)
+        thr_b = self._thrB(B)
         # extension: no compaction at all for a 1x1 layer on the candidate path - the
         # contraction walks the candidate list and skips pixels whose raw bit is not set
         # (cb_conv_update_masked); this layer's own index list is then never materialised
@@ -634,13 +645,13 @@ class CBConv2d(nn.Module):
             cg.detect_sparse_compact(input, self.prevInput, s["raw_bits"], self.threshold, mode, candidates,
                                      self.kernel_size, s["idx"], s["count"], s["sdc_sync"], aux=aux,
                                      bits_are_clear=s.get("raw_clear", False), dil_bits=s["dil_bits"],
-                                     clear_raw=sparse_next, streams=self._streams(B))
+                                     clear_raw=sparse_next, streams=self._streams(B), thr_b=thr_b)
             s["raw_clear"] = sparse_next
             changes = ChangeIndexes(s["idx"], s["count"], (B, H, W), bits=s["dil_bits"])
         elif candidates is not None:
             cg.detect_sparse(input, self.prevInput, s["raw_bits"], self.threshold, mode,
                              candidates, aux=aux,
-                             bits_are_clear=s.get("raw_clear", False))
+                             bits_are_clear=s.get("raw_clear", False), thr_b=thr_b)
             if masked:
                 if "mask_sync" not in s:
                     s["mask_sync"] = torch.zeros(2, dtype=torch.int32, device=input.device)
@@ -651,9 +662,9 @@ class CBConv2d(nn.Module):
                 changes.superset = True
         elif u8norm is not None:
             cg.detect_u8(input, self.prevInput, s["raw_bits"], self.threshold, mode,
-                         u8norm[0], u8norm[1], aux=aux, active=active)
+                         u8norm[0], u8norm[1], aux=aux, active=active, thr_b=thr_b)
         else:
-            cg.detect(input, self.prevInput, s["raw_bits"], self.threshold, mode, aux=aux, active=active)
+            cg.detect(input, self.prevInput, s["raw_bits"], self.threshold, mode, aux=aux, active=active, thr_b=thr_b)
         self._recordDetection()
         return changes, mask
 
@@ -667,6 +678,30 @@ class CBConv2d(nn.Module):
             raise _lib.CBinferError("per-stream change counts of %d streams, the frame has %d (trackStreamChanges)"
                                     % (counts.shape[1], B))
         return counts[l], acc[l]
+
+    def _thrB(self, B):
+        """This layer's row of per-stream thresholds (fp32 [B] on the device) for a frame of B streams, or
+        None when no table is attached (cbinfer_b200.setStreamThresholds)."""
+        if self._thrRow is None:
+            return None
+        table, l, _ = self._thrRow
+        if table.shape[1] != B:
+            raise _lib.CBinferError("per-stream thresholds of %d streams, the frame has %d (setStreamThresholds)"
+                                    % (table.shape[1], B))
+        return table[l]
+
+    def _checkThresholds(self):
+        """Refuse what a frame with per-stream thresholds attached cannot honour."""
+        if self._thrRow is None:
+            return
+        if self.finegrained:
+            raise _lib.CBinferError("per-stream thresholds are not supported on a fine-grained layer")
+        if self.gatherComputationStats:
+            raise _lib.CBinferError("gatherComputationStats thresholds the whole input with the scalar threshold: "
+                                    "it cannot be combined with per-stream thresholds (setStreamThresholds)")
+        if self.threshold != self._thrRow[2]:
+            raise _lib.CBinferError("CBConv2d.threshold was assigned while per-stream thresholds are attached; the "
+                                    "kernels read the table (setStreamThresholds), so the assignment would do nothing")
 
     def _streamMask(self, B):
         """The active-stream mask for a frame of B streams, or None when none is set."""
@@ -690,7 +725,7 @@ class CBConv2d(nn.Module):
             return None
         gemm, packed, bias32 = self._weights(dt, dev)
         return dict(gemm=gemm, packed=packed, bias=bias32, state=self._inBuf, out=self._outBuf,
-                    thr=self.threshold, relu=self.withReLU, count=self._scratch["count"])
+                    thr=self.threshold, thr_b=self._thrB(shape[0]), relu=self.withReLU, count=self._scratch["count"])
 
     def _tryTail(self, input, changeIndexes, gemm, packed, bias32):
         if not self._fusedTail or os.environ.get("CBINFER_FUSE_TAIL", "1") == "0" \
@@ -722,7 +757,8 @@ class CBConv2d(nn.Module):
                        tgt['state'], tgt['packed'], tgt['bias'], tgt['out'], tgt['relu'], tgt['thr'],
                        changeIndexes, C0, C1, C2,
                        _lib.UPDATE_CHANGED if self.feedbackLoop else _lib.UPDATE_ALL,
-                       s["count"], tgt['count'], s["tail_sync"], streams1=rows1, streams2=rows2)
+                       s["count"], tgt['count'], s["tail_sync"], streams1=rows1, streams2=rows2,
+                       thr1_b=self._thrB(B), thr2_b=tgt['thr_b'])
         # the kernel splits its operands on the fly: this layer's operand planes are stale now
         self._auxPlanes = None
         self._recordDetection()
@@ -818,6 +854,7 @@ class CBConv2d(nn.Module):
 
     def forward(self, inp):
         with torch.no_grad():
+            self._checkThresholds()
             if self.finegrained:
                 assert(self.feedbackLoop == False)
                 if self._activeMask is not None:

@@ -139,22 +139,38 @@ def _active_ptr(active, B, device):
     return active.data_ptr()
 
 
-def detect(x, state, raw_bits, threshold, update_mode, aux=None, active=None):
+def _thr_ptr(thr_b, B, device):
+    """Device pointer of a per-stream threshold table (a contiguous fp32 CUDA tensor [B] on the data's
+    device), or None for none (the scalar threshold for every stream)."""
+    if thr_b is None:
+        return None
+    require_cuda(thr_b)
+    if thr_b.dim() != 1 or thr_b.dtype != torch.float32 or not thr_b.is_contiguous() \
+            or thr_b.numel() != B or thr_b.device != device:
+        raise _lib.CBinferError("per-stream thresholds: a contiguous fp32 tensor [%d] on %s is needed, got %s %s on %s"
+                                % (B, device, thr_b.dtype, tuple(thr_b.shape), thr_b.device))
+    return thr_b.data_ptr()
+
+
+def detect(x, state, raw_bits, threshold, update_mode, aux=None, active=None, thr_b=None):
     """cb_change_detect: raw (un-dilated) change bitmap of x vs state; updates state and, when
     given, the auxiliary operand planes `aux` (see _aux_args).  `active`: optional bool / uint8
     CUDA tensor [B], read on the device; a stream with active[b] == 0 is skipped (its bitmap words
-    0, its x not read, its state and planes untouched: cb_change_detect_streams)."""
+    0, its x not read, its state and planes untouched: cb_change_detect_streams).  `thr_b`: optional
+    fp32 CUDA tensor [B] of per-stream thresholds, read on the device instead of `threshold`
+    (cb_change_detect_thr); the same holds for every wrapper below that takes it."""
     require_cuda(x, state, raw_bits)
     B, Cc, H, W = x.shape
     assert state.shape == x.shape and state.dtype == x.dtype
     act = _active_ptr(active, B, x.device)
     mode, hi, lo = _aux_args(aux, state)
-    check(C.cb_change_detect_streams(stream_ptr(x.device), dtype_code(x), x.data_ptr(), *_strides4(x),
-                                     state.data_ptr(), *_strides4(state), mode, hi, lo,
-                                     raw_bits.data_ptr(), B, Cc, H, W, float(threshold), int(update_mode), act))
+    check(C.cb_change_detect_thr(stream_ptr(x.device), dtype_code(x), x.data_ptr(), *_strides4(x),
+                                 state.data_ptr(), *_strides4(state), mode, hi, lo,
+                                 raw_bits.data_ptr(), B, Cc, H, W, float(threshold), int(update_mode), act,
+                                 _thr_ptr(thr_b, B, x.device)))
 
 
-def detect_u8(x, state, raw_bits, threshold, update_mode, divisor, bias, aux=None, active=None):
+def detect_u8(x, state, raw_bits, threshold, update_mode, divisor, bias, aux=None, active=None, thr_b=None):
     """cb_change_detect_u8: detection on a uint8 frame normalised on the fly as u8/divisor + bias
     (the readers' /255 resp. /256 - 0.5); `state` is the fp32 pixel-major state.  Bit-identical to
     :func:`detect` on ``x.float() / divisor + bias``.  `active` as in :func:`detect`."""
@@ -163,14 +179,14 @@ def detect_u8(x, state, raw_bits, threshold, update_mode, divisor, bias, aux=Non
     assert x.dtype == torch.uint8 and state.dtype == torch.float32 and state.shape == x.shape
     act = _active_ptr(active, B, x.device)
     mode, hi, lo = _aux_args(aux, state)
-    check(C.cb_change_detect_u8_streams(stream_ptr(x.device), x.data_ptr(), *_strides4(x),
-                                        state.data_ptr(), *_strides4(state), mode, hi, lo,
-                                        raw_bits.data_ptr(), B, Cc, H, W, float(divisor), float(bias),
-                                        float(threshold), int(update_mode), act))
+    check(C.cb_change_detect_u8_thr(stream_ptr(x.device), x.data_ptr(), *_strides4(x),
+                                    state.data_ptr(), *_strides4(state), mode, hi, lo,
+                                    raw_bits.data_ptr(), B, Cc, H, W, float(divisor), float(bias),
+                                    float(threshold), int(update_mode), act, _thr_ptr(thr_b, B, x.device)))
 
 
 def detect_sparse(x, state, raw_bits, threshold, update_mode, candidates, aux=None,
-                  bits_are_clear=False):
+                  bits_are_clear=False, thr_b=None):
     """cb_change_detect_sparse: the detection test at the candidate pixels only (see the header
     for the exactness conditions).  `candidates` is a :class:`ChangeIndexes` at x's resolution."""
     require_cuda(x, state, raw_bits)
@@ -178,11 +194,11 @@ def detect_sparse(x, state, raw_bits, threshold, update_mode, candidates, aux=No
     assert state.shape == x.shape and state.dtype == x.dtype
     assert tuple(candidates.shape) == (B, H, W)
     mode, hi, lo = _aux_args(aux, state)
-    check(C.cb_change_detect_sparse(stream_ptr(x.device), dtype_code(x), x.data_ptr(), *_strides4(x),
-                                    state.data_ptr(), *_strides4(state), mode, hi, lo,
-                                    candidates.buffer.data_ptr(), candidates.count.data_ptr(),
-                                    raw_bits.data_ptr(), B, Cc, H, W, float(threshold),
-                                    int(update_mode), int(bool(bits_are_clear))))
+    check(C.cb_change_detect_sparse_thr(stream_ptr(x.device), dtype_code(x), x.data_ptr(), *_strides4(x),
+                                        state.data_ptr(), *_strides4(state), mode, hi, lo,
+                                        candidates.buffer.data_ptr(), candidates.count.data_ptr(),
+                                        raw_bits.data_ptr(), B, Cc, H, W, float(threshold),
+                                        int(update_mode), int(bool(bits_are_clear)), _thr_ptr(thr_b, B, x.device)))
 
 
 def _streams_args(streams, B):
@@ -211,7 +227,7 @@ def stream_bucket(changes, shape, streams):
 
 
 def detect_sparse_compact(x, state, raw_bits, threshold, update_mode, candidates, filtSize, idx, count, sync,
-                          aux=None, bits_are_clear=False, dil_bits=None, clear_raw=False, streams=None):
+                          aux=None, bits_are_clear=False, dil_bits=None, clear_raw=False, streams=None, thr_b=None):
     """cb_change_detect_sparse_compact: candidate detection + dilation + ordered compaction in one launch
     (small maps: at most cb_compact_small_max_words() bitmap words).  `sync` = int32[1], zeroed once.
     `streams`: optional (counts int32 [B], accumulator int32 [B] zeroed once): the count split by stream
@@ -221,12 +237,13 @@ def detect_sparse_compact(x, state, raw_bits, threshold, update_mode, candidates
     assert state.shape == x.shape and state.dtype == x.dtype
     assert tuple(candidates.shape) == (B, H, W)
     mode, hi, lo = _aux_args(aux, state)
-    check(C.cb_change_detect_sparse_compact_streams(
+    check(C.cb_change_detect_sparse_compact_thr(
         stream_ptr(x.device), dtype_code(x), x.data_ptr(), *_strides4(x), state.data_ptr(), *_strides4(state),
         mode, hi, lo, candidates.buffer.data_ptr(), candidates.count.data_ptr(), raw_bits.data_ptr(), B, Cc, H, W,
         float(threshold), int(update_mode), int(bool(bits_are_clear)),
         dil_bits.data_ptr() if dil_bits is not None else None, idx.data_ptr(), count.data_ptr(), sync.data_ptr(),
-        (filtSize[0] - 1) // 2, (filtSize[1] - 1) // 2, int(bool(clear_raw)), *_streams_args(streams, B)))
+        (filtSize[0] - 1) // 2, (filtSize[1] - 1) // 2, int(bool(clear_raw)), *_streams_args(streams, B),
+        _thr_ptr(thr_b, B, x.device)))
 
 
 def detect_compact_sparse(*args, **kwargs):
@@ -456,12 +473,12 @@ def conv_update_tiled(state_buf, tile_ws, dil_bits, packed_w, bias_f32, out_buf,
     assert out_buf.shape[:3] == state_buf.shape[:3]
     src, src_lo, pitch = _conv_operands(state_buf, Cin, gemm, aux)
     if pool is not None:
-        # pool = dict(out=pooled map view, next_state=view, next_raw_bits, threshold, mode, aux): the
-        # epilogue also re-pools the touched 2x2 windows and runs the next layer's detection on them
+        # pool = dict(out=pooled map view, next_state=view, next_raw_bits, threshold, mode, aux, optional
+        # thr_b): the epilogue also re-pools the touched 2x2 windows and runs the next layer's detection on them
         po, ns = pool["out"], pool["next_state"]
         assert po.stride(1) == 1 and ns.stride(1) == 1 and po.shape == ns.shape, "pixel-major maps only"
         mode, hi, lo = _aux_args(pool.get("aux"), ns)
-        check(C.cb_conv_update_tiled_pool(stream_ptr(state_buf.device), dtype_code(state_buf), gemm,
+        check(C.cb_conv_update_tiled_pool_thr(stream_ptr(state_buf.device), dtype_code(state_buf), gemm,
                                           src.data_ptr(), src_lo.data_ptr() if src_lo is not None else None,
                                           pitch, tile_ws.data_ptr(), dil_bits.data_ptr(), packed_w.data_ptr(),
                                           bias_f32.data_ptr(), out_buf.data_ptr(), out_buf.shape[3], B, H, W,
@@ -469,7 +486,8 @@ def conv_update_tiled(state_buf, tile_ws, dil_bits, packed_w, bias_f32, out_buf,
                                           po.data_ptr(), po.stride(0), po.stride(2), po.stride(3),
                                           po.size(2), po.size(3), ns.data_ptr(), ns.stride(0), ns.stride(2),
                                           ns.stride(3), mode, hi, lo, pool["next_raw_bits"].data_ptr(),
-                                          float(pool["threshold"]), int(pool["mode"])))
+                                          float(pool["threshold"]), int(pool["mode"]),
+                                          _thr_ptr(pool.get("thr_b"), B, state_buf.device)))
         return
     check(C.cb_conv_update_tiled(stream_ptr(state_buf.device), dtype_code(state_buf), gemm,
                                  src.data_ptr(), src_lo.data_ptr() if src_lo is not None else None,
@@ -480,21 +498,22 @@ def conv_update_tiled(state_buf, tile_ws, dil_bits, packed_w, bias_f32, out_buf,
 
 def tail_update(x_buf, state1_buf, packed1, bias1, out1_buf, relu1, thr1, state2_buf, packed2, bias2,
                 out2_buf, relu2, thr2, candidates, C0, C1, C2, update_mode, count1, count2, sync,
-                streams1=None, streams2=None):
+                streams1=None, streams2=None, thr1_b=None, thr2_b=None):
     """cb_tail_update: two chained 1x1 change-based layers (detect, contraction, detect,
     contraction) for the candidate pixels in one launch; pixel-major fp32 buffers [B,H,W,pitch].
     `streams1` / `streams2`: optional per-stream counts rows of the two layers, as in
-    :func:`detect_sparse_compact` (both or neither)."""
+    :func:`detect_sparse_compact` (both or neither).  `thr1_b` / `thr2_b`: the layers' per-stream thresholds."""
     assert x_buf.dtype == torch.float32 and x_buf.shape[3] == C0 and state1_buf.shape == x_buf.shape
     assert out1_buf.shape[3] == C1 and state2_buf.shape == out1_buf.shape
     B, H, W, _ = x_buf.shape
-    check(C.cb_tail_update_streams(stream_ptr(x_buf.device), x_buf.data_ptr(), state1_buf.data_ptr(),
+    check(C.cb_tail_update_thr(stream_ptr(x_buf.device), x_buf.data_ptr(), state1_buf.data_ptr(),
                            packed1.data_ptr(), bias1.data_ptr(), out1_buf.data_ptr(), int(bool(relu1)),
                            float(thr1), state2_buf.data_ptr(), packed2.data_ptr(), bias2.data_ptr(),
                            out2_buf.data_ptr(), out2_buf.shape[3], int(bool(relu2)), float(thr2),
                            candidates.buffer.data_ptr(), candidates.count.data_ptr(), C0, C1, C2,
                            int(update_mode), count1.data_ptr(), count2.data_ptr(), sync.data_ptr(), B, H * W,
-                           *_streams_args(streams1, B), *_streams_args(streams2, B)))
+                           *_streams_args(streams1, B), *_streams_args(streams2, B),
+                           _thr_ptr(thr1_b, B, x_buf.device), _thr_ptr(thr2_b, B, x_buf.device)))
 
 
 def reset_streams(segments, mask):
@@ -662,7 +681,7 @@ def maxPool2d(input, outputState, changeIndexes, kernelSize=(2, 2), stride=(2, 2
 
 
 def maxPool2d_detect(input, outputState, changeIndexes, next_state, next_raw_bits, threshold,
-                     update_mode, aux=None):
+                     update_mode, aux=None, thr_b=None):
     """cb_maxpool2x2_detect: change-based pooling fused with the next layer's detection (pixel-major
     tensors only; `changeIndexes.bits` required; `next_raw_bits` must be clear)."""
     require_cuda(input, outputState, next_state)
@@ -672,12 +691,13 @@ def maxPool2d_detect(input, outputState, changeIndexes, next_state, next_raw_bit
     for t in (input, outputState, next_state):
         assert t.stride(1) == 1, "pixel-major tensors only"
     mode, hi, lo = _aux_args(aux, next_state)
-    check(C.cb_maxpool2x2_detect(stream_ptr(input.device), dtype_code(input), input.data_ptr(),
+    check(C.cb_maxpool2x2_detect_thr(stream_ptr(input.device), dtype_code(input), input.data_ptr(),
                                  input.stride(0), input.stride(2), input.stride(3),
                                  changeIndexes.buffer.data_ptr(), changeIndexes.count.data_ptr(),
                                  changeIndexes.bits.data_ptr(), outputState.data_ptr(),
                                  outputState.stride(0), outputState.stride(2), outputState.stride(3),
                                  B, Cc, H, W, oH, oW, next_state.data_ptr(), next_state.stride(0),
                                  next_state.stride(2), next_state.stride(3), mode, hi, lo,
-                                 next_raw_bits.data_ptr(), float(threshold), int(update_mode)))
+                                 next_raw_bits.data_ptr(), float(threshold), int(update_mode),
+                                 _thr_ptr(thr_b, B, input.device)))
     return outputState

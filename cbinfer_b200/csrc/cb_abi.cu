@@ -85,18 +85,32 @@ int cb_channel_pitch(int dtype, int C) {
   return (C + v - 1) / v * v;
 }
 
+// per-stream thresholds (the *_thr entry points): fp32 [B] in device memory, or NULL = the scalar
+#define CB_CHECK_THR(thr_b, what) \
+  CB_CHECK_ARG(((uintptr_t)(thr_b) % sizeof(float)) == 0, what ": thr_b is not aligned to 4 bytes")
+
+int cb_change_detect_thr(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
+                         long long x_sy, long long x_sx, void* state, long long s_sb, long long s_sc,
+                         long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
+                         uint32_t* raw_bits, int B, int C, int H, int W, float threshold,
+                         int update_mode, const uint8_t* active, const float* thr_b) {
+  CB_CHECK_ARG(x && state && raw_bits, "change_detect: null pointer");
+  CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect: bad shape");
+  CB_CHECK_THR(thr_b, "change_detect");
+  CB_DISPATCH_DTYPE(dtype, return (launch_detect<T, VEC>((cudaStream_t)stream, x, x_sb, x_sc, x_sy,
+                                                        x_sx, state, s_sb, s_sc, s_sy, s_sx, aux_mode,
+                                                        aux_hi, aux_lo, raw_bits, B, C, H, W, threshold,
+                                                        update_mode, active, thr_b)));
+  return 0;
+}
+
 int cb_change_detect_streams(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
                              long long x_sy, long long x_sx, void* state, long long s_sb, long long s_sc,
                              long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
                              uint32_t* raw_bits, int B, int C, int H, int W, float threshold,
                              int update_mode, const uint8_t* active) {
-  CB_CHECK_ARG(x && state && raw_bits, "change_detect: null pointer");
-  CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect: bad shape");
-  CB_DISPATCH_DTYPE(dtype, return (launch_detect<T, VEC>((cudaStream_t)stream, x, x_sb, x_sc, x_sy,
-                                                        x_sx, state, s_sb, s_sc, s_sy, s_sx, aux_mode,
-                                                        aux_hi, aux_lo, raw_bits, B, C, H, W, threshold,
-                                                        update_mode, active)));
-  return 0;
+  return cb_change_detect_thr(stream, dtype, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy, s_sx, aux_mode,
+                              aux_hi, aux_lo, raw_bits, B, C, H, W, threshold, update_mode, active, nullptr);
 }
 
 int cb_change_detect(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
@@ -108,16 +122,27 @@ int cb_change_detect(void* stream, int dtype, const void* x, long long x_sb, lon
                                   aux_mode, aux_hi, aux_lo, raw_bits, B, C, H, W, threshold, update_mode, nullptr);
 }
 
+int cb_change_detect_u8_thr(void* stream, const uint8_t* x, long long x_sb, long long x_sc,
+                            long long x_sy, long long x_sx, float* state, long long s_sb, long long s_sc,
+                            long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
+                            uint32_t* raw_bits, int B, int C, int H, int W, float divisor, float bias,
+                            float threshold, int update_mode, const uint8_t* active, const float* thr_b) {
+  CB_CHECK_ARG(x && state && raw_bits, "change_detect_u8: null pointer");
+  CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect_u8: bad shape");
+  CB_CHECK_THR(thr_b, "change_detect_u8");
+  return launch_detect_u8((cudaStream_t)stream, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy,
+                          s_sx, aux_mode, aux_hi, aux_lo, raw_bits, B, C, H, W, divisor, bias,
+                          threshold, update_mode, active, thr_b);
+}
+
 int cb_change_detect_u8_streams(void* stream, const uint8_t* x, long long x_sb, long long x_sc,
                                 long long x_sy, long long x_sx, float* state, long long s_sb, long long s_sc,
                                 long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
                                 uint32_t* raw_bits, int B, int C, int H, int W, float divisor, float bias,
                                 float threshold, int update_mode, const uint8_t* active) {
-  CB_CHECK_ARG(x && state && raw_bits, "change_detect_u8: null pointer");
-  CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect_u8: bad shape");
-  return launch_detect_u8((cudaStream_t)stream, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy,
-                          s_sx, aux_mode, aux_hi, aux_lo, raw_bits, B, C, H, W, divisor, bias,
-                          threshold, update_mode, active);
+  return cb_change_detect_u8_thr(stream, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy, s_sx, aux_mode,
+                                 aux_hi, aux_lo, raw_bits, B, C, H, W, divisor, bias, threshold, update_mode,
+                                 active, nullptr);
 }
 
 int cb_change_detect_u8(void* stream, const uint8_t* x, long long x_sb, long long x_sc,
@@ -258,36 +283,49 @@ int cb_pool_compact(void* stream, const uint32_t* in_bits, uint32_t* out_bits, i
   return 0;
 }
 
+int cb_change_detect_sparse_thr(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
+                                long long x_sy, long long x_sx, void* state, long long s_sb,
+                                long long s_sc, long long s_sy, long long s_sx, int aux_mode,
+                                void* aux_hi, void* aux_lo, const int32_t* candidates, const int32_t* n_candidates,
+                                uint32_t* raw_bits, int B, int C, int H, int W, float threshold,
+                                int update_mode, int bits_are_clear, const float* thr_b) {
+  CB_CHECK_ARG(x && state && raw_bits && candidates && n_candidates, "change_detect_sparse: null pointer");
+  CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect_sparse: bad shape");
+  CB_CHECK_THR(thr_b, "change_detect_sparse");
+  CB_DISPATCH_DTYPE(dtype, return (launch_detect_sparse<T, VEC>(
+                               (cudaStream_t)stream, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc,
+                               s_sy, s_sx, aux_mode, aux_hi, aux_lo, candidates, n_candidates, raw_bits,
+                               B, C, H, W,
+                               threshold, update_mode, bits_are_clear, nullptr, thr_b)));
+  return 0;
+}
+
 int cb_change_detect_sparse(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
                             long long x_sy, long long x_sx, void* state, long long s_sb,
                             long long s_sc, long long s_sy, long long s_sx, int aux_mode,
                             void* aux_hi, void* aux_lo, const int32_t* candidates, const int32_t* n_candidates,
                             uint32_t* raw_bits, int B, int C, int H, int W, float threshold,
                             int update_mode, int bits_are_clear) {
-  CB_CHECK_ARG(x && state && raw_bits && candidates && n_candidates, "change_detect_sparse: null pointer");
-  CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect_sparse: bad shape");
-  CB_DISPATCH_DTYPE(dtype, return (launch_detect_sparse<T, VEC>(
-                               (cudaStream_t)stream, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc,
-                               s_sy, s_sx, aux_mode, aux_hi, aux_lo, candidates, n_candidates, raw_bits,
-                               B, C, H, W,
-                               threshold, update_mode, bits_are_clear)));
-  return 0;
+  return cb_change_detect_sparse_thr(stream, dtype, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy, s_sx,
+                                     aux_mode, aux_hi, aux_lo, candidates, n_candidates, raw_bits, B, C, H, W,
+                                     threshold, update_mode, bits_are_clear, nullptr);
 }
 
 int cb_compact_small_max_words(void) { return cb::kCompactWin; }
 
-int cb_change_detect_sparse_compact_streams(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
-                                            long long x_sy, long long x_sx, void* state, long long s_sb,
-                                            long long s_sc, long long s_sy, long long s_sx, int aux_mode,
-                                            void* aux_hi, void* aux_lo, const int32_t* candidates,
-                                            const int32_t* n_candidates, uint32_t* raw_bits, int B, int C, int H,
-                                            int W, float threshold, int update_mode, int bits_are_clear,
-                                            uint32_t* dil_bits, int32_t* idx, int32_t* count, void* sync_ws,
-                                            int kHHalf, int kWHalf, int clear_raw, int32_t* stream_counts,
-                                            int32_t* stream_acc) {
+int cb_change_detect_sparse_compact_thr(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
+                                        long long x_sy, long long x_sx, void* state, long long s_sb,
+                                        long long s_sc, long long s_sy, long long s_sx, int aux_mode,
+                                        void* aux_hi, void* aux_lo, const int32_t* candidates,
+                                        const int32_t* n_candidates, uint32_t* raw_bits, int B, int C, int H,
+                                        int W, float threshold, int update_mode, int bits_are_clear,
+                                        uint32_t* dil_bits, int32_t* idx, int32_t* count, void* sync_ws,
+                                        int kHHalf, int kWHalf, int clear_raw, int32_t* stream_counts,
+                                        int32_t* stream_acc, const float* thr_b) {
   CB_CHECK_ARG(x && state && raw_bits && candidates && n_candidates && idx && count && sync_ws,
                "change_detect_sparse_compact: null pointer");
   CB_CHECK_STREAMS(stream_counts, stream_acc, "change_detect_sparse_compact");
+  CB_CHECK_THR(thr_b, "change_detect_sparse_compact");
   CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect_sparse_compact: bad shape");
   CB_CHECK_ARG(kHHalf >= 0 && kWHalf >= 0 && kWHalf <= 31, "change_detect_sparse_compact: kWHalf must be <= 31");
   CB_CHECK_ARG(raw_bits != dil_bits, "change_detect_sparse_compact: dil_bits must not alias raw_bits");
@@ -303,8 +341,24 @@ int cb_change_detect_sparse_compact_streams(void* stream, int dtype, const void*
   CB_DISPATCH_DTYPE(dtype, return (launch_detect_sparse<T, VEC>(
                                (cudaStream_t)stream, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc,
                                s_sy, s_sx, aux_mode, aux_hi, aux_lo, candidates, n_candidates, raw_bits,
-                               B, C, H, W, threshold, update_mode, bits_are_clear, &fc)));
+                               B, C, H, W, threshold, update_mode, bits_are_clear, &fc, thr_b)));
   return 0;
+}
+
+int cb_change_detect_sparse_compact_streams(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
+                                            long long x_sy, long long x_sx, void* state, long long s_sb,
+                                            long long s_sc, long long s_sy, long long s_sx, int aux_mode,
+                                            void* aux_hi, void* aux_lo, const int32_t* candidates,
+                                            const int32_t* n_candidates, uint32_t* raw_bits, int B, int C, int H,
+                                            int W, float threshold, int update_mode, int bits_are_clear,
+                                            uint32_t* dil_bits, int32_t* idx, int32_t* count, void* sync_ws,
+                                            int kHHalf, int kWHalf, int clear_raw, int32_t* stream_counts,
+                                            int32_t* stream_acc) {
+  return cb_change_detect_sparse_compact_thr(stream, dtype, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy,
+                                             s_sx, aux_mode, aux_hi, aux_lo, candidates, n_candidates, raw_bits,
+                                             B, C, H, W, threshold, update_mode, bits_are_clear, dil_bits, idx,
+                                             count, sync_ws, kHHalf, kWHalf, clear_raw, stream_counts, stream_acc,
+                                             nullptr);
 }
 
 int cb_change_detect_sparse_compact(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
@@ -431,7 +485,8 @@ int cb_conv_tiled_supported(int dtype, int gemm, int B, int H, int W, int Cin, i
 static int conv_update_tiled_impl(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
                          int pitch_in, const void* tile_ws, const uint32_t* dil_bits,
                          const void* packed_w, const float* bias, void* out, int pitch_out, int B,
-                         int H, int W, int Cin, int Cout, int kH, int kW, int relu, const cb::PoolFuse& pf) {
+                         int H, int W, int Cin, int Cout, int kH, int kW, int relu, const cb::PoolFuse& pf,
+                         const float* thr_b) {
   CB_CHECK_ARG(state && tile_ws && dil_bits && packed_w && bias && out, "conv_update_tiled: null pointer");
   CB_CHECK_ARG(gemm != CB_GEMM_SIMT_F32, "conv_update_tiled: tensor-core modes only");
   const int want_pitch = gemm == CB_GEMM_TC_BF16X3 ? cb::pitch16_of(Cin) : cb_channel_pitch(dtype, Cin);
@@ -442,7 +497,7 @@ static int conv_update_tiled_impl(void* stream, int dtype, int gemm, const void*
   if (B == 0 || H == 0 || W == 0) return 0;
   return cb::umma_conv_update_tiled((cudaStream_t)stream, dtype, gemm, state, state_lo, pitch_in,
                                     (const int32_t*)tile_ws, dil_bits, packed_w, bias, out, pitch_out,
-                                    B, H, W, Cout, kH, kW, relu, pf);
+                                    B, H, W, Cout, kH, kW, relu, pf, thr_b);
 }
 
 int cb_conv_update_tiled(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
@@ -452,7 +507,7 @@ int cb_conv_update_tiled(void* stream, int dtype, int gemm, const void* state, c
   cb::PoolFuse pf;
   memset(&pf, 0, sizeof(pf));
   return conv_update_tiled_impl(stream, dtype, gemm, state, state_lo, pitch_in, tile_ws, dil_bits, packed_w,
-                                bias, out, pitch_out, B, H, W, Cin, Cout, kH, kW, relu, pf);
+                                bias, out, pitch_out, B, H, W, Cin, Cout, kH, kW, relu, pf, nullptr);
 }
 
 #ifdef CB_TILE_TRACE
@@ -479,8 +534,9 @@ static int tiled_pool_impl(void* stream, int dtype, int gemm, const void* state,
                               void* pool_out, long long o_sb, long long o_sy, int o_pitch, int oH, int oW,
                               void* next_state, long long n_sb, long long n_sy, int n_pitch, int aux_mode,
                               void* aux_hi, void* aux_lo, uint32_t* next_raw_bits, float threshold,
-                              int update_mode) {
+                              int update_mode, const float* thr_b) {
   CB_CHECK_ARG(pool_out && next_state && next_raw_bits, "conv_update_tiled_pool: null pointer");
+  CB_CHECK_THR(thr_b, "conv_update_tiled_pool");
   CB_CHECK_ARG(update_mode == CB_UPDATE_NONE || update_mode == CB_UPDATE_CHANGED || update_mode == CB_UPDATE_ALL,
                "conv_update_tiled_pool: bad update_mode %d", update_mode);
   const size_t es = cb::esize(dtype);
@@ -499,7 +555,21 @@ static int tiled_pool_impl(void* stream, int dtype, int gemm, const void* state,
   CB_DISPATCH_DTYPE(dtype, rc = cb::make_aux<T>(pf.aux, aux_mode, aux_hi, aux_lo, next_state, Cout));
   if (rc) return rc;
   return conv_update_tiled_impl(stream, dtype, gemm, state, state_lo, pitch_in, tile_ws, dil_bits, packed_w,
-                                bias, out, pitch_out, B, H, W, Cin, Cout, kH, kW, relu, pf);
+                                bias, out, pitch_out, B, H, W, Cin, Cout, kH, kW, relu, pf, thr_b);
+}
+
+int cb_conv_update_tiled_pool_thr(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
+                                  int pitch_in, const void* tile_ws, const uint32_t* dil_bits,
+                                  const void* packed_w, const float* bias, void* out, int pitch_out, int B,
+                                  int H, int W, int Cin, int Cout, int kH, int kW, int relu,
+                                  void* pool_out, long long o_sb, long long o_sy, int o_pitch, int oH, int oW,
+                                  void* next_state, long long n_sb, long long n_sy, int n_pitch, int aux_mode,
+                                  void* aux_hi, void* aux_lo, uint32_t* next_raw_bits, float threshold,
+                                  int update_mode, const float* thr_b) {
+  return tiled_pool_impl(stream, dtype, gemm, state, state_lo, pitch_in, tile_ws, dil_bits, packed_w, bias, out,
+                         pitch_out, B, H, W, Cin, Cout, kH, kW, relu, pool_out, o_sb, o_sy, o_pitch, oH, oW,
+                         next_state, n_sb, n_sy, n_pitch, aux_mode, aux_hi, aux_lo, next_raw_bits, threshold,
+                         update_mode, thr_b);
 }
 
 int cb_conv_update_tiled_pool(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
@@ -513,7 +583,7 @@ int cb_conv_update_tiled_pool(void* stream, int dtype, int gemm, const void* sta
   return tiled_pool_impl(stream, dtype, gemm, state, state_lo, pitch_in, tile_ws, dil_bits, packed_w, bias, out,
                          pitch_out, B, H, W, Cin, Cout, kH, kW, relu, pool_out, o_sb, o_sy, o_pitch, oH, oW,
                          next_state, n_sb, n_sy, n_pitch, aux_mode, aux_hi, aux_lo, next_raw_bits, threshold,
-                         update_mode);
+                         update_mode, nullptr);
 }
 
 int cb_conv_update_masked_streams(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
@@ -554,19 +624,22 @@ int cb_tail_supported(int dtype, int gemm, int C0, int C1, int C2) {
   return dtype == CB_F32 && gemm == CB_GEMM_TC_BF16X3 && cb::tail_supported(C0, C1, C2) ? 1 : 0;
 }
 
-int cb_tail_update_streams(void* stream, const float* x, float* state1, const void* packed_w1, const float* bias1,
-                           float* out1, int relu1, float thr1, float* state2, const void* packed_w2,
-                           const float* bias2, float* out2, int pitch_out2, int relu2, float thr2,
-                           const int32_t* candidates, const int32_t* n_candidates, int C0, int C1, int C2,
-                           int update_mode, int32_t* count1, int32_t* count2, void* sync_ws, int B, int hw,
-                           int32_t* stream_counts1, int32_t* stream_acc1, int32_t* stream_counts2,
-                           int32_t* stream_acc2) {
+int cb_tail_update_thr(void* stream, const float* x, float* state1, const void* packed_w1, const float* bias1,
+                       float* out1, int relu1, float thr1, float* state2, const void* packed_w2,
+                       const float* bias2, float* out2, int pitch_out2, int relu2, float thr2,
+                       const int32_t* candidates, const int32_t* n_candidates, int C0, int C1, int C2,
+                       int update_mode, int32_t* count1, int32_t* count2, void* sync_ws, int B, int hw,
+                       int32_t* stream_counts1, int32_t* stream_acc1, int32_t* stream_counts2,
+                       int32_t* stream_acc2, const float* thr1_b, const float* thr2_b) {
   CB_CHECK_ARG(x && state1 && packed_w1 && bias1 && out1 && state2 && packed_w2 && bias2 && out2 && candidates &&
                    n_candidates && count1 && count2 && sync_ws, "tail_update: null pointer");
   CB_CHECK_STREAMS(stream_counts1, stream_acc1, "tail_update");
   CB_CHECK_STREAMS(stream_counts2, stream_acc2, "tail_update");
   CB_CHECK_ARG(!stream_counts1 == !stream_counts2, "tail_update: per-stream counts for both layers or neither");
-  CB_CHECK_ARG(!stream_counts1 || (B > 0 && hw > 0), "tail_update: bad shape B = %d, H*W = %d", B, hw);
+  CB_CHECK_ARG(!(stream_counts1 || thr1_b || thr2_b) || (B > 0 && hw > 0), "tail_update: bad shape B = %d, H*W = %d",
+               B, hw);
+  CB_CHECK_THR(thr1_b, "tail_update");
+  CB_CHECK_THR(thr2_b, "tail_update");
   CB_CHECK_ARG(update_mode == CB_UPDATE_NONE || update_mode == CB_UPDATE_CHANGED || update_mode == CB_UPDATE_ALL,
                "tail_update: bad update_mode %d", update_mode);
   CB_CHECK_ARG(((uintptr_t)x % 16) == 0 && ((uintptr_t)state1 % 16) == 0 && ((uintptr_t)out1 % 16) == 0 &&
@@ -581,7 +654,20 @@ int cb_tail_update_streams(void* stream, const float* x, float* state1, const vo
   a.relu1 = relu1; a.relu2 = relu2; a.update = update_mode; a.thr1 = thr1; a.thr2 = thr2;
   a.sc1 = stream_counts1; a.sc2 = stream_counts2; a.acc1 = stream_acc1; a.acc2 = stream_acc2;
   a.hw = hw; a.B = B;
-  return cb::tail_update((cudaStream_t)stream, a, packed_w1, packed_w2);
+  return cb::tail_update((cudaStream_t)stream, a, packed_w1, packed_w2, thr1_b, thr2_b);
+}
+
+int cb_tail_update_streams(void* stream, const float* x, float* state1, const void* packed_w1, const float* bias1,
+                           float* out1, int relu1, float thr1, float* state2, const void* packed_w2,
+                           const float* bias2, float* out2, int pitch_out2, int relu2, float thr2,
+                           const int32_t* candidates, const int32_t* n_candidates, int C0, int C1, int C2,
+                           int update_mode, int32_t* count1, int32_t* count2, void* sync_ws, int B, int hw,
+                           int32_t* stream_counts1, int32_t* stream_acc1, int32_t* stream_counts2,
+                           int32_t* stream_acc2) {
+  return cb_tail_update_thr(stream, x, state1, packed_w1, bias1, out1, relu1, thr1, state2, packed_w2, bias2, out2,
+                            pitch_out2, relu2, thr2, candidates, n_candidates, C0, C1, C2, update_mode, count1,
+                            count2, sync_ws, B, hw, stream_counts1, stream_acc1, stream_counts2, stream_acc2,
+                            nullptr, nullptr);
 }
 
 int cb_tail_update(void* stream, const float* x, float* state1, const void* packed_w1, const float* bias1,
@@ -615,7 +701,7 @@ int cb_maxpool2x2(void* stream, int dtype, const void* x, long long x_sb, long l
     CB_DISPATCH_DTYPE(dtype, (cb::launch(maxpool2x2_detect_kernel<T, VEC, CB_UPDATE_NONE, false>, grid, 256, 0,
                                          (cudaStream_t)stream, (const T*)x, x_sb, x_sy, (int)x_sx, idx, count,
                                          dil_bits, (T*)out, o_sb, o_sy, (int)o_sx, cpp, cb::group_log2(cpp), H, W,
-                                         oH, oW, nullptr, 0ll, 0ll, 0, AuxPlanes{}, nullptr, T{})));
+                                         oH, oW, nullptr, 0ll, 0ll, 0, AuxPlanes{}, nullptr, T{}, nullptr)));
   } else {
     CB_DISPATCH_DTYPE(dtype, (cb::launch(maxpool2x2_kernel<T>, grid, 256, 0, (cudaStream_t)stream, 
                                  (const T*)x, x_sb, x_sc, x_sy, x_sx, idx, count, dil_bits, (T*)out,
@@ -625,14 +711,16 @@ int cb_maxpool2x2(void* stream, int dtype, const void* x, long long x_sb, long l
   return 0;
 }
 
-int cb_maxpool2x2_detect(void* stream, int dtype, const void* x, long long x_sb, long long x_sy,
-                         int x_pitch, const int32_t* idx, const int32_t* count,
-                         const uint32_t* dil_bits, void* out, long long o_sb, long long o_sy,
-                         int o_pitch, int B, int C, int H, int W, int oH, int oW, void* next_state,
-                         long long n_sb, long long n_sy, int n_pitch, int aux_mode, void* aux_hi,
-                         void* aux_lo, uint32_t* next_raw_bits, float threshold, int update_mode) {
+int cb_maxpool2x2_detect_thr(void* stream, int dtype, const void* x, long long x_sb, long long x_sy,
+                             int x_pitch, const int32_t* idx, const int32_t* count,
+                             const uint32_t* dil_bits, void* out, long long o_sb, long long o_sy,
+                             int o_pitch, int B, int C, int H, int W, int oH, int oW, void* next_state,
+                             long long n_sb, long long n_sy, int n_pitch, int aux_mode, void* aux_hi,
+                             void* aux_lo, uint32_t* next_raw_bits, float threshold, int update_mode,
+                             const float* thr_b) {
   CB_CHECK_ARG(x && idx && count && dil_bits && out && next_state && next_raw_bits,
                "maxpool2x2_detect: null pointer");
+  CB_CHECK_THR(thr_b, "maxpool2x2_detect");
   if (B == 0 || H == 0 || W == 0 || C == 0) return 0;
   const size_t es = cb::esize(dtype);
   const int vec = (int)(16 / es);
@@ -646,17 +734,28 @@ int cb_maxpool2x2_detect(void* stream, int dtype, const void* x, long long x_sb,
   const int glog = cb::group_log2(cpp);
   const unsigned grid = (unsigned)(sm_count() * 16);
   cudaStream_t s = (cudaStream_t)stream;
-  return dispatch_update(update_mode, "maxpool2x2_detect", [&](auto U) {
+  return dispatch_thr(thr_b, [&](auto R) { return dispatch_update(update_mode, "maxpool2x2_detect", [&](auto U) {
     CB_DISPATCH_DTYPE(dtype, {
       AuxPlanes aux;
       if (int rc = make_aux<T>(aux, aux_mode, aux_hi, aux_lo, next_state, C)) return rc;
-      cb::launch(maxpool2x2_detect_kernel<T, VEC, U>, grid, 256, 0, s, (const T*)x, x_sb, x_sy, x_pitch, idx,
+      cb::launch(maxpool2x2_detect_kernel<T, VEC, U, true, R>, grid, 256, 0, s, (const T*)x, x_sb, x_sy, x_pitch, idx,
                  count, dil_bits, (T*)out, o_sb, o_sy, o_pitch, cpp, glog, H, W, oH, oW, (T*)next_state, n_sb,
-                 n_sy, n_pitch, aux, next_raw_bits, thr_cast<T>(threshold));
+                 n_sy, n_pitch, aux, next_raw_bits, thr_cast<T>(threshold), thr_b);
     })
     CB_CHECK_LAUNCH("maxpool2x2_detect");
     return 0;
-  });
+  }); });
+}
+
+int cb_maxpool2x2_detect(void* stream, int dtype, const void* x, long long x_sb, long long x_sy,
+                         int x_pitch, const int32_t* idx, const int32_t* count,
+                         const uint32_t* dil_bits, void* out, long long o_sb, long long o_sy,
+                         int o_pitch, int B, int C, int H, int W, int oH, int oW, void* next_state,
+                         long long n_sb, long long n_sy, int n_pitch, int aux_mode, void* aux_hi,
+                         void* aux_lo, uint32_t* next_raw_bits, float threshold, int update_mode) {
+  return cb_maxpool2x2_detect_thr(stream, dtype, x, x_sb, x_sy, x_pitch, idx, count, dil_bits, out, o_sb, o_sy,
+                                  o_pitch, B, C, H, W, oH, oW, next_state, n_sb, n_sy, n_pitch, aux_mode, aux_hi,
+                                  aux_lo, next_raw_bits, threshold, update_mode, nullptr);
 }
 
 int cb_reset_streams(void* stream, const uint8_t* mask, int B, const cb_reset_segment* segments,

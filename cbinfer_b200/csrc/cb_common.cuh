@@ -51,6 +51,13 @@ inline int dispatch_update(int update, const char* what, F&& f) {
   }
 }
 
+// per-stream threshold table given?  A compile-time kernel variant (THR), so the kernels launched
+// without one compile exactly as they would without the feature
+template <typename F>
+inline int dispatch_thr(const void* thr_b, F&& f) {
+  return thr_b ? f(std::true_type{}) : f(std::false_type{});
+}
+
 // cooperative != 0: the grid is launched only when ALL its CTAs can be resident at once (kernels whose
 // CTAs wait for each other, e.g. the stream-K finisher spinning on its contributors' flags, must not
 // be half-resident next to another grid on a concurrent stream)

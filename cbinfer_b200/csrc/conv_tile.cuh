@@ -121,12 +121,12 @@ __device__ __forceinline__ uint64_t tile_adesc_base(uint32_t sbo_bytes, int layo
   return ((uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32) | (1ull << 46) | ((uint64_t)layout << 61);
 }
 
-template <typename T, typename TO, bool SPLIT3, int BN>
+template <typename T, typename TO, bool SPLIT3, int BN, bool THR = false>
 __global__ void __launch_bounds__(128 + um_epi(BN), BN <= 16 ? 4 : BN <= 64 ? 2 : 1)
 conv_tile_kernel(const __grid_constant__ CUtensorMap amap_hi, const __grid_constant__ CUtensorMap amap_lo,
                  const __grid_constant__ CUtensorMap wmap, int32_t* tile_ws,
                  const uint32_t* dil_bits, const float* __restrict__ bias,
-                 TO* __restrict__ out, const TileGeom g, const PoolFuse pf) {
+                 TO* __restrict__ out, const TileGeom g, const PoolFuse pf, const float* __restrict__ thr_b) {
 #ifdef CB_TILE_TRACE
   const long long trace_t0 = clock64();
   if (threadIdx.x == 0) {
@@ -401,6 +401,7 @@ conv_tile_kernel(const __grid_constant__ CUtensorMap amap_hi, const __grid_const
       TO* po = reinterpret_cast<TO*>(pf.out) + b * pf.o_sb + yo * pf.o_sy + (long long)xo * pf.op;
       TO* ns = reinterpret_cast<TO*>(pf.nst) + b * pf.n_sb + yo * pf.n_sy + (long long)xo * pf.np;
       const long long opix = ((long long)b * pf.oH + yo) * pf.oW + xo;
+      const TO tthr = stream_thr<THR>(thr_b, b, pthr);        // (THR: pooling) a tile lies in one image
       // What the pooling tail reads from global memory -- the stored values of a touched window's
       // untouched pixels, the next layer's state row of the window's owner -- has not been seen for a
       // frame: with the loads inside the column loop a tile's epilogue was a chain of 8 dependent
@@ -507,7 +508,7 @@ conv_tile_kernel(const __grid_constant__ CUtensorMap amap_hi, const __grid_const
                 const uint4 res = *reinterpret_cast<uint4*>(h);
                 st16(po + co0 + i, res);
                 const uint4 sv = EARLY ? nsv[i / OVEC] : ld16(ns + co0 + i);
-                pchg |= Chunk<TO>::changed(sv, res, pthr);
+                pchg |= Chunk<TO>::changed(sv, res, tthr);
                 if (pf.update == CB_UPDATE_ALL) store_state<TO>(ns + co0 + i, res, pf.aux, opix, co0 + i);
               }
             }
@@ -638,10 +639,10 @@ inline CUtensorMapDataType tmap_dtype() {
                                           : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
 }
 
-template <typename T, typename TO, bool SPLIT3, int BN>
+template <typename T, typename TO, bool SPLIT3, int BN, bool THR = false>
 int launch_conv_tile(cudaStream_t s, const void* state, const void* state_lo, const int32_t* tile_ws,
                      const uint32_t* dil_bits, const void* packed, const float* bias, void* out,
-                     const TilePlan& plan, const PoolFuse& pf) {
+                     const TilePlan& plan, const PoolFuse& pf, const float* thr_b) {
   const TileGeom& g = plan.g;
   auto enc = tensor_map_encoder();
   if (!enc) return fail(3, "conv_update_tiled: cuTensorMapEncodeTiled unavailable");
@@ -674,7 +675,7 @@ int launch_conv_tile(cudaStream_t s, const void* state, const void* state_lo, co
     if (r != CUDA_SUCCESS) return fail(3, "conv_update_tiled: state tensor map failed (%d)", (int)r);
   }
   if (!SPLIT3) amap[1] = amap[0];
-  auto kern = conv_tile_kernel<T, TO, SPLIT3, BN>;
+  auto kern = conv_tile_kernel<T, TO, SPLIT3, BN, THR>;
   static thread_local int attr_dev = -1;
   int dev = 0;
   cudaGetDevice(&dev);
@@ -690,7 +691,7 @@ int launch_conv_tile(cudaStream_t s, const void* state, const void* state_lo, co
   if (grid > max_items) grid = max_items;
   if (grid < 1) grid = 1;
   cb::launch(kern, dim3((unsigned)grid), dim3(128 + um_epi(BN)), (size_t)plan.smem_bytes, s, amap[0], amap[1],
-             wmap, const_cast<int32_t*>(tile_ws), dil_bits, bias, (TO*)out, g, pf);
+             wmap, const_cast<int32_t*>(tile_ws), dil_bits, bias, (TO*)out, g, pf, thr_b);
   CB_CHECK_LAUNCH("conv_update_tiled");
   return 0;
 }
@@ -715,7 +716,7 @@ inline int umma_conv_update_tiled(cudaStream_t s, int dtype, int gemm, const voi
                                   const void* state_lo, int Cp, const int32_t* tile_ws,
                                   const uint32_t* dil_bits, const void* packed, const float* bias,
                                   void* out, int Op, int B, int H, int W, int Cout, int kH, int kW,
-                                  int relu, const PoolFuse& pf) {
+                                  int relu, const PoolFuse& pf, const float* thr_b) {
   TilePlan plan;
   umma_tile_plan(plan, dtype, gemm, Cp, B, H, W, Cout, Op, kH, kW, relu);
   CB_CHECK_ARG(plan.ok, "conv_update_tiled: layer shape not supported by the tile path");
@@ -726,13 +727,18 @@ inline int umma_conv_update_tiled(cudaStream_t s, int dtype, int gemm, const voi
                "conv_update_tiled: state must be 16-byte and packed weights 128-byte aligned");
   const int bn = umma_bn(gemm, Cout);
   CB_CHECK_ARG(!pf.out || tile_pool_ok(gemm, Cout), "conv_update_tiled: fused pooling needs Cout <= 64, a multiple of 16");
+  // per-stream thresholds belong to the fused detection: only the pooling tiles (N <= 64) have the THR variant
+  CB_CHECK_ARG(!thr_b || (pf.out && bn <= 64), "conv_update_tiled: per-stream thresholds need the fused pooling");
+#define CB_TBN_THR(T_, TO_, S3_, N_)                                                               \
+  return thr_b ? launch_conv_tile<T_, TO_, S3_, N_, true>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf, thr_b) \
+               : launch_conv_tile<T_, TO_, S3_, N_>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf, nullptr);
 #define CB_TBN(T_, TO_, S3_)                                                                       \
   switch (bn) {                                                                                    \
-    case 16: return launch_conv_tile<T_, TO_, S3_, 16>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf);   \
-    case 32: return launch_conv_tile<T_, TO_, S3_, 32>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf);   \
-    case 64: return launch_conv_tile<T_, TO_, S3_, 64>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf);   \
-    case 128: return launch_conv_tile<T_, TO_, S3_, 128>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf); \
-    case 256: return launch_conv_tile<T_, TO_, S3_, 256>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf); \
+    case 16: CB_TBN_THR(T_, TO_, S3_, 16)                                                          \
+    case 32: CB_TBN_THR(T_, TO_, S3_, 32)                                                          \
+    case 64: CB_TBN_THR(T_, TO_, S3_, 64)                                                          \
+    case 128: return launch_conv_tile<T_, TO_, S3_, 128>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf, nullptr); \
+    case 256: return launch_conv_tile<T_, TO_, S3_, 256>(s, state, state_lo, tile_ws, dil_bits, packed, bias, out, plan, pf, nullptr); \
     default: return fail(2, "conv_update_tiled: unsupported N tile %d", bn);                      \
   }
   if (bf16x3) { CB_TBN(__nv_bfloat16, float, true) }
@@ -744,6 +750,7 @@ inline int umma_conv_update_tiled(cudaStream_t s, int dtype, int gemm, const voi
     default: return fail(2, "conv_update_tiled: bad dtype %d", dtype);
   }
 #undef CB_TBN
+#undef CB_TBN_THR
 }
 
 }  // namespace cb

@@ -16,11 +16,30 @@
 // kernels decide per bitmap word (a word never spans two images, rows are padded to whole words).
 // A word of a stream with active[b] == 0 is written as 0 and nothing of that stream's x, state or
 // operand planes is loaded or stored; every block barrier is still reached by all threads.
+//
+// Per-stream thresholds (`thr_b`, fp32 [B] on the device, may be null = the scalar `thr` for every
+// stream): every kernel that tests a threshold reads stream b's value once per decision unit (a
+// bitmap word, a candidate) and rounds it to T with thr_cast, as the host rounds the scalar.  The
+// table is a compile-time variant (THR): without it the kernels are the ones compiled before it existed.
 #pragma once
 #include "cb_common.cuh"
 #include "compact.cuh"
 
 namespace cb {
+
+template <typename T> __host__ __device__ inline T thr_cast(float t);
+template <> __host__ __device__ inline float thr_cast<float>(float t) { return t; }
+template <> __host__ __device__ inline __half thr_cast<__half>(float t) { return __float2half_rn(t); }
+template <> __host__ __device__ inline __nv_bfloat16 thr_cast<__nv_bfloat16>(float t) {
+  return __float2bfloat16_rn(t);
+}
+
+// stream b's threshold: thr_b[b] rounded to T (THR), or the scalar
+template <bool THR, typename T>
+__device__ __forceinline__ T stream_thr(const float* __restrict__ thr_b, int b, T thr) {
+  if constexpr (THR) return thr_cast<T>(__ldg(thr_b + b));
+  else return thr;
+}
 
 template <typename T, int VEC>
 __device__ __forceinline__ uint4 merge_tail(uint4 xv, const uint4& sv, int tail) {
@@ -138,12 +157,13 @@ __device__ __forceinline__ bool pixel_changed_scalar(const T* xp, long long x_sc
 // U chunk-iterations are batched: all 2*U 16-byte loads of a batch are issued before the first
 // ballot, so every lane keeps 2*U loads in flight (the ballots would otherwise serialise them).
 // wlog = log2(warps per word): a block of 8 warps covers 8 >> wlog words.
-template <typename T, int VEC, int UPDATE, int U>
+template <typename T, int VEC, int UPDATE, int U, bool THR = false>
 __global__ void __launch_bounds__(kDetWarps * 32)
 detect_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int xp,
                   T* __restrict__ st, long long s_sb, long long s_sy, int sp, AuxPlanes aux,
                   uint32_t* __restrict__ bits, int B, int H, int W, int C, int Wd, T thr,
-                  unsigned cpv_magic, int wlog, const uint8_t* __restrict__ active) {
+                  unsigned cpv_magic, int wlog, const uint8_t* __restrict__ active,
+                  const float* __restrict__ thr_b) {
   __shared__ unsigned s_word[kDetWarps];
   const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
   const int wpw = 1 << wlog;
@@ -176,6 +196,7 @@ detect_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int x
     sb = st + b * s_sb + y * s_sy + (long long)x0 * sp;
     nq = (active && !__ldg(active + b)) ? 0 : npx * cpv;   // skipped stream: no loads, word 0
     pixbase = ((long long)b * H + y) * W + x0;
+    const T tb = stream_thr<THR>(thr_b, b, thr);
 
     bool mychg = false;                      // flag of pixel `lane` (this warp's slice only)
     const int plo = lane * cpv, phi = plo + cpv;
@@ -202,7 +223,7 @@ detect_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int x
       for (int u = 0; u < U; ++u) {
         bool f = false;
         if (valid[u]) {
-          f = Chunk<T>::changed(sv[u], xv[u], thr);
+          f = Chunk<T>::changed(sv[u], xv[u], tb);
           if (UPDATE == CB_UPDATE_ALL) store_state<T>(sptr[u], xv[u], aux, pixbase + pxs[u], ccs[u] * VEC);
         }
         const unsigned bal = __ballot_sync(0xffffffffu, f);
@@ -246,12 +267,13 @@ detect_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int x
 // applied on the fly with IEEE division and addition, so the result is bit-identical to detecting on
 // the host-normalised fp32 frame, at a quarter of the host->device bytes.  Otherwise divisor and bias
 // are unused.
-template <typename T, int VEC, int UPDATE, typename S = T>
+template <typename T, int VEC, int UPDATE, typename S = T, bool THR = false>
 __global__ void __launch_bounds__(256)
 detect_narrow_kernel(const S* __restrict__ x, long long x_sb, long long x_sc, long long x_sy,
                      long long x_sx, T* __restrict__ st, long long s_sb, long long s_sy,
                      AuxPlanes aux, uint32_t* __restrict__ bits, int B, int H, int W, int C,
-                     int Wd, T thr, float divisor, float bias, const uint8_t* __restrict__ active) {
+                     int Wd, T thr, float divisor, float bias, const uint8_t* __restrict__ active,
+                     const float* __restrict__ thr_b) {
   constexpr bool kU8 = std::is_same<S, uint8_t>::value;
   const float* lut = nullptr;
   if constexpr (kU8) {
@@ -279,7 +301,7 @@ detect_narrow_kernel(const S* __restrict__ x, long long x_sb, long long x_sc, lo
       if constexpr (kU8) ne[c] = lut[__ldcs(xp + c * x_sc)];
       else ne[c] = ld_stream(xp + c * x_sc);
     }
-    f = Chunk<T>::changed(sv, nv, thr);
+    f = Chunk<T>::changed(sv, nv, stream_thr<THR>(thr_b, b, thr));
     if (UPDATE == CB_UPDATE_ALL || (UPDATE == CB_UPDATE_CHANGED && f))
       store_state<T>(sp, nv, aux, ((long long)b * H + y) * W + xx, 0);
   }
@@ -307,7 +329,8 @@ struct PlanarWord {
 __device__ __forceinline__ void planar_words_setup(PlanarWord* wi, unsigned* s_word, int word0, int nw,
                                                    long long nwords, int H, int W, int Wd, long long x_sb,
                                                    long long x_sy, long long x_sx, long long s_sb,
-                                                   long long s_sy, int sp, const uint8_t* active = nullptr) {
+                                                   long long s_sy, int sp, const uint8_t* active = nullptr,
+                                                   const float* thr_b = nullptr, float* s_thr = nullptr) {
   if (threadIdx.x < (unsigned)nw) {
     const long long word = (long long)word0 + threadIdx.x;
     PlanarWord w = {0, 0, 0, 0};
@@ -323,6 +346,7 @@ __device__ __forceinline__ void planar_words_setup(PlanarWord* wi, unsigned* s_w
       w.xoff = b * x_sb + y * x_sy + x0 * x_sx;
       w.soff = b * s_sb + y * s_sy + (long long)x0 * sp;
       w.pix = (b * H + y) * W + x0;
+      if (thr_b) s_thr[threadIdx.x] = __ldg(thr_b + b);   // a block's words may lie in two streams
     }
     wi[threadIdx.x] = w;
     s_word[threadIdx.x] = 0u;
@@ -365,19 +389,22 @@ __device__ __forceinline__ void planar_flag(unsigned* s_word, int w, unsigned m)
   }
 }
 
-template <typename T, int VEC, int UPDATE>
+template <typename T, int VEC, int UPDATE, bool THR = false>
 __global__ void __launch_bounds__(256)
 detect_planar_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, long long x_sy,
                      T* __restrict__ st, long long s_sb, long long s_sy, int sp, AuxPlanes aux,
                      uint32_t* __restrict__ bits, int B, int H, int W, int C, int Wd, T thr,
-                     unsigned cpv_magic, int cps, int nw, const uint8_t* __restrict__ active) {
+                     unsigned cpv_magic, int cps, int nw, const uint8_t* __restrict__ active,
+                     const float* __restrict__ thr_b) {
   extern __shared__ __align__(16) unsigned char dp_smem[];
   uint4* xs = reinterpret_cast<uint4*>(dp_smem);                 // [nw*32][cps]
   __shared__ unsigned s_word[kPlanarMaxWords];
   __shared__ PlanarWord wi[kPlanarMaxWords];
+  __shared__ float s_thr[kPlanarMaxWords];                       // thr_b: each word's stream threshold
   const long long nwords = (long long)B * H * Wd;
   const int word0 = blockIdx.x * nw;
-  planar_words_setup(wi, s_word, word0, nw, nwords, H, W, Wd, x_sb, x_sy, 1, s_sb, s_sy, sp, active);
+  planar_words_setup(wi, s_word, word0, nw, nwords, H, W, Wd, x_sb, x_sy, 1, s_sb, s_sy, sp, active,
+                     THR ? thr_b : nullptr, s_thr);
   const int cpv = (C + VEC - 1) / VEC, tail = C % VEC;
   planar_load_tile<T, VEC>(xs, wi, x, x_sc, 1, nw, cpv, cps, C, cpv_magic);
   __syncthreads();
@@ -393,7 +420,7 @@ detect_planar_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, lo
       T* sptr = st + wi[w].soff + (long long)px * sp + cc * VEC;
       const uint4 sv = ld16(sptr);
       if (tail && cc == cpv - 1) xv = merge_tail<T, VEC>(xv, sv, tail);
-      if (Chunk<T>::changed(sv, xv, thr)) m = 1u << px;
+      if (Chunk<T>::changed(sv, xv, THR ? thr_cast<T>(s_thr[w]) : thr)) m = 1u << px;
       if (UPDATE == CB_UPDATE_ALL) store_state<T>(sptr, xv, aux, wi[w].pix + px, cc * VEC);
     }
     planar_flag(s_word, w, m);
@@ -423,29 +450,24 @@ inline int planar_words_per_block(int cpv, int cps) {
   return nw;
 }
 
-template <typename T, int UPDATE>
+template <typename T, int UPDATE, bool THR = false>
 __global__ void __launch_bounds__(256)
 detect_generic_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, long long x_sy,
                       long long x_sx, T* __restrict__ st, long long s_sb, long long s_sc,
                       long long s_sy, long long s_sx, AuxPlanes aux,
                       uint32_t* __restrict__ bits, int B, int H, int W, int C, int Wd, T thr,
-                      const uint8_t* __restrict__ active) {
+                      const uint8_t* __restrict__ active, const float* __restrict__ thr_b) {
   unsigned warp;
   int b, y, xx;
   if (!warp_word(warp, b, y, xx, B, H, Wd)) return;
   const bool f = xx < W && (!active || __ldg(active + b)) && pixel_changed_scalar<T, UPDATE>(x + b * x_sb + y * x_sy + xx * x_sx, x_sc,
                                                             st + b * s_sb + y * s_sy + xx * s_sx, s_sc, C,
-                                                            thr, aux, ((long long)b * H + y) * W + xx);
+                                                            stream_thr<THR>(thr_b, b, thr), aux,
+                                                            ((long long)b * H + y) * W + xx);
   const unsigned word = __ballot_sync(0xffffffffu, f);
   if ((threadIdx.x & 31) == 0) bits[warp] = word;
 }
 
-template <typename T> __host__ __device__ inline T thr_cast(float t);
-template <> __host__ __device__ inline float thr_cast<float>(float t) { return t; }
-template <> __host__ __device__ inline __half thr_cast<__half>(float t) { return __float2half_rn(t); }
-template <> __host__ __device__ inline __nv_bfloat16 thr_cast<__nv_bfloat16>(float t) {
-  return __float2bfloat16_rn(t);
-}
 
 
 template <typename T>
@@ -488,7 +510,7 @@ int launch_detect(cudaStream_t stream, const void* x, long long x_sb, long long 
                   long long x_sy, long long x_sx, void* state, long long s_sb, long long s_sc,
                   long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
                   uint32_t* bits, int B, int C, int H, int W, float threshold, int update,
-                  const uint8_t* active) {
+                  const uint8_t* active, const float* thr_b) {
   const int Wd = (W + 31) / 32;
   const long long words = (long long)B * H * Wd;
   if (words == 0) return 0;
@@ -516,31 +538,31 @@ int launch_detect(cudaStream_t stream, const void* x, long long x_sb, long long 
   const long long blocks = vec_ok ? vec_blocks : (words + 7) / 8;
   CB_CHECK_ARG(blocks < (1ll << 31) && words < (1ll << 31), "change_detect: image too large");
   dim3 grid((unsigned)blocks), block(256);
-  return dispatch_update(update, "change_detect", [&](auto U) {
+  return dispatch_thr(thr_b, [&](auto R) { return dispatch_update(update, "change_detect", [&](auto U) {
     if (vec_ok) {
       if (cpv >= 4)
-        cb::launch(detect_vec_kernel<T, VEC, U, 4>, grid, block, 0, stream, (const T*)x, x_sb, x_sy, (int)x_sx,
-                   (T*)state, s_sb, s_sy, (int)s_sx, aux, bits, B, H, W, C, Wd, thr, magic, wlog, active);
+        cb::launch(detect_vec_kernel<T, VEC, U, 4, R>, grid, block, 0, stream, (const T*)x, x_sb, x_sy, (int)x_sx,
+                   (T*)state, s_sb, s_sy, (int)s_sx, aux, bits, B, H, W, C, Wd, thr, magic, wlog, active, thr_b);
       else
-        cb::launch(detect_vec_kernel<T, VEC, U, 2>, grid, block, 0, stream, (const T*)x, x_sb, x_sy, (int)x_sx,
-                   (T*)state, s_sb, s_sy, (int)s_sx, aux, bits, B, H, W, C, Wd, thr, magic, wlog, active);
+        cb::launch(detect_vec_kernel<T, VEC, U, 2, R>, grid, block, 0, stream, (const T*)x, x_sb, x_sy, (int)x_sx,
+                   (T*)state, s_sb, s_sy, (int)s_sx, aux, bits, B, H, W, C, Wd, thr, magic, wlog, active, thr_b);
     } else if (narrow_ok) {
-      cb::launch(detect_narrow_kernel<T, VEC, U>, grid, block, 0, stream, (const T*)x, x_sb, x_sc, x_sy, x_sx,
-                 (T*)state, s_sb, s_sy, aux, bits, B, H, W, C, Wd, thr, 0.f, 0.f, active);
+      cb::launch(detect_narrow_kernel<T, VEC, U, T, R>, grid, block, 0, stream, (const T*)x, x_sb, x_sc, x_sy, x_sx,
+                 (T*)state, s_sb, s_sy, aux, bits, B, H, W, C, Wd, thr, 0.f, 0.f, active, thr_b);
     } else if (planar_ok) {
       if (planar_smem > 48 * 1024)
-        cudaFuncSetAttribute(detect_planar_kernel<T, VEC, U>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+        cudaFuncSetAttribute(detect_planar_kernel<T, VEC, U, R>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                              (int)planar_smem);
-      cb::launch(detect_planar_kernel<T, VEC, U>, dim3((unsigned)((words + planar_nw - 1) / planar_nw)), block,
+      cb::launch(detect_planar_kernel<T, VEC, U, R>, dim3((unsigned)((words + planar_nw - 1) / planar_nw)), block,
                  planar_smem, stream, (const T*)x, x_sb, x_sc, x_sy, (T*)state, s_sb, s_sy, (int)s_sx, aux, bits,
-                 B, H, W, C, Wd, thr, magic, cps, planar_nw, active);
+                 B, H, W, C, Wd, thr, magic, cps, planar_nw, active, thr_b);
     } else {
-      cb::launch(detect_generic_kernel<T, U>, grid, block, 0, stream, (const T*)x, x_sb, x_sc, x_sy, x_sx,
-                 (T*)state, s_sb, s_sc, s_sy, s_sx, aux, bits, B, H, W, C, Wd, thr, active);
+      cb::launch(detect_generic_kernel<T, U, R>, grid, block, 0, stream, (const T*)x, x_sb, x_sc, x_sy, x_sx,
+                 (T*)state, s_sb, s_sc, s_sy, s_sx, aux, bits, B, H, W, C, Wd, thr, active, thr_b);
     }
     CB_CHECK_LAUNCH("change_detect");
     return 0;
-  });
+  }); });
 }
 
 
@@ -549,7 +571,7 @@ inline int launch_detect_u8(cudaStream_t stream, const void* x, long long x_sb, 
                             long long s_sc, long long s_sy, long long s_sx, int aux_mode,
                             void* aux_hi, void* aux_lo, uint32_t* bits, int B, int C, int H, int W,
                             float divisor, float bias, float threshold, int update,
-                            const uint8_t* active) {
+                            const uint8_t* active, const float* thr_b) {
   const int Wd = (W + 31) / 32;
   const long long words = (long long)B * H * Wd;
   if (words == 0) return 0;
@@ -561,13 +583,13 @@ inline int launch_detect_u8(cudaStream_t stream, const void* x, long long x_sb, 
   if (int rc = make_aux<float>(aux, aux_mode, aux_hi, aux_lo, state, C)) return rc;
   const long long blocks = (words + 7) / 8;
   CB_CHECK_ARG(blocks < (1ll << 31), "change_detect_u8: image too large");
-  return dispatch_update(update, "change_detect_u8", [&](auto U) {
-    cb::launch(detect_narrow_kernel<float, 4, U, uint8_t>, dim3((unsigned)blocks), dim3(256), 0, stream,
+  return dispatch_thr(thr_b, [&](auto R) { return dispatch_update(update, "change_detect_u8", [&](auto U) {
+    cb::launch(detect_narrow_kernel<float, 4, U, uint8_t, R>, dim3((unsigned)blocks), dim3(256), 0, stream,
                (const uint8_t*)x, x_sb, x_sc, x_sy, x_sx, (float*)state, s_sb, s_sy, aux, bits, B, H, W, C, Wd,
-               threshold, divisor, bias, active);
+               threshold, divisor, bias, active, thr_b);
     CB_CHECK_LAUNCH("change_detect_u8");
     return 0;
-  });
+  }); });
 }
 
 
@@ -592,13 +614,14 @@ struct FusedCompact {
   int B;
 };
 
-template <typename T, int VEC, int UPDATE, bool FUSE = false, bool TRACK = false>
+template <typename T, int VEC, int UPDATE, bool FUSE = false, bool TRACK = false, bool THR = false>
 __global__ void __launch_bounds__(256)
 detect_sparse_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int xp,
                          T* __restrict__ st, long long s_sb, long long s_sy, int sp,
                          AuxPlanes aux, const int32_t* __restrict__ cand,
                          const int32_t* __restrict__ ncand, uint32_t* __restrict__ bits, int H,
-                         int W, int C, int Wd, T thr, int glog, FusedCompact fc) {
+                         int W, int C, int Wd, T thr, int glog, FusedCompact fc,
+                         const float* __restrict__ thr_b) {
   const int n = *ncand;
   const int lane = threadIdx.x & 31;
   const int G = 1 << glog, ppw = 32 >> glog;
@@ -612,6 +635,7 @@ detect_sparse_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy
     const long long j = j0 + sub;
     const bool have = j < n;
     int b = 0, y = 0, xx = 0, gpix = 0;
+    T tb = thr;
     if (have) {
       const int pix = __ldg(cand + j);
       gpix = pix;
@@ -619,6 +643,7 @@ detect_sparse_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy
       const int p = pix - b * P;
       y = p / W;
       xx = p - y * W;
+      tb = stream_thr<THR>(thr_b, b, thr);
     }
     const T* xb = x + b * x_sb + y * x_sy + (long long)xx * xp;
     T* sb = st + b * s_sb + y * s_sy + (long long)xx * sp;
@@ -628,7 +653,7 @@ detect_sparse_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy
         uint4 xv = ldg16(xb + cc * VEC);
         const uint4 sv = ld16(sb + cc * VEC);
         if (tail && cc == cpv - 1) xv = merge_tail<T, VEC>(xv, sv, tail);
-        f |= Chunk<T>::changed(sv, xv, thr);
+        f |= Chunk<T>::changed(sv, xv, tb);
         if (UPDATE == CB_UPDATE_ALL) store_state<T>(sb + cc * VEC, xv, aux, gpix, cc * VEC);
       }
     }
@@ -662,13 +687,14 @@ detect_sparse_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy
   }
 }
 
-template <typename T, int UPDATE>
+template <typename T, int UPDATE, bool THR = false>
 __global__ void __launch_bounds__(256)
 detect_sparse_generic_kernel(const T* __restrict__ x, long long x_sb, long long x_sc,
                              long long x_sy, long long x_sx, T* __restrict__ st, long long s_sb,
                              long long s_sc, long long s_sy, long long s_sx, AuxPlanes aux,
                              const int32_t* __restrict__ cand, const int32_t* __restrict__ ncand,
-                             uint32_t* __restrict__ bits, int H, int W, int C, int Wd, T thr) {
+                             uint32_t* __restrict__ bits, int H, int W, int C, int Wd, T thr,
+                             const float* __restrict__ thr_b) {
   const int n = *ncand;
   const int P = H * W;
   for (long long j = (long long)blockIdx.x * blockDim.x + threadIdx.x; j < n;
@@ -678,7 +704,7 @@ detect_sparse_generic_kernel(const T* __restrict__ x, long long x_sb, long long 
     const int y = p / W, xx = p - y * W;
     const T* xp = x + b * x_sb + y * x_sy + xx * x_sx;
     T* sp = st + b * s_sb + y * s_sy + xx * s_sx;
-    if (pixel_changed_scalar<T, UPDATE>(xp, x_sc, sp, s_sc, C, thr, aux, (long long)pix))
+    if (pixel_changed_scalar<T, UPDATE>(xp, x_sc, sp, s_sc, C, stream_thr<THR>(thr_b, b, thr), aux, (long long)pix))
       atomicOr(bits + ((long long)b * H + y) * Wd + (xx >> 5), 1u << (xx & 31));
   }
 }
@@ -689,7 +715,7 @@ int launch_detect_sparse(cudaStream_t stream, const void* x, long long x_sb, lon
                          long long s_sc, long long s_sy, long long s_sx, int aux_mode,
                          void* aux_hi, void* aux_lo, const int32_t* cand, const int32_t* ncand, uint32_t* bits, int B, int C,
                          int H, int W, float threshold, int update, int bits_are_clear,
-                         const FusedCompact* fuse = nullptr) {
+                         const FusedCompact* fuse, const float* thr_b) {
   const int Wd = (W + 31) / 32;
   const long long words = (long long)B * H * Wd;
   if (words == 0) return 0;
@@ -711,22 +737,22 @@ int launch_detect_sparse(cudaStream_t stream, const void* x, long long x_sb, lon
   CB_CHECK_ARG(!fuse || (vec_ok && words <= kCompactWin), "change_detect_sparse_compact: needs pixel-major "
                "tensors and a bitmap of at most %d words", kCompactWin);
   FusedCompact fc = fuse ? *fuse : FusedCompact{nullptr, nullptr, nullptr, nullptr, 0, 0, 0, 0, nullptr, nullptr, 0};
-  return dispatch_update(update, "change_detect_sparse", [&](auto U) {
+  return dispatch_thr(thr_b, [&](auto R) { return dispatch_update(update, "change_detect_sparse", [&](auto U) {
     if (vec_ok && fuse && fc.stream_counts)
-      cb::launch(detect_sparse_vec_kernel<T, VEC, U, true, true>, grid, 256, 0, stream, (const T*)x, x_sb, x_sy,
-                 (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand, ncand, bits, H, W, C, Wd, thr, glog, fc);
+      cb::launch(detect_sparse_vec_kernel<T, VEC, U, true, true, R>, grid, 256, 0, stream, (const T*)x, x_sb, x_sy,
+                 (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand, ncand, bits, H, W, C, Wd, thr, glog, fc, thr_b);
     else if (vec_ok && fuse)
-      cb::launch(detect_sparse_vec_kernel<T, VEC, U, true>, grid, 256, 0, stream, (const T*)x, x_sb, x_sy,
-                 (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand, ncand, bits, H, W, C, Wd, thr, glog, fc);
+      cb::launch(detect_sparse_vec_kernel<T, VEC, U, true, false, R>, grid, 256, 0, stream, (const T*)x, x_sb, x_sy,
+                 (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand, ncand, bits, H, W, C, Wd, thr, glog, fc, thr_b);
     else if (vec_ok)
-      cb::launch(detect_sparse_vec_kernel<T, VEC, U, false>, grid, 256, 0, stream, (const T*)x, x_sb, x_sy,
-                 (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand, ncand, bits, H, W, C, Wd, thr, glog, fc);
+      cb::launch(detect_sparse_vec_kernel<T, VEC, U, false, false, R>, grid, 256, 0, stream, (const T*)x, x_sb, x_sy,
+                 (int)x_sx, (T*)state, s_sb, s_sy, (int)s_sx, aux, cand, ncand, bits, H, W, C, Wd, thr, glog, fc, thr_b);
     else
-      cb::launch(detect_sparse_generic_kernel<T, U>, grid, 256, 0, stream, (const T*)x, x_sb, x_sc, x_sy, x_sx,
-                 (T*)state, s_sb, s_sc, s_sy, s_sx, aux, cand, ncand, bits, H, W, C, Wd, thr);
+      cb::launch(detect_sparse_generic_kernel<T, U, R>, grid, 256, 0, stream, (const T*)x, x_sb, x_sc, x_sy, x_sx,
+                 (T*)state, s_sb, s_sc, s_sy, s_sx, aux, cand, ncand, bits, H, W, C, Wd, thr, thr_b);
     CB_CHECK_LAUNCH("change_detect_sparse");
     return 0;
-  });
+  }); });
 }
 
 }  // namespace cb

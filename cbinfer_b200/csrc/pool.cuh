@@ -108,15 +108,16 @@ maxpool2x2_kernel(const T* __restrict__ x, long long x_sb, long long x_sc, long 
 // compaction, sparse detection) and is exact for the same reason candidate detection is: only
 // re-pooled pixels can differ from what the next layer saw last frame.  Without DETECT the next-layer
 // arguments and UPDATE are unused, and `bits` may be null (then every listed pixel recomputes its
-// window).
-template <typename T, int VEC, int UPDATE, bool DETECT = true>
+// window).  THR (with DETECT): thr_b holds the next layer's per-stream thresholds, fp32 [B], one load
+// per window.
+template <typename T, int VEC, int UPDATE, bool DETECT = true, bool THR = false>
 __global__ void __launch_bounds__(256)
 maxpool2x2_detect_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int xp,
                          const int32_t* __restrict__ idx, const int32_t* __restrict__ count,
                          const uint32_t* __restrict__ bits, T* __restrict__ out, long long o_sb,
                          long long o_sy, int op, int cpp, int glog, int H, int W, int oH, int oW,
                          T* __restrict__ nst, long long n_sb, long long n_sy, int np, AuxPlanes aux,
-                         uint32_t* __restrict__ nbits, T thr) {
+                         uint32_t* __restrict__ nbits, T thr, const float* __restrict__ thr_b) {
   const int n = *count;
   const int lane = threadIdx.x & 31;
   const int G = 1 << glog, ppw = 32 >> glog;                // lanes per pixel, pixels per warp
@@ -147,6 +148,7 @@ maxpool2x2_detect_kernel(const T* __restrict__ x, long long x_sb, long long x_sy
     const long long opix = ((long long)b * oH + yo) * oW + xo;
     bool f = false;
     if (work) {
+      const T tb = stream_thr<DETECT && THR>(thr_b, b, thr);
       for (int cc = gl; cc < cpp; cc += G) {
         const T* q = base + cc * VEC;
         uint4 v00 = ldg16(q), v01 = v00, v10 = v00, v11 = v00;
@@ -159,7 +161,7 @@ maxpool2x2_detect_kernel(const T* __restrict__ x, long long x_sb, long long x_sy
         const uint4 res = window_max16<T, VEC>(v00, v01, v10, v11);
         st16(o + cc * VEC, res);
         if (DETECT) {
-          f |= Chunk<T>::changed(sv, res, thr);
+          f |= Chunk<T>::changed(sv, res, tb);
           if (UPDATE == CB_UPDATE_ALL) store_state<T>(ns + cc * VEC, res, aux, opix, cc * VEC);
         }
       }

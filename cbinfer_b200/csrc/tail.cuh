@@ -61,10 +61,11 @@ __device__ __forceinline__ uint32_t tail_sw128(int r, int k) {
   return (uint32_t)((r >> 3) * 1024 + (r & 7) * 128 + ((((k & 63) >> 3) ^ (r & 7)) << 4) + (k & 7) * 2);
 }
 
-template <int N1, bool TRACK>
+template <int N1, bool TRACK, bool THR>
 __global__ void __launch_bounds__(TAIL_THREADS)
 tail_kernel(const __grid_constant__ CUtensorMap w1map, const __grid_constant__ CUtensorMap w2map,
-            const TailArgs a) {
+            const TailArgs a, const float* __restrict__ thr1_b, const float* __restrict__ thr2_b) {
+  // THR: per-stream thresholds of the two layers (fp32 [B] each, b = pixel / hw), each may be null = thr1 / thr2
   extern __shared__ __align__(1024) uint8_t smem[];
   constexpr int A_KB = TAIL_ROWS * UM_ROW_BYTES;             // one K block of an A plane: 16 KB
   const int tid = threadIdx.x, lane = tid & 31;
@@ -162,6 +163,12 @@ tail_kernel(const __grid_constant__ CUtensorMap w1map, const __grid_constant__ C
         const int j = tile * rpt + rr;
         if (lane < RPW && rr < rpt && j < n) mypix = __ldg(a.cand + j);
       }
+      // THR: row i's layer-1 threshold, fetched by lane i with its index, so the load is in flight with
+      // the row loads below rather than after them
+      float mythr1 = a.thr1;
+      if constexpr (THR) {
+        if (thr1_b && mypix >= 0) mythr1 = __ldg(thr1_b + mypix / a.hw);
+      }
 #pragma unroll 1
       for (int r0 = 0; r0 < RPW; r0 += RB) {
         uint4 xv[RB][2], sv[RB][2];
@@ -185,8 +192,9 @@ tail_kernel(const __grid_constant__ CUtensorMap w1map, const __grid_constant__ C
         for (int i = 0; i < RB; ++i) {
           const int r = warp * RPW + r0 + i;
           bool f = false;
+          const float t1 = THR ? __shfl_sync(0xffffffffu, mythr1, r0 + i) : a.thr1;
 #pragma unroll
-          for (int h = 0; h < 2; ++h) f |= Chunk<float>::changed(sv[i][h], xv[i][h], a.thr1);
+          for (int h = 0; h < 2; ++h) f |= Chunk<float>::changed(sv[i][h], xv[i][h], THR ? t1 : a.thr1);
           const bool chg = __ballot_sync(0xffffffffu, f) != 0u && pix[i] >= 0;
           if (lane == 0) ctrl->flag1[r] = chg ? pix[i] : -1;
 #pragma unroll
@@ -250,6 +258,8 @@ tail_kernel(const __grid_constant__ CUtensorMap w1map, const __grid_constant__ C
 #pragma unroll
       for (int i = 0; i < N1 / 4; ++i)
         s2v[i] = (pix1 >= 0 && 4 * i < a.C1) ? ld16(s2 + 4 * i) : make_uint4(0, 0, 0, 0);
+      // (THR: layer 2's threshold of the row, also fetched while the MMAs run)
+      const float t2 = THR && thr2_b && pix1 >= 0 ? __ldg(thr2_b + pix1 / a.hw) : a.thr2;
       mbar_wait(&ctrl->mma1, par);
       tc_fence_after();
       const uint32_t trow = tmem + ((uint32_t)(warp * 32) << 16);
@@ -272,7 +282,7 @@ tail_kernel(const __grid_constant__ CUtensorMap w1map, const __grid_constant__ C
                                        __float_as_uint(f[i + 3]));
             st16(o1 + c0 + i, v);
             const uint4 sv = s2v[(c0 + i) >> 2];
-            f2 |= Chunk<float>::changed(sv, v, a.thr2);
+            f2 |= Chunk<float>::changed(sv, v, THR ? t2 : a.thr2);   // (a.thr2 read here, as without THR)
             if (a.update == CB_UPDATE_ALL) st16(s2 + c0 + i, v);
           }
           // layer 2's operand tile (K = C1 <= 64: one K block), rows of unchanged pixels are ignored later
@@ -368,7 +378,8 @@ inline bool tail_supported(int C0, int C1, int C2) {
   return C0 % 64 == 0 && C0 >= 64 && C0 <= 256 && (C1 == 16 || C1 == 32 || C1 == 64) && C2 >= 1 && C2 <= 16;
 }
 
-inline int tail_update(cudaStream_t s, const TailArgs& a, const void* packed1, const void* packed2) {
+inline int tail_update(cudaStream_t s, const TailArgs& a, const void* packed1, const void* packed2,
+                       const float* thr1_b, const float* thr2_b) {
   CB_CHECK_ARG(tail_supported(a.C0, a.C1, a.C2), "tail_update: unsupported channel counts %d -> %d -> %d", a.C0,
                a.C1, a.C2);
   CB_CHECK_ARG(a.xp == a.C0 && a.p1 == a.C1 && a.p2 >= a.C2 && (a.p2 % 4) == 0,
@@ -401,25 +412,27 @@ inline int tail_update(cudaStream_t s, const TailArgs& a, const void* packed1, c
   const size_t smem = (size_t)2 * nkb1 * TAIL_ROWS * UM_ROW_BYTES + (size_t)2 * nkb1 * N1 * UM_ROW_BYTES +
                       2 * 16 * UM_ROW_BYTES + sizeof(TailCtrl) + 64;
   const unsigned grid = (unsigned)sm_count();
-#define CB_TAIL(N_, TR_)                                                                             \
+#define CB_TAIL(N_, TR_, TH_)                                                                          \
   {                                                                                                  \
     static thread_local int adev = -1;                                                               \
     int dev = 0;                                                                                     \
     cudaGetDevice(&dev);                                                                             \
     if (adev != dev) {                                                                               \
-      if (cudaFuncSetAttribute(tail_kernel<N_, TR_>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024) != cudaSuccess) \
+      if (cudaFuncSetAttribute(tail_kernel<N_, TR_, TH_>, cudaFuncAttributeMaxDynamicSharedMemorySize, 226 * 1024) != cudaSuccess) \
         return fail(3, "tail_update: cannot reserve shared memory");                                \
       adev = dev;                                                                                    \
     }                                                                                                \
-    cb::launch(tail_kernel<N_, TR_>, dim3(grid), dim3(TAIL_THREADS), smem, s, m1, m2, a);            \
+    cb::launch(tail_kernel<N_, TR_, TH_>, dim3(grid), dim3(TAIL_THREADS), smem, s, m1, m2, a, thr1_b, thr2_b);       \
   }
-  const bool track = a.sc1 != nullptr;
+#define CB_TAIL_THR(N_, TR_) { if (thr) CB_TAIL(N_, TR_, true) else CB_TAIL(N_, TR_, false) }
+  const bool track = a.sc1 != nullptr, thr = thr1_b || thr2_b;
   switch (N1) {
-    case 16: if (track) CB_TAIL(16, true) else CB_TAIL(16, false) break;
-    case 32: if (track) CB_TAIL(32, true) else CB_TAIL(32, false) break;
-    case 64: if (track) CB_TAIL(64, true) else CB_TAIL(64, false) break;
+    case 16: if (track) CB_TAIL_THR(16, true) else CB_TAIL_THR(16, false) break;
+    case 32: if (track) CB_TAIL_THR(32, true) else CB_TAIL_THR(32, false) break;
+    case 64: if (track) CB_TAIL_THR(64, true) else CB_TAIL_THR(64, false) break;
     default: return fail(2, "tail_update: bad mid channel count %d", N1);
   }
+#undef CB_TAIL_THR
 #undef CB_TAIL
   CB_CHECK_LAUNCH("tail_update");
   return 0;

@@ -183,6 +183,18 @@ class FramePipeline(object):
         with torch.cuda.stream(self.compute):
             resetStreams(self.model, streams)
 
+    def setStreamThresholds(self, table):
+        """Write new per-stream thresholds (see cbinfer_b200.setStreamThresholds, including which streams
+        restart): enqueued on the compute stream, so they apply from the next `submit`ted frame on; frames
+        already submitted are computed with the old values.  The captured graphs stay valid: they read the
+        table the model had when they were captured, so one must be attached before the pipeline is built."""
+        from . import setStreamThresholds, streamThresholds
+        streamThresholds(self.model)                 # raises if the graphs were captured without a table
+        if table is None:
+            raise CBinferError("FramePipeline.setStreamThresholds: the graphs read the table; it cannot be detached")
+        with torch.cuda.stream(self.compute):
+            setStreamThresholds(self.model, table)
+
     def wait(self, slot):
         self.out_done[slot].synchronize()
         return self.out_host[slot]

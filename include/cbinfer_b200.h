@@ -366,6 +366,67 @@ int cb_maxpool2x2_detect(void* stream, int dtype, const void* x, long long x_sb,
                          long long n_sb, long long n_sy, int n_pitch, int aux_mode, void* aux_hi,
                          void* aux_lo, uint32_t* next_raw_bits, float threshold, int update_mode);
 
+/* ---- per-stream thresholds --------------------------------------------------------------------
+ * The *_thr entry points are the newest variant of each threshold-taking call above plus thr_b: fp32
+ * [B] in device memory, read on the device (capturable in a CUDA graph; a replay reads the values the
+ * buffer holds then), or NULL = the scalar threshold for every stream (then exactly the call without
+ * it, which forwards here with NULL).  Pixel p of stream b (b = p / (H*W)) is tested against thr_b[b]
+ * instead of the scalar, rounded to the data type exactly as the scalar is (fp16 / bf16: round to
+ * nearest), so a stream b computes bit for bit what the call computes with threshold = thr_b[b].
+ * For cb_maxpool2x2_detect_thr and cb_conv_update_tiled_pool_thr thr_b is the NEXT layer's (the one
+ * whose detection runs in the kernel); cb_tail_update_thr takes one table per layer (thr1_b, thr2_b,
+ * each may be NULL) and needs B and hw whenever one of them is given.  thr_b must be 4-byte aligned.
+ * No reference counterpart (the reference is batch 1; DESIGN.md section 3.15). */
+int cb_change_detect_thr(void* stream, int dtype,
+                         const void* x, long long x_sb, long long x_sc, long long x_sy, long long x_sx,
+                         void* state, long long s_sb, long long s_sc, long long s_sy, long long s_sx,
+                         int aux_mode, void* aux_hi, void* aux_lo, uint32_t* raw_bits, int B, int C,
+                         int H, int W, float threshold, int update_mode, const uint8_t* active,
+                         const float* thr_b);
+int cb_change_detect_u8_thr(void* stream, const uint8_t* x, long long x_sb, long long x_sc,
+                            long long x_sy, long long x_sx, float* state, long long s_sb, long long s_sc,
+                            long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
+                            uint32_t* raw_bits, int B, int C, int H, int W, float divisor, float bias,
+                            float threshold, int update_mode, const uint8_t* active, const float* thr_b);
+int cb_change_detect_sparse_thr(void* stream, int dtype,
+                                const void* x, long long x_sb, long long x_sc, long long x_sy, long long x_sx,
+                                void* state, long long s_sb, long long s_sc, long long s_sy, long long s_sx,
+                                int aux_mode, void* aux_hi, void* aux_lo,
+                                const int32_t* candidates, const int32_t* n_candidates,
+                                uint32_t* raw_bits, int B, int C, int H, int W, float threshold,
+                                int update_mode, int bits_are_clear, const float* thr_b);
+int cb_change_detect_sparse_compact_thr(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
+                                        long long x_sy, long long x_sx, void* state, long long s_sb,
+                                        long long s_sc, long long s_sy, long long s_sx, int aux_mode,
+                                        void* aux_hi, void* aux_lo, const int32_t* candidates,
+                                        const int32_t* n_candidates, uint32_t* raw_bits, int B, int C, int H,
+                                        int W, float threshold, int update_mode, int bits_are_clear,
+                                        uint32_t* dil_bits, int32_t* idx, int32_t* count, void* sync_ws,
+                                        int kHHalf, int kWHalf, int clear_raw, int32_t* stream_counts,
+                                        int32_t* stream_acc, const float* thr_b);
+int cb_maxpool2x2_detect_thr(void* stream, int dtype, const void* x, long long x_sb, long long x_sy,
+                             int x_pitch, const int32_t* idx, const int32_t* count,
+                             const uint32_t* dil_bits, void* out, long long o_sb, long long o_sy,
+                             int o_pitch, int B, int C, int H, int W, int oH, int oW, void* next_state,
+                             long long n_sb, long long n_sy, int n_pitch, int aux_mode, void* aux_hi,
+                             void* aux_lo, uint32_t* next_raw_bits, float threshold, int update_mode,
+                             const float* thr_b);
+int cb_conv_update_tiled_pool_thr(void* stream, int dtype, int gemm, const void* state, const void* state_lo,
+                                  int pitch_in, const void* tile_ws, const uint32_t* dil_bits,
+                                  const void* packed_w, const float* bias, void* out, int pitch_out, int B,
+                                  int H, int W, int Cin, int Cout, int kH, int kW, int relu,
+                                  void* pool_out, long long o_sb, long long o_sy, int o_pitch, int oH, int oW,
+                                  void* next_state, long long n_sb, long long n_sy, int n_pitch, int aux_mode,
+                                  void* aux_hi, void* aux_lo, uint32_t* next_raw_bits, float threshold,
+                                  int update_mode, const float* thr_b);
+int cb_tail_update_thr(void* stream, const float* x, float* state1, const void* packed_w1, const float* bias1,
+                       float* out1, int relu1, float thr1, float* state2, const void* packed_w2,
+                       const float* bias2, float* out2, int pitch_out2, int relu2, float thr2,
+                       const int32_t* candidates, const int32_t* n_candidates, int C0, int C1, int C2,
+                       int update_mode, int32_t* count1, int32_t* count2, void* sync_ws, int B, int hw,
+                       int32_t* stream_counts1, int32_t* stream_acc1, int32_t* stream_counts2,
+                       int32_t* stream_acc2, const float* thr1_b, const float* thr2_b);
+
 /* ---- per-stream state reset -----------------------------------------------------------------
  * Starts a new sequence in some streams of a batch without touching the others: for every b with
  * mask[b] != 0 (mask: uint8[B] in device memory, read on the device), stream b's slice of every
