@@ -19,7 +19,7 @@ __all__ = ['CBConv2d', 'CBPoolMax2d', 'ChangeIndexes', 'subsitute', 'convertRecu
            'propChangeIndexesOf1x1', 'clearMemory', 'getStateTensors', 'convert',
            'tuneThresholdParameters', 'convertPools', 'shareWorkspace', 'resetStreams',
            'setActiveStreams', 'trackStreamChanges', 'streamChangeCounts', 'setStreamThresholds',
-           'streamThresholds']
+           'streamThresholds', 'setStreamZones']
 
 verbose = False
 
@@ -371,6 +371,65 @@ def streamThresholds(net):
         if type(c) is CBConv2d and c._thrRow is not None:
             return c._thrRow[0]
     raise CBinferError("streamThresholds: no per-stream thresholds are attached (setStreamThresholds)")
+
+
+def setStreamZones(net, zones):
+    """Exclude regions of each video stream's frame from change detection: a burned-in clock, a waving
+    tree, a privacy mask.  The zone belongs to the frame-taking layer, the first CBConv2d under `net` in
+    named_modules() order; its qualified name is returned.  `zones` is a bool or uint8 tensor [B, H, W]
+    (non-zero = watched) on the host or on the model's CUDA device; None detaches it.
+
+    While a zone is attached, that layer's dense change scan treats every pixel of stream b outside
+    zones[b] as unchanged: it is not compared, and its state and operand planes are not written.  A pixel
+    whose state holds +inf (never accepted: a fresh model, or a stream reset by resetStreams and not run
+    since) is tested as usual.  Stream b then computes exactly what the model without a zone computes
+    when each excluded pixel with a finite state is replaced by the value the first layer's state holds
+    for it (DESIGN.md section 3.16).  Every later layer is driven by the first layer's change bits, so
+    nothing else changes; a zone may be widened or narrowed between any two frames without a restart.
+
+    The first call allocates one device bitmap (plus an int8 staging map); later calls with the same
+    [B, H, W] rewrite that buffer on the current stream, so CUDA graphs captured after the first call read
+    the zone as it is at each replay.  A host zone is uploaded with an ordinary asynchronous copy; a CUDA
+    zone is converted on the device, which makes the call capturable.  The zone survives clearMemory.
+    Frames of another B, H or W, frames wider than one 16-byte state pixel (> 4 fp32 or > 8 fp16 / bf16
+    channels) and change sets handed to the zone layer raise at forward.  Fine-grained layers,
+    gatherComputationStats and CPU models are not supported."""
+    named = [(name, c) for name, c in net.named_modules() if type(c) is CBConv2d]
+    if not named:
+        raise CBinferError("setStreamZones: the model has no CBConv2d")
+    name, first = named[0]
+    if zones is None:
+        first._zone = None
+        return name
+    if first.finegrained or (first._auxPlanes is not None and first._auxPlanes[0] == 'fg'):
+        raise CBinferError("setStreamZones: a fine-grained layer's detection (cb_fg_detect) takes no zone")
+    if first.gatherComputationStats:
+        raise CBinferError("setStreamZones: gatherComputationStats reads the whole input")
+    if not isinstance(zones, torch.Tensor) or zones.dim() != 3 or zones.dtype not in (torch.bool, torch.uint8):
+        raise CBinferError("setStreamZones: a bool or uint8 tensor [B, H, W] is needed, got %s"
+                           % ("%s %s" % (zones.dtype, tuple(zones.shape)) if isinstance(zones, torch.Tensor)
+                              else type(zones).__name__))
+    dev = first.weight.device
+    if dev.type != "cuda":
+        raise CBinferError("setStreamZones: the model is on %s; the zone lives on a CUDA device" % dev)
+    if zones.is_cuda and zones.device != dev:
+        raise CBinferError("setStreamZones: the zone is on %s, the model on %s" % (zones.device, dev))
+    shape = tuple(zones.shape)
+    if min(shape) < 1:
+        raise CBinferError("setStreamZones: an empty zone %s" % (shape,))
+    if first._zone is not None and first._zone[1] == shape:
+        bits, _, stage = first._zone
+    else:
+        bits = torch.zeros(_cg.C.cb_bitmap_words(*shape), dtype=torch.int32, device=dev)
+        stage = torch.empty(shape, dtype=torch.int8, device=dev)
+    with torch.cuda.device(dev):
+        if zones.is_cuda:
+            stage.copy_(zones)
+        else:
+            stage.copy_(zones.to(torch.int8), non_blocking=True)
+        _cg.check(_cg.C.cb_map_to_bits(_cg.stream_ptr(dev), stage.data_ptr(), bits.data_ptr(), *shape))
+    first._zone = (bits, shape, stage)
+    return name
 
 
 def getStateTensors(net):

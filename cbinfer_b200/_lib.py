@@ -39,6 +39,7 @@ SYMBOLS = [
     "cb_change_detect_thr", "cb_change_detect_u8_thr", "cb_change_detect_sparse_thr",
     "cb_change_detect_sparse_compact_thr", "cb_maxpool2x2_detect_thr", "cb_conv_update_tiled_pool_thr",
     "cb_tail_update_thr",
+    "cb_change_detect_zone", "cb_change_detect_u8_zone",
 ]
 
 
@@ -140,6 +141,9 @@ def _load():
                  "cb_tail_update_streams"):
         tables = 2 if name == "cb_tail_update_streams" else 1
         sig[name.replace("_streams", "") + "_thr"] = (i32, sig[name][1] + [vp] * tables)
+    # the *_zone variants: the *_thr arguments + the watched-pixel zone bitmap
+    for name in ("cb_change_detect_thr", "cb_change_detect_u8_thr"):
+        sig[name.replace("_thr", "_zone")] = (i32, sig[name][1] + [vp])
     for name, (res, args) in sig.items():
         fn = getattr(lib, name)
         fn.restype = res

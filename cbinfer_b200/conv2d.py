@@ -245,6 +245,9 @@ class CBConv2d(nn.Module):
         # per-stream thresholds (cbinfer_b200.setStreamThresholds): (table fp32 [L,B], this layer's row l, the
         # scalar threshold when the table was attached), or None = the scalar threshold for every stream
         self._thrRow = None
+        # watched-pixel zone of the frame-taking layer (cbinfer_b200.setStreamZones): (bitmap int32
+        # [B*H*Wd], (B, H, W), int8 staging map [B, H, W]), or None = every pixel watched
+        self._zone = None
         self._lastPlain = None    # was the last frame's input plain (not a change set)?  None: no frame yet
         self._wsHolder = cg.ConvWorkspace()    # shared per model by pycbinfer.convert()
         self.register_buffer('prevInput', self.weight.data.new_empty(0))
@@ -280,7 +283,7 @@ class CBConv2d(nn.Module):
         super(CBConv2d, self).__setstate__(state)
         self._setDefaultValues()
         for name in ('_fusedPool', '_fusedTail', '_inVersion', '_outVersion', '_activeMask', '_streamRow', '_thrRow',
-                     '_lastPlain'):
+                     '_zone', '_lastPlain'):
             self.__dict__.setdefault(name, None)
 
     # ---- state ---------------------------------------------------------------------------
@@ -494,6 +497,9 @@ class CBConv2d(nn.Module):
         # upstream kernel already ran part of this frame.  This layer records that work itself: the
         # upstream module read its state (_fusedDetectTarget, _tailTarget) right before the launch,
         # nothing since reads _fresh or _lastThr, and kernels bump no tensor versions.
+        # (a DetectionDone for the zone layer reports its own dense scan: nothing runs upstream of it)
+        if self._zone is not None and handed is not None and not isinstance(handed, DetectionDone):
+            raise _lib.CBinferError("the zone layer (setStreamZones) takes plain frames; it was handed a change set")
         if isinstance(handed, (DetectionDone, FrameDone)):
             _checkOwner(handed, self)
             self._recordDetection()
@@ -529,6 +535,7 @@ class CBConv2d(nn.Module):
                 input = input.float().div(u8norm[0]).add(u8norm[1])     # rare paths: plain fp32
                 u8norm = None
             dt = torch.float32
+        self._zoneBits(input.shape, dt)  # (a frame the zone does not fit raises before any state is touched)
 
         if not self._stateAllocated(input.shape, dt, dev):
             # a fresh output map needs every pixel recomputed: the input state goes too
@@ -550,6 +557,9 @@ class CBConv2d(nn.Module):
         s = self._scratch
 
         if self.gatherComputationStats:
+            if self._zone is not None:
+                raise _lib.CBinferError("gatherComputationStats reads the whole input: it cannot be combined "
+                                        "with a zone (setStreamZones)")
             if self._activeMask is not None:
                 raise _lib.CBinferError("gatherComputationStats reads the whole input: it cannot be combined "
                                         "with an active-stream mask (setActiveStreams)")
@@ -662,9 +672,11 @@ class CBConv2d(nn.Module):
                 changes.superset = True
         elif u8norm is not None:
             cg.detect_u8(input, self.prevInput, s["raw_bits"], self.threshold, mode,
-                         u8norm[0], u8norm[1], aux=aux, active=active, thr_b=thr_b)
+                         u8norm[0], u8norm[1], aux=aux, active=active, thr_b=thr_b,
+                         zone=self._zoneBits(input.shape, torch.float32))
         else:
-            cg.detect(input, self.prevInput, s["raw_bits"], self.threshold, mode, aux=aux, active=active, thr_b=thr_b)
+            cg.detect(input, self.prevInput, s["raw_bits"], self.threshold, mode, aux=aux, active=active, thr_b=thr_b,
+                      zone=self._zoneBits(input.shape, input.dtype))
         self._recordDetection()
         return changes, mask
 
@@ -689,6 +701,20 @@ class CBConv2d(nn.Module):
             raise _lib.CBinferError("per-stream thresholds of %d streams, the frame has %d (setStreamThresholds)"
                                     % (table.shape[1], B))
         return table[l]
+
+    def _zoneBits(self, shape, dtype):
+        """The zone bitmap for a frame of `shape` whose state has `dtype`, or None when no zone is attached
+        (cbinfer_b200.setStreamZones).  A frame the zone does not fit raises."""
+        if self._zone is None:
+            return None
+        bits, zshape, _ = self._zone
+        B, C_, H, W = shape
+        if (B, H, W) != zshape:
+            raise _lib.CBinferError("the zone (setStreamZones) is [B, H, W] = %s, the frame is %s" % (list(zshape), [B, H, W]))
+        if C_ * torch.empty(0, dtype=dtype).element_size() > 16:
+            raise _lib.CBinferError("a zone (setStreamZones) needs a frame of at most one 16-byte state pixel; "
+                                    "this one has %d %s channels" % (C_, dtype))
+        return bits
 
     def _checkThresholds(self):
         """Refuse what a frame with per-stream thresholds attached cannot honour."""
@@ -857,6 +883,8 @@ class CBConv2d(nn.Module):
             self._checkThresholds()
             if self.finegrained:
                 assert(self.feedbackLoop == False)
+                if self._zone is not None:
+                    raise _lib.CBinferError("a zone (setStreamZones) is not supported on a fine-grained layer")
                 if self._activeMask is not None:
                     raise _lib.CBinferError("an active-stream mask is not supported on a fine-grained layer")
                 return self.forward_fg(inp)

@@ -152,37 +152,54 @@ def _thr_ptr(thr_b, B, device):
     return thr_b.data_ptr()
 
 
-def detect(x, state, raw_bits, threshold, update_mode, aux=None, active=None, thr_b=None):
+def _zone_ptr(zone, B, H, W, device):
+    """Device pointer of a watched-pixel zone (a contiguous int32 CUDA bitmap [B, H, ceil(W/32)] on the
+    data's device, as cb_map_to_bits writes it), or None for none (every pixel watched)."""
+    if zone is None:
+        return None
+    require_cuda(zone)
+    words = C.cb_bitmap_words(B, H, W)
+    if zone.dtype != torch.int32 or not zone.is_contiguous() or zone.numel() != words or zone.device != device:
+        raise _lib.CBinferError("zone: a contiguous int32 bitmap of %d words on %s is needed, got %s %s on %s"
+                                % (words, device, zone.dtype, tuple(zone.shape), zone.device))
+    return zone.data_ptr()
+
+
+def detect(x, state, raw_bits, threshold, update_mode, aux=None, active=None, thr_b=None, zone=None):
     """cb_change_detect: raw (un-dilated) change bitmap of x vs state; updates state and, when
     given, the auxiliary operand planes `aux` (see _aux_args).  `active`: optional bool / uint8
     CUDA tensor [B], read on the device; a stream with active[b] == 0 is skipped (its bitmap words
     0, its x not read, its state and planes untouched: cb_change_detect_streams).  `thr_b`: optional
     fp32 CUDA tensor [B] of per-stream thresholds, read on the device instead of `threshold`
-    (cb_change_detect_thr); the same holds for every wrapper below that takes it."""
+    (cb_change_detect_thr); the same holds for every wrapper below that takes it.  `zone`: optional
+    int32 bitmap of watched pixels (see _zone_ptr); an excluded pixel whose state is finite counts as
+    unchanged and is neither read nor written (cb_change_detect_zone)."""
     require_cuda(x, state, raw_bits)
     B, Cc, H, W = x.shape
     assert state.shape == x.shape and state.dtype == x.dtype
     act = _active_ptr(active, B, x.device)
     mode, hi, lo = _aux_args(aux, state)
-    check(C.cb_change_detect_thr(stream_ptr(x.device), dtype_code(x), x.data_ptr(), *_strides4(x),
-                                 state.data_ptr(), *_strides4(state), mode, hi, lo,
-                                 raw_bits.data_ptr(), B, Cc, H, W, float(threshold), int(update_mode), act,
-                                 _thr_ptr(thr_b, B, x.device)))
+    check(C.cb_change_detect_zone(stream_ptr(x.device), dtype_code(x), x.data_ptr(), *_strides4(x),
+                                  state.data_ptr(), *_strides4(state), mode, hi, lo,
+                                  raw_bits.data_ptr(), B, Cc, H, W, float(threshold), int(update_mode), act,
+                                  _thr_ptr(thr_b, B, x.device), _zone_ptr(zone, B, H, W, x.device)))
 
 
-def detect_u8(x, state, raw_bits, threshold, update_mode, divisor, bias, aux=None, active=None, thr_b=None):
+def detect_u8(x, state, raw_bits, threshold, update_mode, divisor, bias, aux=None, active=None, thr_b=None,
+              zone=None):
     """cb_change_detect_u8: detection on a uint8 frame normalised on the fly as u8/divisor + bias
     (the readers' /255 resp. /256 - 0.5); `state` is the fp32 pixel-major state.  Bit-identical to
-    :func:`detect` on ``x.float() / divisor + bias``.  `active` as in :func:`detect`."""
+    :func:`detect` on ``x.float() / divisor + bias``.  `active`, `thr_b` and `zone` as in :func:`detect`."""
     require_cuda(x, state, raw_bits)
     B, Cc, H, W = x.shape
     assert x.dtype == torch.uint8 and state.dtype == torch.float32 and state.shape == x.shape
     act = _active_ptr(active, B, x.device)
     mode, hi, lo = _aux_args(aux, state)
-    check(C.cb_change_detect_u8_thr(stream_ptr(x.device), x.data_ptr(), *_strides4(x),
-                                    state.data_ptr(), *_strides4(state), mode, hi, lo,
-                                    raw_bits.data_ptr(), B, Cc, H, W, float(divisor), float(bias),
-                                    float(threshold), int(update_mode), act, _thr_ptr(thr_b, B, x.device)))
+    check(C.cb_change_detect_u8_zone(stream_ptr(x.device), x.data_ptr(), *_strides4(x),
+                                     state.data_ptr(), *_strides4(state), mode, hi, lo,
+                                     raw_bits.data_ptr(), B, Cc, H, W, float(divisor), float(bias),
+                                     float(threshold), int(update_mode), act, _thr_ptr(thr_b, B, x.device),
+                                     _zone_ptr(zone, B, H, W, x.device)))
 
 
 def detect_sparse(x, state, raw_bits, threshold, update_mode, candidates, aux=None,

@@ -89,19 +89,33 @@ int cb_channel_pitch(int dtype, int C) {
 #define CB_CHECK_THR(thr_b, what) \
   CB_CHECK_ARG(((uintptr_t)(thr_b) % sizeof(float)) == 0, what ": thr_b is not aligned to 4 bytes")
 
+// watched-pixel zone (the *_zone entry points): uint32 [B, H, Wd] bitmap in device memory, or NULL
+#define CB_CHECK_ZONE(zone, what) \
+  CB_CHECK_ARG(((uintptr_t)(zone) % sizeof(uint32_t)) == 0, what ": zone is not aligned to 4 bytes")
+
+int cb_change_detect_zone(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
+                          long long x_sy, long long x_sx, void* state, long long s_sb, long long s_sc,
+                          long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
+                          uint32_t* raw_bits, int B, int C, int H, int W, float threshold,
+                          int update_mode, const uint8_t* active, const float* thr_b, const uint32_t* zone) {
+  CB_CHECK_ARG(x && state && raw_bits, "change_detect: null pointer");
+  CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect: bad shape");
+  CB_CHECK_THR(thr_b, "change_detect");
+  CB_CHECK_ZONE(zone, "change_detect");
+  CB_DISPATCH_DTYPE(dtype, return (launch_detect<T, VEC>((cudaStream_t)stream, x, x_sb, x_sc, x_sy,
+                                                        x_sx, state, s_sb, s_sc, s_sy, s_sx, aux_mode,
+                                                        aux_hi, aux_lo, raw_bits, B, C, H, W, threshold,
+                                                        update_mode, active, thr_b, zone)));
+  return 0;
+}
+
 int cb_change_detect_thr(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
                          long long x_sy, long long x_sx, void* state, long long s_sb, long long s_sc,
                          long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
                          uint32_t* raw_bits, int B, int C, int H, int W, float threshold,
                          int update_mode, const uint8_t* active, const float* thr_b) {
-  CB_CHECK_ARG(x && state && raw_bits, "change_detect: null pointer");
-  CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect: bad shape");
-  CB_CHECK_THR(thr_b, "change_detect");
-  CB_DISPATCH_DTYPE(dtype, return (launch_detect<T, VEC>((cudaStream_t)stream, x, x_sb, x_sc, x_sy,
-                                                        x_sx, state, s_sb, s_sc, s_sy, s_sx, aux_mode,
-                                                        aux_hi, aux_lo, raw_bits, B, C, H, W, threshold,
-                                                        update_mode, active, thr_b)));
-  return 0;
+  return cb_change_detect_zone(stream, dtype, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy, s_sx, aux_mode,
+                               aux_hi, aux_lo, raw_bits, B, C, H, W, threshold, update_mode, active, thr_b, nullptr);
 }
 
 int cb_change_detect_streams(void* stream, int dtype, const void* x, long long x_sb, long long x_sc,
@@ -122,17 +136,29 @@ int cb_change_detect(void* stream, int dtype, const void* x, long long x_sb, lon
                                   aux_mode, aux_hi, aux_lo, raw_bits, B, C, H, W, threshold, update_mode, nullptr);
 }
 
+int cb_change_detect_u8_zone(void* stream, const uint8_t* x, long long x_sb, long long x_sc,
+                             long long x_sy, long long x_sx, float* state, long long s_sb, long long s_sc,
+                             long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
+                             uint32_t* raw_bits, int B, int C, int H, int W, float divisor, float bias,
+                             float threshold, int update_mode, const uint8_t* active, const float* thr_b,
+                             const uint32_t* zone) {
+  CB_CHECK_ARG(x && state && raw_bits, "change_detect_u8: null pointer");
+  CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect_u8: bad shape");
+  CB_CHECK_THR(thr_b, "change_detect_u8");
+  CB_CHECK_ZONE(zone, "change_detect_u8");
+  return launch_detect_u8((cudaStream_t)stream, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy,
+                          s_sx, aux_mode, aux_hi, aux_lo, raw_bits, B, C, H, W, divisor, bias,
+                          threshold, update_mode, active, thr_b, zone);
+}
+
 int cb_change_detect_u8_thr(void* stream, const uint8_t* x, long long x_sb, long long x_sc,
                             long long x_sy, long long x_sx, float* state, long long s_sb, long long s_sc,
                             long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
                             uint32_t* raw_bits, int B, int C, int H, int W, float divisor, float bias,
                             float threshold, int update_mode, const uint8_t* active, const float* thr_b) {
-  CB_CHECK_ARG(x && state && raw_bits, "change_detect_u8: null pointer");
-  CB_CHECK_ARG(B >= 0 && C > 0 && H >= 0 && W >= 0, "change_detect_u8: bad shape");
-  CB_CHECK_THR(thr_b, "change_detect_u8");
-  return launch_detect_u8((cudaStream_t)stream, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy,
-                          s_sx, aux_mode, aux_hi, aux_lo, raw_bits, B, C, H, W, divisor, bias,
-                          threshold, update_mode, active, thr_b);
+  return cb_change_detect_u8_zone(stream, x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy, s_sx, aux_mode,
+                                  aux_hi, aux_lo, raw_bits, B, C, H, W, divisor, bias, threshold, update_mode,
+                                  active, thr_b, nullptr);
 }
 
 int cb_change_detect_u8_streams(void* stream, const uint8_t* x, long long x_sb, long long x_sc,

@@ -21,6 +21,13 @@
 // stream): every kernel that tests a threshold reads stream b's value once per decision unit (a
 // bitmap word, a candidate) and rounds it to T with thr_cast, as the host rounds the scalar.  The
 // table is a compile-time variant (THR): without it the kernels are the ones compiled before it existed.
+//
+// Watched-pixel zone (`zone`, uint32 [B, H, Wd] on the device in the bitmap layout, may be null = every
+// pixel watched): detect_narrow_kernel only, as a compile-time variant (ZONE).  A warp loads its word's
+// zone word once; a lane whose bit is 0 and whose state is finite in every real channel is reported
+// unchanged without reading x or writing its state / operand planes.  A state pixel holding +inf in a
+// real channel (never accepted: fresh or reset stream) is tested as usual.  Exactly the result of the
+// call without a zone on the frame whose excluded finite pixels hold the state's values (threshold >= 0).
 #pragma once
 #include "cb_common.cuh"
 #include "compact.cuh"
@@ -267,13 +274,27 @@ detect_vec_kernel(const T* __restrict__ x, long long x_sb, long long x_sy, int x
 // applied on the fly with IEEE division and addition, so the result is bit-identical to detecting on
 // the host-normalised fp32 frame, at a quarter of the host->device bytes.  Otherwise divisor and bias
 // are unused.
-template <typename T, int VEC, int UPDATE, typename S = T, bool THR = false>
+// +inf in one of the first C elements of a state chunk: a pixel that was never accepted
+__device__ __forceinline__ bool is_pos_inf(float v) { return __float_as_uint(v) == 0x7f800000u; }
+__device__ __forceinline__ bool is_pos_inf(__half v) { return __half_as_ushort(v) == 0x7c00u; }
+__device__ __forceinline__ bool is_pos_inf(__nv_bfloat16 v) { return __bfloat16_as_ushort(v) == 0x7f80u; }
+template <typename T, int VEC>
+__device__ __forceinline__ bool chunk_unaccepted(const uint4& v, int C) {
+  const T* e = reinterpret_cast<const T*>(&v);
+  bool r = false;
+#pragma unroll
+  for (int c = 0; c < VEC; ++c)
+    if (c < C) r |= is_pos_inf(e[c]);
+  return r;
+}
+
+template <typename T, int VEC, int UPDATE, typename S = T, bool THR = false, bool ZONE = false>
 __global__ void __launch_bounds__(256)
 detect_narrow_kernel(const S* __restrict__ x, long long x_sb, long long x_sc, long long x_sy,
                      long long x_sx, T* __restrict__ st, long long s_sb, long long s_sy,
                      AuxPlanes aux, uint32_t* __restrict__ bits, int B, int H, int W, int C,
                      int Wd, T thr, float divisor, float bias, const uint8_t* __restrict__ active,
-                     const float* __restrict__ thr_b) {
+                     const float* __restrict__ thr_b, const uint32_t* __restrict__ zone) {
   constexpr bool kU8 = std::is_same<S, uint8_t>::value;
   const float* lut = nullptr;
   if constexpr (kU8) {
@@ -295,15 +316,32 @@ detect_narrow_kernel(const S* __restrict__ x, long long x_sb, long long x_sc, lo
     const uint4 sv = ld16_stream(sp);
     uint4 nv = sv;                             // pad lanes keep the state's (zero) value
     T* ne = reinterpret_cast<T*>(&nv);
+    auto load_x = [&]() {
 #pragma unroll
-    for (int c = 0; c < VEC; ++c) {
-      if (c >= C) continue;
-      if constexpr (kU8) ne[c] = lut[__ldcs(xp + c * x_sc)];
-      else ne[c] = ld_stream(xp + c * x_sc);
+      for (int c = 0; c < VEC; ++c) {
+        if (c >= C) continue;
+        if constexpr (kU8) ne[c] = lut[__ldcs(xp + c * x_sc)];
+        else ne[c] = ld_stream(xp + c * x_sc);
+      }
+    };
+    bool test = true;
+    if constexpr (ZONE) {
+      // watched pixels load x without waiting for the state; an excluded one only if it was never accepted
+      test = (__ldg(zone + warp) >> (threadIdx.x & 31)) & 1u;
+      if (test) {
+        load_x();
+      } else if (chunk_unaccepted<T, VEC>(sv, C)) {
+        load_x();
+        test = true;
+      }
+    } else {
+      load_x();
     }
-    f = Chunk<T>::changed(sv, nv, stream_thr<THR>(thr_b, b, thr));
-    if (UPDATE == CB_UPDATE_ALL || (UPDATE == CB_UPDATE_CHANGED && f))
-      store_state<T>(sp, nv, aux, ((long long)b * H + y) * W + xx, 0);
+    if (test) {
+      f = Chunk<T>::changed(sv, nv, stream_thr<THR>(thr_b, b, thr));
+      if (UPDATE == CB_UPDATE_ALL || (UPDATE == CB_UPDATE_CHANGED && f))
+        store_state<T>(sp, nv, aux, ((long long)b * H + y) * W + xx, 0);
+    }
   }
   const unsigned word = __ballot_sync(0xffffffffu, f);
   if ((threadIdx.x & 31) == 0) bits[warp] = word;
@@ -510,7 +548,7 @@ int launch_detect(cudaStream_t stream, const void* x, long long x_sb, long long 
                   long long x_sy, long long x_sx, void* state, long long s_sb, long long s_sc,
                   long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
                   uint32_t* bits, int B, int C, int H, int W, float threshold, int update,
-                  const uint8_t* active, const float* thr_b) {
+                  const uint8_t* active, const float* thr_b, const uint32_t* zone) {
   const int Wd = (W + 31) / 32;
   const long long words = (long long)B * H * Wd;
   if (words == 0) return 0;
@@ -518,10 +556,23 @@ int launch_detect(cudaStream_t stream, const void* x, long long x_sb, long long 
   const size_t es = sizeof(T);
   AuxPlanes aux;
   if (int rc = make_aux<T>(aux, aux_mode, aux_hi, aux_lo, state, C)) return rc;
+  // the narrow kernel: state pixel = one 16-byte chunk, any x strides
+  const bool narrow_fits = s_sc == 1 && s_sx == VEC && C <= VEC && ((s_sy * es) % 16) == 0 &&
+                           ((s_sb * es) % 16) == 0 && ((uintptr_t)state % 16) == 0;
+  if (zone) {                                 // only the narrow kernel has the ZONE variant
+    CB_CHECK_ARG(narrow_fits, "change_detect: a zone needs a state pixel of one 16-byte chunk (C <= %d, pixel-major "
+                 "state of pitch %d, 16-byte aligned)", VEC, VEC);
+    CB_CHECK_ARG((words + 7) / 8 < (1ll << 31) && words < (1ll << 31), "change_detect: image too large");
+    return dispatch_thr(thr_b, [&](auto R) { return dispatch_update(update, "change_detect", [&](auto U) {
+      cb::launch(detect_narrow_kernel<T, VEC, U, T, R, true>, dim3((unsigned)((words + 7) / 8)), dim3(256), 0,
+                 stream, (const T*)x, x_sb, x_sc, x_sy, x_sx, (T*)state, s_sb, s_sy, aux, bits, B, H, W, C, Wd, thr,
+                 0.f, 0.f, active, thr_b, zone);
+      CB_CHECK_LAUNCH("change_detect");
+      return 0;
+    }); });
+  }
   const bool vec_ok = pixel_major_ok<T, VEC>(x, x_sb, x_sc, x_sy, x_sx, state, s_sb, s_sc, s_sy, s_sx, C);
-  const bool narrow_ok = !vec_ok && s_sc == 1 && s_sx == VEC && C <= VEC &&
-                         ((s_sy * es) % 16) == 0 && ((s_sb * es) % 16) == 0 &&
-                         ((uintptr_t)state % 16) == 0;
+  const bool narrow_ok = !vec_ok && narrow_fits;
   const int cpv = (C + VEC - 1) / VEC;
   const unsigned magic = cpv > 1 ? (unsigned)((0x100000000ull + cpv - 1) / cpv) : 0u;
   // planar x, pixel-major multi-chunk state: transposed through shared memory (detect_planar_kernel)
@@ -548,7 +599,7 @@ int launch_detect(cudaStream_t stream, const void* x, long long x_sb, long long 
                    (T*)state, s_sb, s_sy, (int)s_sx, aux, bits, B, H, W, C, Wd, thr, magic, wlog, active, thr_b);
     } else if (narrow_ok) {
       cb::launch(detect_narrow_kernel<T, VEC, U, T, R>, grid, block, 0, stream, (const T*)x, x_sb, x_sc, x_sy, x_sx,
-                 (T*)state, s_sb, s_sy, aux, bits, B, H, W, C, Wd, thr, 0.f, 0.f, active, thr_b);
+                 (T*)state, s_sb, s_sy, aux, bits, B, H, W, C, Wd, thr, 0.f, 0.f, active, thr_b, nullptr);
     } else if (planar_ok) {
       if (planar_smem > 48 * 1024)
         cudaFuncSetAttribute(detect_planar_kernel<T, VEC, U, R>, cudaFuncAttributeMaxDynamicSharedMemorySize,
@@ -571,7 +622,7 @@ inline int launch_detect_u8(cudaStream_t stream, const void* x, long long x_sb, 
                             long long s_sc, long long s_sy, long long s_sx, int aux_mode,
                             void* aux_hi, void* aux_lo, uint32_t* bits, int B, int C, int H, int W,
                             float divisor, float bias, float threshold, int update,
-                            const uint8_t* active, const float* thr_b) {
+                            const uint8_t* active, const float* thr_b, const uint32_t* zone) {
   const int Wd = (W + 31) / 32;
   const long long words = (long long)B * H * Wd;
   if (words == 0) return 0;
@@ -584,9 +635,14 @@ inline int launch_detect_u8(cudaStream_t stream, const void* x, long long x_sb, 
   const long long blocks = (words + 7) / 8;
   CB_CHECK_ARG(blocks < (1ll << 31), "change_detect_u8: image too large");
   return dispatch_thr(thr_b, [&](auto R) { return dispatch_update(update, "change_detect_u8", [&](auto U) {
-    cb::launch(detect_narrow_kernel<float, 4, U, uint8_t, R>, dim3((unsigned)blocks), dim3(256), 0, stream,
-               (const uint8_t*)x, x_sb, x_sc, x_sy, x_sx, (float*)state, s_sb, s_sy, aux, bits, B, H, W, C, Wd,
-               threshold, divisor, bias, active, thr_b);
+    if (zone)
+      cb::launch(detect_narrow_kernel<float, 4, U, uint8_t, R, true>, dim3((unsigned)blocks), dim3(256), 0, stream,
+                 (const uint8_t*)x, x_sb, x_sc, x_sy, x_sx, (float*)state, s_sb, s_sy, aux, bits, B, H, W, C, Wd,
+                 threshold, divisor, bias, active, thr_b, zone);
+    else
+      cb::launch(detect_narrow_kernel<float, 4, U, uint8_t, R>, dim3((unsigned)blocks), dim3(256), 0, stream,
+                 (const uint8_t*)x, x_sb, x_sc, x_sy, x_sx, (float*)state, s_sb, s_sy, aux, bits, B, H, W, C, Wd,
+                 threshold, divisor, bias, active, thr_b, nullptr);
     CB_CHECK_LAUNCH("change_detect_u8");
     return 0;
   }); });

@@ -195,6 +195,24 @@ class FramePipeline(object):
         with torch.cuda.stream(self.compute):
             setStreamThresholds(self.model, table)
 
+    def setStreamZones(self, zones):
+        """Write a new watched-pixel zone of the same [B, H, W] (see cbinfer_b200.setStreamZones): enqueued on
+        the compute stream, so it applies from the next `submit`ted frame on.  The captured graphs read the
+        zone buffer the model had when they were captured, so one must be attached before the pipeline is
+        built, and it cannot be detached or reshaped through the pipeline."""
+        from . import CBConv2d, setStreamZones
+        first = next(c for c in self.model.modules() if type(c) is CBConv2d)
+        if first._zone is None:
+            raise CBinferError("FramePipeline.setStreamZones: the graphs were captured without a zone; attach one "
+                               "(cbinfer_b200.setStreamZones) before building the pipeline")
+        if zones is None:
+            raise CBinferError("FramePipeline.setStreamZones: the graphs read the zone; it cannot be detached")
+        if not isinstance(zones, torch.Tensor) or tuple(zones.shape) != first._zone[1]:
+            raise CBinferError("FramePipeline.setStreamZones: the graphs read a zone [B, H, W] = %s"
+                               % (list(first._zone[1]),))
+        with torch.cuda.stream(self.compute):
+            setStreamZones(self.model, zones)
+
     def wait(self, slot):
         self.out_done[slot].synchronize()
         return self.out_host[slot]

@@ -427,6 +427,34 @@ int cb_tail_update_thr(void* stream, const float* x, float* state1, const void* 
                        int32_t* stream_counts1, int32_t* stream_acc1, int32_t* stream_counts2,
                        int32_t* stream_acc2, const float* thr1_b, const float* thr2_b);
 
+/* ---- watched-pixel zones ----------------------------------------------------------------------
+ * cb_change_detect_zone / cb_change_detect_u8_zone are cb_change_detect_thr / cb_change_detect_u8_thr
+ * plus zone: a uint32 bitmap [B, H, Wd] (Wd = cb_bitmap_row_words(W); bit x % 32 of word x / 32, bits at
+ * or beyond W ignored) in device memory, read on the device (capturable; a replay reads what the buffer
+ * holds then), or NULL = every pixel watched (then exactly the call without it, which forwards here with
+ * NULL).  A pixel of stream b whose zone bit is 0 counts as unchanged: its x is not read, its bit is 0 and
+ * its state and operand planes are not written, under every update_mode.  Exception: a pixel whose state
+ * holds +inf in one of its C channels (never accepted: a fresh state, or a stream reset by
+ * cb_reset_streams) is tested as usual, so an excluded area never hands +inf to the contraction.
+ * Rule: with a threshold >= 0, the call computes bit for bit what the call without a zone computes on
+ * the frame x' that equals x at watched pixels and at pixels with +inf in their state, and equals the
+ * state elsewhere.  The active mask wins: a skipped stream's words are 0 and its zone is not read.
+ * A zone needs the narrow kernel: C <= 16 / element size and a pixel-major state of exactly one
+ * 16-byte chunk per pixel (any x strides); other layouts, and a zone not aligned to 4 bytes, get
+ * status 2.  No reference counterpart (DESIGN.md section 3.16). */
+int cb_change_detect_zone(void* stream, int dtype,
+                          const void* x, long long x_sb, long long x_sc, long long x_sy, long long x_sx,
+                          void* state, long long s_sb, long long s_sc, long long s_sy, long long s_sx,
+                          int aux_mode, void* aux_hi, void* aux_lo, uint32_t* raw_bits, int B, int C,
+                          int H, int W, float threshold, int update_mode, const uint8_t* active,
+                          const float* thr_b, const uint32_t* zone);
+int cb_change_detect_u8_zone(void* stream, const uint8_t* x, long long x_sb, long long x_sc,
+                             long long x_sy, long long x_sx, float* state, long long s_sb, long long s_sc,
+                             long long s_sy, long long s_sx, int aux_mode, void* aux_hi, void* aux_lo,
+                             uint32_t* raw_bits, int B, int C, int H, int W, float divisor, float bias,
+                             float threshold, int update_mode, const uint8_t* active, const float* thr_b,
+                             const uint32_t* zone);
+
 /* ---- per-stream state reset -----------------------------------------------------------------
  * Starts a new sequence in some streams of a batch without touching the others: for every b with
  * mask[b] != 0 (mask: uint8[B] in device memory, read on the device), stream b's slice of every
